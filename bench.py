@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: test-point predictions/sec (mean + variance + gradient, M=250, D=10, FP64).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 * workload = BASELINE.json configs[1]: the tests/benchmark.py-style synthetic GaussianProcess
   (M=250, D=10, all-U(0,1) model, seed 0), 1e8 FP64 test points PER GPU generated on the device
@@ -41,6 +41,7 @@ M, D = 250, 10
 F_PER_POINT = 2 * M * M + M * (5 * D + 6) + D + 1          # 139,011 flop (+ M exp), SURVEY.md section 8d
 BYTES_PER_POINT = 8 * D + 8 * (2 + D)                      # 176 B
 METRIC = "test-point predictions/sec (mean+var+grad, M=250, D=10, FP64)"
+DUMP_POINTS = 1 << 19                                      # 12 doubles per point: 48 MiB of --dump-outputs at most
 
 
 def parse():
@@ -56,7 +57,29 @@ def parse():
     ap.add_argument("--no-configs", action="store_true", help="skip the cfg 1/3/4/5 block")
     ap.add_argument("--multi-points", type=float, default=1e7, help="host-resident points per GPU of the one-process e2e (N > 1)")
     ap.add_argument("--tripwire", type=int, default=100000, help="prefix and random-subset size of the oracle check")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed (rank 0) as DIR/<name>.npy in float64: "
+                         "every point up to %d points, beyond that the same seeded sample of that many points" % DUMP_POINTS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(dirname, outputs, n):
+    """Write outputs[name] (first axis = the step's n points) as dirname/<name>.npy, float64, on a fixed sample of rows
+    so that two builds given the same arguments can be compared output for output."""
+    os.makedirs(dirname, exist_ok=True)
+    idx = np.arange(n) if n <= DUMP_POINTS else np.sort(np.random.default_rng(0).choice(n, DUMP_POINTS, replace=False))
+    for name, a in outputs.items():
+        if a is None:
+            continue
+        if hasattr(a, "cpu"):   # torch tensor: gather the sample on its device
+            import torch
+            a = a[torch.from_numpy(idx).to(a.device)].cpu().numpy()
+        else:
+            a = np.asarray(a)[idx]
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def workload_config(n_points):
@@ -373,8 +396,10 @@ def run_reference(args, rank, world):
         orc.predict(model["inputs"], model["theta"], model["invQ"], model["invQt"], testing[:20000])
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        orc.predict(model["inputs"], model["theta"], model["invQ"], model["invQt"], testing, chunk=100000)
+        res = orc.predict(model["inputs"], model["theta"], model["invQ"], model["invQt"], testing, chunk=100000)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("mu", "var", "deriv"), res)), npts)
     value = npts * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "points/s", "n_gpus": args.gpus,
@@ -482,6 +507,8 @@ def main():
                          torch.randint(0, N, (nt,), device=dev, generator=torch.Generator(device=dev).manual_seed(7))])
         trip = {"t": testing[idx].cpu().numpy(), "mu": out["mu"][idx].cpu().numpy(), "var": out["var"][idx].cpu().numpy(),
                 "deriv": out["deriv"][idx].cpu().numpy(), "n_prefix": nt, "n_random": nt}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, out, N)
     # ---- configs[1] as written: 1e8 points IN TOTAL, N/G per GPU (strong scaling) ---------------------------------
     strong = None
     Ns = int(round(1e8)) // world

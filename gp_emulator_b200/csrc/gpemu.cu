@@ -563,8 +563,7 @@ int predict_device(gpe_model* m, const double* testing, int64_t N, double* mu, d
         const size_t smem = ((size_t)kTinyTN * (f.Mp + 4) + work) * 8;
         const int grid = (int)((N + kTinyTN - 1) / kTinyTN) * kTinyCluster;
         g_launches.fetch_add(1, std::memory_order_relaxed);
-        static const uint32_t shrink_t = getenv("GPE_DEBUG_SHRINK_SMEM") ? (uint32_t)atoi(getenv("GPE_DEBUG_SHRINK_SMEM")) : 0u;
-        CUDA_TRY(launch_tiny(m->DP, p, grid, smem - std::min<size_t>(shrink_t, smem), st));   // (dev aid: see the fused launch)
+        CUDA_TRY(launch_tiny(m->DP, p, grid, smem, st));
         mean_done = true;
         var = nullptr;
     }
@@ -601,10 +600,7 @@ int predict_device(gpe_model* m, const double* testing, int64_t N, double* mu, d
         }
         const int64_t ntiles = (N + f.TN - 1) / f.TN;
         const int grid = (int)std::min<int64_t>(ntiles, (int64_t)m->sms * f.ctas_per_sm);
-        // dev aid for tests/test_gpu_parity.py::test_smem_guard_traps: launch with less dynamic shared memory than the
-        // carve-up needs; the kernel-entry guard must turn that into a launch error
-        static const uint32_t shrink = getenv("GPE_DEBUG_SHRINK_SMEM") ? (uint32_t)atoi(getenv("GPE_DEBUG_SHRINK_SMEM")) : 0u;
-        CUDA_TRY(launch_full(m->DP, f.cfg, p, grid, f.smem - std::min(shrink, f.smem), st));
+        CUDA_TRY(launch_full(m->DP, f.cfg, p, grid, f.smem, st));
         mean_done = true;
     }
     const bool need_mean = !mean_done && (mu != nullptr || deriv != nullptr);

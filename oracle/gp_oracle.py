@@ -7,12 +7,12 @@ missing instead of falling back to this file.
 
 Parity pinning: the reference package is Python-2 only (print statements, xrange, tab/space mixing,
 ``import _gpu_predict`` at module scope), so it cannot be imported as-is.  ``tests/golden/make_golden.py``
-loads the reference *source text* from /root/reference at generation time, applies a purely mechanical
+loads the reference *source text* from a checkout of it at generation time, applies a purely mechanical
 py2->py3 token conversion in memory, executes it, and freezes its outputs into ``tests/golden/*.npz``.
 ``tests/test_oracle.py`` checks every function below against those frozen reference outputs, so this
 oracle is pinned to outputs of the reference itself.
 
-Each function cites the reference file:line it follows (paths relative to /root/reference).
+Each function cites the reference file:line it follows (paths relative to the reference checkout).
 """
 from __future__ import annotations
 

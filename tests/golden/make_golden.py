@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Freeze outputs of the REFERENCE implementation into tests/golden/*.npz.
 
-Run in the build container only (needs /root/reference); the fixtures it writes are committed and travel
-to the GPU box, the reference does not.
+Needs a checkout of the reference project; the fixtures it writes are committed, so the tests need neither the
+reference nor this script.
 
 The reference package is Python 2 (print statements, xrange, tab/space mixing) and imports its compiled
 ``_gpu_predict`` at module scope, so it cannot be imported.  This script reads the reference *source text*,
@@ -20,7 +20,7 @@ goldens is therefore the reference's own numpy/scipy code:
   per-band bank pattern (E x predict + hessian on shared inputs)   tests/test_perband_emulator.py:22-47
   MultivariateEmulator(X=, y=, hyperparams=) with 20 PCs x 2101 wavelengths (BASELINE config 4)
 
-    python tests/golden/make_golden.py [--only S1500]
+    python tests/golden/make_golden.py REFERENCE_DIR [--only S1500]
 """
 import hashlib
 import os
@@ -30,7 +30,9 @@ import types
 
 import numpy as np
 
-REF = "/root/reference"
+if len(sys.argv) < 2 or sys.argv[1].startswith("-"):
+    sys.exit(__doc__)
+REF = sys.argv[1]
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 from oracle import gp_oracle as orc  # noqa: E402  (input generators only; outputs come from the reference)

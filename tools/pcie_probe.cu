@@ -96,8 +96,7 @@ int main(int argc, char** argv) {
         f = fopen("/sys/kernel/mm/transparent_hugepage/enabled", "r");
         if (f && fgets(line, sizeof(line), f)) printf("THP: %s", line);
         if (f) fclose(f);
-        f = fopen("/proc/sys/vm/nr_hugepages", "w");     // try to reserve 2 MB pages for the HUGETLB case (root on the box)
-        if (f) { fprintf(f, "%d\n", (int)(G * 2 * (total >> 21) + 64)); fclose(f); }
+        // the HUGETLB case runs only when the host already has 2 MB pages reserved: the probe changes no host setting
     }
     for (int g = 0; g < G; ++g) { auto c = local_cpus(g); printf("gpu %d local cpus: %zu (first %d)\n", g, c.size(), c.empty() ? -1 : c[0]); }
     std::vector<int> all, lo, hi, one{0};
