@@ -95,6 +95,7 @@ struct BankMeanPlan {
 
 struct gpe_model {
     int device = 0, M = 0, D = 0, DP = 0, sms = 0;
+    const DpKernels* kern = nullptr;   // launchers compiled for DP (NULL: D > 32, generic kernels)
     double b = 0;
     double sqrt_w[32];
     bool has_invQ = false;
@@ -167,73 +168,6 @@ struct gpe_multi {
 };
 
 namespace {
-
-int pick_dp(int D) {
-    for (int i = 0; i < kNumDp; ++i)
-        if (kDpList[i] >= D) return kDpList[i];
-    return -1;
-}
-
-cudaError_t launch_full(int DP, int cfg, const FullParams& p, int grid, size_t smem, cudaStream_t st) {
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    switch (DP) {
-        case 2: return launch_full_dp2(cfg, p, grid, smem, st);
-        case 4: return launch_full_dp4(cfg, p, grid, smem, st);
-        case 6: return launch_full_dp6(cfg, p, grid, smem, st);
-        case 8: return launch_full_dp8(cfg, p, grid, smem, st);
-        case 10: return launch_full_dp10(cfg, p, grid, smem, st);
-        case 12: return launch_full_dp12(cfg, p, grid, smem, st);
-        case 16: return launch_full_dp16(cfg, p, grid, smem, st);
-        case 24: return launch_full_dp24(cfg, p, grid, smem, st);
-        case 32: return launch_full_dp32(cfg, p, grid, smem, st);
-        default: return cudaErrorInvalidValue;
-    }
-}
-
-cudaError_t launch_mean(int DP, bool hess, const MeanParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-    if (p.smem_need == 0 || p.smem_need > smem) return cudaErrorInvalidConfiguration;   // carve-up vs launch (see MeanParams)
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    switch (DP) {
-        case 2: return launch_mean_dp2(hess, p, grid, smem, st);
-        case 4: return launch_mean_dp4(hess, p, grid, smem, st);
-        case 6: return launch_mean_dp6(hess, p, grid, smem, st);
-        case 8: return launch_mean_dp8(hess, p, grid, smem, st);
-        case 10: return launch_mean_dp10(hess, p, grid, smem, st);
-        case 12: return launch_mean_dp12(hess, p, grid, smem, st);
-        case 16: return launch_mean_dp16(hess, p, grid, smem, st);
-        case 24: return launch_mean_dp24(hess, p, grid, smem, st);
-        case 32: return launch_mean_dp32(hess, p, grid, smem, st);
-        default: return cudaErrorInvalidValue;
-    }
-}
-
-cudaError_t launch_tiny(int DP, const TinyParams& p, int grid, size_t smem, cudaStream_t st) {
-    switch (DP) {
-        case 2: return launch_tiny_dp2(p, grid, smem, st);
-        case 4: return launch_tiny_dp4(p, grid, smem, st);
-        case 6: return launch_tiny_dp6(p, grid, smem, st);
-        case 8: return launch_tiny_dp8(p, grid, smem, st);
-        case 10: return launch_tiny_dp10(p, grid, smem, st);
-        case 12: return launch_tiny_dp12(p, grid, smem, st);
-        case 16: return launch_tiny_dp16(p, grid, smem, st);
-        default: return cudaErrorInvalidValue;
-    }
-}
-
-cudaError_t launch_bank_mean(int DP, int G, bool grad, const BankMeanParams& p, dim3 grid, size_t smem, cudaStream_t st) {
-    if (p.smem_need == 0 || p.smem_need > smem) return cudaErrorInvalidConfiguration;
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    switch (DP) {
-        case 2: return launch_bank_mean_dp2(G, grad, p, grid, smem, st);
-        case 4: return launch_bank_mean_dp4(G, grad, p, grid, smem, st);
-        case 6: return launch_bank_mean_dp6(G, grad, p, grid, smem, st);
-        case 8: return launch_bank_mean_dp8(G, grad, p, grid, smem, st);
-        case 10: return launch_bank_mean_dp10(G, grad, p, grid, smem, st);
-        case 12: return launch_bank_mean_dp12(G, grad, p, grid, smem, st);
-        case 16: return launch_bank_mean_dp16(G, grad, p, grid, smem, st);
-        default: return cudaErrorInvalidValue;
-    }
-}
 
 // Group size and shared-memory carve-up of k_bank_mean for a bank of E emulators: the G that minimises the FP64
 // instruction count  ceil(E / G) (G (2D + 12) + 2D)  (means only: G (D + 11) + 2D) among the compiled ones; invalid when
@@ -357,6 +291,13 @@ uint32_t mean_extent(const MeanPlan& mp, int D, int DP, bool hess) {
     return ext;
 }
 
+// cudaMalloc + copy of a host image.
+template <typename T>
+cudaError_t upload(T** d, const std::vector<T>& h) {
+    const cudaError_t e = cudaMalloc((void**)d, h.size() * sizeof(T));
+    return e == cudaSuccess ? cudaMemcpy(*d, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice) : e;
+}
+
 // [nchunks][ JC*DP sqrt(w)-scaled inputs | JC b*alpha ], zero padded
 std::vector<double> pack_xchunks(int M, int D, int DP, int JC, int nchunks, const double* inputs,
                                  const double* sqrt_w, const double* invQt, double b) {
@@ -395,13 +336,13 @@ int check_device(int device, int* sms) {
 // beyond that, and for the shapes the fused kernel does not cover, the direct kernel runs.
 constexpr double kHessFusedMaxR2 = 2000.0;
 
-int build_hessian_operand(gpe_model* m, const double* inputs, const double* invQt) {
+cudaError_t build_hessian_operand(gpe_model* m, const double* inputs, const double* invQt) {
     const FullPlan& f = m->full;
     const int M = m->M, D = m->D;
     memset(m->centre, 0, sizeof(m->centre));
     m->hess_fused_ok = false;
-    if (getenv("GPE_HESS_DIRECT") != nullptr) return GPE_OK;   // dev aid: always use the direct Hessian kernels
-    if (!f.valid || f.kbh < 1 || f.NC > M || f.NC > f.Mp) return GPE_OK;
+    if (getenv("GPE_HESS_DIRECT") != nullptr) return cudaSuccess;   // dev aid: always use the direct Hessian kernels
+    if (!f.valid || f.kbh < 1 || f.NC > M || f.NC > f.Mp) return cudaSuccess;
     double r2max = 0.0;
     for (int d = 0; d < D; ++d) {
         double lo = inputs[d], hi = inputs[d];
@@ -410,7 +351,7 @@ int build_hessian_operand(gpe_model* m, const double* inputs, const double* invQ
         const double r = m->sqrt_w[d] * 0.5 * (hi - lo);
         r2max = std::max(r2max, r * r);
     }
-    if (!(r2max <= kHessFusedMaxR2)) return GPE_OK;
+    if (!(r2max <= kHessFusedMaxR2)) return cudaSuccess;
     std::vector<double> pt((size_t)f.kblk * f.NC * 4, 0.0);
     std::vector<double> xp(D);
     for (int j = 0; j < M; ++j) {
@@ -420,11 +361,42 @@ int build_hessian_operand(gpe_model* m, const double* inputs, const double* invQ
         for (int d = 0; d < D; ++d)
             for (int e = d; e < D; ++e, ++col) pt[((size_t)(j >> 2) * f.NC + col) * 4 + (j & 3)] = ba * xp[d] * xp[e];
     }
-    cudaError_t e = cudaMalloc((void**)&m->d_ptiled, pt.size() * 8);
-    if (e == cudaSuccess) e = cudaMemcpy(m->d_ptiled, pt.data(), pt.size() * 8, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) return fail(GPE_ERR_CUDA, "model upload failed: %s", cudaGetErrorString(e));
-    m->hess_fused_ok = true;
-    return GPE_OK;
+    const cudaError_t e = upload(&m->d_ptiled, pt);
+    m->hess_fused_ok = e == cudaSuccess;
+    return e;
+}
+
+// K* scratch of the two-launch variance path (1024 < M <= GPE_MAX_TRAIN) and of the generic kernels (D > 32), and with
+// invQ the s_tiled image with the contraction padded to Mp (the scratch pads are zero): d_stiled then has Mp / 4 k-blocks.
+cudaError_t setup_large(gpe_model* m, const double* invQ) {
+    const int M = m->M;
+    m->large_Mp = (M + 63) / 64 * 64;
+    m->large_kblk = m->large_Mp / 4;
+    m->large_nstage = 6;
+    m->large_chunk = 16 * (int64_t)m->sms * 4;
+    const size_t scratch = (size_t)(m->large_chunk / 16) * m->large_kblk * 64 * 8;
+    cudaError_t e = cudaMalloc((void**)&m->d_kscratch, scratch);
+    if (e == cudaSuccess) e = cudaMemset(m->d_kscratch, 0, scratch);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&m->scratch_free, cudaEventDisableTiming);
+    if (e != cudaSuccess || !invQ || M > GPE_MAX_TRAIN) return e;
+    const size_t Mp = (size_t)m->large_Mp;
+    std::vector<double> st((size_t)m->large_kblk * Mp * 4, 0.0);
+    for (int j = 0; j < M; ++j)
+        for (int i = 0; i < M; ++i) st[((size_t)(i >> 2) * Mp + j) * 4 + (i & 3)] = invQ[(size_t)j * M + i];
+    e = upload(&m->d_stiled, st);
+    m->large_valid = e == cudaSuccess;
+    return e;
+}
+
+// k_var_large over n points whose K* is in the model's scratch (1024 < M <= GPE_MAX_TRAIN, and D > 32).
+cudaError_t var_large(const gpe_model* m, double* var, int64_t ld_var, int64_t n, cudaStream_t st) {
+    VarLargeParams v;
+    memset(&v, 0, sizeof(v));
+    v.kstar = m->d_kscratch; v.s_tiled = m->d_stiled; v.var = var; v.ld_var = ld_var; v.N = n;
+    v.Mp = m->large_Mp; v.kblk = m->large_kblk; v.npass = (m->large_Mp + kVlPass - 1) / kVlPass;
+    v.nstage = m->large_nstage; v.b = m->b;
+    const size_t smem = 128 + kVlWarps * kVlTN * 8 + (size_t)v.nstage * kVlStageBytes;
+    return launch_var_large(v, (int)std::min<int64_t>((n + kVlTN - 1) / kVlTN, m->sms), smem, st);
 }
 
 // D > 32 (predict_generic.cuh): K* of a sub-batch into the model's scratch, then gradient / variance / Hessian from it.
@@ -435,7 +407,6 @@ int predict_generic(gpe_model* m, const double* testing, int64_t N, double* mu, 
         return fail(GPE_ERR_UNSUPPORTED, "variance contraction supports M <= %d (got M = %d)", GPE_MAX_TRAIN, m->M);
     const int D = m->D;
     const size_t smem_k = ((size_t)(kGenTN + kGenJC) * (D + 1) + 128) * 8;
-    CUDA_TRY(cudaFuncSetAttribute(k_generic_kstar, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_k));
     std::lock_guard<std::mutex> scratch_lock(m->scratch_mu);   // one caller at a time between wait and record (see below)
     CUDA_TRY(cudaStreamWaitEvent(st, m->scratch_free, 0));
     for (int64_t n0 = 0; n0 < N; n0 += m->large_chunk) {
@@ -451,44 +422,50 @@ int predict_generic(gpe_model* m, const double* testing, int64_t N, double* mu, 
         p.kstar = m->d_kscratch; p.mu_tmp = m->d_gen_mu;
         p.M = m->M; p.D = D; p.kblk = m->large_kblk;
         const int64_t tiles = (n + kGenTN - 1) / kGenTN;
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        k_generic_kstar<<<(unsigned)std::min<int64_t>(tiles, (int64_t)m->sms * 4), kGenThreads, smem_k, st>>>(p);
-        CUDA_TRY(cudaGetLastError());
-        if (deriv != nullptr) {
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-            k_generic_grad<<<dim3((unsigned)std::min<int64_t>(tiles, (int64_t)m->sms * 8), (unsigned)std::min((D + 15) / 16, 16)),
-                             kGenThreads, 0, st>>>(p);
-            CUDA_TRY(cudaGetLastError());
-        }
-        if (var != nullptr) {
-            VarLargeParams v;
-            memset(&v, 0, sizeof(v));
-            v.kstar = m->d_kscratch; v.s_tiled = m->d_stiled; v.var = var + n0 * ld_var; v.ld_var = ld_var; v.N = n;
-            v.Mp = m->large_Mp; v.kblk = m->large_kblk; v.npass = (m->large_Mp + kVlPass - 1) / kVlPass;
-            v.nstage = m->large_nstage; v.b = m->b;
-            const size_t smem = 128 + kVlWarps * kVlTN * 8 + (size_t)v.nstage * kVlStageBytes;
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-            CUDA_TRY(launch_var_large(v, (int)std::min<int64_t>((n + kVlTN - 1) / kVlTN, m->sms), smem, st));
-        }
-        if (hess != nullptr) {
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-            k_generic_hess<<<(unsigned)std::min<int64_t>(n, (int64_t)m->sms * 8), kGenThreads, 0, st>>>(p);
-            CUDA_TRY(cudaGetLastError());
-        }
+        CUDA_TRY(launch_kernel(k_generic_kstar, (unsigned)std::min<int64_t>(tiles, (int64_t)m->sms * 4), kGenThreads, smem_k, st, p));
+        if (deriv != nullptr)
+            CUDA_TRY(launch_kernel(k_generic_grad, dim3((unsigned)std::min<int64_t>(tiles, (int64_t)m->sms * 8), (unsigned)std::min((D + 15) / 16, 16)),
+                                   kGenThreads, 0, st, p));
+        if (var != nullptr) CUDA_TRY(var_large(m, var + n0 * ld_var, ld_var, n, st));
+        if (hess != nullptr) CUDA_TRY(launch_kernel(k_generic_hess, (unsigned)std::min<int64_t>(n, (int64_t)m->sms * 8), kGenThreads, 0, st, p));
     }
     CUDA_TRY(cudaEventRecord(m->scratch_free, st));
     return GPE_OK;
 }
 
-// Whether a mean + variance + gradient call of call_N points takes the cluster path (predict_tiny.cuh): the fused plan's
-// resident training chunk, a compiled DP, and few enough points (GPE_TINY_MAX overrides the threshold, GPE_NO_TINY disables).
-bool tiny_ok(const gpe_model* m, int64_t call_N) {
+// Which kernels a call of call_N points runs on a model: predict_device follows it, gpe_model_plan reports it.
+enum class Path { generic, large, tiny, fused, mean };
+struct CallPlan {
+    Path path;                        // what computes a variance (mean: the model has no variance path)
+    const FullPlan* full = nullptr;   // plan of a fused launch: the main one, or 16-point tiles for a small call
+    bool fuse_hess = false;           // a requested Hessian rides on the fused launch
+};
+
+CallPlan plan_call(const gpe_model* m, int64_t call_N, bool var, bool hess) {
+    CallPlan c;
+    if (m->generic) { c.path = Path::generic; return c; }
+    // The cluster path for a mean + variance + gradient call (predict_tiny.cuh): the fused plan's resident training
+    // chunk, a compiled DP, and few enough points (GPE_TINY_MAX overrides the threshold, GPE_NO_TINY disables).
     static const bool no_tiny = getenv("GPE_NO_TINY") != nullptr;
     static const int64_t env_max = getenv("GPE_TINY_MAX") ? atoll(getenv("GPE_TINY_MAX")) : -1;
     // two clusters per 8 SMs: measured at M = 250 (tools/tiny_threshold_probe.py, synchronous device calls) the cluster path
     // takes 37.9 us against 49.3 us at 500 points and draws level with the 16-point plan at 1000
-    const int64_t n_max = env_max >= 0 ? env_max : kTinyTN * (int64_t)(2 * m->sms / kTinyCluster);
-    return !no_tiny && m->full.valid && m->full.cfg == 0 && m->full.nchunks == 1 && m->DP <= 16 && call_N <= n_max;
+    const int64_t tiny_max = env_max >= 0 ? env_max : kTinyTN * (int64_t)(2 * m->sms / kTinyCluster);
+    const FullPlan& f = m->full;
+    const bool tiny = m->has_invQ && !no_tiny && f.valid && f.cfg == 0 && f.nchunks == 1 && m->DP <= 16 && call_N <= tiny_max;
+    c.path = tiny ? Path::tiny : f.valid ? Path::fused : m->large_valid ? Path::large : Path::mean;
+    // the Hessian rides on the fused kernel when the model qualifies (build_hessian_operand); without a variance
+    // request that only pays for the 64-point tiles of cfg 0 (measured: 4.6e8 vs 3.6e8 points/s at M = 250, but
+    // 0.98e8 vs 1.10e8 at M = 1000), so larger M keeps the direct kernel for Hessian-only calls
+    // (the HESS variants are built on the plain variance operand: with a symmetric-folded model the Hessian only rides
+    // along when no variance is requested -- phase B is then skipped and the fold does not matter)
+    // (calls small enough for the cluster path take the variance from it whatever else is requested, and the Hessian
+    // from the direct kernel: every output of a call of a given size comes from the same kernel for any combination of flags)
+    c.fuse_hess = hess && m->hess_fused_ok && !tiny && (var ? !m->symmetric : f.cfg == 0);
+    // up to three waves of 16-point tiles finish sooner than one wave of 64-point tiles
+    const bool small = m->full_small.valid && !c.fuse_hess && call_N <= 3 * 16 * (int64_t)m->sms;
+    c.full = small ? &m->full_small : &m->full;
+    return c;
 }
 
 // Launch the kernels for device-resident data on `st`.  Output strides allow bank (point-major) layouts.
@@ -499,19 +476,11 @@ int predict_device(gpe_model* m, const double* testing, int64_t N, double* mu, d
     // summation order depend on it, not on the chunk, so that one call is internally consistent
     if (call_N < 0) call_N = N;
     if (N == 0) return GPE_OK;
-    if (m->generic) return predict_generic(m, testing, N, mu, var, deriv, hess, ld_mu, ld_var, ld_deriv, ld_hess, st);
+    const CallPlan c = plan_call(m, call_N, var != nullptr, hess != nullptr);
+    if (c.path == Path::generic) return predict_generic(m, testing, N, mu, var, deriv, hess, ld_mu, ld_var, ld_deriv, ld_hess, st);
     bool mean_done = false;
     static const bool force_full = getenv("GPE_FORCE_FULL") != nullptr;  // dev aid: time phase A alone
-    // the Hessian rides on the fused kernel when the model qualifies (build_hessian_operand); without a variance
-    // request that only pays for the 64-point tiles of cfg 0 (measured: 4.6e8 vs 3.6e8 points/s at M = 250, but
-    // 0.98e8 vs 1.10e8 at M = 1000), so larger M keeps the direct kernel for Hessian-only calls
-    // (the HESS variants are built on the plain variance operand: with a symmetric-folded model the Hessian only rides
-    // along when no variance is requested -- phase B is then skipped and the fold does not matter)
-    // (calls small enough for the cluster path below take the variance from it whatever else is requested, and the Hessian
-    // from the direct kernel: every output of a call of a given size comes from the same kernel for any combination of flags)
-    const bool tiny = m->has_invQ && tiny_ok(m, call_N);
-    const bool fuse_hess = hess != nullptr && m->hess_fused_ok && !tiny && (var != nullptr ? !m->symmetric : m->full.cfg == 0);
-    if (var != nullptr && m->has_invQ && !m->full.valid && m->large_valid) {
+    if (var != nullptr && c.path == Path::large) {
         // 1024 < M <= GPE_MAX_TRAIN: per sub-batch, K* + mean + gradient (k_predict_mean2<DP, true>) into the scratch,
         // then the column-pass contraction (k_var_large).  The scratch is per model: streams take turns.
         // (two threads on different streams must not both pass the wait before either records: hold the model's
@@ -532,16 +501,8 @@ int predict_device(gpe_model* m, const double* testing, int64_t N, double* mu, d
             p.kstar = m->d_kscratch; p.kblk = m->large_kblk;
             memcpy(p.sqrt_w, m->sqrt_w, sizeof(p.sqrt_w));
             const int64_t mtiles = (n + kMeanTN - 1) / kMeanTN;
-            CUDA_TRY(launch_mean(m->DP, false, p, dim3((unsigned)std::min<int64_t>(mtiles, (int64_t)m->sms * 12)), m->mean.smem, st));
-            VarLargeParams v;
-            memset(&v, 0, sizeof(v));
-            v.kstar = m->d_kscratch; v.s_tiled = m->d_stiled; v.var = var + n0 * ld_var; v.ld_var = ld_var; v.N = n;
-            v.Mp = m->large_Mp; v.kblk = m->large_kblk; v.npass = (m->large_Mp + kVlPass - 1) / kVlPass;
-            v.nstage = m->large_nstage; v.b = m->b;
-            const size_t smem = 128 + kVlWarps * kVlTN * 8 + (size_t)v.nstage * kVlStageBytes;
-            const int64_t vtiles = (n + kVlTN - 1) / kVlTN;
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-            CUDA_TRY(launch_var_large(v, (int)std::min<int64_t>(vtiles, m->sms), smem, st));
+            CUDA_TRY(m->kern->mean(false, p, dim3((unsigned)std::min<int64_t>(mtiles, (int64_t)m->sms * 12)), m->mean.smem, st));
+            CUDA_TRY(var_large(m, var + n0 * ld_var, ld_var, n, st));
         }
         CUDA_TRY(cudaEventRecord(m->scratch_free, st));
         mean_done = true;
@@ -549,7 +510,7 @@ int predict_device(gpe_model* m, const double* testing, int64_t N, double* mu, d
     }
     // A handful of points (up to two clusters per 8 SMs): the latency path, one 8-CTA cluster per 16-point tile
     // (predict_tiny.cuh).  Needs the fused plan's resident training chunk; a Hessian request goes the usual way.
-    if (var != nullptr && tiny) {
+    if (var != nullptr && c.path == Path::tiny) {
         const FullPlan& f = m->full;
         TinyParams p;
         memset(&p, 0, sizeof(p));
@@ -562,18 +523,15 @@ int predict_device(gpe_model* m, const double* testing, int64_t N, double* mu, d
                                               (size_t)16 * 16 * (m->DP + 1), (size_t)8 * 16 * 32});
         const size_t smem = ((size_t)kTinyTN * (f.Mp + 4) + work) * 8;
         const int grid = (int)((N + kTinyTN - 1) / kTinyTN) * kTinyCluster;
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        CUDA_TRY(launch_tiny(m->DP, p, grid, smem, st));
+        CUDA_TRY(m->kern->tiny(p, grid, smem, st));
         mean_done = true;
         var = nullptr;
     }
-    if (var != nullptr || fuse_hess || (force_full && m->full.valid)) {
+    if (var != nullptr || c.fuse_hess || (force_full && m->full.valid)) {
         if (var != nullptr && !m->has_invQ) return fail(GPE_ERR_INVALID, "variance requested but the model was created without invQ");
         if (!m->full.valid)
             return fail(GPE_ERR_UNSUPPORTED, "variance contraction supports M <= %d (got M = %d)", GPE_MAX_TRAIN, m->M);
-        // up to three waves of 16-point tiles finish sooner than one wave of 64-point tiles
-        const bool small = m->full_small.valid && !fuse_hess && call_N <= 3 * 16 * (int64_t)m->sms;
-        const FullPlan& f = small ? m->full_small : m->full;
+        const FullPlan& f = *c.full;
         FullParams p;
         memset(&p, 0, sizeof(p));
         p.testing = testing; p.N = N; p.mu = mu; p.var = var; p.deriv = deriv;
@@ -593,14 +551,14 @@ int predict_device(gpe_model* m, const double* testing, int64_t N, double* mu, d
         p.stage_bytes = f.stage_bytes; p.ts_bytes = f.ts_bytes;
         memcpy(p.sqrt_w, m->sqrt_w, sizeof(p.sqrt_w));
         p.trace = g_trace;
-        if (fuse_hess) {
+        if (c.fuse_hess) {
             p.hess = hess; p.ld_hess = ld_hess; p.p_tiled = m->d_ptiled; p.kbh = f.kbh; p.nit_h = f.nit_h; p.off_hts = f.off_hts;
             memcpy(p.centre, m->centre, sizeof(p.centre));
             hess = nullptr;   // done by this launch
         }
         const int64_t ntiles = (N + f.TN - 1) / f.TN;
         const int grid = (int)std::min<int64_t>(ntiles, (int64_t)m->sms * f.ctas_per_sm);
-        CUDA_TRY(launch_full(m->DP, f.cfg, p, grid, f.smem, st));
+        CUDA_TRY(m->kern->full(f.cfg, p, grid, f.smem, st));
         mean_done = true;
     }
     const bool need_mean = !mean_done && (mu != nullptr || deriv != nullptr);
@@ -623,7 +581,7 @@ int predict_device(gpe_model* m, const double* testing, int64_t N, double* mu, d
         const int mult = env_mult > 0 ? env_mult : (do_hess ? 8 : 12);
         const int grid = (int)std::min<int64_t>(ntiles, (int64_t)m->sms * mult);
         const size_t smem = do_hess ? m->mean.smem_hess : m->mean.smem;
-        CUDA_TRY(launch_mean(m->DP, do_hess, p, dim3(grid), smem, st));
+        CUDA_TRY(m->kern->mean(do_hess, p, dim3(grid), smem, st));
     }
     return GPE_OK;
 }
@@ -691,27 +649,81 @@ int run_per_device(int G, const int* devices, Fn fn) {
     return GPE_OK;
 }
 
-// Host-resident FP64 predict of one model: its share of a call of call_N points (the whole call unless `shared`
-// hands out the chunks of a multi-device call).  Caller holds m->host_mu.
-int model_stream(gpe_model* m, const double* testing, int64_t N, double* mu, double* var, double* deriv, double* hess,
-                 const StreamPlan* shared_plan = nullptr, ChunkSource* shared = nullptr, const Relay* relay = nullptr) {
-    const int64_t D = m->D;
+// Request check of every entry point.  outs are the entry point's output arrays in GPE_WANT_* bit order (mu, var,
+// deriv, hess, fwd, deriv_full), as many as it has: an array whose flag is clear is dropped; a set flag with a NULL
+// array, or a call that asks for nothing, is an error.
+template <typename... T>
+int take_outputs(unsigned flags, T*&... outs) {
+    unsigned bit = GPE_WANT_MU;
+    bool missing = false, any = false;
+    auto take = [&](auto*& o) {
+        if (!(flags & bit)) o = nullptr;
+        else if (!o) missing = true;
+        any = any || o != nullptr;
+        bit <<= 1;
+    };
+    (take(outs), ...);
+    if (missing) return fail(GPE_ERR_INVALID, "an output flag is set but its array is NULL");
+    if (!any) return fail(GPE_ERR_INVALID, "no output requested");
+    return GPE_OK;
+}
+
+// The streamed arrays of one host-resident call, in the order its chunk launch reads them: idx[k] is the chunk array
+// of the call kind's k-th array (-1: not streamed).
+struct CallIo {
     IoList in, out;
-    in.add(testing, D);
-    const int i_mu = mu ? out.add(mu, 1) : -1, i_var = var ? out.add(var, 1) : -1, i_der = deriv ? out.add(deriv, D) : -1,
-              i_hes = hess ? out.add(hess, D * D) : -1;
-    StreamPlan pl = shared_plan ? *shared_plan : plan_stream(in.v, in.n, out.v, out.n, N, 8, 64 * (int64_t)m->sms, 1, true);
-    int rc = prepare_slots(m->slots, pl, in.v, in.n, out.v, out.n, 8);
+    int idx[6] = {-1, -1, -1, -1, -1, -1};
+    template <typename T>
+    T* at(void* const* chunk, int k) const { return idx[k] >= 0 ? (T*)chunk[idx[k]] : nullptr; }
+};
+
+// Single GP: testing in; mu, var, deriv, hess out (idx 0-3).
+CallIo model_io(int64_t D, const void* testing, const void* mu, const void* var, const void* deriv, const void* hess) {
+    CallIo io;
+    io.in.add(testing, D);
+    io.idx[0] = mu ? io.out.add(mu, 1) : -1;
+    io.idx[1] = var ? io.out.add(var, 1) : -1;
+    io.idx[2] = deriv ? io.out.add(deriv, D) : -1;
+    io.idx[3] = hess ? io.out.add(hess, D * D) : -1;
+    return io;
+}
+
+// The part of a multi-device call that one pipeline runs: the call's shared chunk plan and cursor, the device's relay.
+struct SharedCall {
+    const StreamPlan* plan;
+    ChunkSource* src;
+    const Relay* relay;
+};
+
+// Chunk plan of a call of N points: for one pipeline of its own (shared_by = 0: the mapped-buffer path is open to tiny
+// calls), or shared by that many pipelines pulling from one cursor.
+StreamPlan stream_plan(const CallIo& io, int64_t N, size_t ES, int sms, int shared_by = 0) {
+    return plan_stream(io.in.v, io.in.n, io.out.v, io.out.n, N, ES, 64 * (int64_t)sms, std::max(shared_by, 1), shared_by == 0);
+}
+
+// Run a host-resident call of N points through an owner's slots (caller holds the owner's host_mu): with a plan and a
+// cursor of its own, or with `shared` its share of a multi-device call.  launch(n0, n, d_ins, d_outs, stream) enqueues
+// the kernels of one chunk (host_stream.h).
+template <typename Launch>
+int stream_call(Slot* slots, int device, int sms, const CallIo& io, int64_t N, size_t ES, const SharedCall* shared,
+                Launch launch) {
+    const StreamPlan pl = shared ? *shared->plan : stream_plan(io, N, ES, sms);
+    int rc = prepare_slots(slots, pl, io.in.v, io.in.n, io.out.v, io.out.n, ES);
     if (rc) return rc;
     std::atomic<int64_t> cursor{0};
-    ChunkSource src = shared ? *shared : ChunkSource{&cursor, N, pl.CH};
-    const int64_t call_N = src.N;   // plan choices that change the summation order follow the size of the API call
-    return stream_host(m->slots, m->device, pl, src, 8, in.v, in.n, out.v, out.n,
+    const ChunkSource src = shared ? *shared->src : ChunkSource{&cursor, N, pl.CH};
+    return stream_host(slots, device, pl, src, ES, io.in.v, io.in.n, io.out.v, io.out.n, launch, shared ? shared->relay : nullptr);
+}
+
+// Host-resident FP64 predict of one model.  Plan choices that change the summation order follow the size N of the API
+// call, not of a chunk.
+int model_stream(gpe_model* m, int64_t N, const CallIo& io, const SharedCall* shared = nullptr) {
+    const int64_t D = m->D;
+    return stream_call(m->slots, m->device, m->sms, io, N, 8, shared,
                        [&](int64_t, int64_t n, void* const* di, void* const* dout, cudaStream_t st) {
-                           auto at = [&](int i) { return i >= 0 ? (double*)dout[i] : nullptr; };
-                           return predict_device(m, (const double*)di[0], n, at(i_mu), at(i_var), at(i_der), at(i_hes), 1, 1,
-                                                 D, D * D, st, call_N);
-                       }, relay);
+                           return predict_device(m, (const double*)di[0], n, io.at<double>(dout, 0), io.at<double>(dout, 1),
+                                                 io.at<double>(dout, 2), io.at<double>(dout, 3), 1, 1, D, D * D, st, N);
+                       });
 }
 
 // ---- PCA back-projection: out (R, W) = A (R, E) . basis (E, W): kernels and launcher in project.cu ----------------
@@ -764,8 +776,7 @@ int ensure_tf32(gpe_model* m) {
         for (int d = 0; d < D; ++d) xa[(size_t)j * DP + d] = (float)(m->sqrt_w[d] * m->h_inputs[(size_t)j * D + d]);
         xa[(size_t)Mp * DP + j] = (float)(m->b * m->h_invQt[j]);
     }
-    CUDA_TRY(cudaMalloc((void**)&m->d_xa_f32, xa.size() * 4));
-    CUDA_TRY(cudaMemcpy(m->d_xa_f32, xa.data(), xa.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(upload(&m->d_xa_f32, xa));
     if (!m->h_invQ.empty()) {
         // B operand: slab s holds invQ[j][32 s .. 32 s + 31] for every output column j as a [Mp][128 B] image with
         // the 16-byte chunk index XOR-ed by (j % 8): exactly what a SWIZZLE_128B K-major UMMA descriptor reads.
@@ -782,10 +793,8 @@ int ensure_tf32(gpe_model* m) {
                 bh[at] = hi;
                 bl[at] = host_tf32_rna(x - hf);
             }
-        CUDA_TRY(cudaMalloc((void**)&m->d_bslabs, bh.size() * 4));
-        CUDA_TRY(cudaMemcpy(m->d_bslabs, bh.data(), bh.size() * 4, cudaMemcpyHostToDevice));
-        CUDA_TRY(cudaMalloc((void**)&m->d_bslabs_lo, bl.size() * 4));
-        CUDA_TRY(cudaMemcpy(m->d_bslabs_lo, bl.data(), bl.size() * 4, cudaMemcpyHostToDevice));
+        CUDA_TRY(upload(&m->d_bslabs, bh));
+        CUDA_TRY(upload(&m->d_bslabs_lo, bl));
     }
     m->tf = fast;
     m->tfx = prec;
@@ -803,7 +812,6 @@ int predict_device_f32(gpe_model* m, const float* testing, int64_t N, float* mu,
     const Tf32Plan& t = x3 ? m->tfx : m->tf;
     const int64_t ntiles = (N + kTfTN - 1) / kTfTN;
     const int grid = (int)std::min<int64_t>(ntiles, m->sms);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
     if (t.big) {
         Tf32BigParams p;
         memset(&p, 0, sizeof(p));
@@ -893,7 +901,9 @@ int gpe_model_create_ex(int device, int M, int D, const double* inputs, const do
     if (rc) return rc;
     CUDA_TRY(cudaSetDevice(device));
     gpe_model* m = new gpe_model();
-    m->device = device; m->M = M; m->D = D; m->DP = pick_dp(D); m->sms = sms;
+    m->device = device; m->M = M; m->D = D; m->sms = sms;
+    m->kern = dp_kernels(D);
+    m->DP = m->kern ? m->kern->DP : -1;
     m->b = expX[D];
     for (int d = 0; d < 32; ++d) m->sqrt_w[d] = (d < D) ? std::sqrt(expX[d]) : 0.0;
     m->has_invQ = invQ != nullptr;
@@ -903,36 +913,17 @@ int gpe_model_create_ex(int device, int M, int D, const double* inputs, const do
         // (predict_generic.cuh); the symmetric fold does not apply (k_var_large reads the plain operand)
         m->generic = true;
         m->symmetric = false;
-        m->large_Mp = (M + 63) / 64 * 64;
-        m->large_kblk = m->large_Mp / 4;
-        m->large_nstage = 6;
-        m->large_chunk = 16 * (int64_t)m->sms * 4;
         std::vector<double> xs((size_t)M * D), al(M), sq(D);
         for (int d = 0; d < D; ++d) sq[d] = std::sqrt(expX[d]);
         for (int j = 0; j < M; ++j) {
             for (int d = 0; d < D; ++d) xs[(size_t)j * D + d] = sq[d] * inputs[(size_t)j * D + d];
             al[j] = m->b * invQt[j];
         }
-        const size_t scratch = (size_t)(m->large_chunk / 16) * m->large_kblk * 64 * 8;
-        cudaError_t e = cudaMalloc((void**)&m->d_gen_xs, xs.size() * 8);
-        if (e == cudaSuccess) e = cudaMemcpy(m->d_gen_xs, xs.data(), xs.size() * 8, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&m->d_gen_alpha, al.size() * 8);
-        if (e == cudaSuccess) e = cudaMemcpy(m->d_gen_alpha, al.data(), al.size() * 8, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&m->d_gen_sqw, sq.size() * 8);
-        if (e == cudaSuccess) e = cudaMemcpy(m->d_gen_sqw, sq.data(), sq.size() * 8, cudaMemcpyHostToDevice);
+        cudaError_t e = setup_large(m, invQ);
+        if (e == cudaSuccess) e = upload(&m->d_gen_xs, xs);
+        if (e == cudaSuccess) e = upload(&m->d_gen_alpha, al);
+        if (e == cudaSuccess) e = upload(&m->d_gen_sqw, sq);
         if (e == cudaSuccess) e = cudaMalloc((void**)&m->d_gen_mu, (size_t)m->large_chunk * 8);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&m->d_kscratch, scratch);
-        if (e == cudaSuccess) e = cudaMemset(m->d_kscratch, 0, scratch);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&m->scratch_free, cudaEventDisableTiming);
-        if (e == cudaSuccess && invQ && M <= GPE_MAX_TRAIN) {
-            const size_t Mp = (size_t)m->large_Mp;
-            std::vector<double> st((size_t)m->large_kblk * Mp * 4, 0.0);
-            for (int j = 0; j < M; ++j)
-                for (int i = 0; i < M; ++i) st[((size_t)(i >> 2) * Mp + j) * 4 + (i & 3)] = invQ[(size_t)j * M + i];
-            e = cudaMalloc((void**)&m->d_stiled, st.size() * 8);
-            if (e == cudaSuccess) e = cudaMemcpy(m->d_stiled, st.data(), st.size() * 8, cudaMemcpyHostToDevice);
-            m->large_valid = e == cudaSuccess;
-        }
         if (e != cudaSuccess) { gpe_model_destroy(m); return fail(GPE_ERR_CUDA, "model upload failed: %s", cudaGetErrorString(e)); }
         *out = m;
         return GPE_OK;
@@ -942,17 +933,11 @@ int gpe_model_create_ex(int device, int M, int D, const double* inputs, const do
     if (invQ && M <= 1024) m->h_invQ.assign(invQ, invQ + (size_t)M * M);
     for (int d = 0; d <= D; ++d) m->h_expx[d] = expX[d];
     m->mean = plan_mean(M, D, m->DP);
-    {
-        std::vector<double> xc = pack_xchunks(M, D, m->DP, m->mean.JC, m->mean.nchunks, inputs, m->sqrt_w, invQt, m->b);
-        cudaError_t e = cudaMalloc((void**)&m->d_xchunks_mean, xc.size() * 8);
-        if (e == cudaSuccess) e = cudaMemcpy(m->d_xchunks_mean, xc.data(), xc.size() * 8, cudaMemcpyHostToDevice);
-        if (e != cudaSuccess) { gpe_model_destroy(m); return fail(GPE_ERR_CUDA, "model upload failed: %s", cudaGetErrorString(e)); }
-    }
-    if (invQ) {
+    cudaError_t e = upload(&m->d_xchunks_mean, pack_xchunks(M, D, m->DP, m->mean.JC, m->mean.nchunks, inputs, m->sqrt_w, invQt, m->b));
+    if (e == cudaSuccess && invQ) {
         m->full = plan_full(M, D, m->DP);
         if (m->full.valid) {
             const FullPlan& f = m->full;
-            std::vector<double> xc = pack_xchunks(M, D, m->DP, f.JC, f.nchunks, inputs, m->sqrt_w, invQt, m->b);
             // s_tiled[kb][j][c] = invQ[j][4 kb + c]
             std::vector<double> st((size_t)f.kblk * f.Mp * 4, 0.0);
             for (int j = 0; j < M; ++j)
@@ -962,38 +947,19 @@ int gpe_model_create_ex(int device, int M, int D, const double* inputs, const do
                         v = (i < j) ? invQ[(size_t)j * M + i] + invQ[(size_t)i * M + j] : (i == j ? v : 0.0);
                     st[((size_t)(i >> 2) * f.Mp + j) * 4 + (i & 3)] = v;
                 }
-            cudaError_t e = cudaMalloc((void**)&m->d_xchunks_full, xc.size() * 8);
-            if (e == cudaSuccess) e = cudaMemcpy(m->d_xchunks_full, xc.data(), xc.size() * 8, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) e = cudaMalloc((void**)&m->d_stiled, st.size() * 8);
-            if (e == cudaSuccess) e = cudaMemcpy(m->d_stiled, st.data(), st.size() * 8, cudaMemcpyHostToDevice);
-            if (e != cudaSuccess) { gpe_model_destroy(m); return fail(GPE_ERR_CUDA, "model upload failed: %s", cudaGetErrorString(e)); }
-            rc = build_hessian_operand(m, inputs, invQt);
-            if (rc) { gpe_model_destroy(m); return rc; }
+            e = upload(&m->d_xchunks_full, pack_xchunks(M, D, m->DP, f.JC, f.nchunks, inputs, m->sqrt_w, invQt, m->b));
+            if (e == cudaSuccess) e = upload(&m->d_stiled, st);
+            if (e == cudaSuccess) e = build_hessian_operand(m, inputs, invQt);
             // low-latency plan for small batches: a 64-point tile costs ~45 us at M = 250 even for one point
             if (f.cfg == 0 && f.Mp % 64 == 0 && getenv("GPE_NO_SMALL_PLAN") == nullptr) {
                 FullPlan fs = plan_full(M, D, m->DP, f.Mp);
                 if (fs.valid && fs.JC == f.JC && fs.nchunks == f.nchunks && fs.kblk == f.kblk) m->full_small = fs;
             }
         } else if (M <= GPE_MAX_TRAIN) {
-            // beyond the fused kernel: s_tiled with the contraction padded to Mp (the K* scratch pads are zero)
-            m->large_Mp = (M + 63) / 64 * 64;
-            m->large_kblk = m->large_Mp / 4;
-            m->large_nstage = 6;
-            m->large_chunk = 16 * (int64_t)m->sms * 4;
-            const size_t Mp = (size_t)m->large_Mp;
-            std::vector<double> st((size_t)m->large_kblk * Mp * 4, 0.0);
-            for (int j = 0; j < M; ++j)
-                for (int i = 0; i < M; ++i) st[((size_t)(i >> 2) * Mp + j) * 4 + (i & 3)] = invQ[(size_t)j * M + i];
-            const size_t scratch = (size_t)(m->large_chunk / 16) * m->large_kblk * 64 * 8;
-            cudaError_t e = cudaMalloc((void**)&m->d_stiled, st.size() * 8);
-            if (e == cudaSuccess) e = cudaMemcpy(m->d_stiled, st.data(), st.size() * 8, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) e = cudaMalloc((void**)&m->d_kscratch, scratch);
-            if (e == cudaSuccess) e = cudaMemset(m->d_kscratch, 0, scratch);
-            if (e == cudaSuccess) e = cudaEventCreateWithFlags(&m->scratch_free, cudaEventDisableTiming);
-            if (e != cudaSuccess) { gpe_model_destroy(m); return fail(GPE_ERR_CUDA, "model upload failed: %s", cudaGetErrorString(e)); }
-            m->large_valid = true;
+            e = setup_large(m, invQ);   // beyond the fused kernel: the two-launch variance path
         }
     }
+    if (e != cudaSuccess) { gpe_model_destroy(m); return fail(GPE_ERR_CUDA, "model upload failed: %s", cudaGetErrorString(e)); }
     *out = m;
     return GPE_OK;
 }
@@ -1023,28 +989,25 @@ int gpe_model_destroy(gpe_model* m) {
 // roofline instead of a hard-coded name).  Returns the number of characters written.
 int gpe_model_plan(gpe_model* m, int64_t N, char* buf, int len) {
     if (!m || !buf || len <= 0) return 0;
-    auto full_name = [&](const FullPlan& f, char* out, int n) {
-        // template arguments as instantiated in predict_full_inst.cu: <MT, NT, WR, WC, DP, MINB, KB, FULLNT, SYM, HESS>
-        static const int MT[3] = {4, 4, 2}, WR[3] = {2, 1, 1}, WC[3] = {4, 8, 8}, MINB[3] = {1, 1, 1}, KB[3] = {2, 1, 1};
-        const int nt_inst = f.cfg == 0 ? f.nt_act : (f.cfg == 1 ? (f.nt_act >= 5 && f.nt_act <= 7 ? f.nt_act : 8)
-                                                                  : (f.nt_act >= 9 && f.nt_act <= 15 ? f.nt_act : 16));
-        return snprintf(out, n, "k_predict_full<%d,%d,%d,%d,%d,%d,%d,%s,%s,false> (cfg %d: %d-point tiles, Mp=%d, %d-stage TMA ring, %u B smem)",
-                        MT[f.cfg], nt_inst, WR[f.cfg], WC[f.cfg], m->DP, MINB[f.cfg], KB[f.cfg], nt_inst == f.nt_act ? "true" : "false",
-                        m->symmetric ? "true" : "false", f.cfg, f.TN, f.Mp, f.nstage, f.smem);
-    };
-    if (m->generic)
-        return snprintf(buf, len, "k_generic_kstar + k_generic_grad%s (D = %d > 32: generic kernels on the K* scratch)",
-                        m->large_valid ? " + k_var_large" : "", m->D);
-    if (m->has_invQ && tiny_ok(m, N))
-        return snprintf(buf, len, "k_predict_tiny<%d> (one 8-CTA cluster per 16-point tile, Mp=%d)", m->DP, m->full.Mp);
-    if (m->full.valid) {
-        const bool small = m->full_small.valid && N <= 3 * 16 * (int64_t)m->sms;
-        return full_name(small ? m->full_small : m->full, buf, len);
+    const CallPlan c = plan_call(m, N, true, false);
+    switch (c.path) {
+        case Path::generic:
+            return snprintf(buf, len, "k_generic_kstar + k_generic_grad%s (D = %d > 32: generic kernels on the K* scratch)",
+                            m->large_valid ? " + k_var_large" : "", m->D);
+        case Path::tiny:
+            return snprintf(buf, len, "k_predict_tiny<%d> (one 8-CTA cluster per 16-point tile, Mp=%d)", m->DP, m->full.Mp);
+        case Path::fused: {
+            const FullPlan& f = *c.full;
+            const int n = std::min(m->kern->full_name(f.cfg, f.nt_act, m->symmetric, buf, len), len - 1);
+            return n + snprintf(buf + n, len - n, " (cfg %d: %d-point tiles, Mp=%d, %d-stage TMA ring, %u B smem)", f.cfg, f.TN,
+                                f.Mp, f.nstage, f.smem);
+        }
+        case Path::large:
+            return snprintf(buf, len, "k_predict_mean2<%d,true> + k_var_large (Mp=%d, %d k-blocks, %d-stage ring)", m->DP,
+                            m->large_Mp, m->large_kblk, m->large_nstage);
+        case Path::mean: break;
     }
-    if (m->large_valid)
-        return snprintf(buf, len, "k_predict_mean2<%d,true> + k_var_large (Mp=%d, %d k-blocks, %d-stage ring)", m->DP, m->large_Mp,
-                        m->large_kblk, m->large_nstage);
-    return snprintf(buf, len, "k_predict_mean2<%d,false> (no invQ: mean + gradient only)", m->DP);
+    return snprintf(buf, len, "%s<%d,false> (no invQ: mean + gradient only)", m->kern->mean_name(), m->DP);
 }
 
 int gpe_predict(gpe_model* m, const double* testing, int64_t N, double* mu, double* var, double* deriv, double* hess,
@@ -1054,19 +1017,12 @@ int gpe_predict(gpe_model* m, const double* testing, int64_t N, double* mu, doub
     if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
     if (N == 0) return GPE_OK;
     if (!testing) return fail(GPE_ERR_INVALID, "testing is NULL");
-    if (!(flags & GPE_WANT_MU)) mu = nullptr;
-    if (!(flags & GPE_WANT_VAR)) var = nullptr;
-    if (!(flags & GPE_WANT_DERIV)) deriv = nullptr;
-    if (!(flags & GPE_WANT_HESS)) hess = nullptr;
-    if ((flags & GPE_WANT_MU) && !mu) return fail(GPE_ERR_INVALID, "GPE_WANT_MU set but mu is NULL");
-    if ((flags & GPE_WANT_VAR) && !var) return fail(GPE_ERR_INVALID, "GPE_WANT_VAR set but var is NULL");
-    if ((flags & GPE_WANT_DERIV) && !deriv) return fail(GPE_ERR_INVALID, "GPE_WANT_DERIV set but deriv is NULL");
-    if ((flags & GPE_WANT_HESS) && !hess) return fail(GPE_ERR_INVALID, "GPE_WANT_HESS set but hess is NULL");
-    if (!mu && !var && !deriv && !hess) return fail(GPE_ERR_INVALID, "no output requested");
+    int rc = take_outputs(flags, mu, var, deriv, hess);
+    if (rc) return rc;
     CUDA_TRY(cudaSetDevice(m->device));
     if (flags & GPE_HOST_PTRS) {
         std::lock_guard<std::mutex> lock(m->host_mu);
-        return model_stream(m, testing, N, mu, var, deriv, hess);
+        return model_stream(m, N, model_io(m->D, testing, mu, var, deriv, hess));
     }
     return predict_device(m, testing, N, mu, var, deriv, hess, 1, 1, m->D, (int64_t)m->D * m->D,
                           (cudaStream_t)stream);
@@ -1079,13 +1035,8 @@ int gpe_predict_f32(gpe_model* m, const float* testing, int64_t N, float* mu, fl
     if (N == 0) return GPE_OK;
     if (!testing) return fail(GPE_ERR_INVALID, "testing is NULL");
     if (flags & GPE_WANT_HESS) return fail(GPE_ERR_UNSUPPORTED, "the single-precision path has no Hessian output");
-    if (!(flags & GPE_WANT_MU)) mu = nullptr;
-    if (!(flags & GPE_WANT_VAR)) var = nullptr;
-    if (!(flags & GPE_WANT_DERIV)) deriv = nullptr;
-    if ((flags & GPE_WANT_MU) && !mu) return fail(GPE_ERR_INVALID, "GPE_WANT_MU set but mu is NULL");
-    if ((flags & GPE_WANT_VAR) && !var) return fail(GPE_ERR_INVALID, "GPE_WANT_VAR set but var is NULL");
-    if ((flags & GPE_WANT_DERIV) && !deriv) return fail(GPE_ERR_INVALID, "GPE_WANT_DERIV set but deriv is NULL");
-    if (!mu && !var && !deriv) return fail(GPE_ERR_INVALID, "no output requested");
+    int rc = take_outputs(flags, mu, var, deriv);
+    if (rc) return rc;
     CUDA_TRY(cudaSetDevice(m->device));
     // variance mode: 3xTF32 split unless asked otherwise -- except for M > 256, where the FP32 accumulation of the
     // long sums dominates the error anyway (1.1e-5 vs 1.5e-5 at M = 1000) and the split costs 3.6x: there the
@@ -1094,18 +1045,11 @@ int gpe_predict_f32(gpe_model* m, const float* testing, int64_t N, float* mu, fl
     std::lock_guard<std::mutex> lock(m->host_mu);   // also covers the lazy packing of the FP32 operands
     if (!(flags & GPE_HOST_PTRS)) return predict_device_f32(m, testing, N, mu, var, deriv, fast, (cudaStream_t)stream);
     // host pointers: the same overlapped pipeline as the FP64 path
-    const int64_t D = m->D;
-    IoList in, out;
-    in.add(testing, D);
-    const int i_mu = mu ? out.add(mu, 1) : -1, i_var = var ? out.add(var, 1) : -1, i_der = deriv ? out.add(deriv, D) : -1;
-    const StreamPlan pl = plan_stream(in.v, in.n, out.v, out.n, N, 4, 64 * (int64_t)m->sms, 1, true);
-    int rc = prepare_slots(m->slots, pl, in.v, in.n, out.v, out.n, 4);
-    if (rc) return rc;
-    std::atomic<int64_t> cursor{0};
-    return stream_host(m->slots, m->device, pl, ChunkSource{&cursor, N, pl.CH}, 4, in.v, in.n, out.v, out.n,
+    const CallIo io = model_io(m->D, testing, mu, var, deriv, nullptr);
+    return stream_call(m->slots, m->device, m->sms, io, N, 4, nullptr,
                        [&](int64_t, int64_t n, void* const* di, void* const* dout, cudaStream_t st) {
-                           auto at = [&](int i) { return i >= 0 ? (float*)dout[i] : nullptr; };
-                           return predict_device_f32(m, (const float*)di[0], n, at(i_mu), at(i_var), at(i_der), fast, st);
+                           return predict_device_f32(m, (const float*)di[0], n, io.at<float>(dout, 0), io.at<float>(dout, 1),
+                                                     io.at<float>(dout, 2), fast, st);
                        });
 }
 
@@ -1202,7 +1146,7 @@ int bank_predict_device(gpe_bank* b, const double* testing, int64_t N, double* m
         const int64_t ntiles = (N + kBankTN - 1) / kBankTN;
         const int resident = grad ? 2 : 3;   // CTAs per SM (launch bounds of k_bank_mean)
         const int gx = (int)std::min<int64_t>(ntiles, std::max<int64_t>(1, (int64_t)m0->sms * resident / g.ngroups));
-        CUDA_TRY(launch_bank_mean(m0->DP, g.G, grad != 0, p, dim3(gx, (unsigned)g.ngroups), g.smem, stream));
+        CUDA_TRY(m0->kern->bank_mean(g.G, grad != 0, p, dim3(gx, (unsigned)g.ngroups), g.smem, stream));
         return GPE_OK;
     }
     if (hess != nullptr || (!with_var && (mu != nullptr || deriv != nullptr))) {
@@ -1225,7 +1169,7 @@ int bank_predict_device(gpe_bank* b, const double* testing, int64_t N, double* m
         const int64_t ntiles = (N + kMeanTN - 1) / kMeanTN;
         const int gx = (int)std::min<int64_t>(ntiles, std::max<int64_t>(1, (int64_t)m0->sms * 8 / E));
         const size_t smem = do_hess ? m0->mean.smem_hess : m0->mean.smem;
-        CUDA_TRY(launch_mean(m0->DP, do_hess, p, dim3(gx, (unsigned)E), smem, stream));
+        CUDA_TRY(m0->kern->mean(do_hess, p, dim3(gx, (unsigned)E), smem, stream));
     }
     return GPE_OK;
 }
@@ -1238,7 +1182,6 @@ int bank_project_device(gpe_bank* b, const double* mu, const double* deriv, int6
     auto run = [&](const double* A, int64_t R, int RD, int64_t ldn, int64_t lde, int64_t ldd, double* o) -> cudaError_t {
         for (int e0 = 0; e0 < E; e0 += 32) {
             const int Es = std::min(32, E - e0);
-            g_launches.fetch_add(1);
             cudaError_t e = project_rows(A + (int64_t)e0 * lde, R, RD, ldn, lde, ldd, b->d_basis + (size_t)(e0 / 4) * b->Wp * 4, Es, W,
                                          b->Wp, o, e0 > 0, st);
             if (e != cudaSuccess) return e;
@@ -1310,52 +1253,57 @@ int bank_cost_device(gpe_bank* b, const double* testing, int64_t N, const double
         int rc = bank_predict_device(b, testing + n0 * D, n, d_mu, nullptr, d_der, nullptr, st, call_N);
         if (rc) return rc;
         const int grid = (int)std::min<int64_t>((n + 3) / 4, (int64_t)sms * 16);
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        k_bank_cost<<<grid, 128, (size_t)4 * E * 8, st>>>(d_mu, d_der, obs + n0 * obs_ld, obs_ld, weights,
-                                                          cost ? cost + n0 : nullptr, grad ? grad + n0 * D : nullptr, n,
-                                                          (int)E, (int)D);
-        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(launch_kernel(k_bank_cost, grid, 128, (size_t)4 * E * 8, st, d_mu, d_der, obs + n0 * obs_ld, obs_ld, weights,
+                               cost ? cost + n0 : nullptr, grad ? grad + n0 * D : nullptr, n, (int)E, (int)D));
     }
     CUDA_TRY(cudaEventRecord(b->cost_free, st));
     return GPE_OK;
 }
 
-// Host-resident bank call through the streaming pipeline: any of the point-major bank outputs plus the back-projected
-// spectra / Jacobians; the PC means / gradients a projection consumes stay on the device as chunk intermediates when
-// the caller did not ask for them.  Caller holds b->host_mu.
-int bank_stream(gpe_bank* b, const double* testing, int64_t N, double* mu, double* var, double* deriv, double* hess,
-                double* fwd, double* deriv_full, const StreamPlan* shared_plan = nullptr, ChunkSource* shared = nullptr,
-                const Relay* relay = nullptr) {
+// Bank: testing in; mu, var, deriv, hess, fwd, deriv_full out (idx 0-5).  The PC means / gradients a projection consumes
+// stay on the device as chunk intermediates (host NULL) when the caller did not ask for them.
+CallIo bank_io(const gpe_bank* b, const double* testing, double* mu, double* var, double* deriv, double* hess, double* fwd,
+               double* deriv_full) {
     const int64_t E = b->E, D = b->D, W = b->W;
-    IoList in, out;
-    in.add(testing, D);
-    const int i_mu = (mu || fwd) ? out.add(mu, E) : -1;
-    const int i_var = var ? out.add(var, E) : -1;
-    const int i_der = (deriv || deriv_full) ? out.add(deriv, E * D) : -1;
-    const int i_hes = hess ? out.add(hess, E * D * D) : -1;
-    const int i_fwd = fwd ? out.add(fwd, W) : -1;
-    const int i_dfl = deriv_full ? out.add(deriv_full, D * W) : -1;
-    const int sms = b->models[0]->sms;
-    StreamPlan pl = shared_plan ? *shared_plan : plan_stream(in.v, in.n, out.v, out.n, N, 8, 64 * (int64_t)sms, 1, true);
-    int rc = prepare_slots(b->slots, pl, in.v, in.n, out.v, out.n, 8);
-    if (rc) return rc;
-    std::atomic<int64_t> cursor{0};
-    ChunkSource src = shared ? *shared : ChunkSource{&cursor, N, pl.CH};
-    return stream_host(b->slots, b->device, pl, src, 8, in.v, in.n, out.v, out.n,
+    CallIo io;
+    io.in.add(testing, D);
+    io.idx[0] = (mu || fwd) ? io.out.add(mu, E) : -1;
+    io.idx[1] = var ? io.out.add(var, E) : -1;
+    io.idx[2] = (deriv || deriv_full) ? io.out.add(deriv, E * D) : -1;
+    io.idx[3] = hess ? io.out.add(hess, E * D * D) : -1;
+    io.idx[4] = fwd ? io.out.add(fwd, W) : -1;
+    io.idx[5] = deriv_full ? io.out.add(deriv_full, D * W) : -1;
+    return io;
+}
+
+// Host-resident bank call through the streaming pipeline: any of the point-major bank outputs plus the back-projected
+// spectra / Jacobians.  Caller holds b->host_mu.
+int bank_stream(gpe_bank* b, int64_t N, const CallIo& io, const SharedCall* shared = nullptr) {
+    return stream_call(b->slots, b->device, b->models[0]->sms, io, N, 8, shared,
                        [&](int64_t, int64_t n, void* const* di, void* const* dout, cudaStream_t st) {
-                           auto at = [&](int i) { return i >= 0 ? (double*)dout[i] : nullptr; };
-                           int r = bank_predict_device(b, (const double*)di[0], n, at(i_mu), at(i_var), at(i_der), at(i_hes), st, N);
-                           if (r == GPE_OK && (i_fwd >= 0 || i_dfl >= 0))
-                               r = bank_project_device(b, at(i_mu), at(i_der), n, at(i_fwd), at(i_dfl), st);
+                           double *mu = io.at<double>(dout, 0), *deriv = io.at<double>(dout, 2);
+                           double *fwd = io.at<double>(dout, 4), *deriv_full = io.at<double>(dout, 5);
+                           int r = bank_predict_device(b, (const double*)di[0], n, mu, io.at<double>(dout, 1), deriv,
+                                                       io.at<double>(dout, 3), st, N);
+                           if (r == GPE_OK && (fwd || deriv_full)) r = bank_project_device(b, mu, deriv, n, fwd, deriv_full, st);
                            return r;
-                       }, relay);
+                       });
+}
+
+// Bank cost: testing and, unless obs_ld = 0, the per-point observations (idx 0) in; cost, grad out (idx 1, 2).
+CallIo cost_io(const gpe_bank* b, const double* testing, const double* obs, int64_t obs_ld, double* cost, double* grad) {
+    CallIo io;
+    io.in.add(testing, b->D);
+    io.idx[0] = obs_ld != 0 ? io.in.add(obs, b->E) : -1;
+    io.idx[1] = cost ? io.out.add(cost, 1) : -1;
+    io.idx[2] = grad ? io.out.add(grad, b->D) : -1;
+    return io;
 }
 
 // Host-resident gpe_bank_cost: test points (and per-point observations) stream in, cost / gradient stream out.
-int bank_cost_stream(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
-                     double* cost, double* grad, const StreamPlan* shared_plan = nullptr, ChunkSource* shared = nullptr,
-                     const Relay* relay = nullptr) {
-    const int64_t E = b->E, D = b->D;
+int bank_cost_stream(gpe_bank* b, int64_t N, const double* obs, int64_t obs_ld, const double* weights, const CallIo& io,
+                     const SharedCall* shared = nullptr) {
+    const int64_t E = b->E;
     if (obs_ld != 0 && obs_ld != E) return fail(GPE_ERR_INVALID, "host observations must be contiguous: obs_ld = E or 0");
     // the shared observation vector and the weights are small: one upload per call
     const size_t aux_n = (size_t)(obs_ld == 0 ? E : 0) + (weights ? E : 0);
@@ -1367,22 +1315,12 @@ int bank_cost_stream(gpe_bank* b, const double* testing, int64_t N, const double
         if (obs_ld == 0) { CUDA_TRY(cudaMemcpy(p, obs, (size_t)E * 8, cudaMemcpyHostToDevice)); d_obs1 = p; p += E; }
         if (weights) { CUDA_TRY(cudaMemcpy(p, weights, (size_t)E * 8, cudaMemcpyHostToDevice)); d_w = p; }
     }
-    IoList in, out;
-    in.add(testing, D);
-    const int i_obs = obs_ld != 0 ? in.add(obs, E) : -1;
-    const int i_cost = cost ? out.add(cost, 1) : -1, i_grad = grad ? out.add(grad, D) : -1;
-    const int sms = b->models[0]->sms;
-    StreamPlan pl = shared_plan ? *shared_plan : plan_stream(in.v, in.n, out.v, out.n, N, 8, 64 * (int64_t)sms, 1, true);
-    int rc = prepare_slots(b->slots, pl, in.v, in.n, out.v, out.n, 8);
-    if (rc) return rc;
-    std::atomic<int64_t> cursor{0};
-    ChunkSource src = shared ? *shared : ChunkSource{&cursor, N, pl.CH};
-    return stream_host(b->slots, b->device, pl, src, 8, in.v, in.n, out.v, out.n,
+    return stream_call(b->slots, b->device, b->models[0]->sms, io, N, 8, shared,
                        [&](int64_t, int64_t n, void* const* di, void* const* dout, cudaStream_t st) {
-                           return bank_cost_device(b, (const double*)di[0], n, i_obs >= 0 ? (const double*)di[i_obs] : d_obs1,
-                                                   i_obs >= 0 ? E : 0, d_w, i_cost >= 0 ? (double*)dout[i_cost] : nullptr,
-                                                   i_grad >= 0 ? (double*)dout[i_grad] : nullptr, st, N);
-                       }, relay);
+                           const double* d_obs = obs_ld != 0 ? io.at<const double>(di, 0) : d_obs1;
+                           return bank_cost_device(b, (const double*)di[0], n, d_obs, obs_ld != 0 ? E : 0, d_w,
+                                                   io.at<double>(dout, 1), io.at<double>(dout, 2), st, N);
+                       });
 }
 
 int bank_check_outputs(gpe_bank* b, int64_t N, const double* testing, double*& mu, double*& var, double*& deriv, double*& hess,
@@ -1390,16 +1328,8 @@ int bank_check_outputs(gpe_bank* b, int64_t N, const double* testing, double*& m
     if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
     if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
     if (N > 0 && !testing) return fail(GPE_ERR_INVALID, "testing is NULL");
-    if (!(flags & GPE_WANT_MU)) mu = nullptr;
-    if (!(flags & GPE_WANT_VAR)) var = nullptr;
-    if (!(flags & GPE_WANT_DERIV)) deriv = nullptr;
-    if (!(flags & GPE_WANT_HESS)) hess = nullptr;
-    if (!(flags & GPE_WANT_FWD)) fwd = nullptr;
-    if (!(flags & GPE_WANT_DERIV_FULL)) deriv_full = nullptr;
-    if (((flags & GPE_WANT_MU) && !mu) || ((flags & GPE_WANT_VAR) && !var) || ((flags & GPE_WANT_DERIV) && !deriv) ||
-        ((flags & GPE_WANT_HESS) && !hess) || ((flags & GPE_WANT_FWD) && !fwd) || ((flags & GPE_WANT_DERIV_FULL) && !deriv_full))
-        return fail(GPE_ERR_INVALID, "an output flag is set but its array is NULL");
-    if (!mu && !var && !deriv && !hess && !fwd && !deriv_full) return fail(GPE_ERR_INVALID, "no output requested");
+    int rc = take_outputs(flags, mu, var, deriv, hess, fwd, deriv_full);
+    if (rc) return rc;
     if (var && !b->models[0]->has_invQ) return fail(GPE_ERR_INVALID, "variance requested but the bank was created without invQ");
     if ((fwd || deriv_full) && !b->d_basis) return fail(GPE_ERR_INVALID, "bank was created without basis functions");
     return GPE_OK;
@@ -1558,9 +1488,37 @@ void multi_free_relays(gpe_multi* mm) {
     mm->relays.clear();
 }
 
-// Chunk plan of a call that G pipelines share.
-StreamPlan plan_shared(const IoList& in, const IoList& out, int64_t N, int sms, int G) {
-    return plan_stream(in.v, in.n, out.v, out.n, N, 8, 64 * (int64_t)sms, G, false);
+// One host-resident call on the devices of mm; run(owner, shared) streams an owner's share of it (caller holds the
+// owner's host_mu; shared NULL: the whole call).  With one device, or up to solo_max points, the call is one chunk: the
+// first device serves it on the calling thread (no thread fan-out, and the mapped-buffer path for the reference's
+// one-point calls stays available) -- same kernels, same result; solo_max < 0 always fans out.  Otherwise one thread per
+// device pulls the chunks of one shared plan from one cursor.  The kernel plan (tile size) follows the size of the whole
+// call, so G devices reproduce one device bit for bit.
+template <typename Owner, typename Run>
+int fan_out(gpe_multi* mm, const std::vector<Owner*>& owners, int sms, const CallIo& io, int64_t N, int64_t solo_max, Run run) {
+    const int G = (int)owners.size();
+    if (solo_max >= 0 && (G == 1 || N <= solo_max)) {
+        DeviceRestore restore_device;
+        CUDA_TRY(cudaSetDevice(owners[0]->device));
+        std::lock_guard<std::mutex> lock(owners[0]->host_mu);
+        return run(owners[0], nullptr);
+    }
+    const StreamPlan pl = stream_plan(io, N, 8, sms, G);
+    std::atomic<int64_t> cursor{0};
+    ChunkSource src{&cursor, N, pl.CH};
+    // large page-locked calls: decide (once per handle) whether some devices should send their host traffic through a
+    // partner's PCIe link
+    const bool relay_ok = pl.in_direct && pl.out_direct && N >= 4 * pl.CH;
+    if (relay_ok) multi_route(mm);
+    return run_per_device(G, mm->devices.data(), [&](int g) {
+        Owner* o = owners[g];
+        std::lock_guard<std::mutex> lock(o->host_mu);   // also guards the buffers of the device's relay
+        int rc = GPE_OK;
+        const Relay* relay = (relay_ok && mm->routed && !mm->relays.empty()) ? multi_relay(mm, g, pl, io.in, io.out, &rc) : nullptr;
+        if (rc) return rc;
+        const SharedCall shared{&pl, &src, relay};
+        return run(o, &shared);
+    });
 }
 
 }  // namespace
@@ -1588,8 +1546,7 @@ int gpe_bank_create(int device, int E, int M, int D, const double* inputs, const
             ent[e2].xchunks = b->models[e2]->d_xchunks_mean;
             memcpy(ent[e2].sqrt_w, b->models[e2]->sqrt_w, sizeof(ent[e2].sqrt_w));
         }
-        cudaError_t e = cudaMalloc((void**)&b->d_entries, sizeof(MeanBankEntry) * E);
-        if (e == cudaSuccess) e = cudaMemcpy(b->d_entries, ent.data(), sizeof(MeanBankEntry) * E, cudaMemcpyHostToDevice);
+        const cudaError_t e = upload(&b->d_entries, ent);
         if (e != cudaSuccess) { gpe_bank_destroy(b); return fail(GPE_ERR_CUDA, "bank upload failed: %s", cudaGetErrorString(e)); }
     }
     {
@@ -1618,13 +1575,10 @@ int gpe_bank_create(int device, int E, int M, int D, const double* inputs, const
                 std::vector<double> gx((size_t)g.nchunks * g.JC * XP, 0.0);
                 for (int j = 0; j < M; ++j)
                     for (int d = 0; d < D; ++d) gx[(size_t)j * XP + d] = inputs[(size_t)j * D + d];
-                e = cudaMalloc((void**)&b->d_gx, gx.size() * 8);
-                if (e == cudaSuccess) e = cudaMemcpy(b->d_gx, gx.data(), gx.size() * 8, cudaMemcpyHostToDevice);
+                e = upload(&b->d_gx, gx);
             }
-            if (e == cudaSuccess) e = cudaMalloc((void**)&b->d_galpha[grad], galpha.size() * 8);
-            if (e == cudaSuccess) e = cudaMemcpy(b->d_galpha[grad], galpha.data(), galpha.size() * 8, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess) e = cudaMalloc((void**)&b->d_gw[grad], gw.size() * 8);
-            if (e == cudaSuccess) e = cudaMemcpy(b->d_gw[grad], gw.data(), gw.size() * 8, cudaMemcpyHostToDevice);
+            if (e == cudaSuccess) e = upload(&b->d_galpha[grad], galpha);
+            if (e == cudaSuccess) e = upload(&b->d_gw[grad], gw);
             if (e != cudaSuccess) { gpe_bank_destroy(b); return fail(GPE_ERR_CUDA, "bank upload failed: %s", cudaGetErrorString(e)); }
             b->gplan[grad] = g;
         }
@@ -1637,8 +1591,7 @@ int gpe_bank_create(int device, int E, int M, int D, const double* inputs, const
         std::vector<double> bt((size_t)ks_alloc * b->Wp * 4, 0.0);
         for (int e2 = 0; e2 < E; ++e2)
             for (int w = 0; w < W; ++w) bt[((size_t)(e2 >> 2) * b->Wp + w) * 4 + (e2 & 3)] = basis[(size_t)e2 * W + w];
-        cudaError_t e = cudaMalloc((void**)&b->d_basis, bt.size() * 8);
-        if (e == cudaSuccess) e = cudaMemcpy(b->d_basis, bt.data(), bt.size() * 8, cudaMemcpyHostToDevice);
+        const cudaError_t e = upload(&b->d_basis, bt);
         if (e != cudaSuccess) { gpe_bank_destroy(b); return fail(GPE_ERR_CUDA, "basis upload failed: %s", cudaGetErrorString(e)); }
     }
     *out = b;
@@ -1673,7 +1626,7 @@ int gpe_bank_predict_ex(gpe_bank* b, const double* testing, int64_t N, double* m
     CUDA_TRY(cudaSetDevice(b->device));
     if (flags & GPE_HOST_PTRS) {
         std::lock_guard<std::mutex> lock(b->host_mu);
-        return bank_stream(b, testing, N, mu, var, deriv, hess, fwd, deriv_full);
+        return bank_stream(b, N, bank_io(b, testing, mu, var, deriv, hess, fwd, deriv_full));
     }
     // device pointers: a projection needs the PC means / gradients materialised by the caller
     if (fwd && !mu) return fail(GPE_ERR_INVALID, "device-pointer projection: GPE_WANT_FWD needs GPE_WANT_MU (the PC means) too");
@@ -1712,7 +1665,7 @@ int gpe_bank_cost_host(gpe_bank* b, const double* testing, int64_t N, const doub
     if (!cost && !grad) return fail(GPE_ERR_INVALID, "no output requested");
     CUDA_TRY(cudaSetDevice(b->device));
     std::lock_guard<std::mutex> lock(b->host_mu);
-    return bank_cost_stream(b, testing, N, obs, obs_ld, weights, cost, grad);
+    return bank_cost_stream(b, N, obs, obs_ld, weights, cost_io(b, testing, obs, obs_ld, cost, grad));
 }
 
 int gpe_bank_project(gpe_bank* b, const double* mu, const double* deriv, int64_t N, double* fwd, double* deriv_full,
@@ -1791,46 +1744,13 @@ int gpe_multi_predict(gpe_multi* mm, const double* testing, int64_t N, double* m
     if (!mm || mm->models.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a single-GP handle");
     if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
     if (N == 0) return GPE_OK;
-    if (!(flags & GPE_WANT_MU)) mu = nullptr;
-    if (!(flags & GPE_WANT_VAR)) var = nullptr;
-    if (!(flags & GPE_WANT_DERIV)) deriv = nullptr;
-    if (!(flags & GPE_WANT_HESS)) hess = nullptr;
-    if (((flags & GPE_WANT_MU) && !mu) || ((flags & GPE_WANT_VAR) && !var) || ((flags & GPE_WANT_DERIV) && !deriv) ||
-        ((flags & GPE_WANT_HESS) && !hess) || !(mu || var || deriv || hess) || !testing)
-        return fail(GPE_ERR_INVALID, "output flag set with a NULL array, or nothing requested");
-    const int G = (int)mm->models.size();
+    if (!testing) return fail(GPE_ERR_INVALID, "testing is NULL");
+    int rc = take_outputs(flags, mu, var, deriv, hess);
+    if (rc) return rc;
     gpe_model* m0 = mm->models[0];
-    const int64_t D = m0->D;
-    if (G == 1 || N <= 3 * 64 * (int64_t)m0->sms) {
-        // a call this small is one chunk: the first device serves it on the calling thread (no thread fan-out, and the
-        // mapped-buffer path for the reference's one-point calls stays available) -- same kernels, same result
-        DeviceRestore restore_device;
-        CUDA_TRY(cudaSetDevice(m0->device));
-        std::lock_guard<std::mutex> lock(m0->host_mu);
-        return model_stream(m0, testing, N, mu, var, deriv, hess);
-    }
-    IoList in, out;
-    in.add(testing, D);
-    if (mu) out.add(mu, 1);
-    if (var) out.add(var, 1);
-    if (deriv) out.add(deriv, D);
-    if (hess) out.add(hess, D * D);
-    const StreamPlan pl = plan_shared(in, out, N, m0->sms, G);
-    std::atomic<int64_t> cursor{0};
-    ChunkSource src{&cursor, N, pl.CH};
-    // large page-locked calls: decide (once per handle) whether some devices should send their host traffic through a
-    // partner's PCIe link
-    const bool relay_ok = pl.in_direct && pl.out_direct && N >= 4 * pl.CH;
-    if (relay_ok) multi_route(mm);
-    // the kernel plan (tile size) follows the size of the whole call, so G devices reproduce one device bit for bit
-    return run_per_device(G, mm->devices.data(), [&](int g) {
-        gpe_model* m = mm->models[g];
-        std::lock_guard<std::mutex> lock(m->host_mu);
-        int rc = GPE_OK;
-        const Relay* relay = (relay_ok && mm->routed && !mm->relays.empty()) ? multi_relay(mm, g, pl, in, out, &rc) : nullptr;
-        if (rc) return rc;
-        return model_stream(m, testing, N, mu, var, deriv, hess, &pl, &src, relay);
-    });
+    const CallIo io = model_io(m0->D, testing, mu, var, deriv, hess);
+    return fan_out(mm, mm->models, m0->sms, io, N, 3 * 64 * (int64_t)m0->sms,
+                   [&](gpe_model* m, const SharedCall* shared) { return model_stream(m, N, io, shared); });
 }
 
 int gpe_multi_predict_device(gpe_multi* mm, const double* const* testing, const int64_t* N, double* const* mu,
@@ -1849,16 +1769,13 @@ int gpe_multi_predict_device(gpe_multi* mm, const double* const* testing, const 
     for (int g = 0; g < G; ++g) {
         if (N[g] == 0) continue;
         gpe_model* m = mm->models[g];
-        double* o_mu = (flags & GPE_WANT_MU) && mu ? mu[g] : nullptr;
-        double* o_var = (flags & GPE_WANT_VAR) && var ? var[g] : nullptr;
-        double* o_der = (flags & GPE_WANT_DERIV) && deriv ? deriv[g] : nullptr;
-        double* o_hes = (flags & GPE_WANT_HESS) && hess ? hess[g] : nullptr;
         if (!testing[g]) return fail(GPE_ERR_INVALID, "testing[%d] is NULL", g);
-        if (((flags & GPE_WANT_MU) && !o_mu) || ((flags & GPE_WANT_VAR) && !o_var) || ((flags & GPE_WANT_DERIV) && !o_der) ||
-            ((flags & GPE_WANT_HESS) && !o_hes) || !(o_mu || o_var || o_der || o_hes))
-            return fail(GPE_ERR_INVALID, "device %d: output flag set with a NULL array, or nothing requested", mm->devices[g]);
+        double *o_mu = mu ? mu[g] : nullptr, *o_var = var ? var[g] : nullptr;
+        double *o_der = deriv ? deriv[g] : nullptr, *o_hes = hess ? hess[g] : nullptr;
+        int rc = take_outputs(flags, o_mu, o_var, o_der, o_hes);
+        if (rc) return rc;
         CUDA_TRY(cudaSetDevice(m->device));
-        int rc = predict_device(m, testing[g], N[g], o_mu, o_var, o_der, o_hes, 1, 1, m->D, (int64_t)m->D * m->D,
+        rc = predict_device(m, testing[g], N[g], o_mu, o_var, o_der, o_hes, 1, 1, m->D, (int64_t)m->D * m->D,
                                 streams ? (cudaStream_t)streams[g] : nullptr, call_N);
         if (rc) return rc;
     }
@@ -1873,35 +1790,10 @@ int gpe_multi_bank_predict(gpe_multi* mm, const double* testing, int64_t N, doub
     int rc = bank_check_outputs(b0, N, testing, mu, var, deriv, hess, fwd, deriv_full, flags);
     if (rc) return rc;
     if (N == 0) return GPE_OK;
-    const int G = (int)mm->banks.size();
-    const int64_t E = b0->E, D = b0->D, W = b0->W;
-    if (G == 1 || N <= 64 * (int64_t)b0->models[0]->sms) {   // one chunk: served by the first device on the calling thread
-        DeviceRestore restore_device;
-        CUDA_TRY(cudaSetDevice(b0->device));
-        std::lock_guard<std::mutex> lock(b0->host_mu);
-        return bank_stream(b0, testing, N, mu, var, deriv, hess, fwd, deriv_full);
-    }
-    IoList in, out;   // same arrays, same order as bank_stream builds them: the plan only needs widths and pinned-ness
-    in.add(testing, D);
-    if (mu || fwd) out.add(mu, E);
-    if (var) out.add(var, E);
-    if (deriv || deriv_full) out.add(deriv, E * D);
-    if (hess) out.add(hess, E * D * D);
-    if (fwd) out.add(fwd, W);
-    if (deriv_full) out.add(deriv_full, D * W);
-    const StreamPlan pl = plan_shared(in, out, N, b0->models[0]->sms, G);
-    std::atomic<int64_t> cursor{0};
-    ChunkSource src{&cursor, N, pl.CH};
-    const bool relay_ok = pl.in_direct && pl.out_direct && N >= 4 * pl.CH;
-    if (relay_ok) multi_route(mm);
-    return run_per_device(G, mm->devices.data(), [&](int g) {
-        gpe_bank* b = mm->banks[g];
-        std::lock_guard<std::mutex> lock(b->host_mu);
-        int rc = GPE_OK;
-        const Relay* relay = (relay_ok && mm->routed && !mm->relays.empty()) ? multi_relay(mm, g, pl, in, out, &rc) : nullptr;
-        if (rc) return rc;
-        return bank_stream(b, testing, N, mu, var, deriv, hess, fwd, deriv_full, &pl, &src, relay);
-    });
+    const int sms = b0->models[0]->sms;
+    const CallIo io = bank_io(b0, testing, mu, var, deriv, hess, fwd, deriv_full);
+    return fan_out(mm, mm->banks, sms, io, N, 64 * (int64_t)sms,
+                   [&](gpe_bank* b, const SharedCall* shared) { return bank_stream(b, N, io, shared); });
 }
 
 int gpe_multi_bank_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
@@ -1913,26 +1805,9 @@ int gpe_multi_bank_cost(gpe_multi* mm, const double* testing, int64_t N, const d
     if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
     if (!cost && !grad) return fail(GPE_ERR_INVALID, "no output requested");
     gpe_bank* b0 = mm->banks[0];
-    const int G = (int)mm->banks.size();
-    const int64_t E = b0->E, D = b0->D;
-    IoList in, out;
-    in.add(testing, D);
-    if (obs_ld != 0) in.add(obs, E);
-    if (cost) out.add(cost, 1);
-    if (grad) out.add(grad, D);
-    const StreamPlan pl = plan_shared(in, out, N, b0->models[0]->sms, G);
-    std::atomic<int64_t> cursor{0};
-    ChunkSource src{&cursor, N, pl.CH};
-    const bool relay_ok = pl.in_direct && pl.out_direct && N >= 4 * pl.CH;
-    if (relay_ok) multi_route(mm);
-    return run_per_device(G, mm->devices.data(), [&](int g) {
-        gpe_bank* b = mm->banks[g];
-        std::lock_guard<std::mutex> lock(b->host_mu);
-        int rc = GPE_OK;
-        const Relay* relay = (relay_ok && mm->routed && !mm->relays.empty()) ? multi_relay(mm, g, pl, in, out, &rc) : nullptr;
-        if (rc) return rc;
-        return bank_cost_stream(b, testing, N, obs, obs_ld, weights, cost, grad, &pl, &src, relay);
-    });
+    const CallIo io = cost_io(b0, testing, obs, obs_ld, cost, grad);
+    return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1,
+                   [&](gpe_bank* b, const SharedCall* shared) { return bank_cost_stream(b, N, obs, obs_ld, weights, io, shared); });
 }
 
 }  // extern "C"

@@ -1,6 +1,8 @@
-// Host-side declarations of the per-DP kernel launchers (defined in predict_full_inst.cu, one object per DP).
+// Host-side launch helper and the per-DP kernel launchers (defined in predict_full_inst.cu, one object per DP).
 #pragma once
 #include <cuda_runtime.h>
+#include <utility>
+#include "host_common.h"
 #include "predict_full.cuh"
 #include "predict_mean.cuh"
 #include "predict_bank_mean.cuh"
@@ -11,12 +13,32 @@
 
 namespace gpe {
 
-#define GPE_DECL_DP(DPV)                                                                                          \
-    cudaError_t launch_full_dp##DPV(int cfg, const FullParams& p, int grid, size_t smem, cudaStream_t st);         \
-    cudaError_t launch_mean_dp##DPV(bool hess, const MeanParams& p, dim3 grid, size_t smem, cudaStream_t st);   \
-    cudaError_t launch_bank_mean_dp##DPV(int G, bool grad, const BankMeanParams& p, dim3 grid, size_t smem, cudaStream_t st); \
-    cudaError_t launch_tiny_dp##DPV(const TinyParams& p, int grid, size_t smem, cudaStream_t st);
+// Launch `kern` on `st` with `smem` bytes of dynamic shared memory and count the launch (gpe_launch_count).  The
+// shared-memory opt-in is per function AND per device: it is set on every launch (microseconds) so that multi-device
+// processes stay correct.
+template <typename... P, typename... A>
+cudaError_t launch_kernel(void (*kern)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A&&... args) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kern<<<grid, block, smem, st>>>(std::forward<A>(args)...);
+    count_launch();
+    return cudaGetLastError();
+}
 
+// The kernels compiled for one padded input dimension DP.
+struct DpKernels {
+    int DP;
+    cudaError_t (*full)(int cfg, const FullParams& p, int grid, size_t smem, cudaStream_t st);
+    cudaError_t (*mean)(bool hess, const MeanParams& p, dim3 grid, size_t smem, cudaStream_t st);
+    cudaError_t (*bank_mean)(int G, bool grad, const BankMeanParams& p, dim3 grid, size_t smem, cudaStream_t st);
+    cudaError_t (*tiny)(const TinyParams& p, int grid, size_t smem, cudaStream_t st);
+    // name of the fused instance `full` runs for (cfg, nt_act, symmetric); characters written, as snprintf
+    int (*full_name)(int cfg, int nt_act, bool symmetric, char* buf, int len);
+    // template name of the kernel `mean` runs for mean + gradient without the K* scratch
+    const char* (*mean_name)();
+};
+
+#define GPE_DECL_DP(DPV) extern const DpKernels kKernelsDp##DPV;
 GPE_DECL_DP(2)
 GPE_DECL_DP(4)
 GPE_DECL_DP(6)
@@ -27,6 +49,15 @@ GPE_DECL_DP(16)
 GPE_DECL_DP(24)
 GPE_DECL_DP(32)
 #undef GPE_DECL_DP
+
+// The kernels of the smallest compiled DP >= D (NULL: D > 32, no per-D compiled kernels).
+inline const DpKernels* dp_kernels(int D) {
+    static const DpKernels* const table[] = {&kKernelsDp2,  &kKernelsDp4,  &kKernelsDp6,  &kKernelsDp8, &kKernelsDp10,
+                                             &kKernelsDp12, &kKernelsDp16, &kKernelsDp24, &kKernelsDp32};
+    for (const DpKernels* k : table)
+        if (k->DP >= D) return k;
+    return nullptr;
+}
 
 cudaError_t launch_tf32(int DP, bool x3, const Tf32Params& p, int grid, size_t smem, cudaStream_t st);
 cudaError_t launch_tf32_big(int DP, bool x3, const Tf32BigParams& p, int grid, size_t smem, cudaStream_t st);
@@ -45,9 +76,5 @@ inline bool bank_group_ok(int DP, int G, bool grad) {
     return false;
 }
 static const int kTfDpList[] = {4, 8, 12, 16, 32};
-
-// padded input dimensions that have compiled kernels, ascending
-static const int kDpList[] = {2, 4, 6, 8, 10, 12, 16, 24, 32};
-static const int kNumDp = sizeof(kDpList) / sizeof(kDpList[0]);
 
 }  // namespace gpe

@@ -7,11 +7,7 @@ namespace gpe {
 
 template <int DP, bool X3>
 static cudaError_t launch_dp(const Tf32Params& p, int grid, size_t smem, cudaStream_t st) {
-    auto kern = k_predict_tf32<DP, X3>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    kern<<<grid, kTfThreads, smem, st>>>(p);
-    return cudaGetLastError();
+    return launch_kernel(k_predict_tf32<DP, X3>, grid, kTfThreads, smem, st, p);
 }
 
 cudaError_t launch_tf32(int DP, bool x3, const Tf32Params& p, int grid, size_t smem, cudaStream_t st) {
@@ -30,11 +26,7 @@ cudaError_t launch_tf32(int DP, bool x3, const Tf32Params& p, int grid, size_t s
 
 template <int DP, bool X3>
 static cudaError_t launch_big_dp(const Tf32BigParams& p, int grid, size_t smem, cudaStream_t st) {
-    auto kern = k_predict_tf32_big<DP, X3>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    kern<<<grid, kTfThreads, smem, st>>>(p);
-    return cudaGetLastError();
+    return launch_kernel(k_predict_tf32_big<DP, X3>, grid, kTfThreads, smem, st, p);
 }
 
 cudaError_t launch_tf32_big(int DP, bool x3, const Tf32BigParams& p, int grid, size_t smem, cudaStream_t st) {

@@ -5,10 +5,7 @@
 namespace gpe {
 
 cudaError_t launch_var_large(const VarLargeParams& p, int grid, size_t smem, cudaStream_t st) {
-    cudaError_t e = cudaFuncSetAttribute(k_var_large, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    k_var_large<<<grid, kVlWarps * 32, smem, st>>>(p);
-    return cudaGetLastError();
+    return launch_kernel(k_var_large, grid, kVlWarps * 32, smem, st, p);
 }
 
 }  // namespace gpe

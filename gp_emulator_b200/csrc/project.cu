@@ -143,16 +143,13 @@ template <int KS>
 cudaError_t launch_project(const double* A, int64_t R, int RD, int64_t ldn, int64_t lde, int64_t ldd,
                            const double* b_tiled, int E, int W, int Wp, double* out, int accumulate, cudaStream_t st) {
     const size_t psmem = 128 + 2 * (size_t)KS * kProjCols * 4 * 8 + 8 * 16 * kProjPitch * 8;
-    cudaError_t e = cudaFuncSetAttribute(k_project<KS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem);
-    if (e != cudaSuccess) return e;
     // few row blocks: spread the column groups over gridDim.y so that about one wave of CTAs is in flight
     const int64_t nrb = (R + kProjRows - 1) / kProjRows;
     int dev = 0, sms = 148;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const int gy = (int)std::max<int64_t>(1, std::min<int64_t>(Wp / kProjCols, (int64_t)sms / nrb));
-    k_project<KS><<<dim3((unsigned)nrb, (unsigned)gy), kProjThreads, psmem, st>>>(A, R, RD, ldn, lde, ldd, b_tiled, E, W, Wp, out,
-                                                                                accumulate);
-    return cudaGetLastError();
+    return launch_kernel(k_project<KS>, dim3((unsigned)nrb, (unsigned)gy), kProjThreads, psmem, st, A, R, RD, ldn, lde, ldd, b_tiled, E,
+                         W, Wp, out, accumulate);
 }
 
 // ---- tensor-map variant ------------------------------------------------------------------------------------------
@@ -342,11 +339,8 @@ template <int KS, int WRG>
 cudaError_t launch_project_tma(const double* A, int64_t R, int RD, int64_t ldn, int64_t lde, int64_t ldd, const double* b_tiled,
                                int E, int W, int Wp, const CUtensorMap& even, const CUtensorMap& odd, double* out, cudaStream_t st) {
     const size_t psmem = 128 + 2 * (size_t)KS * kProjCols * 4 * 8 + 2 * (size_t)WRG * 16 * kProjCols * 8;
-    cudaError_t e = cudaFuncSetAttribute(k_project_tma<KS, WRG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem);
-    if (e != cudaSuccess) return e;
-    k_project_tma<KS, WRG><<<(unsigned)((R + WRG * 32 - 1) / (WRG * 32)), WRG * 128, psmem, st>>>(A, R, RD, ldn, lde, ldd, b_tiled, E, W, Wp,
-                                                                                           even, odd, out);
-    return cudaGetLastError();
+    return launch_kernel(k_project_tma<KS, WRG>, (unsigned)((R + WRG * 32 - 1) / (WRG * 32)), WRG * 128, psmem, st, A, R, RD, ldn, lde,
+                         ldd, b_tiled, E, W, Wp, even, odd, out);
 }
 
 }  // namespace

@@ -31,6 +31,7 @@
 #include "../../include/gpemu.h"
 #include "gpe_math.cuh"
 #include "host_common.h"
+#include "launch.h"
 
 namespace gpe {
 
@@ -583,12 +584,8 @@ int gpe_trainer_eval(gpe_trainer* t, int B, const int* target_index, const doubl
         p.x = t->d_x; p.targets = t->d_targets; p.thetas = t->d_theta; p.tidx = t->d_tidx; p.work = t->d_work;
         p.loglik = t->d_ll; p.grad = t->d_grad; p.status = t->d_status; p.M = t->M; p.D = t->D;
         p.trace = g_train_trace;
-        // per function AND per device: set on every launch so multi-device processes stay correct
         auto kern = t->NB == 32 ? k_train_eval<32> : (t->NB == 16 ? k_train_eval<16> : k_train_eval<8>);
-        TR_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)t->smem));
-        kern<<<nb, kTrainThreads, t->smem, t->st>>>(p);
-        count_launch();
-        TR_TRY(cudaGetLastError());
+        TR_TRY(launch_kernel(kern, nb, kTrainThreads, t->smem, t->st, p));
         TR_TRY(cudaMemcpyAsync(loglik + b0, t->d_ll, (size_t)nb * 8, cudaMemcpyDeviceToHost, t->st));
         TR_TRY(cudaMemcpyAsync(grad + (size_t)b0 * G, t->d_grad, (size_t)nb * G * 8, cudaMemcpyDeviceToHost, t->st));
         TR_TRY(cudaMemcpyAsync(status + b0, t->d_status, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, t->st));
