@@ -47,6 +47,11 @@ def main():
     truth = toy_model(y_test, wl)
     print("batch of %d: rms emulation error %.2e (signal rms %.2f)" % (len(y_test), np.sqrt(np.mean((fwd_all - truth) ** 2)),
                                                                        np.sqrt(np.mean(truth ** 2))))
+    noise = np.random.RandomState(1).standard_normal(len(wl))                # 3b. spectrum misfit
+    cost, grad = emu.cost(y_test, truth[3] + 0.01 * noise)                   # spectra and Jacobians stay in the kernel
+    best = int(np.argmin(cost))
+    print("misfit of 1000 candidates against one observed spectrum: best candidate %d (cost %.3f), true one is 3 "
+          "(cost %.3f); gradients %s" % (best, cost[best], cost[3], grad.shape))
 
     bands = [40, 120, 200, 280, 360]                                          # 4. per-band GPs
     from gp_emulator_b200.training import fit_bank

@@ -148,6 +148,7 @@ struct gpe_bank {
     Slot slots[3];
     double* d_aux = nullptr;     // shared observation vector + weights of a host-pointer gpe_bank_cost call
     size_t aux_cap = 0;
+    cudaEvent_t aux_ready = nullptr;   // recorded after their upload, on the stream of the call's first chunk
     // gpe_bank_cost: per-chunk mu / deriv scratch, shared by every stream that reduces with this bank
     std::mutex cost_mu;
     double* cost_d = nullptr;
@@ -1224,40 +1225,76 @@ __global__ void __launch_bounds__(128) k_bank_cost(const double* __restrict__ mu
     }
 }
 
-int bank_cost_device(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
-                     double* cost, double* grad, cudaStream_t st, int64_t call_N = -1) {
+// The chunk walk of the bank's cost calls on `st`: the bank means (and, with `grad`, their input gradients) of whole
+// waves of 64-point tiles, at most 256 MB of them, go to the bank's cost scratch, and reduce(aux, mu, deriv, n0, n) consumes
+// each chunk.  The scratch starts with aux_n doubles that the reducer may fill with per-call operands.
+template <typename Reduce>
+int bank_cost_walk(gpe_bank* b, const double* testing, int64_t N, bool grad, int64_t aux_n, cudaStream_t st, int64_t call_N,
+                   Reduce reduce) {
     if (call_N < 0) call_N = N;
     const int64_t E = b->E, D = b->D;
     const int64_t per_point = E * (1 + (grad ? D : 0));
     // points per chunk: whole waves of 64-point tiles, scratch bounded by 256 MB
     int64_t chunk = std::max<int64_t>(64, (((int64_t)256 << 20) / (per_point * 8)) / 64 * 64);
     chunk = std::min(chunk, (N + 63) / 64 * 64);
+    const size_t need = (size_t)(aux_n + chunk * per_point);
     std::lock_guard<std::mutex> lock(b->cost_mu);
     if (!b->cost_free) CUDA_TRY(cudaEventCreateWithFlags(&b->cost_free, cudaEventDisableTiming));
     // the scratch may still be read by a reduction enqueued on another stream
     CUDA_TRY(cudaStreamWaitEvent(st, b->cost_free, 0));
-    if (b->cost_cap < (size_t)(chunk * per_point)) {
+    if (b->cost_cap < need) {
         if (b->cost_d) {
             CUDA_TRY(cudaEventSynchronize(b->cost_free));
             CUDA_TRY(cudaFree(b->cost_d));
             b->cost_d = nullptr; b->cost_cap = 0;
         }
-        CUDA_TRY(cudaMalloc((void**)&b->cost_d, (size_t)(chunk * per_point) * 8));
-        b->cost_cap = (size_t)(chunk * per_point);
+        CUDA_TRY(cudaMalloc((void**)&b->cost_d, need * 8));
+        b->cost_cap = need;
     }
-    double* d_mu = b->cost_d;
-    double* d_der = grad ? b->cost_d + chunk * E : nullptr;
-    const int sms = b->models[0]->sms;
+    double* aux = b->cost_d;
+    double* d_mu = b->cost_d + aux_n;
+    double* d_der = grad ? d_mu + chunk * E : nullptr;
     for (int64_t n0 = 0; n0 < N; n0 += chunk) {
         const int64_t n = std::min(chunk, N - n0);
         int rc = bank_predict_device(b, testing + n0 * D, n, d_mu, nullptr, d_der, nullptr, st, call_N);
+        if (rc == GPE_OK) rc = reduce(aux, d_mu, d_der, n0, n);
         if (rc) return rc;
-        const int grid = (int)std::min<int64_t>((n + 3) / 4, (int64_t)sms * 16);
-        CUDA_TRY(launch_kernel(k_bank_cost, grid, 128, (size_t)4 * E * 8, st, d_mu, d_der, obs + n0 * obs_ld, obs_ld, weights,
-                               cost ? cost + n0 : nullptr, grad ? grad + n0 * D : nullptr, n, (int)E, (int)D));
     }
     CUDA_TRY(cudaEventRecord(b->cost_free, st));
     return GPE_OK;
+}
+
+int bank_cost_device(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                     double* cost, double* grad, cudaStream_t st, int64_t call_N = -1) {
+    const int64_t E = b->E, D = b->D;
+    const int sms = b->models[0]->sms;
+    return bank_cost_walk(b, testing, N, grad != nullptr, 0, st, call_N,
+                          [&](double*, const double* d_mu, const double* d_der, int64_t n0, int64_t n) -> int {
+                              const int grid = (int)std::min<int64_t>((n + 3) / 4, (int64_t)sms * 16);
+                              CUDA_TRY(launch_kernel(k_bank_cost, grid, 128, (size_t)4 * E * 8, st, d_mu, d_der, obs + n0 * obs_ld,
+                                                     obs_ld, weights, cost ? cost + n0 : nullptr, grad ? grad + n0 * D : nullptr,
+                                                     n, (int)E, (int)D));
+                              return GPE_OK;
+                          });
+}
+
+// Misfit of the back-projected spectra against observed ones (k_forward_cost, project.cu): the same walk, the spectra and
+// Jacobians exist only as tiles inside the kernel.  The weights and the shared observation go to the scratch once per
+// call, zero-padded to the basis image's width.
+int bank_forward_cost_device(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                             const double* weights, double* cost, double* grad, cudaStream_t st, int64_t call_N = -1) {
+    const int D = b->D, W = b->W, Wp = b->Wp;
+    // calls of a few points spread the column groups over CTAs; their partial sums follow the aux operands in the scratch
+    const int gy = forward_cost_split(call_N < 0 ? N : call_N, W);
+    const int64_t part_n = gy > 1 ? (int64_t)gy * ((N + 63) / 64 * 64) * (1 + b->E) : 0;
+    return bank_cost_walk(b, testing, N, grad != nullptr, 2 * (int64_t)Wp + part_n, st, call_N,
+                          [&](double* aux, const double* d_mu, const double* d_der, int64_t n0, int64_t n) -> int {
+                              if (n0 == 0) CUDA_TRY(forward_cost_aux(weights, obs_ld == 0 ? obs : nullptr, W, Wp, aux, st));
+                              CUDA_TRY(forward_cost_rows(d_mu, d_der, n, b->E, D, obs + n0 * obs_ld, obs_ld, aux, b->d_basis, W,
+                                                         Wp, gy, aux + 2 * Wp, cost ? cost + n0 : nullptr,
+                                                         grad ? grad + n0 * D : nullptr, st));
+                              return GPE_OK;
+                          });
 }
 
 // Bank: testing in; mu, var, deriv, hess, fwd, deriv_full out (idx 0-5).  The PC means / gradients a projection consumes
@@ -1290,37 +1327,66 @@ int bank_stream(gpe_bank* b, int64_t N, const CallIo& io, const SharedCall* shar
                        });
 }
 
-// Bank cost: testing and, unless obs_ld = 0, the per-point observations (idx 0) in; cost, grad out (idx 1, 2).
-CallIo cost_io(const gpe_bank* b, const double* testing, const double* obs, int64_t obs_ld, double* cost, double* grad) {
+// Bank cost of observations K wide (E: the bank's own outputs, W: its spectra): testing and, unless obs_ld = 0, the
+// per-point observations (idx 0) in; cost, grad out (idx 1, 2).
+CallIo cost_io(const gpe_bank* b, int64_t K, const double* testing, const double* obs, int64_t obs_ld, double* cost, double* grad) {
     CallIo io;
     io.in.add(testing, b->D);
-    io.idx[0] = obs_ld != 0 ? io.in.add(obs, b->E) : -1;
+    io.idx[0] = obs_ld != 0 ? io.in.add(obs, K) : -1;
     io.idx[1] = cost ? io.out.add(cost, 1) : -1;
     io.idx[2] = grad ? io.out.add(grad, b->D) : -1;
     return io;
 }
 
-// Host-resident gpe_bank_cost: test points (and per-point observations) stream in, cost / gradient stream out.
-int bank_cost_stream(gpe_bank* b, int64_t N, const double* obs, int64_t obs_ld, const double* weights, const CallIo& io,
-                     const SharedCall* shared = nullptr) {
-    const int64_t E = b->E;
-    if (obs_ld != 0 && obs_ld != E) return fail(GPE_ERR_INVALID, "host observations must be contiguous: obs_ld = E or 0");
-    // the shared observation vector and the weights are small: one upload per call
-    const size_t aux_n = (size_t)(obs_ld == 0 ? E : 0) + (weights ? E : 0);
+typedef int (*CostDevice)(gpe_bank*, const double*, int64_t, const double*, int64_t, const double*, double*, double*, cudaStream_t,
+                          int64_t);
+
+// Host-resident cost call (bank_cost_device or bank_forward_cost_device, observations K wide): test points (and
+// per-point observations) stream in, cost / gradient stream out.
+int bank_cost_stream(gpe_bank* b, int64_t K, CostDevice cost_device, int64_t N, const double* obs, int64_t obs_ld,
+                     const double* weights, const CallIo& io, const SharedCall* shared = nullptr) {
+    if (obs_ld != 0 && obs_ld != K) return fail(GPE_ERR_INVALID, "host observations must be contiguous: obs_ld = %s or 0", K == b->E ? "E" : "W");
+    // the shared observation vector and the weights are small: one upload per call, enqueued ahead of this pipeline's first
+    // chunk; its later chunks (other slot streams) wait for it.  (Every chunk of the previous call has finished: the
+    // buffer is free.)
+    const size_t aux_n = (size_t)(obs_ld == 0 ? K : 0) + (weights ? K : 0);
     double *d_obs1 = nullptr, *d_w = nullptr;
     if (aux_n > 0) {
         int rc = ensure_buf((void**)&b->d_aux, &b->aux_cap, aux_n * 8, false);
         if (rc) return rc;
-        double* p = b->d_aux;
-        if (obs_ld == 0) { CUDA_TRY(cudaMemcpy(p, obs, (size_t)E * 8, cudaMemcpyHostToDevice)); d_obs1 = p; p += E; }
-        if (weights) { CUDA_TRY(cudaMemcpy(p, weights, (size_t)E * 8, cudaMemcpyHostToDevice)); d_w = p; }
+        if (!b->aux_ready) CUDA_TRY(cudaEventCreateWithFlags(&b->aux_ready, cudaEventDisableTiming));
+        d_obs1 = obs_ld == 0 ? b->d_aux : nullptr;
+        d_w = weights ? b->d_aux + (obs_ld == 0 ? K : 0) : nullptr;
     }
+    bool uploaded = false;
     return stream_call(b->slots, b->device, b->models[0]->sms, io, N, 8, shared,
                        [&](int64_t, int64_t n, void* const* di, void* const* dout, cudaStream_t st) {
+                           if (aux_n > 0 && !uploaded) {
+                               if (d_obs1) CUDA_TRY(cudaMemcpyAsync(d_obs1, obs, (size_t)K * 8, cudaMemcpyHostToDevice, st));
+                               if (d_w) CUDA_TRY(cudaMemcpyAsync(d_w, weights, (size_t)K * 8, cudaMemcpyHostToDevice, st));
+                               CUDA_TRY(cudaEventRecord(b->aux_ready, st));
+                               uploaded = true;
+                           } else if (aux_n > 0) {
+                               CUDA_TRY(cudaStreamWaitEvent(st, b->aux_ready, 0));
+                           }
                            const double* d_obs = obs_ld != 0 ? io.at<const double>(di, 0) : d_obs1;
-                           return bank_cost_device(b, (const double*)di[0], n, d_obs, obs_ld != 0 ? E : 0, d_w,
-                                                   io.at<double>(dout, 1), io.at<double>(dout, 2), st, N);
+                           return cost_device(b, (const double*)di[0], n, d_obs, obs_ld != 0 ? K : 0, d_w,
+                                              io.at<double>(dout, 1), io.at<double>(dout, 2), st, N);
                        });
+}
+
+// Request check of the forward-cost calls (device: obs_ld = 0 or >= W; the host calls check obs_ld = 0 or W).
+int forward_cost_check(gpe_bank* b, int64_t N, const double* testing, const double* obs, int64_t obs_ld, const double* cost,
+                       const double* grad) {
+    if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
+    if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
+    if (!b->d_basis) return fail(GPE_ERR_INVALID, "bank was created without basis functions");
+    if (!cost && !grad) return fail(GPE_ERR_INVALID, "no output requested");
+    if (N > 0 && (!testing || !obs)) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
+    if (obs_ld != 0 && obs_ld < b->W) return fail(GPE_ERR_INVALID, "obs_ld must be 0 (one observed spectrum) or >= W");
+    if (forward_cost_smem(b->E) > kSmemMax)
+        return fail(GPE_ERR_UNSUPPORTED, "the forward cost supports banks of up to 96 emulators (got %d)", b->E);
+    return GPE_OK;
 }
 
 int bank_check_outputs(gpe_bank* b, int64_t N, const double* testing, double*& mu, double*& var, double*& deriv, double*& hess,
@@ -1611,6 +1677,7 @@ int gpe_bank_destroy(gpe_bank* b) {
         if (b->d_gw[i]) cudaFree(b->d_gw[i]);
     }
     if (b->d_aux) cudaFree(b->d_aux);
+    if (b->aux_ready) cudaEventDestroy(b->aux_ready);
     if (b->cost_d) cudaFree(b->cost_d);
     if (b->cost_free) cudaEventDestroy(b->cost_free);
     delete b;
@@ -1665,7 +1732,27 @@ int gpe_bank_cost_host(gpe_bank* b, const double* testing, int64_t N, const doub
     if (!cost && !grad) return fail(GPE_ERR_INVALID, "no output requested");
     CUDA_TRY(cudaSetDevice(b->device));
     std::lock_guard<std::mutex> lock(b->host_mu);
-    return bank_cost_stream(b, N, obs, obs_ld, weights, cost_io(b, testing, obs, obs_ld, cost, grad));
+    return bank_cost_stream(b, b->E, bank_cost_device, N, obs, obs_ld, weights, cost_io(b, b->E, testing, obs, obs_ld, cost, grad));
+}
+
+int gpe_bank_forward_cost(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                          const double* weights, double* cost, double* grad, void* stream) {
+    NvtxRange nvtx_range("gpe_bank_forward_cost");
+    int rc = forward_cost_check(b, N, testing, obs, obs_ld, cost, grad);
+    if (rc || N == 0) return rc;
+    CUDA_TRY(cudaSetDevice(b->device));
+    return bank_forward_cost_device(b, testing, N, obs, obs_ld, weights, cost, grad, (cudaStream_t)stream);
+}
+
+int gpe_bank_forward_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                               const double* weights, double* cost, double* grad) {
+    NvtxRange nvtx_range("gpe_bank_forward_cost_host");
+    int rc = forward_cost_check(b, N, testing, obs, obs_ld, cost, grad);
+    if (rc || N == 0) return rc;
+    CUDA_TRY(cudaSetDevice(b->device));
+    std::lock_guard<std::mutex> lock(b->host_mu);
+    return bank_cost_stream(b, b->W, bank_forward_cost_device, N, obs, obs_ld, weights,
+                            cost_io(b, b->W, testing, obs, obs_ld, cost, grad));
 }
 
 int gpe_bank_project(gpe_bank* b, const double* mu, const double* deriv, int64_t N, double* fwd, double* deriv_full,
@@ -1805,9 +1892,23 @@ int gpe_multi_bank_cost(gpe_multi* mm, const double* testing, int64_t N, const d
     if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
     if (!cost && !grad) return fail(GPE_ERR_INVALID, "no output requested");
     gpe_bank* b0 = mm->banks[0];
-    const CallIo io = cost_io(b0, testing, obs, obs_ld, cost, grad);
-    return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1,
-                   [&](gpe_bank* b, const SharedCall* shared) { return bank_cost_stream(b, N, obs, obs_ld, weights, io, shared); });
+    const CallIo io = cost_io(b0, b0->E, testing, obs, obs_ld, cost, grad);
+    return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
+        return bank_cost_stream(b, b->E, bank_cost_device, N, obs, obs_ld, weights, io, shared);
+    });
+}
+
+int gpe_multi_bank_forward_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                                const double* weights, double* cost, double* grad) {
+    NvtxRange nvtx_range("gpe_multi_bank_forward_cost");
+    if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
+    gpe_bank* b0 = mm->banks[0];
+    int rc = forward_cost_check(b0, N, testing, obs, obs_ld, cost, grad);
+    if (rc || N == 0) return rc;
+    const CallIo io = cost_io(b0, b0->W, testing, obs, obs_ld, cost, grad);
+    return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
+        return bank_cost_stream(b, b->W, bank_forward_cost_device, N, obs, obs_ld, weights, io, shared);
+    });
 }
 
 }  // extern "C"

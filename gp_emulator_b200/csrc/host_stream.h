@@ -50,6 +50,10 @@ constexpr int64_t kZeroCopyMax = 16384;   // host calls of up to this many point
                                           // (tools/zero_copy_probe.py: 1000 points 71 -> 58 us, 16000 points 470 -> 300 us)
 constexpr size_t kSlotOutBytes = (size_t)512 << 20;   // cap of one slot's result buffer: bounds chunks of wide outputs
                                                       // (bank Hessians: 57 KB per point, spectra: 17 KB per point)
+constexpr size_t kSlotInBytes = (size_t)1 << 30;      // cap of one slot's input buffer: bounds chunks of wide inputs (observed
+                                                      // spectra: 17 KB per point).  Binds only above 512 doubles per point
+                                                      // (kPipeChunk x 4 KB): test points (D <= GPE_MAX_INPUTS = 256) never
+                                                      // reach it, band observations only where D + E > 512
 constexpr int kMaxIo = 8;
 
 struct Slot {
@@ -227,13 +231,16 @@ inline StreamPlan plan_stream(const IoSpec* ins, int nin, const IoSpec* outs, in
     const bool tiny = N <= 3 * wave;
     pl.out_direct = pl.in_direct || !tiny;
     for (int i = 0; i < nout && pl.out_direct; ++i) pl.out_direct = is_pinned_or_null(outs[i].host);
-    int64_t per_out = 0;
+    int64_t per_in = 0, per_out = 0;
+    for (int i = 0; i < nin; ++i) per_in += ins[i].width;
     for (int i = 0; i < nout; ++i) per_out += outs[i].width;
-    // wide outputs bound the chunk through the slot's result buffer, in whole waves where that leaves at least one
+    // wide outputs (inputs) bound the chunk through the slot's result (input) buffer, in whole waves where that leaves at
+    // least one
     int64_t cap = kPipeChunk;
     size_t slot_bytes = kSlotOutBytes;
     if (const char* e = getenv("GPE_SLOT_OUT_BYTES")) slot_bytes = (size_t)atoll(e);   // dev aid: force chunk seams in tests
     if (per_out > 0) cap = std::min<int64_t>(cap, (int64_t)(slot_bytes / ((size_t)per_out * ES)));
+    if (per_in > 0) cap = std::min<int64_t>(cap, (int64_t)(kSlotInBytes / ((size_t)per_in * ES)));
     if (cap >= wave) cap = cap / wave * wave;
     cap = std::max<int64_t>(cap, 1);
     const bool direct = pl.in_direct && pl.out_direct;

@@ -66,6 +66,17 @@ cudaError_t launch_var_large(const VarLargeParams& p, int grid, size_t smem, cud
 // at + e lde (project.cu)
 cudaError_t project_rows(const double* A, int64_t R, int RD, int64_t ldn, int64_t lde, int64_t ldd, const double* b_tiled, int E,
                          int W, int Wp, double* out, int accumulate, cudaStream_t st);
+// Forward cost of R rows (project.cu): cost (R) = 1/2 sum_w l_w (fwd - obs)^2 and, with grad, grad (R, D) of it, from the bank
+// means mu (R, E) and gradients deriv (R, E, D); obs (R, obs_ld) or, obs_ld = 0, the shared observation in aux.
+// aux (2 Wp) is filled by forward_cost_aux: weights (NULL: 1) and the shared observation (NULL: none), zero-padded to Wp.
+cudaError_t forward_cost_aux(const double* weights, const double* obs1, int W, int Wp, double* aux, cudaStream_t st);
+cudaError_t forward_cost_rows(const double* mu, const double* deriv, int64_t R, int E, int D, const double* obs, int64_t obs_ld,
+                              const double* aux, const double* b_tiled, int W, int Wp, int gy, double* part, double* cost,
+                              double* grad, cudaStream_t st);
+size_t forward_cost_smem(int E);   // dynamic shared memory of forward_cost_rows for a bank of E emulators
+// Column split gy of forward_cost_rows for a call of call_N points: > 1 (the column groups spread over gy CTAs per row tile,
+// partial sums in part (gy, R, 1 + E)) when the row tiles alone leave most SMs idle.  A function of the call, not of a chunk.
+int forward_cost_split(int64_t call_N, int W);
 // group sizes the shared-difference bank kernel (predict_bank_mean.cuh) is compiled for: the G x (DP + 1) accumulators
 // of a thread (G without the gradient) have to stay in registers
 inline bool bank_group_ok(int DP, int G, bool grad) {

@@ -296,6 +296,291 @@ __global__ void __launch_bounds__(WRG * 128, (KS <= 5 ? (WRG == 1 ? 3 : 2) : 1))
     if (tid == 0) tma_store_wait_read();   // shared memory must outlive the last copy's reads
 }
 
+// ---- forward cost: the misfit of the back-projected spectra, reduced without materialising them ------------------
+//   cost_n = 1/2 sum_w l_w (fwd_nw - obs_nw)^2,  grad_nd = sum_w l_w (fwd_nw - obs_nw) deriv_full_ndw
+//          = sum_e deriv_ned s_ne  with  s (N, E) = u . basis^T,  u = l o (fwd - obs)           (multivariate_gp.py:216,218)
+// CTA = 32 rows, 8 warps as 2 (16 rows) x 4 (32 columns of each 128-column group).  The basis streams through the
+// two-stage TMA ring of k_project_tma; the fwd tile is formed by the same DMMA sequence as there (accumulators from
+// zero, k-steps ascending; slices of 32 emulators each from zero, added in slice order), so an observation equal to the
+// library's own fwd leaves a residual of exactly zero.  Residual and cost stay in registers.  The C fragment of u (lane:
+// row lane / 4, columns 2 (lane % 4) + h) is the A operand of two k-steps of s = u . basis^T with k <-> column
+// 2 (lane % 4) + h, B read from the staged basis group: no shared-memory round trip.  The four column warps add their
+// partial s through shared memory once per row tile, in a fixed order.
+//   KS: k-steps of 4 emulators per slice (4, 6 or 8; zero-padded emulators add exact zeros); nsl > 1: slices of 32
+//   emulators (KS = 8), all staged per group; A fragments are then re-read per slice, and with GRAD the W sweep runs
+//   once per slice of s (registers hold the s of one slice).
+//   aux = [weights padded to Wp with zeros | shared observation padded to Wp], so the tail group adds exact zeros.
+constexpr int kFcThreads = 256, kFcRows = 32, kFcPitch = 33;
+template <int KS, bool GRAD>
+__global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost(const double* __restrict__ mu, const double* __restrict__ deriv,
+                                                                int64_t R, int E, int D, const double* __restrict__ obs,
+                                                                int64_t obs_ld, const double* __restrict__ aux,
+                                                                const double* __restrict__ b_tiled, int W, int Wp, int nsl,
+                                                                double* __restrict__ cost, double* __restrict__ grad,
+                                                                double* __restrict__ part) {
+    extern __shared__ __align__(128) unsigned char psm[];
+    constexpr int NT = KS / 2;                                   // n-tiles of 8 emulators per slice of s
+    const int kstg = nsl == 1 ? KS : 8 * nsl;                    // k-steps staged per column group
+    const uint32_t stage_doubles = (uint32_t)kstg * kProjCols * 4, ks_bytes = kProjCols * 4 * 8;
+    uint64_t* full = reinterpret_cast<uint64_t*>(psm);           // [2]
+    double* stage = reinterpret_cast<double*>(psm + 128);        // [2][kstg][128][4]
+    double* red_s = stage + 2 * (size_t)stage_doubles;           // [4 column warps][32 rows][kFcPitch]
+    double* red_c = red_s + 4 * kFcRows * kFcPitch;              // [4 column warps][32 rows]
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int wr = warp >> 2, wc = warp & 3;
+    smem_guard(128u + 2u * stage_doubles * 8u + (4u * kFcRows * kFcPitch + 4u * kFcRows) * 8u);
+    const int64_t t0 = (int64_t)blockIdx.x * kFcRows;
+    // column groups y, y + gy, ... of this CTA (gy = gridDim.y > 1: a few rows, the groups spread over CTAs; the partial
+    // sums go to `part` [gy][R][1 + E] and k_forward_cost_finish adds them in the order of y)
+    const int gy = (int)gridDim.y, y0 = (int)blockIdx.y, ngroups = Wp / kProjCols;
+    const int ng = (ngroups - y0 + gy - 1) / gy, nsweep = GRAD ? nsl : 1, nitems = nsweep * ng;
+    if (tid == 0) {
+        mbar_init(&full[0], 1);
+        mbar_init(&full[1], 1);
+        fence_mbar_init();
+    }
+    __syncthreads();
+    auto load_item = [&](int it, int st) {   // thread 0: every staged k-step of the item's column group
+        const int g = y0 + (it % ng) * gy;
+        mbar_arrive_expect_tx(&full[st], (uint32_t)kstg * ks_bytes);
+        for (int ks = 0; ks < kstg; ++ks)
+            tma_bulk_g2s(stage + (size_t)st * stage_doubles + (size_t)ks * kProjCols * 4,
+                         b_tiled + ((size_t)ks * Wp + (size_t)g * kProjCols) * 4, ks_bytes, &full[st]);
+    };
+    if (tid == 0) {
+        load_item(0, 0);
+        if (nitems > 1) load_item(1, 1);
+    }
+    // A fragments of slice sl: lane holds mu[row = 16 wr + 8 i + lane / 4][e = 32 sl + 4 ks + lane % 4]
+    double a[2][KS];
+    auto load_a = [&](int sl) {
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+            const int64_t r = t0 + 16 * wr + 8 * i + (lane >> 2);
+#pragma unroll
+            for (int ks = 0; ks < KS; ++ks) {
+                const int e = 32 * sl + 4 * ks + (lane & 3);
+                a[i][ks] = (r < R && e < E) ? mu[r * E + e] : 0.0;
+            }
+        }
+    };
+    if (nsl == 1) load_a(0);
+    // observations of this lane's C-fragment elements: [i][j][h] = obs[row 16 wr + 8 i + lane / 4][column 8 j + 2 (lane % 4) + h
+    // of the warp's 32], zero past W
+    const double* obs1 = obs_ld == 0 ? aux + Wp : nullptr;
+    double ob[2][4][2];
+    auto load_obs = [&](int g) {
+        const int c0 = g * kProjCols + wc * 32 + 2 * (lane & 3);
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {
+            const int64_t r = t0 + 16 * wr + 8 * i + (lane >> 2);
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    const int w = c0 + 8 * j + h;
+                    ob[i][j][h] = obs1 ? obs1[w] : ((r < R && w < W) ? obs[r * obs_ld + w] : 0.0);
+                }
+        }
+    };
+    load_obs(y0);
+    double c[2] = {0.0, 0.0};                                    // per-lane share of sum u r of rows i
+    double s[2][NT][2];
+#pragma unroll
+    for (int i = 0; i < 2; ++i)
+#pragma unroll
+        for (int nt = 0; nt < NT; ++nt) s[i][nt][0] = s[i][nt][1] = 0.0;
+    uint32_t par = 0;
+    for (int it = 0; it < nitems; ++it) {
+        const int g = y0 + (it % ng) * gy, so = it / ng, st = it & 1;
+        const bool last = it % ng == ng - 1;
+        mbar_wait(&full[st], (par >> st) & 1u);
+        par ^= 1u << st;
+        const double* sb = stage + (size_t)st * stage_doubles;
+        // 1. fwd tile of the warp: 16 rows x 32 columns
+        double f[2][4][2];
+        for (int sl = 0; sl < nsl; ++sl) {
+            if (nsl > 1) load_a(sl);
+            const double* bs = sb + (size_t)sl * 8 * kProjCols * 4 + (size_t)(wc * 32 + (lane >> 2)) * 4 + (lane & 3);
+            double acc[2][4][2];
+#pragma unroll
+            for (int i = 0; i < 2; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
+#pragma unroll
+            for (int ks = 0; ks < KS; ++ks) {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const double bf = bs[(size_t)ks * kProjCols * 4 + j * 32];
+#pragma unroll
+                    for (int i = 0; i < 2; ++i) dmma_m8n8k4(acc[i][j][0], acc[i][j][1], a[i][ks], bf);
+                }
+            }
+#pragma unroll
+            for (int i = 0; i < 2; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) f[i][j][h] = sl == 0 ? acc[i][j][h] : f[i][j][h] + acc[i][j][h];
+        }
+        // 2. residual, weighted residual u (kept in f), cost
+        const int c0 = g * kProjCols + wc * 32 + 2 * (lane & 3);
+#pragma unroll
+        for (int i = 0; i < 2; ++i)
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    const double r = f[i][j][h] - ob[i][j][h];
+                    const double u = aux[c0 + 8 * j + h] * r;
+                    if (so == 0) c[i] = fma(u, r, c[i]);
+                    f[i][j][h] = u;
+                }
+        if (it + 1 < nitems) load_obs(y0 + ((it + 1) % ng) * gy);   // in flight during the s update and the next wait
+        // 3. s (rows x emulators of slice so) += u . basis^T over this warp's 32 columns: 8 k-steps (j, h)
+        if (GRAD) {
+            const double* bsl = sb + (size_t)so * 8 * kProjCols * 4;
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    const int cl = wc * 32 + 8 * j + 2 * (lane & 3) + h;
+#pragma unroll
+                    for (int nt = 0; nt < NT; ++nt) {
+                        // B[k = lane % 4][n = lane / 4] = basis[e = 8 nt + lane / 4][column cl]
+                        const double bf = bsl[((size_t)(2 * nt + (lane >> 4)) * kProjCols + cl) * 4 + ((lane >> 2) & 3)];
+#pragma unroll
+                        for (int i = 0; i < 2; ++i) dmma_m8n8k4(s[i][nt][0], s[i][nt][1], f[i][j][h], bf);
+                    }
+                }
+        }
+        __syncthreads();   // every warp is done with this stage: refill it
+        if (tid == 0 && it + 2 < nitems) load_item(it + 2, st);
+        if (so == 0 && last) {
+            // 4a. cost of the tile's rows: lanes of a row, then the four column warps, in a fixed order
+#pragma unroll
+            for (int i = 0; i < 2; ++i) {
+                double v = c[i] + __shfl_xor_sync(0xffffffffu, c[i], 1);
+                v += __shfl_xor_sync(0xffffffffu, v, 2);
+                if ((lane & 3) == 0) red_c[wc * kFcRows + 16 * wr + 8 * i + (lane >> 2)] = v;
+            }
+            __syncthreads();
+            if (tid < kFcRows && t0 + tid < R) {
+                const double v = ((red_c[tid] + red_c[kFcRows + tid]) + red_c[2 * kFcRows + tid]) + red_c[3 * kFcRows + tid];
+                if (gy > 1) part[((size_t)y0 * R + t0 + tid) * (1 + E)] = v;
+                else if (cost) cost[t0 + tid] = 0.5 * v;
+            }
+        }
+        if (GRAD && last) {
+            // 4b. grad_nd (+)= sum_{e in slice so} deriv_ned s_ne
+#pragma unroll
+            for (int i = 0; i < 2; ++i)
+#pragma unroll
+                for (int nt = 0; nt < NT; ++nt)
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) {
+                        red_s[(wc * kFcRows + 16 * wr + 8 * i + (lane >> 2)) * kFcPitch + 8 * nt + 2 * (lane & 3) + h] = s[i][nt][h];
+                        s[i][nt][h] = 0.0;
+                    }
+            __syncthreads();
+            const int es = min(32, E - 32 * so);
+            for (int k = tid; k < kFcRows * es; k += kFcThreads) {
+                const int rl = k / es, e = k - rl * es;
+                double* q = red_s + rl * kFcPitch + e;
+                *q = ((q[0] + q[kFcRows * kFcPitch]) + q[2 * kFcRows * kFcPitch]) + q[3 * kFcRows * kFcPitch];
+            }
+            __syncthreads();
+            if (gy > 1) {
+                for (int k = tid; k < kFcRows * es; k += kFcThreads) {
+                    const int rl = k / es, e = k - rl * es;
+                    if (t0 + rl < R) part[((size_t)y0 * R + t0 + rl) * (1 + E) + 1 + 32 * so + e] = red_s[rl * kFcPitch + e];
+                }
+            }
+            for (int k = tid; k < kFcRows * D && gy == 1; k += kFcThreads) {
+                const int rl = k / D, d = k - rl * D;
+                const int64_t r = t0 + rl;
+                if (r >= R) continue;
+                const double* dp = deriv + (r * E + 32 * so) * D + d;
+                double v = 0.0;
+                for (int e = 0; e < es; ++e) v = fma(dp[(size_t)e * D], red_s[rl * kFcPitch + e], v);
+                grad[r * D + d] = so == 0 ? v : grad[r * D + d] + v;
+            }
+            __syncthreads();   // red_s is rewritten by the next sweep
+        }
+    }
+}
+
+// aux = [weights or 1, zero past W | shared observation, zero past W] (one launch per call)
+__global__ void k_forward_cost_aux(const double* __restrict__ weights, const double* __restrict__ obs1, int W, int Wp,
+                                   double* __restrict__ aux) {
+    for (int w = blockIdx.x * blockDim.x + threadIdx.x; w < Wp; w += gridDim.x * blockDim.x) {
+        aux[w] = w < W ? (weights ? weights[w] : 1.0) : 0.0;
+        if (obs1) aux[Wp + w] = w < W ? obs1[w] : 0.0;
+    }
+}
+
+// Column-split calls: cost_r = 1/2 sum_y part[y][r][0], s_re = sum_y part[y][r][1 + e], grad_rd = sum_e deriv_red s_re
+__global__ void k_forward_cost_finish(const double* __restrict__ part, const double* __restrict__ deriv, int64_t R, int E, int D,
+                                      int gy, double* __restrict__ cost, double* __restrict__ grad) {
+    const int64_t pitch = (int64_t)R * (1 + E);
+    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < R * (D + 1); k += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t r = k / (D + 1);
+        const int d = (int)(k - r * (D + 1)) - 1;               // -1: the cost
+        const double* p = part + r * (1 + E);
+        if (d < 0) {
+            double v = 0.0;
+            for (int y = 0; y < gy; ++y) v += p[y * pitch];
+            if (cost) cost[r] = 0.5 * v;
+        } else if (grad) {
+            double v = 0.0;
+            for (int e = 0; e < E; ++e) {
+                double se = 0.0;
+                for (int y = 0; y < gy; ++y) se += p[y * pitch + 1 + e];
+                v = fma(deriv[(r * E + e) * D + d], se, v);
+            }
+            grad[r * D + d] = v;
+        }
+    }
+}
+
+int forward_cost_split(int64_t call_N, int W) {
+    int dev = 0, sms = 148;
+    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int64_t tiles = (call_N + kFcRows - 1) / kFcRows, ngroups = (W + kProjCols - 1) / kProjCols;
+    return (int)std::max<int64_t>(1, std::min<int64_t>(ngroups, (int64_t)sms / tiles));
+}
+
+size_t forward_cost_smem(int E) {
+    const int nsl = (E + 31) / 32, ks = (E + 3) / 4;
+    const int kstg = nsl == 1 ? (ks <= 4 ? 4 : ks <= 6 ? 6 : 8) : 8 * nsl;
+    return 128 + 2 * (size_t)kstg * kProjCols * 4 * 8 + (4 * (size_t)kFcRows * kFcPitch + 4 * kFcRows) * 8;
+}
+
+cudaError_t forward_cost_aux(const double* weights, const double* obs1, int W, int Wp, double* aux, cudaStream_t st) {
+    return launch_kernel(k_forward_cost_aux, (unsigned)((Wp + 255) / 256), 256, 0, st, weights, obs1, W, Wp, aux);
+}
+
+cudaError_t forward_cost_rows(const double* mu, const double* deriv, int64_t R, int E, int D, const double* obs, int64_t obs_ld,
+                              const double* aux, const double* b_tiled, int W, int Wp, int gy, double* part, double* cost,
+                              double* grad, cudaStream_t st) {
+    const int nsl = (E + 31) / 32, ks = (E + 3) / 4;
+    const size_t smem = forward_cost_smem(E);
+    const dim3 grid((unsigned)((R + kFcRows - 1) / kFcRows), (unsigned)gy);
+    cudaError_t e;
+#define GPE_FC(KSV)                                                                                                          \
+    e = grad ? launch_kernel(k_forward_cost<KSV, true>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs, obs_ld, aux,     \
+                             b_tiled, W, Wp, nsl, cost, grad, part)                                                          \
+             : launch_kernel(k_forward_cost<KSV, false>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs, obs_ld, aux,    \
+                             b_tiled, W, Wp, nsl, cost, grad, part)
+    if (nsl == 1 && ks <= 4) GPE_FC(4);
+    else if (nsl == 1 && ks <= 6) GPE_FC(6);
+    else GPE_FC(8);
+#undef GPE_FC
+    if (e != cudaSuccess || gy == 1) return e;
+    return launch_kernel(k_forward_cost_finish, (unsigned)((R * (D + 1) + 127) / 128), 128, 0, st, part, deriv, R, E, D, gy, cost,
+                         grad);
+}
+
 namespace {
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,

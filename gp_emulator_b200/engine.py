@@ -505,31 +505,50 @@ class DeviceBank(_Handle):
         (``gpe_bank_cost``).  ``obs`` is (E,) -- one observation for every point -- or (N, E); ``weights`` (E,) or None.
         numpy in -> numpy out (streamed below the C ABI, all devices of the bank); torch CUDA in -> torch CUDA out
         (asynchronous on the current stream, single-device banks)."""
-        D, E = self.D, self.E
         lib = _lib.load()
+        return self._reduce(testing, obs, weights, want_grad, self.E,
+                            lib.gpe_multi_bank_cost if self.multi else lib.gpe_bank_cost_host, lib.gpe_bank_cost)
+
+    def forward_cost(self, testing, obs, weights=None, want_grad=True):
+        """Least-squares misfit of the back-projected spectra against observed spectra, per point:
+        ``cost (N,) = 1/2 sum_w w_w (fwd_nw - obs_nw)^2`` and ``grad (N, D) = sum_w w_w (fwd_nw - obs_nw) deriv_full_ndw``
+        (``gpe_bank_forward_cost``), with fwd / deriv_full those of ``predict(project=True, project_deriv=True)``.  The
+        spectra never leave the kernel.  ``obs`` is (W,) -- one observed spectrum for every point -- or (N, W);
+        ``weights`` (W,) or None.  numpy in -> numpy out (streamed below the C ABI, all devices of the bank); torch CUDA
+        in -> torch CUDA out (asynchronous on the current stream, single-device banks)."""
+        if self.W == 0:
+            raise GpemuError("bank has no basis functions to project onto")
+        lib = _lib.load()
+        return self._reduce(testing, obs, weights, want_grad, self.W,
+                            lib.gpe_multi_bank_forward_cost if self.multi else lib.gpe_bank_forward_cost_host,
+                            lib.gpe_bank_forward_cost)
+
+    def _reduce(self, testing, obs, weights, want_grad, K, host_fn, device_fn):
+        """Shape checks and routing of the cost calls (observations K wide): host arrays to host_fn, CUDA tensors to
+        device_fn on the current stream."""
+        D = self.D
         if not _is_torch(testing):
             th = f64c(testing)
             if th.ndim != 2 or th.shape[1] != D:
                 raise ValueError(f"testing must be float64 (N, {D})")
             N = th.shape[0]
             o = f64c(obs.cpu().numpy() if _is_torch(obs) else obs)
-            if o.shape == (E,):
+            if o.shape == (K,):
                 obs_ld = 0
-            elif o.shape == (N, E):
-                obs_ld = E
+            elif o.shape == (N, K):
+                obs_ld = K
             else:
-                raise ValueError(f"obs must be ({E},) or ({N}, {E})")
+                raise ValueError(f"obs must be ({K},) or ({N}, {K})")
             wt = None
             if weights is not None:
                 wt = f64c(weights.cpu().numpy() if _is_torch(weights) else weights)
-                if wt.shape != (E,):
-                    raise ValueError(f"weights must be ({E},)")
+                if wt.shape != (K,):
+                    raise ValueError(f"weights must be ({K},)")
             out = {"cost": np.empty(N)}
             if want_grad:
                 out["grad"] = np.empty((N, D))
             if N > 0:
-                fn = lib.gpe_multi_bank_cost if self.multi else lib.gpe_bank_cost_host
-                check(fn(self._h, addr(th), N, addr(o), obs_ld, addr(wt), addr(out["cost"]), addr(out.get("grad"))))
+                check(host_fn(self._h, addr(th), N, addr(o), obs_ld, addr(wt), addr(out["cost"]), addr(out.get("grad"))))
             return out
         if self.multi:
             raise ValueError("a multi-device bank takes host arrays; use one DeviceBank per device for CUDA tensors")
@@ -541,23 +560,23 @@ class DeviceBank(_Handle):
         N = t.shape[0]
         o = torch.as_tensor(np.asarray(obs, dtype=np.float64) if not _is_torch(obs) else obs, dtype=torch.float64,
                             device=dev).contiguous()
-        if tuple(o.shape) == (E,):
+        if tuple(o.shape) == (K,):
             obs_ld = 0
-        elif tuple(o.shape) == (N, E):
-            obs_ld = E
+        elif tuple(o.shape) == (N, K):
+            obs_ld = K
         else:
-            raise ValueError(f"obs must be ({E},) or ({N}, {E})")
+            raise ValueError(f"obs must be ({K},) or ({N}, {K})")
         wt = None
         if weights is not None:
             wt = torch.as_tensor(np.asarray(weights, dtype=np.float64) if not _is_torch(weights) else weights,
                                  dtype=torch.float64, device=dev).contiguous()
-            if tuple(wt.shape) != (E,):
-                raise ValueError(f"weights must be ({E},)")
+            if tuple(wt.shape) != (K,):
+                raise ValueError(f"weights must be ({K},)")
         out = {"cost": torch.empty(N, dtype=torch.float64, device=dev)}
         if want_grad:
             out["grad"] = torch.empty(N, D, dtype=torch.float64, device=dev)
-        check(lib.gpe_bank_cost(self._h, addr(t), N, addr(o), obs_ld, addr(wt), addr(out["cost"]),
-                                addr(out.get("grad")), _current_stream_ptr(self.device)))
+        check(device_fn(self._h, addr(t), N, addr(o), obs_ld, addr(wt), addr(out["cost"]),
+                        addr(out.get("grad")), _current_stream_ptr(self.device)))
         return out
 
     def forward(self, testing, want_deriv=True):

@@ -164,6 +164,27 @@ class MultivariateEmulator(object):
             return (fwd[0], dfull[0]) if do_deriv else fwd[0]
         return (fwd, dfull) if do_deriv else fwd
 
+    def cost(self, y, obs, weights=None, do_deriv=True):
+        """Misfit of the reconstructed output at parameter vector(s) ``y`` against observed output(s) ``obs`` and its
+        gradient in ``y``: ``cost = 1/2 sum_w weights_w (fwd_w - obs_w)^2``, ``grad_d = sum_w weights_w (fwd_w - obs_w)
+        deriv_dw`` with fwd / deriv those of ``predict``, reduced on the device without forming them.
+
+        ``obs`` (N_full,) is shared by every point, (N, N_full) is one per point; ``weights`` (N_full,) or None (all 1).
+        One point: returns ``(cost: float, grad (N_params,))``; N points: ``(cost (N,), grad (N, N_params))``;
+        ``do_deriv=False``: the cost alone.  Host arrays or CUDA tensors, as ``predict``.
+        """
+        bank = self._device_bank()
+        if isinstance(y, np.ndarray) or not hasattr(y, "is_cuda"):
+            y2 = np.atleast_2d(y)
+        else:
+            y2 = y if y.dim() == 2 else y.reshape(1, -1)
+        out = bank.forward_cost(y2, obs, weights, want_grad=do_deriv)
+        c, g = out["cost"], out.get("grad")
+        if y2.shape[0] == 1:
+            c0 = float(c[0]) if isinstance(c, np.ndarray) else c[0]
+            return (c0, g[0]) if do_deriv else c0
+        return (c, g) if do_deriv else c
+
     def predict_pcs(self, y, do_unc=True, do_deriv=True):
         """PC-space outputs for N points: dict with mu (N, P), var (N, P), deriv (N, P, D)."""
         return self._device_bank().predict(np.atleast_2d(y), want_var=do_unc, want_deriv=do_deriv)

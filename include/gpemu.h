@@ -178,9 +178,26 @@ int gpe_bank_cost(gpe_bank* b, const double* testing, int64_t N, const double* o
 int gpe_bank_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                        const double* weights, double* cost, double* grad);
 
+/* Least-squares cost of the bank's back-projected spectra against observed spectra and its input gradient, per point:
+ *   cost_n = 1/2 sum_w l_w (fwd_nw - obs_nw)^2          fwd = mu . basis           (gp_emulator/multivariate_gp.py:216)
+ *   grad_nd =    sum_w l_w (fwd_nw - obs_nw) deriv_full_ndw    deriv_full_ndw = sum_e deriv_ned basis_ew   (:218)
+ * fwd and deriv are the bank's own PC means and gradients: the values gpe_bank_predict_ex returns with GPE_WANT_FWD and
+ * GPE_WANT_DERIV_FULL.  The residual is formed per wavelength, in one fused kernel, so neither fwd (N, W) nor
+ * deriv_full (N, D, W) is ever written to memory.  An observation equal to the library's own fwd gives exactly 0.
+ *   obs (N, W) with obs_ld >= W, or one (W) spectrum shared by every point with obs_ld = 0; weights (W) or NULL (all 1);
+ *   cost (N) or NULL; grad (N, D) or NULL (not both).  The bank needs a basis, and at most 96 emulators.
+ * Non-finite values propagate as in the formula above evaluated in numpy (no masking): a NaN observation gives a NaN
+ * cost and gradient even where its weight is 0. Results do not depend on chunking, pointer placement or the device count.
+ * Device pointers, asynchronous on `stream`; N = 0 launches nothing. */
+int gpe_bank_forward_cost(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                          const double* weights, double* cost, double* grad, void* stream);
+/* The same for host arrays (obs_ld = W or 0), streamed in chunks; synchronous. */
+int gpe_bank_forward_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                               const double* weights, double* cost, double* grad);
+
 /* Banks on several devices, host arrays, one call: the bank counterpart of gpe_multi_create / gpe_multi_predict
  * (same handle type; destroy with gpe_multi_destroy).  Arguments as gpe_bank_create / gpe_bank_predict_ex /
- * gpe_bank_cost_host. */
+ * gpe_bank_cost_host / gpe_bank_forward_cost_host. */
 int gpe_multi_bank_create(int n_devices, const int* devices, int E, int M, int D, const double* inputs,
                           const double* expX, const double* invQt, const double* invQ, const double* basis, int W,
                           gpe_multi** out);
@@ -188,6 +205,8 @@ int gpe_multi_bank_predict(gpe_multi* mm, const double* testing, int64_t N, doub
                            double* hess, double* fwd, double* deriv_full, unsigned flags);
 int gpe_multi_bank_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                         const double* weights, double* cost, double* grad);
+int gpe_multi_bank_forward_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                                const double* weights, double* cost, double* grad);
 
 /* PCA back-projection of bank means: fwd (N, W) = mu (N, E) @ basis (E, W)
  * (the accumulation `fwd += pred_mu * basis_functions[i]`, gp_emulator/multivariate_gp.py:216, batched
