@@ -1000,8 +1000,8 @@ int gpe_model_plan(gpe_model* m, int64_t N, char* buf, int len) {
         case Path::fused: {
             const FullPlan& f = *c.full;
             const int n = std::min(m->kern->full_name(f.cfg, f.nt_act, m->symmetric, buf, len), len - 1);
-            return n + snprintf(buf + n, len - n, " (cfg %d: %d-point tiles, Mp=%d, %d-stage TMA ring, %u B smem)", f.cfg, f.TN,
-                                f.Mp, f.nstage, f.smem);
+            return n + snprintf(buf + n, len - n, " (cfg %d: %d-point tiles, Mp=%d, %d-stage TMA ring, %u B smem, JC=%d, nchunks=%d)",
+                                f.cfg, f.TN, f.Mp, f.nstage, f.smem, f.JC, f.nchunks);
         }
         case Path::large:
             return snprintf(buf, len, "k_predict_mean2<%d,true> + k_var_large (Mp=%d, %d k-blocks, %d-stage ring)", m->DP,
