@@ -29,7 +29,8 @@ SYMBOLS = (
     "gpe_multi_destroy", "gpe_multi_bank_create", "gpe_multi_bank_predict", "gpe_multi_bank_cost",
     "gpe_bank_create", "gpe_bank_destroy", "gpe_bank_predict", "gpe_bank_predict_ex",
     "gpe_bank_cost", "gpe_bank_cost_host", "gpe_bank_forward_cost", "gpe_bank_forward_cost_host",
-    "gpe_multi_bank_forward_cost", "gpe_bank_project", "gpe_bank_forward", "gpe_measure_fp64_peaks", "gpe_launch_count",
+    "gpe_multi_bank_forward_cost", "gpe_bank_cost_ex", "gpe_bank_cost_host_ex", "gpe_bank_forward_cost_ex",
+    "gpe_bank_forward_cost_host_ex", "gpe_multi_bank_cost_ex", "gpe_multi_bank_forward_cost_ex", "gpe_bank_project", "gpe_bank_forward", "gpe_measure_fp64_peaks", "gpe_launch_count",
     "gpe_trainer_create", "gpe_trainer_eval", "gpe_trainer_destroy",
 )
 
@@ -107,6 +108,13 @@ def load():
     lib.gpe_bank_forward_cost_host.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, dp, dp]
     lib.gpe_multi_bank_forward_cost.restype = C.c_int
     lib.gpe_multi_bank_forward_cost.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, dp, dp]
+    for name in ("gpe_bank_cost_ex", "gpe_bank_forward_cost_ex"):
+        getattr(lib, name).restype = C.c_int
+        getattr(lib, name).argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, dp, dp, dp, C.c_void_p]
+    for name in ("gpe_bank_cost_host_ex", "gpe_bank_forward_cost_host_ex", "gpe_multi_bank_cost_ex",
+                 "gpe_multi_bank_forward_cost_ex"):
+        getattr(lib, name).restype = C.c_int
+        getattr(lib, name).argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, dp, dp, dp]
     lib.gpe_bank_project.restype = C.c_int
     lib.gpe_bank_project.argtypes = [C.c_void_p, dp, dp, C.c_int64, dp, dp, C.c_void_p]
     lib.gpe_bank_forward.restype = C.c_int

@@ -1225,15 +1225,90 @@ __global__ void __launch_bounds__(128) k_bank_cost(const double* __restrict__ mu
     }
 }
 
+// Exact Hessian of a bank cost, per point (DESIGN 4.6c), from the chunk scratch of bank_cost_walk:
+//   hess_n = sum_e c_ne H_ne + G_n^T A G_n,   G_n = deriv (E, D), H_ne = hs (E, D, D)
+//   band cost (s == NULL):     c = w o (mu - obs), formed here; A = diag(w) (C == NULL)
+//   forward cost (s != NULL):  c = s (n, E) from k_forward_cost;  A = C (E, E) from k_forward_cost_curv
+// A CTA takes P points at a time: their c (and, with C, T = C G_n) go to shared memory, then one thread per point and
+// upper-triangle entry i <= j sums over e in ascending order and writes (i, j) and (j, i): hess_n == hess_n^T bit for bit.
+__global__ void __launch_bounds__(256) k_cost_hess(const double* __restrict__ mu, const double* __restrict__ obs, int64_t obs_ld,
+                                                   const double* __restrict__ weights, const double* __restrict__ s,
+                                                   const double* __restrict__ C, const double* __restrict__ deriv,
+                                                   const double* __restrict__ hs, int64_t n, int E, int D, int P,
+                                                   double* __restrict__ hess) {
+    extern __shared__ double ch_s[];                     // [P][E] c, then (C) [P][E][D] T
+    double* cs = ch_s;
+    double* T = ch_s + (size_t)P * E;
+    const int tid = threadIdx.x, nt = D * (D + 1) / 2;
+    const int64_t ED = (int64_t)E * D, EDD = ED * D;
+    for (int64_t p0 = (int64_t)blockIdx.x * P; p0 < n; p0 += (int64_t)gridDim.x * P) {
+        const int np = n - p0 < P ? (int)(n - p0) : P;
+        for (int k = tid; k < np * E; k += blockDim.x) {
+            const int pl = k / E, e = k - pl * E;
+            const int64_t pt = p0 + pl;
+            cs[k] = s ? s[pt * E + e] : (weights ? weights[e] : 1.0) * (mu[pt * E + e] - obs[pt * obs_ld + e]);
+        }
+        if (C) {
+            for (int64_t k = tid; k < np * ED; k += blockDim.x) {
+                const int pl = (int)(k / ED), e = (int)((k - pl * ED) / D), d = (int)(k - pl * ED - (int64_t)e * D);
+                const double* g = deriv + (p0 + pl) * ED + d;
+                double v = 0.0;
+                for (int f = 0; f < E; ++f) v = fma(C[(int64_t)e * E + f], g[(int64_t)f * D], v);
+                T[k] = v;
+            }
+        }
+        __syncthreads();
+        for (int k = tid; k < np * nt; k += blockDim.x) {
+            const int pl = k / nt;
+            int q = k - pl * nt, i = 0;
+            while (q >= D - i) { q -= D - i; ++i; }
+            const int j = i + q;
+            const int64_t pt = p0 + pl;
+            const double* g = deriv + pt * ED;
+            const double* h = hs + pt * EDD + i * D + j;
+            const double* c = cs + (size_t)pl * E;
+            double a = 0.0, gn = 0.0;
+            for (int e = 0; e < E; ++e) a = fma(c[e], h[(int64_t)e * D * D], a);
+            if (C) {
+                const double* t = T + (size_t)pl * ED + j;
+                for (int e = 0; e < E; ++e) gn = fma(g[(int64_t)e * D + i], t[(int64_t)e * D], gn);
+            } else {
+                for (int e = 0; e < E; ++e) gn = fma((weights ? weights[e] : 1.0) * g[(int64_t)e * D + i], g[(int64_t)e * D + j], gn);
+            }
+            const double v = a + gn;
+            hess[pt * D * D + i * D + j] = v;
+            hess[pt * D * D + j * D + i] = v;
+        }
+        __syncthreads();
+    }
+}
+
+// Launch of k_cost_hess over n points: as many points per CTA as fill its 256 threads with upper-triangle entries, within
+// 48 KB of shared memory (at least one point: a forward cost of 96 emulators at D = 256 takes 194 KB).
+int cost_hess(const double* mu, const double* obs, int64_t obs_ld, const double* weights, const double* s, const double* C,
+              const double* deriv, const double* hs, int64_t n, int E, int D, int sms, double* hess, cudaStream_t st) {
+    const int nt = D * (D + 1) / 2;
+    const size_t per = (size_t)E * (C ? 1 + D : 1);
+    const int P = (int)std::max<size_t>(1, std::min<size_t>(std::max(1, 256 / nt), ((size_t)48 << 10) / (per * 8)));
+    const size_t smem = (size_t)P * per * 8;
+    if (smem > kSmemMax) return fail(GPE_ERR_UNSUPPORTED, "cost Hessian: %zu bytes of shared memory per point", smem);
+    const int grid = (int)std::min<int64_t>((n + P - 1) / P, (int64_t)sms * 8);
+    CUDA_TRY(launch_kernel(k_cost_hess, grid, 256, smem, st, mu, obs, obs_ld, weights, s, C, deriv, hs, n, E, D, P, hess));
+    return GPE_OK;
+}
+
 // The chunk walk of the bank's cost calls on `st`: the bank means (and, with `grad`, their input gradients) of whole
-// waves of 64-point tiles, at most 256 MB of them, go to the bank's cost scratch, and reduce(aux, mu, deriv, n0, n) consumes
-// each chunk.  The scratch starts with aux_n doubles that the reducer may fill with per-call operands.
+// waves of 64-point tiles, at most 256 MB of them, go to the bank's cost scratch, and reduce(aux, mu, deriv, hs, ext, n0, n)
+// consumes each chunk.  The scratch starts with aux_n doubles that the reducer may fill with per-call operands.  With
+// `hess`, a second pass after the unchanged first one fills hs (n, E, D, D) (and deriv, if the first pass did not), and ext
+// holds ext_pp doubles per point for the reducer: cost and gradient are those of the same call without `hess`.  A 64-point
+// chunk is allocated even where it exceeds the 256 MB (wide Hessians: 96 emulators at D = 256).
 template <typename Reduce>
-int bank_cost_walk(gpe_bank* b, const double* testing, int64_t N, bool grad, int64_t aux_n, cudaStream_t st, int64_t call_N,
-                   Reduce reduce) {
+int bank_cost_walk(gpe_bank* b, const double* testing, int64_t N, bool grad, bool hess, int64_t aux_n, int64_t ext_pp,
+                   cudaStream_t st, int64_t call_N, Reduce reduce) {
     if (call_N < 0) call_N = N;
     const int64_t E = b->E, D = b->D;
-    const int64_t per_point = E * (1 + (grad ? D : 0));
+    const int64_t per_point = E * (1 + (grad || hess ? D : 0)) + (hess ? E * D * D + ext_pp : 0);
     // points per chunk: whole waves of 64-point tiles, scratch bounded by 256 MB
     int64_t chunk = std::max<int64_t>(64, (((int64_t)256 << 20) / (per_point * 8)) / 64 * 64);
     chunk = std::min(chunk, (N + 63) / 64 * 64);
@@ -1253,11 +1328,15 @@ int bank_cost_walk(gpe_bank* b, const double* testing, int64_t N, bool grad, int
     }
     double* aux = b->cost_d;
     double* d_mu = b->cost_d + aux_n;
-    double* d_der = grad ? d_mu + chunk * E : nullptr;
+    double* d_der = grad || hess ? d_mu + chunk * E : nullptr;
+    double* d_hes = hess ? d_der + chunk * E * D : nullptr;
+    double* d_ext = hess ? d_hes + chunk * E * D * D : nullptr;
     for (int64_t n0 = 0; n0 < N; n0 += chunk) {
         const int64_t n = std::min(chunk, N - n0);
-        int rc = bank_predict_device(b, testing + n0 * D, n, d_mu, nullptr, d_der, nullptr, st, call_N);
-        if (rc == GPE_OK) rc = reduce(aux, d_mu, d_der, n0, n);
+        int rc = bank_predict_device(b, testing + n0 * D, n, d_mu, nullptr, grad ? d_der : nullptr, nullptr, st, call_N);
+        if (rc == GPE_OK && hess)
+            rc = bank_predict_device(b, testing + n0 * D, n, nullptr, nullptr, grad ? nullptr : d_der, d_hes, st, call_N);
+        if (rc == GPE_OK) rc = reduce(aux, d_mu, d_der, d_hes, d_ext, n0, n);
         if (rc) return rc;
     }
     CUDA_TRY(cudaEventRecord(b->cost_free, st));
@@ -1265,35 +1344,50 @@ int bank_cost_walk(gpe_bank* b, const double* testing, int64_t N, bool grad, int
 }
 
 int bank_cost_device(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
-                     double* cost, double* grad, cudaStream_t st, int64_t call_N = -1) {
+                     double* cost, double* grad, double* hess, cudaStream_t st, int64_t call_N = -1) {
     const int64_t E = b->E, D = b->D;
     const int sms = b->models[0]->sms;
-    return bank_cost_walk(b, testing, N, grad != nullptr, 0, st, call_N,
-                          [&](double*, const double* d_mu, const double* d_der, int64_t n0, int64_t n) -> int {
-                              const int grid = (int)std::min<int64_t>((n + 3) / 4, (int64_t)sms * 16);
-                              CUDA_TRY(launch_kernel(k_bank_cost, grid, 128, (size_t)4 * E * 8, st, d_mu, d_der, obs + n0 * obs_ld,
-                                                     obs_ld, weights, cost ? cost + n0 : nullptr, grad ? grad + n0 * D : nullptr,
-                                                     n, (int)E, (int)D));
-                              return GPE_OK;
+    return bank_cost_walk(b, testing, N, grad != nullptr, hess != nullptr, 0, 0, st, call_N,
+                          [&](double*, const double* d_mu, const double* d_der, const double* d_hes, double*, int64_t n0,
+                              int64_t n) -> int {
+                              if (cost || grad) {
+                                  const int grid = (int)std::min<int64_t>((n + 3) / 4, (int64_t)sms * 16);
+                                  CUDA_TRY(launch_kernel(k_bank_cost, grid, 128, (size_t)4 * E * 8, st, d_mu, d_der,
+                                                         obs + n0 * obs_ld, obs_ld, weights, cost ? cost + n0 : nullptr,
+                                                         grad ? grad + n0 * D : nullptr, n, (int)E, (int)D));
+                              }
+                              if (!hess) return GPE_OK;
+                              return cost_hess(d_mu, obs + n0 * obs_ld, obs_ld, weights, nullptr, nullptr, d_der, d_hes, n, (int)E,
+                                               (int)D, sms, hess + n0 * D * D, st);
                           });
 }
 
 // Misfit of the back-projected spectra against observed ones (k_forward_cost, project.cu): the same walk, the spectra and
 // Jacobians exist only as tiles inside the kernel.  The weights and the shared observation go to the scratch once per
 // call, zero-padded to the basis image's width.
+//   With hess, k_forward_cost also stores s = (l o (fwd - obs)) . basis^T (n, E) in the chunk scratch, and C = basis .
+// diag(l) . basis^T (E, E) follows the partial sums in the aux area, formed once per call: the Gauss-Newton term G^T C G
+// then costs E^2 D + E D^2 per point instead of D^2 W.
 int bank_forward_cost_device(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
-                             const double* weights, double* cost, double* grad, cudaStream_t st, int64_t call_N = -1) {
-    const int D = b->D, W = b->W, Wp = b->Wp;
+                             const double* weights, double* cost, double* grad, double* hess, cudaStream_t st,
+                             int64_t call_N = -1) {
+    const int D = b->D, W = b->W, Wp = b->Wp, E = b->E;
     // calls of a few points spread the column groups over CTAs; their partial sums follow the aux operands in the scratch
     const int gy = forward_cost_split(call_N < 0 ? N : call_N, W);
-    const int64_t part_n = gy > 1 ? (int64_t)gy * ((N + 63) / 64 * 64) * (1 + b->E) : 0;
-    return bank_cost_walk(b, testing, N, grad != nullptr, 2 * (int64_t)Wp + part_n, st, call_N,
-                          [&](double* aux, const double* d_mu, const double* d_der, int64_t n0, int64_t n) -> int {
+    const int64_t part_n = gy > 1 ? (int64_t)gy * ((N + 63) / 64 * 64) * (1 + E) : 0;
+    const int64_t aux_n = 2 * (int64_t)Wp + part_n + (hess ? (int64_t)E * E : 0);
+    return bank_cost_walk(b, testing, N, grad != nullptr, hess != nullptr, aux_n, E, st, call_N,
+                          [&](double* aux, const double* d_mu, const double* d_der, const double* d_hes, double* d_s,
+                              int64_t n0, int64_t n) -> int {
+                              double* C = hess ? aux + 2 * Wp + part_n : nullptr;
                               if (n0 == 0) CUDA_TRY(forward_cost_aux(weights, obs_ld == 0 ? obs : nullptr, W, Wp, aux, st));
-                              CUDA_TRY(forward_cost_rows(d_mu, d_der, n, b->E, D, obs + n0 * obs_ld, obs_ld, aux, b->d_basis, W,
+                              if (n0 == 0 && hess) CUDA_TRY(forward_cost_curv(b->d_basis, aux, E, Wp, C, st));
+                              CUDA_TRY(forward_cost_rows(d_mu, d_der, n, E, D, obs + n0 * obs_ld, obs_ld, aux, b->d_basis, W,
                                                          Wp, gy, aux + 2 * Wp, cost ? cost + n0 : nullptr,
-                                                         grad ? grad + n0 * D : nullptr, st));
-                              return GPE_OK;
+                                                         grad ? grad + n0 * D : nullptr, d_s, st));
+                              if (!hess) return GPE_OK;
+                              return cost_hess(nullptr, nullptr, 0, nullptr, d_s, C, d_der, d_hes, n, E, D, b->models[0]->sms,
+                                               hess + n0 * D * D, st);
                           });
 }
 
@@ -1328,21 +1422,23 @@ int bank_stream(gpe_bank* b, int64_t N, const CallIo& io, const SharedCall* shar
 }
 
 // Bank cost of observations K wide (E: the bank's own outputs, W: its spectra): testing and, unless obs_ld = 0, the
-// per-point observations (idx 0) in; cost, grad out (idx 1, 2).
-CallIo cost_io(const gpe_bank* b, int64_t K, const double* testing, const double* obs, int64_t obs_ld, double* cost, double* grad) {
+// per-point observations (idx 0) in; cost, grad, hess out (idx 1, 2, 3).
+CallIo cost_io(const gpe_bank* b, int64_t K, const double* testing, const double* obs, int64_t obs_ld, double* cost, double* grad,
+               double* hess) {
     CallIo io;
     io.in.add(testing, b->D);
     io.idx[0] = obs_ld != 0 ? io.in.add(obs, K) : -1;
     io.idx[1] = cost ? io.out.add(cost, 1) : -1;
     io.idx[2] = grad ? io.out.add(grad, b->D) : -1;
+    io.idx[3] = hess ? io.out.add(hess, (int64_t)b->D * b->D) : -1;
     return io;
 }
 
-typedef int (*CostDevice)(gpe_bank*, const double*, int64_t, const double*, int64_t, const double*, double*, double*, cudaStream_t,
-                          int64_t);
+typedef int (*CostDevice)(gpe_bank*, const double*, int64_t, const double*, int64_t, const double*, double*, double*, double*,
+                          cudaStream_t, int64_t);
 
 // Host-resident cost call (bank_cost_device or bank_forward_cost_device, observations K wide): test points (and
-// per-point observations) stream in, cost / gradient stream out.
+// per-point observations) stream in, cost / gradient / Hessian stream out.
 int bank_cost_stream(gpe_bank* b, int64_t K, CostDevice cost_device, int64_t N, const double* obs, int64_t obs_ld,
                      const double* weights, const CallIo& io, const SharedCall* shared = nullptr) {
     if (obs_ld != 0 && obs_ld != K) return fail(GPE_ERR_INVALID, "host observations must be contiguous: obs_ld = %s or 0", K == b->E ? "E" : "W");
@@ -1371,17 +1467,17 @@ int bank_cost_stream(gpe_bank* b, int64_t K, CostDevice cost_device, int64_t N, 
                            }
                            const double* d_obs = obs_ld != 0 ? io.at<const double>(di, 0) : d_obs1;
                            return cost_device(b, (const double*)di[0], n, d_obs, obs_ld != 0 ? K : 0, d_w,
-                                              io.at<double>(dout, 1), io.at<double>(dout, 2), st, N);
+                                              io.at<double>(dout, 1), io.at<double>(dout, 2), io.at<double>(dout, 3), st, N);
                        });
 }
 
 // Request check of the forward-cost calls (device: obs_ld = 0 or >= W; the host calls check obs_ld = 0 or W).
 int forward_cost_check(gpe_bank* b, int64_t N, const double* testing, const double* obs, int64_t obs_ld, const double* cost,
-                       const double* grad) {
+                       const double* grad, const double* hess) {
     if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
     if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
     if (!b->d_basis) return fail(GPE_ERR_INVALID, "bank was created without basis functions");
-    if (!cost && !grad) return fail(GPE_ERR_INVALID, "no output requested");
+    if (!cost && !grad && !hess) return fail(GPE_ERR_INVALID, "no output requested");
     if (N > 0 && (!testing || !obs)) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
     if (obs_ld != 0 && obs_ld < b->W) return fail(GPE_ERR_INVALID, "obs_ld must be 0 (one observed spectrum) or >= W");
     if (forward_cost_smem(b->E) > kSmemMax)
@@ -1709,50 +1805,71 @@ int gpe_bank_predict(gpe_bank* b, const double* testing, int64_t N, double* mu, 
                                flags & ~(unsigned)(GPE_WANT_FWD | GPE_WANT_DERIV_FULL), stream);
 }
 
-int gpe_bank_cost(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
-                  double* cost, double* grad, void* stream) {
+int gpe_bank_cost_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                     double* cost, double* grad, double* hess, void* stream) {
     NvtxRange nvtx_range("gpe_bank_cost");
     if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
     if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
     if (N == 0) return GPE_OK;
     if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
-    if (!cost && !grad) return fail(GPE_ERR_INVALID, "no output requested");
+    if (!cost && !grad && !hess) return fail(GPE_ERR_INVALID, "no output requested");
     if (obs_ld != 0 && obs_ld < b->E) return fail(GPE_ERR_INVALID, "obs_ld must be 0 (one observation vector) or >= E");
     CUDA_TRY(cudaSetDevice(b->device));
-    return bank_cost_device(b, testing, N, obs, obs_ld, weights, cost, grad, (cudaStream_t)stream);
+    return bank_cost_device(b, testing, N, obs, obs_ld, weights, cost, grad, hess, (cudaStream_t)stream);
 }
 
-int gpe_bank_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
-                       const double* weights, double* cost, double* grad) {
+int gpe_bank_cost(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                  double* cost, double* grad, void* stream) {
+    return gpe_bank_cost_ex(b, testing, N, obs, obs_ld, weights, cost, grad, nullptr, stream);
+}
+
+int gpe_bank_cost_host_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                          const double* weights, double* cost, double* grad, double* hess) {
     NvtxRange nvtx_range("gpe_bank_cost_host");
     if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
     if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
     if (N == 0) return GPE_OK;
     if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
-    if (!cost && !grad) return fail(GPE_ERR_INVALID, "no output requested");
+    if (!cost && !grad && !hess) return fail(GPE_ERR_INVALID, "no output requested");
     CUDA_TRY(cudaSetDevice(b->device));
     std::lock_guard<std::mutex> lock(b->host_mu);
-    return bank_cost_stream(b, b->E, bank_cost_device, N, obs, obs_ld, weights, cost_io(b, b->E, testing, obs, obs_ld, cost, grad));
+    return bank_cost_stream(b, b->E, bank_cost_device, N, obs, obs_ld, weights,
+                            cost_io(b, b->E, testing, obs, obs_ld, cost, grad, hess));
+}
+
+int gpe_bank_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                       const double* weights, double* cost, double* grad) {
+    return gpe_bank_cost_host_ex(b, testing, N, obs, obs_ld, weights, cost, grad, nullptr);
+}
+
+int gpe_bank_forward_cost_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                             const double* weights, double* cost, double* grad, double* hess, void* stream) {
+    NvtxRange nvtx_range("gpe_bank_forward_cost");
+    int rc = forward_cost_check(b, N, testing, obs, obs_ld, cost, grad, hess);
+    if (rc || N == 0) return rc;
+    CUDA_TRY(cudaSetDevice(b->device));
+    return bank_forward_cost_device(b, testing, N, obs, obs_ld, weights, cost, grad, hess, (cudaStream_t)stream);
 }
 
 int gpe_bank_forward_cost(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                           const double* weights, double* cost, double* grad, void* stream) {
-    NvtxRange nvtx_range("gpe_bank_forward_cost");
-    int rc = forward_cost_check(b, N, testing, obs, obs_ld, cost, grad);
-    if (rc || N == 0) return rc;
-    CUDA_TRY(cudaSetDevice(b->device));
-    return bank_forward_cost_device(b, testing, N, obs, obs_ld, weights, cost, grad, (cudaStream_t)stream);
+    return gpe_bank_forward_cost_ex(b, testing, N, obs, obs_ld, weights, cost, grad, nullptr, stream);
 }
 
-int gpe_bank_forward_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
-                               const double* weights, double* cost, double* grad) {
+int gpe_bank_forward_cost_host_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                                  const double* weights, double* cost, double* grad, double* hess) {
     NvtxRange nvtx_range("gpe_bank_forward_cost_host");
-    int rc = forward_cost_check(b, N, testing, obs, obs_ld, cost, grad);
+    int rc = forward_cost_check(b, N, testing, obs, obs_ld, cost, grad, hess);
     if (rc || N == 0) return rc;
     CUDA_TRY(cudaSetDevice(b->device));
     std::lock_guard<std::mutex> lock(b->host_mu);
     return bank_cost_stream(b, b->W, bank_forward_cost_device, N, obs, obs_ld, weights,
-                            cost_io(b, b->W, testing, obs, obs_ld, cost, grad));
+                            cost_io(b, b->W, testing, obs, obs_ld, cost, grad, hess));
+}
+
+int gpe_bank_forward_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                               const double* weights, double* cost, double* grad) {
+    return gpe_bank_forward_cost_host_ex(b, testing, N, obs, obs_ld, weights, cost, grad, nullptr);
 }
 
 int gpe_bank_project(gpe_bank* b, const double* mu, const double* deriv, int64_t N, double* fwd, double* deriv_full,
@@ -1883,32 +2000,42 @@ int gpe_multi_bank_predict(gpe_multi* mm, const double* testing, int64_t N, doub
                    [&](gpe_bank* b, const SharedCall* shared) { return bank_stream(b, N, io, shared); });
 }
 
-int gpe_multi_bank_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
-                        const double* weights, double* cost, double* grad) {
+int gpe_multi_bank_cost_ex(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                           const double* weights, double* cost, double* grad, double* hess) {
     NvtxRange nvtx_range("gpe_multi_bank_cost");
     if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
     if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
     if (N == 0) return GPE_OK;
     if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
-    if (!cost && !grad) return fail(GPE_ERR_INVALID, "no output requested");
+    if (!cost && !grad && !hess) return fail(GPE_ERR_INVALID, "no output requested");
     gpe_bank* b0 = mm->banks[0];
-    const CallIo io = cost_io(b0, b0->E, testing, obs, obs_ld, cost, grad);
+    const CallIo io = cost_io(b0, b0->E, testing, obs, obs_ld, cost, grad, hess);
     return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
         return bank_cost_stream(b, b->E, bank_cost_device, N, obs, obs_ld, weights, io, shared);
     });
 }
 
-int gpe_multi_bank_forward_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
-                                const double* weights, double* cost, double* grad) {
+int gpe_multi_bank_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                        const double* weights, double* cost, double* grad) {
+    return gpe_multi_bank_cost_ex(mm, testing, N, obs, obs_ld, weights, cost, grad, nullptr);
+}
+
+int gpe_multi_bank_forward_cost_ex(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                                   const double* weights, double* cost, double* grad, double* hess) {
     NvtxRange nvtx_range("gpe_multi_bank_forward_cost");
     if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
     gpe_bank* b0 = mm->banks[0];
-    int rc = forward_cost_check(b0, N, testing, obs, obs_ld, cost, grad);
+    int rc = forward_cost_check(b0, N, testing, obs, obs_ld, cost, grad, hess);
     if (rc || N == 0) return rc;
-    const CallIo io = cost_io(b0, b0->W, testing, obs, obs_ld, cost, grad);
+    const CallIo io = cost_io(b0, b0->W, testing, obs, obs_ld, cost, grad, hess);
     return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
         return bank_cost_stream(b, b->W, bank_forward_cost_device, N, obs, obs_ld, weights, io, shared);
     });
+}
+
+int gpe_multi_bank_forward_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                                const double* weights, double* cost, double* grad) {
+    return gpe_multi_bank_forward_cost_ex(mm, testing, N, obs, obs_ld, weights, cost, grad, nullptr);
 }
 
 }  // extern "C"

@@ -70,9 +70,12 @@ cudaError_t project_rows(const double* A, int64_t R, int RD, int64_t ldn, int64_
 // means mu (R, E) and gradients deriv (R, E, D); obs (R, obs_ld) or, obs_ld = 0, the shared observation in aux.
 // aux (2 Wp) is filled by forward_cost_aux: weights (NULL: 1) and the shared observation (NULL: none), zero-padded to Wp.
 cudaError_t forward_cost_aux(const double* weights, const double* obs1, int W, int Wp, double* aux, cudaStream_t st);
+// s_out (R, E) or NULL: with it, s = (l o (fwd - obs)) . basis^T is stored too, and grad may be NULL.
 cudaError_t forward_cost_rows(const double* mu, const double* deriv, int64_t R, int E, int D, const double* obs, int64_t obs_ld,
                               const double* aux, const double* b_tiled, int W, int Wp, int gy, double* part, double* cost,
-                              double* grad, cudaStream_t st);
+                              double* grad, double* s_out, cudaStream_t st);
+// C (E, E) = basis . diag(weights in aux) . basis^T, exactly symmetric.
+cudaError_t forward_cost_curv(const double* b_tiled, const double* aux, int E, int Wp, double* C, cudaStream_t st);
 size_t forward_cost_smem(int E);   // dynamic shared memory of forward_cost_rows for a bank of E emulators
 // Column split gy of forward_cost_rows for a call of call_N points: > 1 (the column groups spread over gy CTAs per row tile,
 // partial sums in part (gy, R, 1 + E)) when the row tiles alone leave most SMs idle.  A function of the call, not of a chunk.

@@ -310,14 +310,16 @@ __global__ void __launch_bounds__(WRG * 128, (KS <= 5 ? (WRG == 1 ? 3 : 2) : 1))
 //   emulators (KS = 8), all staged per group; A fragments are then re-read per slice, and with GRAD the W sweep runs
 //   once per slice of s (registers hold the s of one slice).
 //   aux = [weights padded to Wp with zeros | shared observation padded to Wp], so the tail group adds exact zeros.
+//   HESS (with GRAD): s itself goes to s_out (R, E) as well, the curvature coefficients of the cost's Hessian
+//   (k_cost_hess); grad may then be NULL.
 constexpr int kFcThreads = 256, kFcRows = 32, kFcPitch = 33;
-template <int KS, bool GRAD>
+template <int KS, bool GRAD, bool HESS>
 __global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost(const double* __restrict__ mu, const double* __restrict__ deriv,
                                                                 int64_t R, int E, int D, const double* __restrict__ obs,
                                                                 int64_t obs_ld, const double* __restrict__ aux,
                                                                 const double* __restrict__ b_tiled, int W, int Wp, int nsl,
                                                                 double* __restrict__ cost, double* __restrict__ grad,
-                                                                double* __restrict__ part) {
+                                                                double* __restrict__ part, double* __restrict__ s_out) {
     extern __shared__ __align__(128) unsigned char psm[];
     constexpr int NT = KS / 2;                                   // n-tiles of 8 emulators per slice of s
     const int kstg = nsl == 1 ? KS : 8 * nsl;                    // k-steps staged per column group
@@ -495,8 +497,13 @@ __global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost(const double* __
                     const int rl = k / es, e = k - rl * es;
                     if (t0 + rl < R) part[((size_t)y0 * R + t0 + rl) * (1 + E) + 1 + 32 * so + e] = red_s[rl * kFcPitch + e];
                 }
+            } else if (HESS) {
+                for (int k = tid; k < kFcRows * es; k += kFcThreads) {
+                    const int rl = k / es, e = k - rl * es;
+                    if (t0 + rl < R) s_out[(t0 + rl) * E + 32 * so + e] = red_s[rl * kFcPitch + e];
+                }
             }
-            for (int k = tid; k < kFcRows * D && gy == 1; k += kFcThreads) {
+            for (int k = tid; k < kFcRows * D && gy == 1 && (!HESS || grad); k += kFcThreads) {
                 const int rl = k / D, d = k - rl * D;
                 const int64_t r = t0 + rl;
                 if (r >= R) continue;
@@ -519,9 +526,31 @@ __global__ void k_forward_cost_aux(const double* __restrict__ weights, const dou
     }
 }
 
+// C (E, E) = basis . diag(l) . basis^T, the Gauss-Newton operand of the forward cost's Hessian (k_cost_hess), from the
+// tiled basis image and the padded weights in aux (one launch per call).  One warp per entry e <= f: lanes stride over
+// w, then a fixed butterfly; the entry is written to (e, f) and (f, e), so C is exactly symmetric.
+__global__ void k_forward_cost_curv(const double* __restrict__ b_tiled, const double* __restrict__ aux, int E, int Wp,
+                                    double* __restrict__ C) {
+    const int lane = threadIdx.x & 31;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; k < (int64_t)E * E; k += nwarps) {
+        const int e = (int)(k / E), f = (int)(k - (int64_t)e * E);
+        if (f < e) continue;
+        const double* be = b_tiled + (size_t)(e >> 2) * Wp * 4 + (e & 3);
+        const double* bf = b_tiled + (size_t)(f >> 2) * Wp * 4 + (f & 3);
+        double v = 0.0;
+        for (int w = lane; w < Wp; w += 32) v = fma(be[(size_t)4 * w] * aux[w], bf[(size_t)4 * w], v);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if (lane == 0) C[(int64_t)e * E + f] = C[(int64_t)f * E + e] = v;
+    }
+}
+
 // Column-split calls: cost_r = 1/2 sum_y part[y][r][0], s_re = sum_y part[y][r][1 + e], grad_rd = sum_e deriv_red s_re
+// (HESS: s also to s_out (R, E), by the threads of d = 0)
+template <bool HESS>
 __global__ void k_forward_cost_finish(const double* __restrict__ part, const double* __restrict__ deriv, int64_t R, int E, int D,
-                                      int gy, double* __restrict__ cost, double* __restrict__ grad) {
+                                      int gy, double* __restrict__ cost, double* __restrict__ grad, double* __restrict__ s_out) {
     const int64_t pitch = (int64_t)R * (1 + E);
     for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < R * (D + 1); k += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = k / (D + 1);
@@ -531,14 +560,15 @@ __global__ void k_forward_cost_finish(const double* __restrict__ part, const dou
             double v = 0.0;
             for (int y = 0; y < gy; ++y) v += p[y * pitch];
             if (cost) cost[r] = 0.5 * v;
-        } else if (grad) {
+        } else if (grad || HESS) {
             double v = 0.0;
             for (int e = 0; e < E; ++e) {
                 double se = 0.0;
                 for (int y = 0; y < gy; ++y) se += p[y * pitch + 1 + e];
+                if (HESS && d == 0) s_out[r * E + e] = se;
                 v = fma(deriv[(r * E + e) * D + d], se, v);
             }
-            grad[r * D + d] = v;
+            if (grad) grad[r * D + d] = v;
         }
     }
 }
@@ -560,25 +590,33 @@ cudaError_t forward_cost_aux(const double* weights, const double* obs1, int W, i
     return launch_kernel(k_forward_cost_aux, (unsigned)((Wp + 255) / 256), 256, 0, st, weights, obs1, W, Wp, aux);
 }
 
+cudaError_t forward_cost_curv(const double* b_tiled, const double* aux, int E, int Wp, double* C, cudaStream_t st) {
+    const int64_t warps = (int64_t)E * E;
+    return launch_kernel(k_forward_cost_curv, (unsigned)std::min<int64_t>((warps + 7) / 8, 4096), 256, 0, st, b_tiled, aux, E, Wp, C);
+}
+
 cudaError_t forward_cost_rows(const double* mu, const double* deriv, int64_t R, int E, int D, const double* obs, int64_t obs_ld,
                               const double* aux, const double* b_tiled, int W, int Wp, int gy, double* part, double* cost,
-                              double* grad, cudaStream_t st) {
+                              double* grad, double* s_out, cudaStream_t st) {
     const int nsl = (E + 31) / 32, ks = (E + 3) / 4;
     const size_t smem = forward_cost_smem(E);
     const dim3 grid((unsigned)((R + kFcRows - 1) / kFcRows), (unsigned)gy);
     cudaError_t e;
 #define GPE_FC(KSV)                                                                                                          \
-    e = grad ? launch_kernel(k_forward_cost<KSV, true>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs, obs_ld, aux,     \
-                             b_tiled, W, Wp, nsl, cost, grad, part)                                                          \
-             : launch_kernel(k_forward_cost<KSV, false>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs, obs_ld, aux,    \
-                             b_tiled, W, Wp, nsl, cost, grad, part)
+    e = s_out ? launch_kernel(k_forward_cost<KSV, true, true>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs, obs_ld,   \
+                              aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out)                                             \
+        : grad ? launch_kernel(k_forward_cost<KSV, true, false>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs, obs_ld, \
+                               aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out)                                            \
+               : launch_kernel(k_forward_cost<KSV, false, false>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs,       \
+                               obs_ld, aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out)
     if (nsl == 1 && ks <= 4) GPE_FC(4);
     else if (nsl == 1 && ks <= 6) GPE_FC(6);
     else GPE_FC(8);
 #undef GPE_FC
     if (e != cudaSuccess || gy == 1) return e;
-    return launch_kernel(k_forward_cost_finish, (unsigned)((R * (D + 1) + 127) / 128), 128, 0, st, part, deriv, R, E, D, gy, cost,
-                         grad);
+    const unsigned fgrid = (unsigned)((R * (D + 1) + 127) / 128);
+    return s_out ? launch_kernel(k_forward_cost_finish<true>, fgrid, 128, 0, st, part, deriv, R, E, D, gy, cost, grad, s_out)
+                 : launch_kernel(k_forward_cost_finish<false>, fgrid, 128, 0, st, part, deriv, R, E, D, gy, cost, grad, s_out);
 }
 
 namespace {

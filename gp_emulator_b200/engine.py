@@ -499,31 +499,33 @@ class DeviceBank(_Handle):
             self._host_call(th, N, res, flags)
         return res
 
-    def cost(self, testing, obs, weights=None, want_grad=True):
+    def cost(self, testing, obs, weights=None, want_grad=True, want_hess=False):
         """Least-squares misfit of the bank's means against observations, reduced over the emulators on the device:
         ``cost (N,) = 1/2 sum_e w_e (mu_ne - obs_ne)^2`` and ``grad (N, D) = sum_e w_e (mu_ne - obs_ne) deriv_ned``
         (``gpe_bank_cost``).  ``obs`` is (E,) -- one observation for every point -- or (N, E); ``weights`` (E,) or None.
+        ``want_hess``: also ``hess (N, D, D)``, the exact input Hessian of the cost (``gpe_bank_cost_ex``).
         numpy in -> numpy out (streamed below the C ABI, all devices of the bank); torch CUDA in -> torch CUDA out
         (asynchronous on the current stream, single-device banks)."""
         lib = _lib.load()
-        return self._reduce(testing, obs, weights, want_grad, self.E,
-                            lib.gpe_multi_bank_cost if self.multi else lib.gpe_bank_cost_host, lib.gpe_bank_cost)
+        return self._reduce(testing, obs, weights, want_grad, want_hess, self.E,
+                            lib.gpe_multi_bank_cost_ex if self.multi else lib.gpe_bank_cost_host_ex, lib.gpe_bank_cost_ex)
 
-    def forward_cost(self, testing, obs, weights=None, want_grad=True):
+    def forward_cost(self, testing, obs, weights=None, want_grad=True, want_hess=False):
         """Least-squares misfit of the back-projected spectra against observed spectra, per point:
         ``cost (N,) = 1/2 sum_w w_w (fwd_nw - obs_nw)^2`` and ``grad (N, D) = sum_w w_w (fwd_nw - obs_nw) deriv_full_ndw``
         (``gpe_bank_forward_cost``), with fwd / deriv_full those of ``predict(project=True, project_deriv=True)``.  The
         spectra never leave the kernel.  ``obs`` is (W,) -- one observed spectrum for every point -- or (N, W);
-        ``weights`` (W,) or None.  numpy in -> numpy out (streamed below the C ABI, all devices of the bank); torch CUDA
-        in -> torch CUDA out (asynchronous on the current stream, single-device banks)."""
+        ``weights`` (W,) or None.  ``want_hess``: also ``hess (N, D, D)``, the exact input Hessian of the cost
+        (``gpe_bank_forward_cost_ex``).  numpy in -> numpy out (streamed below the C ABI, all devices of the bank); torch
+        CUDA in -> torch CUDA out (asynchronous on the current stream, single-device banks)."""
         if self.W == 0:
             raise GpemuError("bank has no basis functions to project onto")
         lib = _lib.load()
-        return self._reduce(testing, obs, weights, want_grad, self.W,
-                            lib.gpe_multi_bank_forward_cost if self.multi else lib.gpe_bank_forward_cost_host,
-                            lib.gpe_bank_forward_cost)
+        return self._reduce(testing, obs, weights, want_grad, want_hess, self.W,
+                            lib.gpe_multi_bank_forward_cost_ex if self.multi else lib.gpe_bank_forward_cost_host_ex,
+                            lib.gpe_bank_forward_cost_ex)
 
-    def _reduce(self, testing, obs, weights, want_grad, K, host_fn, device_fn):
+    def _reduce(self, testing, obs, weights, want_grad, want_hess, K, host_fn, device_fn):
         """Shape checks and routing of the cost calls (observations K wide): host arrays to host_fn, CUDA tensors to
         device_fn on the current stream."""
         D = self.D
@@ -547,8 +549,11 @@ class DeviceBank(_Handle):
             out = {"cost": np.empty(N)}
             if want_grad:
                 out["grad"] = np.empty((N, D))
+            if want_hess:
+                out["hess"] = np.empty((N, D, D))
             if N > 0:
-                check(host_fn(self._h, addr(th), N, addr(o), obs_ld, addr(wt), addr(out["cost"]), addr(out.get("grad"))))
+                check(host_fn(self._h, addr(th), N, addr(o), obs_ld, addr(wt), addr(out["cost"]), addr(out.get("grad")),
+                              addr(out.get("hess"))))
             return out
         if self.multi:
             raise ValueError("a multi-device bank takes host arrays; use one DeviceBank per device for CUDA tensors")
@@ -575,8 +580,10 @@ class DeviceBank(_Handle):
         out = {"cost": torch.empty(N, dtype=torch.float64, device=dev)}
         if want_grad:
             out["grad"] = torch.empty(N, D, dtype=torch.float64, device=dev)
+        if want_hess:
+            out["hess"] = torch.empty(N, D, D, dtype=torch.float64, device=dev)
         check(device_fn(self._h, addr(t), N, addr(o), obs_ld, addr(wt), addr(out["cost"]),
-                        addr(out.get("grad")), _current_stream_ptr(self.device)))
+                        addr(out.get("grad")), addr(out.get("hess")), _current_stream_ptr(self.device)))
         return out
 
     def forward(self, testing, want_deriv=True):

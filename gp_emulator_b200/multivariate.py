@@ -164,26 +164,29 @@ class MultivariateEmulator(object):
             return (fwd[0], dfull[0]) if do_deriv else fwd[0]
         return (fwd, dfull) if do_deriv else fwd
 
-    def cost(self, y, obs, weights=None, do_deriv=True):
+    def cost(self, y, obs, weights=None, do_deriv=True, do_hess=False):
         """Misfit of the reconstructed output at parameter vector(s) ``y`` against observed output(s) ``obs`` and its
         gradient in ``y``: ``cost = 1/2 sum_w weights_w (fwd_w - obs_w)^2``, ``grad_d = sum_w weights_w (fwd_w - obs_w)
-        deriv_dw`` with fwd / deriv those of ``predict``, reduced on the device without forming them.
+        deriv_dw`` with fwd / deriv those of ``predict``, reduced on the device without forming them.  ``do_hess``: also
+        the exact Hessian in ``y`` (for Newton steps; with weights 1 / sigma^2, ``inv(hess)`` at the optimum is the
+        Laplace approximation of the posterior covariance).
 
         ``obs`` (N_full,) is shared by every point, (N, N_full) is one per point; ``weights`` (N_full,) or None (all 1).
-        One point: returns ``(cost: float, grad (N_params,))``; N points: ``(cost (N,), grad (N, N_params))``;
-        ``do_deriv=False``: the cost alone.  Host arrays or CUDA tensors, as ``predict``.
+        Returns the requested items in the order cost, grad, hess -- one point: ``float``, ``(N_params,)``,
+        ``(N_params, N_params)``; N points: ``(N,)``, ``(N, N_params)``, ``(N, N_params, N_params)`` -- and the cost
+        alone, not in a tuple, when it is the only one.  Host arrays or CUDA tensors, as ``predict``.
         """
         bank = self._device_bank()
         if isinstance(y, np.ndarray) or not hasattr(y, "is_cuda"):
             y2 = np.atleast_2d(y)
         else:
             y2 = y if y.dim() == 2 else y.reshape(1, -1)
-        out = bank.forward_cost(y2, obs, weights, want_grad=do_deriv)
-        c, g = out["cost"], out.get("grad")
+        out = bank.forward_cost(y2, obs, weights, want_grad=do_deriv, want_hess=do_hess)
+        res = [out["cost"]] + ([out["grad"]] if do_deriv else []) + ([out["hess"]] if do_hess else [])
         if y2.shape[0] == 1:
-            c0 = float(c[0]) if isinstance(c, np.ndarray) else c[0]
-            return (c0, g[0]) if do_deriv else c0
-        return (c, g) if do_deriv else c
+            c = res[0]
+            res = [float(c[0]) if isinstance(c, np.ndarray) else c[0]] + [a[0] for a in res[1:]]
+        return tuple(res) if len(res) > 1 else res[0]
 
     def predict_pcs(self, y, do_unc=True, do_deriv=True):
         """PC-space outputs for N points: dict with mu (N, P), var (N, P), deriv (N, P, D)."""

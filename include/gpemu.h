@@ -177,6 +177,18 @@ int gpe_bank_cost(gpe_bank* b, const double* testing, int64_t N, const double* o
 /* The same reduction for host arrays (obs_ld = E or 0), streamed in chunks; synchronous. */
 int gpe_bank_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                        const double* weights, double* cost, double* grad);
+/* gpe_bank_cost / gpe_bank_cost_host plus the exact input Hessian of the cost, hess (N, D, D) or NULL, laid out as
+ * GaussianProcess.hessian:
+ *   hess_n = sum_e w_e (mu_ne - obs_ne) H_ne + sum_e w_e deriv_ne deriv_ne^T      H_ne: the bank's per-emulator Hessians
+ * (the hess of gpe_bank_predict).  Any non-empty subset of cost, grad and hess may be requested; cost and grad are bit
+ * for bit those of the same call without hess.  hess_n equals its transpose bit for bit.  At obs = the bank's own mu the
+ * first sum is exactly 0 and hess_n is the (positive semi-definite) Gauss-Newton term; elsewhere it may be indefinite.
+ * Non-finite values propagate as in the formula evaluated in numpy: a NaN observation gives a NaN Hessian even where its
+ * weight is 0.  Results do not depend on chunking, pointer placement or the device count. */
+int gpe_bank_cost_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                     const double* weights, double* cost, double* grad, double* hess, void* stream);
+int gpe_bank_cost_host_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                          const double* weights, double* cost, double* grad, double* hess);
 
 /* Least-squares cost of the bank's back-projected spectra against observed spectra and its input gradient, per point:
  *   cost_n = 1/2 sum_w l_w (fwd_nw - obs_nw)^2          fwd = mu . basis           (gp_emulator/multivariate_gp.py:216)
@@ -194,6 +206,19 @@ int gpe_bank_forward_cost(gpe_bank* b, const double* testing, int64_t N, const d
 /* The same for host arrays (obs_ld = W or 0), streamed in chunks; synchronous. */
 int gpe_bank_forward_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                                const double* weights, double* cost, double* grad);
+/* gpe_bank_forward_cost / gpe_bank_forward_cost_host plus the exact input Hessian of the cost, hess (N, D, D) or NULL,
+ * laid out as GaussianProcess.hessian:
+ *   hess_n = sum_e s_ne H_ne + deriv_n^T C deriv_n      s_ne = sum_w l_w (fwd_nw - obs_nw) basis_ew,
+ *                                                       C = basis . diag(l) . basis^T (E, E), deriv_n (E, D)
+ * which is sum_w l_w deriv_full_nw deriv_full_nw^T + sum_w l_w (fwd_nw - obs_nw) d2 fwd_nw / dx2 without forming either
+ * per wavelength.  Any non-empty subset of cost, grad and hess may be requested; cost and grad are bit for bit those of
+ * the same call without hess.  hess_n equals its transpose bit for bit.  At obs = the bank's own fwd s is exactly 0 and
+ * hess_n is the (positive semi-definite) Gauss-Newton term.  A NaN observation gives a NaN Hessian even where its weight
+ * is 0, as the formula evaluated in numpy does.  Same limits as gpe_bank_forward_cost (basis, at most 96 emulators). */
+int gpe_bank_forward_cost_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                             const double* weights, double* cost, double* grad, double* hess, void* stream);
+int gpe_bank_forward_cost_host_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                                  const double* weights, double* cost, double* grad, double* hess);
 
 /* Banks on several devices, host arrays, one call: the bank counterpart of gpe_multi_create / gpe_multi_predict
  * (same handle type; destroy with gpe_multi_destroy).  Arguments as gpe_bank_create / gpe_bank_predict_ex /
@@ -207,6 +232,11 @@ int gpe_multi_bank_cost(gpe_multi* mm, const double* testing, int64_t N, const d
                         const double* weights, double* cost, double* grad);
 int gpe_multi_bank_forward_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                                 const double* weights, double* cost, double* grad);
+/* ... with the Hessian hess (N, D, D) or NULL, as gpe_bank_cost_host_ex / gpe_bank_forward_cost_host_ex. */
+int gpe_multi_bank_cost_ex(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                           const double* weights, double* cost, double* grad, double* hess);
+int gpe_multi_bank_forward_cost_ex(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                                   const double* weights, double* cost, double* grad, double* hess);
 
 /* PCA back-projection of bank means: fwd (N, W) = mu (N, E) @ basis (E, W)
  * (the accumulation `fwd += pred_mu * basis_functions[i]`, gp_emulator/multivariate_gp.py:216, batched
