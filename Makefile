@@ -8,7 +8,7 @@ BUILD     := build/obj
 DPS       := 2 4 6 8 10 12 16 24 32
 LIB       := gp_emulator_b200/libgpemu.so
 
-OBJS := $(BUILD)/gpemu.o $(BUILD)/project.o $(BUILD)/peaks.o $(BUILD)/var_large.o $(BUILD)/tf32.o $(BUILD)/train.o $(foreach d,$(DPS),$(BUILD)/inst_dp$(d).o)
+OBJS := $(BUILD)/gpemu.o $(BUILD)/project.o $(BUILD)/invert.o $(BUILD)/peaks.o $(BUILD)/var_large.o $(BUILD)/tf32.o $(BUILD)/train.o $(foreach d,$(DPS),$(BUILD)/inst_dp$(d).o)
 HDRS := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) include/gpemu.h
 
 all: $(LIB)
@@ -24,6 +24,9 @@ $(BUILD)/peaks.o: $(CSRC)/peaks.cu $(HDRS) | $(BUILD)
 
 $(BUILD)/project.o: $(CSRC)/project.cu $(HDRS) | $(BUILD)
 	$(NVCC) $(NVFLAGS) -Xptxas -v -c $< -o $@ 2> $(BUILD)/project.ptxas.log || (cat $(BUILD)/project.ptxas.log; exit 1)
+
+$(BUILD)/invert.o: $(CSRC)/invert.cu $(HDRS) | $(BUILD)
+	$(NVCC) $(NVFLAGS) -Xptxas -v -c $< -o $@ 2> $(BUILD)/invert.ptxas.log || (cat $(BUILD)/invert.ptxas.log; exit 1)
 
 $(BUILD)/var_large.o: $(CSRC)/predict_var_large.cu $(HDRS) | $(BUILD)
 	$(NVCC) $(NVFLAGS) -Xptxas -v -c $< -o $@ 2> $(BUILD)/var_large.ptxas.log || (cat $(BUILD)/var_large.ptxas.log; exit 1)

@@ -7,8 +7,9 @@
 2. build a ``MultivariateEmulator`` (PCA + one GP per component), hyper-parameters fitted with the batched GPU
    training objective (``batched_training=True``; drop the flag for the reference's sequential host fit);
 3. predict spectra + Jacobians, one point (the reference's call) and a batch; score 1000 candidates against an observed
-   spectrum (``emu.cost``), refine the best one with Newton steps on the exact Hessian and print its Laplace posterior
-   standard deviations;
+   spectrum (``emu.cost``), then invert 1000 noisy spectra at once inside the design's bounds (``emu.invert``: bounded
+   Levenberg-Marquardt on the exact Hessian, on the device) and print the retrieved parameters with their Laplace
+   posterior standard deviations;
 4. per-band ``GaussianProcess`` objects: mean / variance / gradient / Hessian, FP64 and single precision;
 5. a per-band bank reduced on the device to a least-squares misfit and its gradient (``DeviceBank.cost``);
 6. store and reload an emulator (``EmulatorStorage``).
@@ -54,21 +55,18 @@ def main():
     best = int(np.argmin(cost))
     print("misfit of 1000 candidates against one observed spectrum: best candidate %d (cost %.3f), true one is 3 "
           "(cost %.3f); gradients %s" % (best, cost[best], cost[3], grad.shape))
-    sigma = 0.01                                                              # 3c. Newton steps + Laplace uncertainty
-    obs, w = truth[3] + sigma * noise, np.full(len(wl), 1.0 / sigma ** 2)     # weights 1 / sigma^2: cost = -log likelihood
-    y, damp = y_test[best].copy(), 0.0
-    c, g, H = emu.cost(y, obs, w, do_hess=True)
-    c_start = c
-    for _ in range(8):                                                        # Newton, damped only when a step fails
-        step = np.linalg.solve(H + damp * np.abs(np.diag(H)).max() * np.eye(len(y)), -g)
-        c_new, g_new, H_new = emu.cost(y + step, obs, w, do_hess=True)
-        if c_new < c:
-            y, c, g, H, damp = y + step, c_new, g_new, H_new, damp / 10
-        else:
-            damp = max(10 * damp, 1e-3)
-    sd = np.sqrt(np.diag(np.linalg.inv(H)))
-    print("Newton from candidate %d: cost %.1f -> %.1f; retrieved %s +- %s (Laplace sd), truth %s" % (
-        best, c_start, c, np.round(y, 4), np.round(sd, 4), np.round(y_test[3], 4)))
+    sigma = 0.01                                                              # 3c. inversion + Laplace uncertainty
+    obs = truth + sigma * np.random.RandomState(2).standard_normal(truth.shape)   # one noisy spectrum per pixel
+    lower, upper = np.array([d.ppf(0.0) for d in dists]), np.array([d.ppf(1.0) for d in dists])
+    y0 = np.tile(0.5 * (lower + upper), (len(obs), 1))
+    t0 = time.perf_counter()                                                  # weights 1 / sigma^2: cost = -log likelihood
+    res = emu.invert(obs, y0, weights=np.full(len(wl), 1.0 / sigma ** 2), bounds=(lower, upper))
+    sd = np.sqrt(np.diagonal(res["cov"], axis1=1, axis2=2))
+    print("inverted %d spectra in %.3f s, status counts %s (converged, max_iter, stalled, nonfinite)" % (
+        len(obs), time.perf_counter() - t0, np.bincount(res["status"], minlength=4).tolist()))
+    print("pixel 3: retrieved %s +- %s (Laplace sd), truth %s; %.0f%% of all retrieved parameters lie within 3 sd of "
+          "the truth" % (np.round(res["x"][3], 4), np.round(sd[3], 4), np.round(y_test[3], 4),
+                         100 * np.mean(np.abs(res["x"] - y_test) <= 3 * sd)))
 
     bands = [40, 120, 200, 280, 360]                                          # 4. per-band GPs
     from gp_emulator_b200.training import fit_bank

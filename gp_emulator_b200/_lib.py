@@ -21,6 +21,10 @@ F32_FAST_TF32 = 0x200
 F32_FORCE_3X = 0x400
 MAX_TRAIN, MAX_INPUTS = 16384, 256
 TRAIN_MAX_M = 1024
+SOLVE_SPECTRA = 0x1000
+SOLVE_MAX_D = 32
+SOLVE_CONVERGED, SOLVE_MAX_ITER, SOLVE_STALLED, SOLVE_NONFINITE = 0, 1, 2, 3
+SOLVE_DEFAULT_MAX_ITER = 50
 
 # every symbol include/gpemu.h declares (tests/test_abi.py checks the header against this list and the .so)
 SYMBOLS = (
@@ -31,8 +35,15 @@ SYMBOLS = (
     "gpe_bank_cost", "gpe_bank_cost_host", "gpe_bank_forward_cost", "gpe_bank_forward_cost_host",
     "gpe_multi_bank_forward_cost", "gpe_bank_cost_ex", "gpe_bank_cost_host_ex", "gpe_bank_forward_cost_ex",
     "gpe_bank_forward_cost_host_ex", "gpe_multi_bank_cost_ex", "gpe_multi_bank_forward_cost_ex", "gpe_bank_project", "gpe_bank_forward", "gpe_measure_fp64_peaks", "gpe_launch_count",
-    "gpe_trainer_create", "gpe_trainer_eval", "gpe_trainer_destroy",
+    "gpe_trainer_create", "gpe_trainer_eval", "gpe_trainer_destroy", "gpe_bank_solve", "gpe_multi_bank_solve",
 )
+
+
+class SolveOpts(C.Structure):
+    """``gpe_solve_opts`` of include/gpemu.h."""
+    _fields_ = [("max_iter", C.c_int), ("ftol", C.c_double), ("xtol", C.c_double), ("gtol", C.c_double),
+                ("lambda0", C.c_double), ("lower", C.c_void_p), ("upper", C.c_void_p), ("prior_mean", C.c_void_p),
+                ("prior_ld", C.c_int64), ("prior_prec", C.c_void_p)]
 
 
 class GpemuError(RuntimeError):
@@ -115,6 +126,12 @@ def load():
                  "gpe_multi_bank_forward_cost_ex"):
         getattr(lib, name).restype = C.c_int
         getattr(lib, name).argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, dp, dp, dp]
+    so = C.POINTER(SolveOpts)
+    lib.gpe_bank_solve.restype = C.c_int
+    lib.gpe_bank_solve.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, so, dp, dp, dp, dp, dp, dp, C.c_uint,
+                                   C.c_void_p]
+    lib.gpe_multi_bank_solve.restype = C.c_int
+    lib.gpe_multi_bank_solve.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, so, dp, dp, dp, dp, dp, dp, C.c_uint]
     lib.gpe_bank_project.restype = C.c_int
     lib.gpe_bank_project.argtypes = [C.c_void_p, dp, dp, C.c_int64, dp, dp, C.c_void_p]
     lib.gpe_bank_forward.restype = C.c_int

@@ -31,6 +31,7 @@
 #include "gpe_math.cuh"
 #include "host_common.h"
 #include "host_stream.h"
+#include "invert.h"
 
 using namespace gpe;
 
@@ -154,6 +155,12 @@ struct gpe_bank {
     double* cost_d = nullptr;
     size_t cost_cap = 0;
     cudaEvent_t cost_free = nullptr;
+    // gpe_bank_solve: solver state and active lists (one solve at a time per bank), the active count read back per iteration
+    std::mutex solve_mu;
+    void* solve_d = nullptr;
+    size_t solve_cap = 0;
+    int* solve_count = nullptr;        // page-locked
+    cudaEvent_t solve_ev = nullptr;
 };
 
 struct gpe_multi {
@@ -1485,6 +1492,176 @@ int forward_cost_check(gpe_bank* b, int64_t N, const double* testing, const doub
     return GPE_OK;
 }
 
+// ---- inversion (DESIGN 4.6d): bounded Levenberg-Marquardt, kernels in invert.cu ------------------------------------
+// Solve of N points on `st` (device arrays), in sub-chunks whose solver scratch stays within 256 MB.  Each iteration
+// evaluates the active trial points with the call's cost (cost, gradient and Hessian; call_N: the kernel plans follow the
+// call, never the active count), runs k_lm_step, compacts the active list in ascending order and reads its length back
+// through page-locked memory; the trial rows (and per-point observation rows, when the list shrank) of the survivors are
+// gathered for the next evaluation.  Synchronous: returns when the outputs are written.
+int bank_solve_device(gpe_bank* b, CostDevice cost_device, int64_t K, const LmProblem& pb, const double* x0, int64_t N,
+                      const double* obs, int64_t obs_ld, const double* weights, double* x, double* cost, double* grad,
+                      double* hess, double* cov, int32_t* info, cudaStream_t st, int64_t call_N) {
+    const int64_t D = b->D, R = lm_state_doubles((int)D);
+    const int64_t per = R + D * D + 2 * D + 1 + (obs_ld > 0 ? K : 0) + 2;   // doubles per point, lists and flag included
+    int64_t sub = std::max<int64_t>(1, std::min<int64_t>(N, (((int64_t)256 << 20) / 8) / per));
+    if (const char* e = getenv("GPE_SOLVE_SUB_POINTS")) sub = std::max<int64_t>(1, std::min<int64_t>(sub, atoll(e)));   // dev aid: force sub-chunks in tests
+    const size_t temp = lm_select_temp(sub);
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
+    const size_t o_state = carve(8 * sub * R), o_xe = carve(8 * sub * D), o_fe = carve(8 * sub), o_ge = carve(8 * sub * D);
+    const size_t o_he = carve(8 * sub * D * D), o_obs = carve(obs_ld > 0 ? 8 * sub * K : 0), o_l0 = carve(4 * sub);
+    const size_t o_l1 = carve(4 * sub), o_flag = carve(4 * sub), o_cnt = carve(4), o_tmp = carve(temp);
+    std::lock_guard<std::mutex> lock(b->solve_mu);
+    int rc = ensure_buf(&b->solve_d, &b->solve_cap, off, false);
+    if (rc) return rc;
+    if (!b->solve_count) CUDA_TRY(cudaMallocHost((void**)&b->solve_count, sizeof(int)));
+    if (!b->solve_ev) CUDA_TRY(cudaEventCreateWithFlags(&b->solve_ev, cudaEventDisableTiming));
+    char* base = (char*)b->solve_d;
+    double* state = (double*)(base + o_state);
+    double *xe = (double*)(base + o_xe), *fe = (double*)(base + o_fe), *ge = (double*)(base + o_ge), *he = (double*)(base + o_he);
+    double* obs_c = (double*)(base + o_obs);
+    int *lists[2] = {(int*)(base + o_l0), (int*)(base + o_l1)}, *flag = (int*)(base + o_flag), *d_cnt = (int*)(base + o_cnt);
+    for (int64_t s0 = 0; s0 < N; s0 += sub) {
+        const int64_t n = std::min(sub, N - s0);
+        LmProblem p = pb;
+        if (p.prior_mean && p.prior_ld > 0) p.prior_mean += s0 * p.prior_ld;
+        const double* o = obs + s0 * obs_ld;
+        CUDA_TRY(lm_init(p, x0 + s0 * D, n, state, xe, lists[0], st));
+        const double* e_obs = o;      // observation rows of the evaluation: the caller's while every point is active
+        int64_t e_ld = obs_ld, act = n;
+        for (int it = 0;; ++it) {
+            int* list = lists[it & 1];
+            int* next_list = lists[(it + 1) & 1];
+            rc = cost_device(b, xe, act, e_obs, e_ld, weights, fe, ge, he, st, call_N);
+            if (rc) return rc;
+            CUDA_TRY(lm_step(p, act, list, fe, ge, he, state, flag, it == 0, st));
+            CUDA_TRY(lm_select(list, flag, act, next_list, d_cnt, base + o_tmp, temp, st));
+            CUDA_TRY(cudaMemcpyAsync(b->solve_count, d_cnt, sizeof(int), cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaEventRecord(b->solve_ev, st));
+            CUDA_TRY(cudaEventSynchronize(b->solve_ev));
+            const int64_t next = *b->solve_count;
+            if (next == 0) break;
+            const bool regather = obs_ld > 0 && next < act;
+            CUDA_TRY(lm_gather(state, (int)D, next_list, next, xe, o, regather ? obs_ld : 0, K, obs_c, st));
+            if (regather) { e_obs = obs_c; e_ld = K; }
+            act = next;
+        }
+        CUDA_TRY(lm_output((int)D, n, state, x + s0 * D, cost ? cost + s0 : nullptr, grad ? grad + s0 * D : nullptr,
+                           hess ? hess + s0 * D * D : nullptr, cov ? cov + s0 * D * D : nullptr, info + 2 * s0, st));
+    }
+    CUDA_TRY(cudaEventRecord(b->solve_ev, st));
+    CUDA_TRY(cudaEventSynchronize(b->solve_ev));
+    return GPE_OK;
+}
+
+constexpr gpe_solve_opts kSolveDefaults = {GPE_SOLVE_DEFAULT_MAX_ITER, 1e-10, 1e-10, 0.0, 1e-3, nullptr, nullptr, nullptr, 0, nullptr};
+
+LmProblem lm_problem(int D, const gpe_solve_opts& o, const double* lower, const double* upper, const double* prior_mean,
+                     int64_t prior_ld, const double* prior_prec) {
+    return LmProblem{D, lower, upper, prior_mean, prior_ld, prior_prec, o.max_iter, o.ftol, o.xtol, o.gtol, o.lambda0};
+}
+
+// Request check of the solve calls; *o = the options with defaults for opts == NULL.  Reads the bounds (device pointers:
+// a D2H copy on the call's stream `st`, so that it sees what the solve will read; the device is set).
+int solve_check(gpe_bank* b, int64_t N, const double* x0, const double* obs, int64_t obs_ld, const gpe_solve_opts* opts,
+                const double* x, const int32_t* info, unsigned flags, bool host, cudaStream_t st, gpe_solve_opts* o) {
+    if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
+    if (flags & ~(GPE_SOLVE_SPECTRA | GPE_HOST_PTRS)) return fail(GPE_ERR_INVALID, "unknown flag bits 0x%x", flags);
+    if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
+    const bool spectra = flags & GPE_SOLVE_SPECTRA;
+    const int D = b->D;
+    const int64_t K = spectra ? b->W : b->E;
+    if (spectra && !b->d_basis) return fail(GPE_ERR_INVALID, "bank was created without basis functions");
+    *o = opts ? *opts : kSolveDefaults;
+    if (o->max_iter < 0) return fail(GPE_ERR_INVALID, "max_iter must be >= 0");
+    if (!(o->ftol >= 0 && o->xtol >= 0 && o->gtol >= 0 && o->lambda0 > 0))
+        return fail(GPE_ERR_INVALID, "ftol, xtol, gtol must be >= 0 and lambda0 > 0");
+    if (o->prior_mean && !o->prior_prec) return fail(GPE_ERR_INVALID, "prior_mean given without prior_prec");
+    if (o->prior_mean && o->prior_ld != 0 && (host ? o->prior_ld != D : o->prior_ld < D))
+        return fail(GPE_ERR_INVALID, "prior_ld must be 0 (one prior mean) or %s D", host ? "=" : ">=");
+    if (obs_ld != 0 && (host ? obs_ld != K : obs_ld < K))
+        return fail(GPE_ERR_INVALID, "obs_ld must be 0 (one observation) or %s %s", host ? "=" : ">=", spectra ? "W" : "E");
+    if (N > 0 && (!x0 || !obs || !x || !info)) return fail(GPE_ERR_INVALID, "x0 / obs / x / info is NULL");
+    if (D > GPE_SOLVE_MAX_D) return fail(GPE_ERR_UNSUPPORTED, "the solver supports D <= %d (got %d)", GPE_SOLVE_MAX_D, D);
+    if (spectra && forward_cost_smem(b->E) > kSmemMax)
+        return fail(GPE_ERR_UNSUPPORTED, "the forward cost supports banks of up to 96 emulators (got %d)", b->E);
+    if (o->lower && o->upper) {
+        double lo[GPE_SOLVE_MAX_D], hi[GPE_SOLVE_MAX_D];
+        if (host) {
+            memcpy(lo, o->lower, D * 8);
+            memcpy(hi, o->upper, D * 8);
+        } else {
+            CUDA_TRY(cudaSetDevice(b->device));
+            CUDA_TRY(cudaMemcpyAsync(lo, o->lower, D * 8, cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaMemcpyAsync(hi, o->upper, D * 8, cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaStreamSynchronize(st));
+        }
+        for (int d = 0; d < D; ++d)
+            if (!(lo[d] <= hi[d])) return fail(GPE_ERR_INVALID, "lower[%d] > upper[%d] (or NaN)", d, d);
+    }
+    return GPE_OK;
+}
+
+// The streamed arrays of a host-resident solve: x0 and, when per point, obs and the prior means in; x, the optional
+// cost / grad / hess / cov and info (8 bytes a point: one double-wide column) out.
+struct SolveIo {
+    CallIo io;
+    int obs = -1, pm = -1, x = -1, cost = -1, grad = -1, hess = -1, cov = -1, info = -1;
+};
+
+SolveIo solve_io(int64_t D, int64_t K, const double* x0, const double* obs, int64_t obs_ld, const gpe_solve_opts& o, double* x,
+                 double* cost, double* grad, double* hess, double* cov, int32_t* info) {
+    SolveIo s;
+    s.io.in.add(x0, D);
+    if (obs_ld != 0) s.obs = s.io.in.add(obs, K);
+    if (o.prior_mean && o.prior_ld != 0) s.pm = s.io.in.add(o.prior_mean, D);
+    s.x = s.io.out.add(x, D);
+    if (cost) s.cost = s.io.out.add(cost, 1);
+    if (grad) s.grad = s.io.out.add(grad, D);
+    if (hess) s.hess = s.io.out.add(hess, D * D);
+    if (cov) s.cov = s.io.out.add(cov, D * D);
+    s.info = s.io.out.add(info, 1);
+    return s;
+}
+
+// Host-resident solve through the bank's pipeline (caller holds b->host_mu): the small per-call operands (shared
+// observation, weights, bounds, shared prior mean, precision) are uploaded once, then every chunk is solved by
+// bank_solve_device as its chunk launch.  A chunk's solve blocks this pipeline's thread until it has finished.
+int bank_solve_stream(gpe_bank* b, bool spectra, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                      const gpe_solve_opts& o, const SolveIo& s, const SharedCall* shared = nullptr) {
+    const int64_t D = b->D, K = spectra ? b->W : b->E;
+    struct Part { const double* src; int64_t n; double* dev; };
+    Part parts[] = {{obs_ld == 0 ? obs : nullptr, K, nullptr}, {weights, K, nullptr}, {o.lower, D, nullptr},
+                    {o.upper, D, nullptr}, {o.prior_ld == 0 ? o.prior_mean : nullptr, D, nullptr}, {o.prior_prec, D * D, nullptr}};
+    size_t total = 0;
+    for (const Part& p : parts) if (p.src) total += (size_t)p.n;
+    if (total > 0) {
+        int rc = ensure_buf((void**)&b->d_aux, &b->aux_cap, total * 8, false);
+        if (rc) return rc;
+        double* at = b->d_aux;
+        for (Part& p : parts) {
+            if (!p.src) continue;
+            CUDA_TRY(cudaMemcpyAsync(at, p.src, (size_t)p.n * 8, cudaMemcpyHostToDevice, cudaStreamLegacy));
+            p.dev = at;
+            at += p.n;
+        }
+        // The chunks run on the slots' non-blocking streams, which are not ordered after the legacy stream, and a copy from
+        // pageable memory may return before its DMA has landed: wait for the copies here.
+        CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));
+    }
+    const LmProblem pb = lm_problem((int)D, o, parts[2].dev, parts[3].dev, parts[4].dev, 0, parts[5].dev);
+    return stream_call(b->slots, b->device, b->models[0]->sms, s.io, N, 8, shared,
+                       [&](int64_t, int64_t n, void* const* di, void* const* dout, cudaStream_t st) {
+                           LmProblem p = pb;
+                           if (s.pm >= 0) { p.prior_mean = (const double*)di[s.pm]; p.prior_ld = D; }
+                           auto out = [&](int k) { return k >= 0 ? (double*)dout[k] : nullptr; };
+                           return bank_solve_device(b, spectra ? bank_forward_cost_device : bank_cost_device, K, p,
+                                                    (const double*)di[0], n, s.obs >= 0 ? (const double*)di[s.obs] : parts[0].dev,
+                                                    obs_ld != 0 ? K : 0, parts[1].dev, out(s.x), out(s.cost), out(s.grad),
+                                                    out(s.hess), out(s.cov), (int32_t*)dout[s.info], st, N);
+                       });
+}
+
 int bank_check_outputs(gpe_bank* b, int64_t N, const double* testing, double*& mu, double*& var, double*& deriv, double*& hess,
                        double*& fwd, double*& deriv_full, unsigned flags) {
     if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
@@ -1776,6 +1953,9 @@ int gpe_bank_destroy(gpe_bank* b) {
     if (b->aux_ready) cudaEventDestroy(b->aux_ready);
     if (b->cost_d) cudaFree(b->cost_d);
     if (b->cost_free) cudaEventDestroy(b->cost_free);
+    if (b->solve_d) cudaFree(b->solve_d);
+    if (b->solve_count) cudaFreeHost(b->solve_count);
+    if (b->solve_ev) cudaEventDestroy(b->solve_ev);
     delete b;
     return GPE_OK;
 }
@@ -1870,6 +2050,26 @@ int gpe_bank_forward_cost_host_ex(gpe_bank* b, const double* testing, int64_t N,
 int gpe_bank_forward_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                                const double* weights, double* cost, double* grad) {
     return gpe_bank_forward_cost_host_ex(b, testing, N, obs, obs_ld, weights, cost, grad, nullptr);
+}
+
+int gpe_bank_solve(gpe_bank* b, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                   const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess, double* cov,
+                   int32_t* info, unsigned flags, void* stream) {
+    NvtxRange nvtx_range("gpe_bank_solve");
+    const bool host = flags & GPE_HOST_PTRS, spectra = flags & GPE_SOLVE_SPECTRA;
+    gpe_solve_opts o;
+    int rc = solve_check(b, N, x0, obs, obs_ld, opts, x, info, flags, host, (cudaStream_t)stream, &o);
+    if (rc || N == 0) return rc;
+    CUDA_TRY(cudaSetDevice(b->device));
+    const int64_t D = b->D, K = spectra ? b->W : b->E;
+    if (host) {
+        std::lock_guard<std::mutex> lock(b->host_mu);
+        return bank_solve_stream(b, spectra, N, obs, obs_ld, weights, o,
+                                 solve_io(D, K, x0, obs, obs_ld, o, x, cost, grad, hess, cov, info));
+    }
+    const LmProblem pb = lm_problem((int)D, o, o.lower, o.upper, o.prior_mean, o.prior_ld, o.prior_prec);
+    return bank_solve_device(b, spectra ? bank_forward_cost_device : bank_cost_device, K, pb, x0, N, obs, obs_ld, weights, x,
+                             cost, grad, hess, cov, info, (cudaStream_t)stream, N);
 }
 
 int gpe_bank_project(gpe_bank* b, const double* mu, const double* deriv, int64_t N, double* fwd, double* deriv_full,
@@ -2036,6 +2236,22 @@ int gpe_multi_bank_forward_cost_ex(gpe_multi* mm, const double* testing, int64_t
 int gpe_multi_bank_forward_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                                 const double* weights, double* cost, double* grad) {
     return gpe_multi_bank_forward_cost_ex(mm, testing, N, obs, obs_ld, weights, cost, grad, nullptr);
+}
+
+int gpe_multi_bank_solve(gpe_multi* mm, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                         const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess, double* cov,
+                         int32_t* info, unsigned flags) {
+    NvtxRange nvtx_range("gpe_multi_bank_solve");
+    if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
+    gpe_bank* b0 = mm->banks[0];
+    const bool spectra = flags & GPE_SOLVE_SPECTRA;
+    gpe_solve_opts o;
+    int rc = solve_check(b0, N, x0, obs, obs_ld, opts, x, info, flags, true, nullptr, &o);
+    if (rc || N == 0) return rc;
+    const SolveIo s = solve_io(b0->D, spectra ? b0->W : b0->E, x0, obs, obs_ld, o, x, cost, grad, hess, cov, info);
+    return fan_out(mm, mm->banks, b0->models[0]->sms, s.io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
+        return bank_solve_stream(b, spectra, N, obs, obs_ld, weights, o, s, shared);
+    });
 }
 
 }  // extern "C"

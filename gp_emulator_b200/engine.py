@@ -586,6 +586,91 @@ class DeviceBank(_Handle):
                         addr(out.get("grad")), addr(out.get("hess")), _current_stream_ptr(self.device)))
         return out
 
+    def invert(self, x0, obs, weights=None, lower=None, upper=None, prior_mean=None, prior_precision=None,
+               max_iter=_lib.SOLVE_DEFAULT_MAX_ITER, ftol=1e-10, xtol=1e-10, gtol=0.0, lambda0=1e-3, want_cov=False):
+        """Per point, the inputs that minimise the band cost of ``cost`` plus an optional Gaussian prior,
+        ``f(x) = cost(x) + 1/2 (x - prior_mean)^T prior_precision (x - prior_mean)``, inside the box ``lower <= x <= upper``:
+        bounded Levenberg-Marquardt on the exact Hessian, every iteration on the device (``gpe_bank_solve``; the
+        algorithm and the stopping tests are stated in include/gpemu.h).
+
+        ``x0`` (N, D) starting points; ``obs`` (E,) or (N, E); ``weights`` (E,) or None; ``lower`` / ``upper`` (D,) or
+        None (entries may be infinite); ``prior_mean`` (D,) or (N, D), ``prior_precision`` (D, D).  Returns a dict:
+        ``x`` (N, D), ``cost`` (N,), ``grad`` (N, D) and ``hess`` (N, D, D) at x (prior included), ``cov`` (N, D, D) =
+        inv(hess) with ``want_cov`` (NaN where hess is not positive definite), ``status`` (N,) int32 (``SOLVE_*`` of
+        ``_lib``) and ``n_iter`` (N,) int32, the evaluations after the first.  numpy in -> numpy out (all devices of the
+        bank); torch CUDA in -> torch CUDA out (single-device banks; the call returns when the results are written)."""
+        return self._solve(False, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
+                           lambda0, want_cov)
+
+    def forward_invert(self, x0, obs, weights=None, lower=None, upper=None, prior_mean=None, prior_precision=None,
+                       max_iter=_lib.SOLVE_DEFAULT_MAX_ITER, ftol=1e-10, xtol=1e-10, gtol=0.0, lambda0=1e-3,
+                       want_cov=False):
+        """``invert`` with the spectrum cost of ``forward_cost``: ``obs`` (W,) or (N, W), ``weights`` (W,) or None."""
+        if self.W == 0:
+            raise GpemuError("bank has no basis functions to project onto")
+        return self._solve(True, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
+                           lambda0, want_cov)
+
+    def _solve(self, spectra, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
+               lambda0, want_cov):
+        D, K = self.D, (self.W if spectra else self.E)
+        lib = _lib.load()
+        dev = _is_torch(x0)
+        if dev:
+            if self.multi:
+                raise ValueError("a multi-device bank takes host arrays; use one DeviceBank per device for CUDA tensors")
+            import torch
+            tdev = torch.device("cuda", self.device)
+            arr = lambda a: None if a is None else torch.as_tensor(
+                a if _is_torch(a) else np.asarray(a, dtype=np.float64), dtype=torch.float64, device=tdev).contiguous()
+            shape = lambda a: tuple(a.shape)
+            empty = lambda *s: torch.empty(*s, dtype=torch.float64, device=tdev)
+            info_empty = lambda n: torch.empty(n, 2, dtype=torch.int32, device=tdev)
+        else:
+            arr = lambda a: None if a is None else f64c(a.cpu().numpy() if _is_torch(a) else a)
+            shape = lambda a: a.shape
+            empty = np.empty
+            info_empty = lambda n: np.empty((n, 2), dtype=np.int32)
+        x0 = arr(x0)
+        if len(shape(x0)) != 2 or shape(x0)[1] != D:
+            raise ValueError(f"x0 must be (N, {D})")
+        N = shape(x0)[0]
+        o = arr(obs)
+        if shape(o) == (K,):
+            obs_ld = 0
+        elif shape(o) == (N, K):
+            obs_ld = K
+        else:
+            raise ValueError(f"obs must be ({K},) or ({N}, {K})")
+        wt, lo, hi, pm, pp = (arr(a) for a in (weights, lower, upper, prior_mean, prior_precision))
+        for name, a, want in (("weights", wt, (K,)), ("lower", lo, (D,)), ("upper", hi, (D,)),
+                              ("prior_precision", pp, (D, D))):
+            if a is not None and shape(a) != want:
+                raise ValueError(f"{name} must be {want}")
+        prior_ld = 0
+        if pm is not None:
+            if shape(pm) == (N, D):
+                prior_ld = D
+            elif shape(pm) != (D,):
+                raise ValueError(f"prior_mean must be ({D},) or ({N}, {D})")
+        opts = _lib.SolveOpts(int(max_iter), float(ftol), float(xtol), float(gtol), float(lambda0), addr(lo), addr(hi),
+                              addr(pm), prior_ld, addr(pp))
+        out = {"x": empty((N, D)), "cost": empty(N), "grad": empty((N, D)), "hess": empty((N, D, D))}
+        if want_cov:
+            out["cov"] = empty((N, D, D))
+        info = info_empty(N)
+        flags = _lib.SOLVE_SPECTRA if spectra else 0
+        args = (addr(x0), N, addr(o), obs_ld, addr(wt), C.byref(opts), addr(out["x"]), addr(out["cost"]),
+                addr(out["grad"]), addr(out["hess"]), addr(out.get("cov")), addr(info))
+        if dev:
+            check(lib.gpe_bank_solve(self._h, *args, flags, _current_stream_ptr(self.device)))
+        elif self.multi:
+            check(lib.gpe_multi_bank_solve(self._h, *args, flags))
+        else:
+            check(lib.gpe_bank_solve(self._h, *args, flags | HOST_PTRS, None))
+        out["status"], out["n_iter"] = info[:, 0], info[:, 1]
+        return out
+
     def forward(self, testing, want_deriv=True):
         """numpy (N, D) -> fwd (N, W) [, deriv_full (N, D, W)]: one call, nothing but the spectra (and Jacobians)
         crosses PCIe.  This is what ``MultivariateEmulator.predict`` (reference multivariate_gp.py:195-222) runs on."""

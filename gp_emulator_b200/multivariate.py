@@ -188,6 +188,35 @@ class MultivariateEmulator(object):
             res = [float(c[0]) if isinstance(c, np.ndarray) else c[0]] + [a[0] for a in res[1:]]
         return tuple(res) if len(res) > 1 else res[0]
 
+    def invert(self, obs, y0, weights=None, bounds=None, prior=None, max_iter=50, ftol=1e-10, xtol=1e-10, gtol=0.0,
+               do_cov=True):
+        """Retrieve the parameters whose reconstructed output best fits ``obs``: per point, the minimiser of ``cost``
+        (plus ``1/2 (y - m)^T P (y - m)`` with ``prior = (m, P)``) inside ``bounds = (lower, upper)``, by bounded
+        Levenberg-Marquardt on the exact Hessian with every iteration on the device (``DeviceBank.forward_invert``).
+        With weights 1 / sigma^2 the cost is a negative log-likelihood and ``cov = inv(hess)`` at the optimum is the
+        Laplace approximation of the posterior covariance.
+
+        ``y0`` (N_params,) or (N, N_params) starting points; ``obs`` (N_full,) shared or (N, N_full) one per point;
+        ``lower`` / ``upper`` (N_params,) or None; ``m`` (N_params,) or (N, N_params), ``P`` (N_params, N_params).
+        Returns a dict ``x``, ``cost``, ``grad``, ``hess``, ``cov`` (with ``do_cov``), ``status``, ``n_iter`` -- one point:
+        ``(N_params,)``, ``float``, ``(N_params,)``, ``(N_params, N_params)``, ..., ``int``, ``int``; N points: the same with
+        a leading N.  Host arrays or CUDA tensors, as ``predict``."""
+        bank = self._device_bank()
+        if isinstance(y0, np.ndarray) or not hasattr(y0, "is_cuda"):
+            y2 = np.atleast_2d(y0)
+        else:
+            y2 = y0 if y0.dim() == 2 else y0.reshape(1, -1)
+        lower, upper = bounds if bounds is not None else (None, None)
+        m, P = prior if prior is not None else (None, None)
+        out = bank.forward_invert(y2, obs, weights, lower=lower, upper=upper, prior_mean=m, prior_precision=P,
+                                  max_iter=max_iter, ftol=ftol, xtol=xtol, gtol=gtol, want_cov=do_cov)
+        if y2.shape[0] == 1:
+            one = {k: v[0] for k, v in out.items()}
+            for k in ("cost", "status", "n_iter"):
+                one[k] = (float if k == "cost" else int)(one[k]) if isinstance(one[k], np.generic) else one[k]
+            return one
+        return out
+
     def predict_pcs(self, y, do_unc=True, do_deriv=True):
         """PC-space outputs for N points: dict with mu (N, P), var (N, P), deriv (N, P, D)."""
         return self._device_bank().predict(np.atleast_2d(y), want_var=do_unc, want_deriv=do_deriv)

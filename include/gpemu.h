@@ -238,6 +238,62 @@ int gpe_multi_bank_cost_ex(gpe_multi* mm, const double* testing, int64_t N, cons
 int gpe_multi_bank_forward_cost_ex(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                                    const double* weights, double* cost, double* grad, double* hess);
 
+/* Inversion: per point, the x in the box lower <= x <= upper that minimises
+ *   f(x) = cost(x) + 1/2 (x - m)^T P (x - m)
+ * where cost is the band cost of gpe_bank_cost_ex (default) or, with GPE_SOLVE_SPECTRA, the spectrum cost of
+ * gpe_bank_forward_cost_ex, and the Gaussian prior (mean m, precision P) is optional.  g = grad + P (x - m) and
+ * H = hess + P.  Levenberg-Marquardt on the exact Hessian, every point independently:
+ *   1. x = clip(x0, lower, upper); evaluate f, g, H there; lambda = lambda0, nu = 2.
+ *   2. Free set F: every d except those with x_d = lower_d, g_d > 0 or x_d = upper_d, g_d < 0.  Solve
+ *      (H_FF + lambda diag(s_F)) delta_F = -g_F by Cholesky, s_d = max(|H_dd|, 1e-12 max_{k in F} |H_kk|); while the
+ *      factorisation fails (H may be indefinite away from the optimum): lambda *= nu, nu *= 2.
+ *   3. x_t = clip(x + delta), delta' = x_t - x, pred = -(g^T delta' + 1/2 delta'^T H delta').
+ *   4. Evaluate f_t, g_t, H_t at x_t; rho = (f - f_t) / pred.  f_t < f and rho > 0: accept x_t,
+ *      lambda *= max(1/3, 1 - (2 rho - 1)^3), nu = 2.  Otherwise lambda *= nu, nu *= 2.
+ * The point stops with (tests in this order after each evaluation: f at x0, ftol, gtol, lambda, xtol, max_iter)
+ *   GPE_SOLVE_NONFINITE  f is not finite at clip(x0): returned there, with what was evaluated there;
+ *   GPE_SOLVE_CONVERGED  an accepted step changed f by at most ftol |f|, or max_F |g_F| <= gtol, or the proposed
+ *                        max |delta'| <= xtol (max |x| + xtol);
+ *   GPE_SOLVE_STALLED    lambda passed 1e20 (failed factorisations and rejected steps both raise it) before a step
+ *                        could be formed;
+ *   GPE_SOLVE_MAX_ITER   max_iter evaluations after the first were used.
+ * Outputs at the returned x (prior included): x (N, D); cost (N), grad (N, D), hess (N, D, D) or NULL; cov (N, D, D) =
+ * inv(H) without damping, symmetric bit for bit, NaN where H is not positive definite, or NULL; info (N, 2) =
+ * (status, evaluations after the first).
+ * Arguments: x0 (N, D); obs and weights as the cost call (obs (N, K) with obs_ld >= K, or (K) with obs_ld = 0; K = E, or
+ * W with GPE_SOLVE_SPECTRA; weights (K) or NULL); opts NULL takes the defaults below.  lower / upper (D) or NULL (no
+ * bound; entries may be -inf / +inf); prior_mean (N, D) rows prior_ld >= D apart, one (D) row with prior_ld = 0, or NULL
+ * (0); prior_prec (D, D), symmetric, or NULL (no prior; a prior_mean then is an error).
+ * Every array follows the call's placement: device pointers on the bank's device, or host pointers with GPE_HOST_PTRS
+ * (host obs_ld = K or 0, host prior_ld = D or 0).  The call is SYNCHRONOUS even with device pointers: it reads the number
+ * of points still active once per iteration.  Iterations stay on the device and converged points are not evaluated again.
+ * Results do not depend on chunking, pointer placement, the device count or the order of the points.
+ * D <= 32; the spectrum cost takes banks of up to 96 emulators (GPE_ERR_UNSUPPORTED beyond). */
+#define GPE_SOLVE_SPECTRA 0x1000u   /* spectrum cost (needs a basis); default: band cost */
+#define GPE_SOLVE_MAX_D 32
+#define GPE_SOLVE_CONVERGED 0
+#define GPE_SOLVE_MAX_ITER 1
+#define GPE_SOLVE_STALLED 2
+#define GPE_SOLVE_NONFINITE 3
+#define GPE_SOLVE_DEFAULT_MAX_ITER 50
+typedef struct gpe_solve_opts {
+    int max_iter;          /* >= 0 (default 50) */
+    double ftol, xtol, gtol;   /* >= 0 (defaults 1e-10, 1e-10, 0) */
+    double lambda0;        /* > 0 (default 1e-3) */
+    const double* lower;
+    const double* upper;
+    const double* prior_mean;
+    int64_t prior_ld;
+    const double* prior_prec;
+} gpe_solve_opts;
+int gpe_bank_solve(gpe_bank* b, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                   const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess, double* cov,
+                   int32_t* info, unsigned flags, void* stream);
+/* The same on every device of a bank handle; host arrays (GPE_HOST_PTRS is implied). */
+int gpe_multi_bank_solve(gpe_multi* mm, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                         const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess, double* cov,
+                         int32_t* info, unsigned flags);
+
 /* PCA back-projection of bank means: fwd (N, W) = mu (N, E) @ basis (E, W)
  * (the accumulation `fwd += pred_mu * basis_functions[i]`, gp_emulator/multivariate_gp.py:216, batched
  * over N points), and optionally deriv_full (N, D, W) = sum_e deriv[n, e, d] * basis[e, w] (:218).
