@@ -8,7 +8,7 @@ BUILD     := build/obj
 DPS       := 2 4 6 8 10 12 16 24 32
 LIB       := gp_emulator_b200/libgpemu.so
 
-OBJS := $(BUILD)/gpemu.o $(BUILD)/project.o $(BUILD)/invert.o $(BUILD)/peaks.o $(BUILD)/var_large.o $(BUILD)/tf32.o $(BUILD)/train.o $(foreach d,$(DPS),$(BUILD)/inst_dp$(d).o)
+OBJS := $(BUILD)/gpemu.o $(BUILD)/project.o $(BUILD)/invert.o $(BUILD)/search.o $(BUILD)/peaks.o $(BUILD)/var_large.o $(BUILD)/tf32.o $(BUILD)/train.o $(foreach d,$(DPS),$(BUILD)/inst_dp$(d).o)
 HDRS := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) include/gpemu.h
 
 all: $(LIB)
@@ -27,6 +27,9 @@ $(BUILD)/project.o: $(CSRC)/project.cu $(HDRS) | $(BUILD)
 
 $(BUILD)/invert.o: $(CSRC)/invert.cu $(HDRS) | $(BUILD)
 	$(NVCC) $(NVFLAGS) -Xptxas -v -c $< -o $@ 2> $(BUILD)/invert.ptxas.log || (cat $(BUILD)/invert.ptxas.log; exit 1)
+
+$(BUILD)/search.o: $(CSRC)/search.cu $(HDRS) | $(BUILD)
+	$(NVCC) $(NVFLAGS) -Xptxas -v -c $< -o $@ 2> $(BUILD)/search.ptxas.log || (cat $(BUILD)/search.ptxas.log; exit 1)
 
 $(BUILD)/var_large.o: $(CSRC)/predict_var_large.cu $(HDRS) | $(BUILD)
 	$(NVCC) $(NVFLAGS) -Xptxas -v -c $< -o $@ 2> $(BUILD)/var_large.ptxas.log || (cat $(BUILD)/var_large.ptxas.log; exit 1)

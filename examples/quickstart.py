@@ -50,20 +50,31 @@ def main():
     truth = toy_model(y_test, wl)
     print("batch of %d: rms emulation error %.2e (signal rms %.2f)" % (len(y_test), np.sqrt(np.mean((fwd_all - truth) ** 2)),
                                                                        np.sqrt(np.mean(truth ** 2))))
-    noise = np.random.RandomState(1).standard_normal(len(wl))                # 3b. spectrum misfit
-    cost, grad = emu.cost(y_test, truth[3] + 0.01 * noise)                   # spectra and Jacobians stay in the kernel
-    best = int(np.argmin(cost))
-    print("misfit of 1000 candidates against one observed spectrum: best candidate %d (cost %.3f), true one is 3 "
-          "(cost %.3f); gradients %s" % (best, cost[best], cost[3], grad.shape))
+    noise = np.random.RandomState(1).standard_normal(len(wl))                # 3b. look-up-table search
+    obs_lut = truth + 0.01 * noise                                            # 1000 observed spectra, one call:
+    found = emu.search(obs_lut, candidates=y_test, k=3)                       # the 3 best of 1000 candidates per pixel
+    print("look-up table: %d of %d pixels pick their own candidate first; pixel 3: candidates %s, costs %s" % (
+        int(np.sum(found["idx"][:, 0] == np.arange(len(obs_lut)))), len(obs_lut), found["idx"][3].tolist(),
+        np.round(found["cost"][3], 3).tolist()))
     sigma = 0.01                                                              # 3c. inversion + Laplace uncertainty
     obs = truth + sigma * np.random.RandomState(2).standard_normal(truth.shape)   # one noisy spectrum per pixel
     lower, upper = np.array([d.ppf(0.0) for d in dists]), np.array([d.ppf(1.0) for d in dists])
-    y0 = np.tile(0.5 * (lower + upper), (len(obs), 1))
-    t0 = time.perf_counter()                                                  # weights 1 / sigma^2: cost = -log likelihood
-    res = emu.invert(obs, y0, weights=np.full(len(wl), 1.0 / sigma ** 2), bounds=(lower, upper))
+    w = np.full(len(wl), 1.0 / sigma ** 2)                                    # weights 1 / sigma^2: cost = -log likelihood
+    state = np.random.get_state()                                             # (later steps keep their draws)
+    np.random.seed(3)
+    table = gpe.lhd(dist=dists, size=2000)                                    # starts: the 4 best rows of a seeded table
+    np.random.set_state(state)
+    t0 = time.perf_counter()
+    res = emu.invert(obs, weights=w, bounds=(lower, upper), candidates=table, n_starts=4)
+    t_seeded = time.perf_counter() - t0
+    t0 = time.perf_counter()
+    mid = emu.invert(obs, np.tile(0.5 * (lower + upper), (len(obs), 1)), weights=w, bounds=(lower, upper))
+    t_mid = time.perf_counter() - t0
+    print("inverted %d spectra from the table in %.3f s (from the box centre: %.3f s); median cost %.1f (box centre: "
+          "%.1f); status counts %s (converged, max_iter, stalled, nonfinite)" % (
+        len(obs), t_seeded, t_mid, np.median(res["cost"]), np.median(mid["cost"]),
+        np.bincount(res["status"], minlength=4).tolist()))
     sd = np.sqrt(np.diagonal(res["cov"], axis1=1, axis2=2))
-    print("inverted %d spectra in %.3f s, status counts %s (converged, max_iter, stalled, nonfinite)" % (
-        len(obs), time.perf_counter() - t0, np.bincount(res["status"], minlength=4).tolist()))
     print("pixel 3: retrieved %s +- %s (Laplace sd), truth %s; %.0f%% of all retrieved parameters lie within 3 sd of "
           "the truth" % (np.round(res["x"][3], 4), np.round(sd[3], 4), np.round(y_test[3], 4),
                          100 * np.mean(np.abs(res["x"] - y_test) <= 3 * sd)))

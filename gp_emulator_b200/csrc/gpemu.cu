@@ -161,6 +161,12 @@ struct gpe_bank {
     size_t solve_cap = 0;
     int* solve_count = nullptr;        // page-locked
     cudaEvent_t solve_ev = nullptr;
+    // gpe_bank_search: candidate table and per-pixel scratch (one search at a time per bank), handed between streams
+    // through search_free
+    std::mutex search_mu;
+    void* search_d = nullptr;
+    size_t search_cap = 0;
+    cudaEvent_t search_free = nullptr;
 };
 
 struct gpe_multi {
@@ -1492,6 +1498,160 @@ int forward_cost_check(gpe_bank* b, int64_t N, const double* testing, const doub
     return GPE_OK;
 }
 
+// ---- candidate search (DESIGN 4.6e): kernels in search.cu ---------------------------------------------------------
+// The search scratch of a call: the candidate table (built once per call) followed by the per-pixel work area of at most
+// P pixels at a time.
+constexpr int64_t kSearchRows = 1 << 16;
+struct SearchScratch {
+    int Kp = 0, gy = 1;
+    int64_t P = 0;
+    double *tbl = nullptr, *ta = nullptr, *mu = nullptr, *aux = nullptr, *C = nullptr;   // table (aux, C: spectrum cost)
+    double *s = nullptr, *zeros = nullptr, *pv = nullptr, *x = nullptr, *cst = nullptr;   // pixels
+    int* pi = nullptr;
+    int64_t* sel = nullptr;
+};
+
+// Lay out and grow the bank's search scratch for a call of call_N pixels (caller holds search_mu).
+int search_prepare(gpe_bank* b, bool spectra, int64_t K, int k, int64_t call_N, SearchScratch* sc) {
+    const int64_t E = b->E, D = b->D;
+    sc->Kp = search_pad(K);
+    sc->gy = search_split(call_N, K);
+    sc->P = std::min<int64_t>(kSearchRows, call_N);
+    const int64_t P = sc->P, gy = sc->gy;
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
+    const size_t o_tbl = carve(8 * (size_t)search_ks((int)E) * sc->Kp * 4), o_ta = carve(8 * (size_t)sc->Kp), o_mu = carve(8 * K * E);
+    const size_t o_aux = carve(spectra ? 16 * (size_t)b->Wp : 0), o_C = carve(spectra ? 8 * E * E : 0);
+    const size_t o_s = carve(8 * P * E), o_z = carve(spectra ? 8 * P * E : 0), o_sel = carve(8 * P * k);
+    const size_t o_pv = carve(gy > 1 ? 8 * gy * P * k : 0), o_pi = carve(gy > 1 ? 4 * gy * P * k : 0);
+    const size_t o_x = carve(8 * P * D), o_cst = carve(8 * P * k);
+    if (!b->search_free) CUDA_TRY(cudaEventCreateWithFlags(&b->search_free, cudaEventDisableTiming));
+    if (b->search_cap < off) CUDA_TRY(cudaEventSynchronize(b->search_free));   // the old scratch may still be in use
+    int rc = ensure_buf(&b->search_d, &b->search_cap, off, false);
+    if (rc) return rc;
+    char* base = (char*)b->search_d;
+    sc->tbl = (double*)(base + o_tbl); sc->ta = (double*)(base + o_ta); sc->mu = (double*)(base + o_mu);
+    sc->aux = spectra ? (double*)(base + o_aux) : nullptr; sc->C = spectra ? (double*)(base + o_C) : nullptr;
+    sc->s = (double*)(base + o_s); sc->zeros = spectra ? (double*)(base + o_z) : nullptr; sc->sel = (int64_t*)(base + o_sel);
+    sc->pv = (double*)(base + o_pv); sc->pi = (int*)(base + o_pi); sc->x = (double*)(base + o_x); sc->cst = (double*)(base + o_cst);
+    return GPE_OK;
+}
+
+// Candidate table on st: the bank means at the K candidates (one call of K points), a_k and the packed image; for the
+// spectrum cost also the padded weights / shared observation (aux) and C = basis . diag(l) . basis^T.
+int search_build_table(gpe_bank* b, const SearchScratch& sc, bool spectra, const double* cand, int64_t K, const double* weights,
+                       const double* obs1, cudaStream_t st) {
+    const int E = b->E;
+    int rc = bank_predict_device(b, cand, K, sc.mu, nullptr, nullptr, nullptr, st, K);
+    if (rc) return rc;
+    if (spectra) {
+        CUDA_TRY(forward_cost_aux(weights, obs1, b->W, b->Wp, sc.aux, st));
+        CUDA_TRY(forward_cost_curv(b->d_basis, sc.aux, E, b->Wp, sc.C, st));
+        CUDA_TRY(cudaMemsetAsync(sc.zeros, 0, (size_t)sc.P * E * 8, st));
+    }
+    CUDA_TRY(search_table(sc.mu, K, E, sc.Kp, spectra ? nullptr : weights, sc.C, sc.tbl, sc.ta, st));
+    return GPE_OK;
+}
+
+// Pixels [0, n) of a call of call_N pixels on st, P at a time: pixel operand s (spectrum cost: s of k_forward_cost at
+// fwd = 0, i.e. -basis . (l o obs)), top-k selection, then per slot j the exact cost of candidate sel[:, j] by the cost
+// call's own path (call_N: the same kernel plans as a cost call of the call's pixels), then the final order.
+int search_rows(gpe_bank* b, const SearchScratch& sc, bool spectra, const double* cand, int k, const double* obs, int64_t obs_ld,
+                const double* weights, int64_t n, int64_t call_N, int64_t* idx, double* cost, cudaStream_t st) {
+    const int E = b->E, D = b->D;
+    const CostDevice cost_device = spectra ? bank_forward_cost_device : bank_cost_device;
+    for (int64_t p0 = 0; p0 < n; p0 += sc.P) {
+        const int64_t m = std::min(sc.P, n - p0);
+        const double* o = obs + p0 * obs_ld;
+        if (spectra)
+            CUDA_TRY(forward_cost_rows(sc.zeros, nullptr, m, E, D, o, obs_ld, sc.aux, b->d_basis, b->W, b->Wp, 1, nullptr, nullptr,
+                                       nullptr, sc.s, st));
+        else
+            CUDA_TRY(search_band_s(o, obs_ld, weights, m, E, sc.s, st));
+        CUDA_TRY(search_topk(sc.s, m, E, sc.tbl, sc.ta, sc.Kp, k, sc.gy, sc.pv, sc.pi, sc.sel, st));
+        for (int j = 0; j < k; ++j) {
+            CUDA_TRY(search_gather(cand, D, sc.sel, k, j, m, sc.x, st));
+            int rc = cost_device(b, sc.x, m, o, obs_ld, weights, sc.cst + (int64_t)j * m, nullptr, nullptr, st, call_N);
+            if (rc) return rc;
+        }
+        CUDA_TRY(search_output(sc.sel, sc.cst, m, k, idx ? idx + p0 * k : nullptr, cost ? cost + p0 * k : nullptr, st));
+    }
+    return GPE_OK;
+}
+
+// Request check of the search calls (device: obs_ld = 0 or >= the observation width; host: 0 or equal to it).
+int search_check(gpe_bank* b, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld, int k,
+                 const int64_t* idx, const double* cost, unsigned flags, bool host) {
+    if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
+    if (flags & ~(GPE_SOLVE_SPECTRA | GPE_HOST_PTRS)) return fail(GPE_ERR_INVALID, "unknown flag bits 0x%x", flags);
+    const bool spectra = flags & GPE_SOLVE_SPECTRA;
+    if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
+    if (K < 1 || K > ((int64_t)1 << 30)) return fail(GPE_ERR_INVALID, "K must be in [1, 2^30] (got %lld)", (long long)K);
+    if (k < 1 || k > GPE_SEARCH_MAX_K || k > K)
+        return fail(GPE_ERR_INVALID, "k must be in [1, min(K, %d)] (got %d)", GPE_SEARCH_MAX_K, k);
+    if (spectra && !b->d_basis) return fail(GPE_ERR_INVALID, "bank was created without basis functions");
+    const int64_t Kw = spectra ? b->W : b->E;
+    if (obs_ld != 0 && (host ? obs_ld != Kw : obs_ld < Kw))
+        return fail(GPE_ERR_INVALID, "obs_ld must be 0 (one observation) or %s %s", host ? "=" : ">=", spectra ? "W" : "E");
+    if (!cand) return fail(GPE_ERR_INVALID, "cand is NULL");
+    if (N > 0 && !obs) return fail(GPE_ERR_INVALID, "obs is NULL");
+    if (!idx && !cost) return fail(GPE_ERR_INVALID, "no output requested");
+    if (search_smem(b->E) > kSmemMax || (spectra && forward_cost_smem(b->E) > kSmemMax) || b->E > 96)
+        return fail(GPE_ERR_UNSUPPORTED, "the search supports banks of up to 96 emulators (got %d)", b->E);
+    return GPE_OK;
+}
+
+// The streamed arrays of a host-resident search: per-point observations (unless shared) in; idx and cost (k 8-byte
+// columns each) out.
+CallIo search_io(int64_t Kw, const double* obs, int64_t obs_ld, int k, int64_t* idx, double* cost) {
+    CallIo io;
+    io.idx[0] = obs_ld != 0 ? io.in.add(obs, Kw) : -1;
+    io.idx[1] = idx ? io.out.add(idx, k) : -1;
+    io.idx[2] = cost ? io.out.add(cost, k) : -1;
+    return io;
+}
+
+// Host-resident search through the bank's pipeline (caller holds b->host_mu): the candidates and the shared operands are
+// uploaded and the table is built once per call, then every chunk of pixels is searched on its slot's stream.  The
+// chunks share the per-pixel scratch: each waits for the previous one through search_free.
+int bank_search_stream(gpe_bank* b, bool spectra, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                       const double* weights, int k, const CallIo& io, const SharedCall* shared = nullptr) {
+    const int64_t D = b->D, Kw = spectra ? b->W : b->E;
+    struct Part { const double* src; int64_t n; double* dev; };
+    Part parts[] = {{cand, K * D, nullptr}, {obs_ld == 0 ? obs : nullptr, Kw, nullptr}, {weights, Kw, nullptr}};
+    size_t total = 0;
+    for (const Part& p : parts) if (p.src) total += ((size_t)p.n + 31) & ~(size_t)31;
+    int rc = ensure_buf((void**)&b->d_aux, &b->aux_cap, total * 8, false);
+    if (rc) return rc;
+    double* at = b->d_aux;
+    for (Part& p : parts) {
+        if (!p.src) continue;
+        CUDA_TRY(cudaMemcpyAsync(at, p.src, (size_t)p.n * 8, cudaMemcpyHostToDevice, cudaStreamLegacy));
+        p.dev = at;
+        at += ((size_t)p.n + 31) & ~(size_t)31;
+    }
+    std::lock_guard<std::mutex> lock(b->search_mu);
+    SearchScratch sc;
+    rc = search_prepare(b, spectra, K, k, N, &sc);
+    if (rc) return rc;
+    CUDA_TRY(cudaStreamWaitEvent(cudaStreamLegacy, b->search_free, 0));
+    rc = search_build_table(b, sc, spectra, parts[0].dev, K, parts[2].dev, parts[1].dev, cudaStreamLegacy);
+    if (rc) return rc;
+    CUDA_TRY(cudaEventRecord(b->search_free, cudaStreamLegacy));
+    // (a copy from pageable memory may return before its DMA has landed: the chunks' streams are not ordered after the
+    // legacy stream, the event orders them)
+    return stream_call(b->slots, b->device, b->models[0]->sms, io, N, 8, shared,
+                       [&](int64_t, int64_t n, void* const* di, void* const* dout, cudaStream_t st) -> int {
+                           CUDA_TRY(cudaStreamWaitEvent(st, b->search_free, 0));
+                           const double* o = obs_ld != 0 ? io.at<const double>(di, 0) : parts[1].dev;
+                           int r = search_rows(b, sc, spectra, parts[0].dev, k, o, obs_ld != 0 ? Kw : 0, parts[2].dev, n, N,
+                                               io.at<int64_t>(dout, 1), io.at<double>(dout, 2), st);
+                           if (r) return r;
+                           CUDA_TRY(cudaEventRecord(b->search_free, st));
+                           return GPE_OK;
+                       });
+}
+
 // ---- inversion (DESIGN 4.6d): bounded Levenberg-Marquardt, kernels in invert.cu ------------------------------------
 // Solve of N points on `st` (device arrays), in sub-chunks whose solver scratch stays within 256 MB.  Each iteration
 // evaluates the active trial points with the call's cost (cost, gradient and Hessian; call_N: the kernel plans follow the
@@ -1956,6 +2116,8 @@ int gpe_bank_destroy(gpe_bank* b) {
     if (b->solve_d) cudaFree(b->solve_d);
     if (b->solve_count) cudaFreeHost(b->solve_count);
     if (b->solve_ev) cudaEventDestroy(b->solve_ev);
+    if (b->search_d) cudaFree(b->search_d);
+    if (b->search_free) cudaEventDestroy(b->search_free);
     delete b;
     return GPE_OK;
 }
@@ -2070,6 +2232,31 @@ int gpe_bank_solve(gpe_bank* b, const double* x0, int64_t N, const double* obs, 
     const LmProblem pb = lm_problem((int)D, o, o.lower, o.upper, o.prior_mean, o.prior_ld, o.prior_prec);
     return bank_solve_device(b, spectra ? bank_forward_cost_device : bank_cost_device, K, pb, x0, N, obs, obs_ld, weights, x,
                              cost, grad, hess, cov, info, (cudaStream_t)stream, N);
+}
+
+int gpe_bank_search(gpe_bank* b, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                    const double* weights, int k, int64_t* idx, double* cost, unsigned flags, void* stream) {
+    NvtxRange nvtx_range("gpe_bank_search");
+    const bool host = flags & GPE_HOST_PTRS, spectra = flags & GPE_SOLVE_SPECTRA;
+    int rc = search_check(b, cand, K, obs, N, obs_ld, k, idx, cost, flags, host);
+    if (rc || N == 0) return rc;
+    CUDA_TRY(cudaSetDevice(b->device));
+    if (host) {
+        std::lock_guard<std::mutex> lock(b->host_mu);
+        return bank_search_stream(b, spectra, cand, K, obs, N, obs_ld, weights, k,
+                                  search_io(spectra ? b->W : b->E, obs, obs_ld, k, idx, cost));
+    }
+    const cudaStream_t st = (cudaStream_t)stream;
+    std::lock_guard<std::mutex> lock(b->search_mu);
+    SearchScratch sc;
+    rc = search_prepare(b, spectra, K, k, N, &sc);
+    if (rc) return rc;
+    CUDA_TRY(cudaStreamWaitEvent(st, b->search_free, 0));
+    rc = search_build_table(b, sc, spectra, cand, K, weights, obs_ld == 0 ? obs : nullptr, st);
+    if (rc == GPE_OK) rc = search_rows(b, sc, spectra, cand, k, obs, obs_ld, weights, N, N, idx, cost, st);
+    if (rc) return rc;
+    CUDA_TRY(cudaEventRecord(b->search_free, st));
+    return GPE_OK;
 }
 
 int gpe_bank_project(gpe_bank* b, const double* mu, const double* deriv, int64_t N, double* fwd, double* deriv_full,
@@ -2251,6 +2438,21 @@ int gpe_multi_bank_solve(gpe_multi* mm, const double* x0, int64_t N, const doubl
     const SolveIo s = solve_io(b0->D, spectra ? b0->W : b0->E, x0, obs, obs_ld, o, x, cost, grad, hess, cov, info);
     return fan_out(mm, mm->banks, b0->models[0]->sms, s.io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
         return bank_solve_stream(b, spectra, N, obs, obs_ld, weights, o, s, shared);
+    });
+}
+
+int gpe_multi_bank_search(gpe_multi* mm, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                          const double* weights, int k, int64_t* idx, double* cost, unsigned flags) {
+    NvtxRange nvtx_range("gpe_multi_bank_search");
+    if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
+    gpe_bank* b0 = mm->banks[0];
+    const bool spectra = flags & GPE_SOLVE_SPECTRA;
+    int rc = search_check(b0, cand, K, obs, N, obs_ld, k, idx, cost, flags, true);
+    if (rc || N == 0) return rc;
+    const CallIo io = search_io(spectra ? b0->W : b0->E, obs, obs_ld, k, idx, cost);
+    // every device builds its own, identical candidate table
+    return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
+        return bank_search_stream(b, spectra, cand, K, obs, N, obs_ld, weights, k, io, shared);
     });
 }
 

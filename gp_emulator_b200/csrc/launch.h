@@ -80,6 +80,28 @@ size_t forward_cost_smem(int E);   // dynamic shared memory of forward_cost_rows
 // Column split gy of forward_cost_rows for a call of call_N points: > 1 (the column groups spread over gy CTAs per row tile,
 // partial sums in part (gy, R, 1 + E)) when the row tiles alone leave most SMs idle.  A function of the call, not of a chunk.
 int forward_cost_split(int64_t call_N, int W);
+// ---- candidate search (search.cu, DESIGN 4.6e) ----
+// k-steps of 4 emulators the table of a bank of E emulators is packed with; dynamic shared memory of search_topk; K rounded
+// up to whole 128-candidate groups
+int search_ks(int E);
+size_t search_smem(int E);
+int search_pad(int64_t K);
+// Candidate split gy of search_topk for a call of call_N pixels: > 1 (the candidate groups spread over gy CTAs per pixel
+// tile, partial lists in part (gy, R, k)) when the pixel tiles alone leave most SMs idle.  A function of the call.
+int search_split(int64_t call_N, int64_t K);
+// tbl [search_ks(E)][Kp][4] and ta (Kp) from the means mu (K, E): band cost with weights w (NULL: 1) when C == NULL,
+// spectrum cost with C (E, E) otherwise
+cudaError_t search_table(const double* mu, int64_t K, int E, int Kp, const double* w, const double* C, double* tbl, double* ta,
+                         cudaStream_t st);
+// Band-cost pixel operand s (R, E) = -(w o obs)
+cudaError_t search_band_s(const double* obs, int64_t obs_ld, const double* w, int64_t R, int E, double* s, cudaStream_t st);
+// sel (R, k): per row the k candidates of the smallest a_k + s_r . m_k, in (score, index) order, -1 where none is left
+cudaError_t search_topk(const double* s, int64_t R, int E, const double* tbl, const double* ta, int Kp, int k, int gy,
+                        double* part_v, int* part_i, int64_t* sel, cudaStream_t st);
+// x (R, D) = cand rows sel[:, j] (row 0 for -1)
+cudaError_t search_gather(const double* cand, int D, const int64_t* sel, int k, int j, int64_t R, double* x, cudaStream_t st);
+// idx / cost (R, k), either may be NULL: the entries of sel with their exact costs cst [k][R], sorted by (cost, index)
+cudaError_t search_output(const int64_t* sel, const double* cst, int64_t R, int k, int64_t* idx, double* cost, cudaStream_t st);
 // group sizes the shared-difference bank kernel (predict_bank_mean.cuh) is compiled for: the G x (DP + 1) accumulators
 // of a thread (G without the gradient) have to stay in registers
 inline bool bank_group_ok(int DP, int G, bool grad) {

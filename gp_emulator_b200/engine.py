@@ -586,8 +586,68 @@ class DeviceBank(_Handle):
                         addr(out.get("grad")), addr(out.get("hess")), _current_stream_ptr(self.device)))
         return out
 
+    def search(self, candidates, obs, weights=None, k=1):
+        """Per point, the ``k`` rows of the candidate table ``candidates`` (K, D) whose band cost (``cost``) against the
+        point's observation is smallest: a look-up-table retrieval, or the starting points of ``invert``
+        (``gpe_bank_search``).  ``obs`` is (E,) -- one point -- or (N, E); ``weights`` (E,) or None; 1 <= k <=
+        min(K, ``SEARCH_MAX_K``).  Returns ``{"idx": (N, k) int64, "cost": (N, k)}``: row n lists the chosen candidates in
+        ascending order of (cost, index), and ``cost`` is bit for bit the ``cost`` of those candidates against row n in a
+        call of the same N points.  Candidates are ranked by the expanded form ``a_k + s_n . m_k`` of the cost, whose
+        rounding may swap candidates whose costs differ by about ``E u (|a_k| + sum_e |s_ne m_ke|)`` (include/gpemu.h).
+        A point with fewer than k candidates of non-NaN score gets ``idx = -1`` and ``cost = NaN`` in its last slots.
+        numpy in -> numpy out (all devices of the bank); a torch CUDA tensor among ``candidates`` / ``obs`` -> torch CUDA
+        out (asynchronous on the current stream, single-device banks)."""
+        return self._search(False, candidates, obs, weights, k)
+
+    def forward_search(self, candidates, obs, weights=None, k=1):
+        """``search`` with the spectrum cost of ``forward_cost``: ``obs`` (W,) or (N, W), ``weights`` (W,) or None."""
+        if self.W == 0:
+            raise GpemuError("bank has no basis functions to project onto")
+        return self._search(True, candidates, obs, weights, k)
+
+    def _search(self, spectra, candidates, obs, weights, k):
+        D, K_obs = self.D, (self.W if spectra else self.E)
+        lib = _lib.load()
+        k = int(k)
+        flags = _lib.SOLVE_SPECTRA if spectra else 0
+        if _is_torch(candidates) or _is_torch(obs):
+            if self.multi:
+                raise ValueError("a multi-device bank takes host arrays; use one DeviceBank per device for CUDA tensors")
+            import torch
+            tdev = torch.device("cuda", self.device)
+            arr = lambda a: None if a is None else torch.as_tensor(
+                a if _is_torch(a) else np.asarray(a, dtype=np.float64), dtype=torch.float64, device=tdev).contiguous()
+            c, o, wt = arr(candidates), arr(obs), arr(weights)
+            shape = lambda a: tuple(a.shape)
+            empty = lambda s, dt: torch.empty(s, dtype=torch.int64 if dt is np.int64 else torch.float64, device=tdev)
+        else:
+            arr = lambda a: None if a is None else f64c(a.cpu().numpy() if _is_torch(a) else a)
+            c, o, wt = arr(candidates), arr(obs), arr(weights)
+            shape = lambda a: a.shape
+            empty = lambda s, dt: np.empty(s, dtype=dt)
+        if len(shape(c)) != 2 or shape(c)[1] != D:
+            raise ValueError(f"candidates must be (K, {D})")
+        if shape(o) == (K_obs,):
+            N, obs_ld = 1, 0
+        elif len(shape(o)) == 2 and shape(o)[1] == K_obs:
+            N, obs_ld = shape(o)[0], K_obs
+        else:
+            raise ValueError(f"obs must be ({K_obs},) or (N, {K_obs})")
+        if wt is not None and shape(wt) != (K_obs,):
+            raise ValueError(f"weights must be ({K_obs},)")
+        out = {"idx": empty((N, k), np.int64), "cost": empty((N, k), np.float64)}
+        args = (addr(c), shape(c)[0], addr(o), N, obs_ld, addr(wt), k, addr(out["idx"]), addr(out["cost"]))
+        if _is_torch(c):
+            check(lib.gpe_bank_search(self._h, *args, flags, _current_stream_ptr(self.device)))
+        elif self.multi:
+            check(lib.gpe_multi_bank_search(self._h, *args, flags))
+        else:
+            check(lib.gpe_bank_search(self._h, *args, flags | HOST_PTRS, None))
+        return out
+
     def invert(self, x0, obs, weights=None, lower=None, upper=None, prior_mean=None, prior_precision=None,
-               max_iter=_lib.SOLVE_DEFAULT_MAX_ITER, ftol=1e-10, xtol=1e-10, gtol=0.0, lambda0=1e-3, want_cov=False):
+               max_iter=_lib.SOLVE_DEFAULT_MAX_ITER, ftol=1e-10, xtol=1e-10, gtol=0.0, lambda0=1e-3, want_cov=False,
+               candidates=None, n_starts=1):
         """Per point, the inputs that minimise the band cost of ``cost`` plus an optional Gaussian prior,
         ``f(x) = cost(x) + 1/2 (x - prior_mean)^T prior_precision (x - prior_mean)``, inside the box ``lower <= x <= upper``:
         bounded Levenberg-Marquardt on the exact Hessian, every iteration on the device (``gpe_bank_solve``; the
@@ -598,21 +658,75 @@ class DeviceBank(_Handle):
         ``x`` (N, D), ``cost`` (N,), ``grad`` (N, D) and ``hess`` (N, D, D) at x (prior included), ``cov`` (N, D, D) =
         inv(hess) with ``want_cov`` (NaN where hess is not positive definite), ``status`` (N,) int32 (``SOLVE_*`` of
         ``_lib``) and ``n_iter`` (N,) int32, the evaluations after the first.  numpy in -> numpy out (all devices of the
-        bank); torch CUDA in -> torch CUDA out (single-device banks; the call returns when the results are written)."""
+        bank); torch CUDA in -> torch CUDA out (single-device banks; the call returns when the results are written).
+
+        Starting points from a candidate table: with ``x0=None`` and ``candidates`` (K, D), the ``n_starts`` best
+        candidates of each point (``search``) are each solved from, and each point keeps the result of the lowest returned
+        cost (prior included; ties go to the better-ranked start, NaN loses).  ``candidate`` (N,) int64 is then added: the
+        index of the winning start in ``candidates``.  A point without a candidate of non-NaN score comes back with status
+        ``SOLVE_NONFINITE``, NaN x and ``n_iter`` 0.  With ``n_starts=1`` the result is that of
+        ``invert(candidates[idx[:, 0]], ...)``, bit for bit."""
         return self._solve(False, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
-                           lambda0, want_cov)
+                           lambda0, want_cov, candidates, n_starts)
 
     def forward_invert(self, x0, obs, weights=None, lower=None, upper=None, prior_mean=None, prior_precision=None,
                        max_iter=_lib.SOLVE_DEFAULT_MAX_ITER, ftol=1e-10, xtol=1e-10, gtol=0.0, lambda0=1e-3,
-                       want_cov=False):
-        """``invert`` with the spectrum cost of ``forward_cost``: ``obs`` (W,) or (N, W), ``weights`` (W,) or None."""
+                       want_cov=False, candidates=None, n_starts=1):
+        """``invert`` with the spectrum cost of ``forward_cost``: ``obs`` (W,) or (N, W), ``weights`` (W,) or None; the
+        starts from ``candidates`` are chosen by ``forward_search``."""
         if self.W == 0:
             raise GpemuError("bank has no basis functions to project onto")
         return self._solve(True, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
-                           lambda0, want_cov)
+                           lambda0, want_cov, candidates, n_starts)
+
+    def _solve_from_candidates(self, spectra, candidates, n_starts, obs, weights, solve):
+        """Multi-start solve: ``solve(x0)`` from each of the ``n_starts`` best candidates, the best result per point."""
+        found = self._search(spectra, candidates, obs, weights, n_starts)
+        idx = found["idx"]
+        if _is_torch(idx):
+            import torch
+            cand = torch.as_tensor(candidates if _is_torch(candidates) else np.asarray(candidates, dtype=np.float64),
+                                   dtype=torch.float64, device=idx.device)
+            where = lambda m, a, b: torch.where(m.reshape(m.shape + (1,) * (a.dim() - 1)), a, b)
+            isnan = torch.isnan
+        else:
+            cand = f64c(candidates.cpu().numpy() if _is_torch(candidates) else candidates)
+            where = lambda m, a, b: np.where(m.reshape(m.shape + (1,) * (a.ndim - 1)), a, b)
+            isnan = np.isnan
+        best, win = None, None
+        for j in range(int(n_starts)):
+            ij = idx[:, j]
+            res = solve(cand[ij.clip(min=0) if _is_torch(ij) else np.clip(ij, 0, None)])
+            if best is None:
+                best, win = res, ij
+                continue
+            c, bc = res["cost"], best["cost"]
+            take = (ij >= 0) & ((c < bc) | (isnan(bc) & ~isnan(c)))
+            best = {key: where(take, res[key], best[key]) for key in best}
+            win = where(take, ij, win)
+        none = idx[:, 0] < 0
+        if bool(none.any()):
+            for key, v in best.items():
+                if key == "status":
+                    best[key] = where(none, v * 0 + _lib.SOLVE_NONFINITE, v)
+                elif key == "n_iter":
+                    best[key] = where(none, v * 0, v)
+                else:
+                    best[key] = where(none, v * float("nan"), v)
+        best["candidate"] = win
+        return best
 
     def _solve(self, spectra, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
-               lambda0, want_cov):
+               lambda0, want_cov, candidates=None, n_starts=1):
+        if x0 is None:
+            if candidates is None:
+                raise ValueError("give the starting points x0 or a candidate table")
+            return self._solve_from_candidates(
+                spectra, candidates, n_starts, obs, weights,
+                lambda s: self._solve(spectra, s, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol,
+                                      xtol, gtol, lambda0, want_cov))
+        if candidates is not None:
+            raise ValueError("give x0 or candidates, not both")
         D, K = self.D, (self.W if spectra else self.E)
         lib = _lib.load()
         dev = _is_torch(x0)

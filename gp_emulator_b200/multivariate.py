@@ -188,8 +188,18 @@ class MultivariateEmulator(object):
             res = [float(c[0]) if isinstance(c, np.ndarray) else c[0]] + [a[0] for a in res[1:]]
         return tuple(res) if len(res) > 1 else res[0]
 
-    def invert(self, obs, y0, weights=None, bounds=None, prior=None, max_iter=50, ftol=1e-10, xtol=1e-10, gtol=0.0,
-               do_cov=True):
+    def search(self, obs, candidates=None, k=1, weights=None):
+        """The ``k`` parameter vectors of the table ``candidates`` (K, N_params) whose reconstructed output fits ``obs``
+        best, by ``cost`` (``DeviceBank.forward_search``); ``candidates=None`` searches the training design ``y_train``.
+        ``obs`` (N_full,) is one observation, (N, N_full) one per point.  Returns ``{"idx", "cost"}``, each ``(k,)`` for
+        one observation and ``(N, k)`` for N, in ascending order of (cost, index); ``idx`` -1 / ``cost`` NaN where fewer
+        than k candidates have a finite ranking score.  Host arrays or CUDA tensors, as ``predict``."""
+        cand = np.atleast_2d(self.y_train) if candidates is None else candidates
+        out = self._device_bank().forward_search(cand, obs, weights, k)
+        return {key: v[0] for key, v in out.items()} if len(obs.shape) == 1 else out
+
+    def invert(self, obs, y0=None, weights=None, bounds=None, prior=None, max_iter=50, ftol=1e-10, xtol=1e-10, gtol=0.0,
+               do_cov=True, candidates=None, n_starts=1):
         """Retrieve the parameters whose reconstructed output best fits ``obs``: per point, the minimiser of ``cost``
         (plus ``1/2 (y - m)^T P (y - m)`` with ``prior = (m, P)``) inside ``bounds = (lower, upper)``, by bounded
         Levenberg-Marquardt on the exact Hessian with every iteration on the device (``DeviceBank.forward_invert``).
@@ -200,20 +210,35 @@ class MultivariateEmulator(object):
         ``lower`` / ``upper`` (N_params,) or None; ``m`` (N_params,) or (N, N_params), ``P`` (N_params, N_params).
         Returns a dict ``x``, ``cost``, ``grad``, ``hess``, ``cov`` (with ``do_cov``), ``status``, ``n_iter`` -- one point:
         ``(N_params,)``, ``float``, ``(N_params,)``, ``(N_params, N_params)``, ..., ``int``, ``int``; N points: the same with
-        a leading N.  Host arrays or CUDA tensors, as ``predict``."""
+        a leading N.  Host arrays or CUDA tensors, as ``predict``.
+
+        Without ``y0`` the starts come from a candidate table (``search``): the ``n_starts`` best rows of ``candidates``
+        (K, N_params) -- the training design ``y_train`` when None -- are each solved from and the lowest cost is kept per
+        point; the result gains ``candidate``, the row of the winning start (``DeviceBank.invert``).  The number of points
+        is then that of ``obs``."""
         bank = self._device_bank()
-        if isinstance(y0, np.ndarray) or not hasattr(y0, "is_cuda"):
-            y2 = np.atleast_2d(y0)
-        else:
-            y2 = y0 if y0.dim() == 2 else y0.reshape(1, -1)
         lower, upper = bounds if bounds is not None else (None, None)
         m, P = prior if prior is not None else (None, None)
-        out = bank.forward_invert(y2, obs, weights, lower=lower, upper=upper, prior_mean=m, prior_precision=P,
-                                  max_iter=max_iter, ftol=ftol, xtol=xtol, gtol=gtol, want_cov=do_cov)
-        if y2.shape[0] == 1:
+        if y0 is None:
+            cand = np.atleast_2d(self.y_train) if candidates is None else candidates
+            one = len(obs.shape) == 1
+            out = bank.forward_invert(None, obs, weights, lower=lower, upper=upper, prior_mean=m, prior_precision=P,
+                                      max_iter=max_iter, ftol=ftol, xtol=xtol, gtol=gtol, want_cov=do_cov,
+                                      candidates=cand, n_starts=n_starts)
+        else:
+            if isinstance(y0, np.ndarray) or not hasattr(y0, "is_cuda"):
+                y2 = np.atleast_2d(y0)
+            else:
+                y2 = y0 if y0.dim() == 2 else y0.reshape(1, -1)
+            one = y2.shape[0] == 1
+            out = bank.forward_invert(y2, obs, weights, lower=lower, upper=upper, prior_mean=m, prior_precision=P,
+                                      max_iter=max_iter, ftol=ftol, xtol=xtol, gtol=gtol, want_cov=do_cov,
+                                      candidates=candidates, n_starts=n_starts)
+        if one:
             one = {k: v[0] for k, v in out.items()}
-            for k in ("cost", "status", "n_iter"):
-                one[k] = (float if k == "cost" else int)(one[k]) if isinstance(one[k], np.generic) else one[k]
+            for k in ("cost", "status", "n_iter", "candidate"):
+                if k in one:
+                    one[k] = (float if k == "cost" else int)(one[k]) if isinstance(one[k], np.generic) else one[k]
             return one
         return out
 

@@ -294,6 +294,34 @@ int gpe_multi_bank_solve(gpe_multi* mm, const double* x0, int64_t N, const doubl
                          const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess, double* cov,
                          int32_t* info, unsigned flags);
 
+/* Candidate search: per point (pixel), the k rows of a candidate table cand (K, D) that fit its observation best -- the
+ * starting points of an inversion, or a look-up-table retrieval.  The cost is the band cost of gpe_bank_cost (default)
+ * or, with GPE_SOLVE_SPECTRA, the spectrum cost of gpe_bank_forward_cost.  With m_k the bank means at candidate k, both
+ * are exactly cost_nk = a_k + s_n . m_k + c_n, where c_n does not depend on k:
+ *   band cost:      a_k = 1/2 sum_e w_e m_ke^2       s_n = -w o obs_n
+ *   spectrum cost:  a_k = 1/2 m_k^T C m_k            s_n = -basis . (l o obs_n)      C = basis . diag(l) . basis^T
+ * Row n of the outputs holds the k candidates with the smallest ranking score a_k + s_n . m_k under the total order
+ * (score, candidate index), reported in ascending order of (exact cost, candidate index): cost[n, j] is, bit for bit,
+ * the cost (only) of gpe_bank_cost / gpe_bank_forward_cost at cand[idx[n, j]] against row n in a call of the same N
+ * points.  The score is rounded: its error is about E u (|a_k| + sum_e |s_ne m_ke|), u = 2^-53, so candidates whose exact
+ * costs differ by less than that may be ranked either way; that is the only way the selected set can differ from an
+ * exact brute force.
+ * Candidates whose score is NaN are never selected.  A point with fewer than k selectable candidates fills its last slots
+ * with idx = -1 and cost = NaN (a NaN observation gives all -1).
+ *   cand (K, D), K >= 1; obs (N, K_obs) with obs_ld >= K_obs, or one (K_obs) row shared by every point with obs_ld = 0,
+ *   K_obs = E (W with GPE_SOLVE_SPECTRA); weights (K_obs) or NULL (all 1); 1 <= k <= min(K, GPE_SEARCH_MAX_K);
+ *   idx (N, k) and cost (N, k) outputs, either (not both) may be NULL.
+ * Every array follows the call's placement: device pointers on the bank's device, asynchronous on `stream`, or host
+ * pointers with GPE_HOST_PTRS (host obs_ld = K_obs or 0), streamed in chunks, synchronous.  N = 0 launches nothing.
+ * Banks of up to 96 emulators (GPE_ERR_UNSUPPORTED beyond).  Results do not depend on chunking, pointer placement, the
+ * device count, the order of the points or the split of the candidates over CTAs. */
+#define GPE_SEARCH_MAX_K 16
+int gpe_bank_search(gpe_bank* b, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                    const double* weights, int k, int64_t* idx, double* cost, unsigned flags, void* stream);
+/* The same on every device of a bank handle; host arrays (GPE_HOST_PTRS is implied).  Each device builds its own table. */
+int gpe_multi_bank_search(gpe_multi* mm, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                          const double* weights, int k, int64_t* idx, double* cost, unsigned flags);
+
 /* PCA back-projection of bank means: fwd (N, W) = mu (N, E) @ basis (E, W)
  * (the accumulation `fwd += pred_mu * basis_functions[i]`, gp_emulator/multivariate_gp.py:216, batched
  * over N points), and optionally deriv_full (N, D, W) = sum_e deriv[n, e, d] * basis[e, w] (:218).
