@@ -11,7 +11,9 @@
    Levenberg-Marquardt on the exact Hessian, on the device) and print the retrieved parameters with their Laplace
    posterior standard deviations;
 4. per-band ``GaussianProcess`` objects: mean / variance / gradient / Hessian, FP64 and single precision;
-5. a per-band bank reduced on the device to a least-squares misfit and its gradient (``DeviceBank.cost``);
+5. a per-band bank reduced on the device to a least-squares misfit and its gradient (``DeviceBank.cost``), then 1000
+   band observations inverted at once with each pixel's own sigma and one band masked on a tenth of the pixels
+   (per-point weights ``(N, bands)``: ``DeviceBank.invert``);
 6. store and reload an emulator (``EmulatorStorage``).
 """
 import os
@@ -97,6 +99,18 @@ def main():
     best = int(np.argmin(out["cost"]))
     print("misfit of 1000 candidates against one observation: best candidate %d (cost %.2f), true one is 3 (cost %.2f)" % (
         best, out["cost"][best], out["cost"][3]))
+    rs = np.random.RandomState(4)                                             # 5b. per-pixel sigma and masked bands
+    sig = 0.005 * rs.uniform(0.5, 3.0, (len(y_test), len(bands)))            # each pixel's own noise level per band
+    obs_b = truth[:, bands] + sig * rs.standard_normal(sig.shape)
+    wb = 1.0 / sig ** 2                                                       # weights (N, bands): one row per pixel
+    masked = rs.random_sample(len(y_test)) < 0.1
+    wb[masked, 2] = 0.0                                                       # band 2 unusable there: weight 0
+    rb = bank.invert(np.tile(0.5 * (lower + upper), (len(y_test), 1)), obs_b, wb, lower=lower, upper=upper, want_cov=True)
+    sdb = np.sqrt(np.diagonal(rb["cov"], axis1=1, axis2=2))
+    print("inverted %d band observations with per-pixel sigma, band %d masked on %d of them: status counts %s; median "
+          "Laplace sd of parameter 0: %.4f with all bands, %.4f with one masked" % (
+        len(y_test), bands[2], int(masked.sum()), np.bincount(rb["status"], minlength=4).tolist(),
+        np.nanmedian(sdb[~masked, 0]), np.nanmedian(sdb[masked, 0])))
 
     with tempfile.TemporaryDirectory() as tmp:                                # 6. storage
         store = gpe.EmulatorStorage(os.path.join(tmp, "emulators"))

@@ -26,6 +26,7 @@ SOLVE_MAX_D = 32
 SOLVE_CONVERGED, SOLVE_MAX_ITER, SOLVE_STALLED, SOLVE_NONFINITE = 0, 1, 2, 3
 SOLVE_DEFAULT_MAX_ITER = 50
 SEARCH_MAX_K = 16
+SEARCH_PW_MAX_E_BANDS, SEARCH_PW_MAX_E_SPECTRA = 48, 12
 
 # every symbol include/gpemu.h declares (tests/test_abi.py checks the header against this list and the .so)
 SYMBOLS = (
@@ -38,6 +39,8 @@ SYMBOLS = (
     "gpe_bank_forward_cost_host_ex", "gpe_multi_bank_cost_ex", "gpe_multi_bank_forward_cost_ex", "gpe_bank_project", "gpe_bank_forward", "gpe_measure_fp64_peaks", "gpe_launch_count",
     "gpe_trainer_create", "gpe_trainer_eval", "gpe_trainer_destroy", "gpe_bank_solve", "gpe_multi_bank_solve",
     "gpe_bank_search", "gpe_multi_bank_search",
+    "gpe_bank_cost_pw", "gpe_bank_solve_pw", "gpe_bank_search_pw", "gpe_multi_bank_cost_pw", "gpe_multi_bank_solve_pw",
+    "gpe_multi_bank_search_pw",
 )
 
 
@@ -139,6 +142,23 @@ def load():
                                     C.c_void_p]
     lib.gpe_multi_bank_search.restype = C.c_int
     lib.gpe_multi_bank_search.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, C.c_int64, dp, C.c_int, dp, dp, C.c_uint]
+    # per-point weights: the same arguments plus weights_ld after weights (the cost calls also take flags)
+    lib.gpe_bank_cost_pw.restype = C.c_int
+    lib.gpe_bank_cost_pw.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, C.c_int64, dp, dp, dp, C.c_uint, C.c_void_p]
+    lib.gpe_multi_bank_cost_pw.restype = C.c_int
+    lib.gpe_multi_bank_cost_pw.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, C.c_int64, dp, dp, dp, C.c_uint]
+    lib.gpe_bank_solve_pw.restype = C.c_int
+    lib.gpe_bank_solve_pw.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, C.c_int64, so, dp, dp, dp, dp, dp, dp,
+                                      C.c_uint, C.c_void_p]
+    lib.gpe_multi_bank_solve_pw.restype = C.c_int
+    lib.gpe_multi_bank_solve_pw.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, dp, C.c_int64, so, dp, dp, dp, dp, dp, dp,
+                                            C.c_uint]
+    lib.gpe_bank_search_pw.restype = C.c_int
+    lib.gpe_bank_search_pw.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, C.c_int64, dp, C.c_int64, C.c_int, dp, dp,
+                                       C.c_uint, C.c_void_p]
+    lib.gpe_multi_bank_search_pw.restype = C.c_int
+    lib.gpe_multi_bank_search_pw.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, C.c_int64, dp, C.c_int64, C.c_int, dp,
+                                             dp, C.c_uint]
     lib.gpe_bank_project.restype = C.c_int
     lib.gpe_bank_project.argtypes = [C.c_void_p, dp, dp, C.c_int64, dp, dp, C.c_void_p]
     lib.gpe_bank_forward.restype = C.c_int

@@ -1209,10 +1209,12 @@ int bank_project_device(gpe_bank* b, const double* mu, const double* deriv, int6
 
 // Least-squares reduction over the emulators of a bank (SURVEY 8f-3: outputs consumed on the fly).  One warp per
 // point: lanes stride over the emulators for the residuals, then lane d accumulates column d of the gradient.
+// PW: per-point weights, row pt at weights + pt * w_ld (DESIGN 4.6f); otherwise one shared row.
+template <bool PW>
 __global__ void __launch_bounds__(128) k_bank_cost(const double* __restrict__ mu, const double* __restrict__ deriv,
                                                    const double* __restrict__ obs, int64_t obs_ld,
                                                    const double* __restrict__ weights, double* __restrict__ cost,
-                                                   double* __restrict__ grad, int64_t n, int E, int D) {
+                                                   double* __restrict__ grad, int64_t n, int E, int D, int64_t w_ld) {
     extern __shared__ double wr_s[];                     // [4 warps][E] weighted residuals
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     double* wr = wr_s + (size_t)w * E;
@@ -1220,7 +1222,7 @@ __global__ void __launch_bounds__(128) k_bank_cost(const double* __restrict__ mu
         double c = 0.0;
         for (int e = lane; e < E; e += 32) {
             const double r = mu[pt * E + e] - obs[pt * obs_ld + e];
-            const double we = weights ? weights[e] : 1.0;
+            const double we = weights ? weights[(PW ? pt * w_ld : 0) + e] : 1.0;
             wr[e] = we * r;
             c = fma(we * r, r, c);
         }
@@ -1244,11 +1246,13 @@ __global__ void __launch_bounds__(128) k_bank_cost(const double* __restrict__ mu
 //   forward cost (s != NULL):  c = s (n, E) from k_forward_cost;  A = C (E, E) from k_forward_cost_curv
 // A CTA takes P points at a time: their c (and, with C, T = C G_n) go to shared memory, then one thread per point and
 // upper-triangle entry i <= j sums over e in ascending order and writes (i, j) and (j, i): hess_n == hess_n^T bit for bit.
+// PW (DESIGN 4.6f): per-point weights w_n at weights + pt * w_ld, and one C_n (E, E) per point at C + pt E^2.
+template <bool PW>
 __global__ void __launch_bounds__(256) k_cost_hess(const double* __restrict__ mu, const double* __restrict__ obs, int64_t obs_ld,
                                                    const double* __restrict__ weights, const double* __restrict__ s,
                                                    const double* __restrict__ C, const double* __restrict__ deriv,
                                                    const double* __restrict__ hs, int64_t n, int E, int D, int P,
-                                                   double* __restrict__ hess) {
+                                                   double* __restrict__ hess, int64_t w_ld) {
     extern __shared__ double ch_s[];                     // [P][E] c, then (C) [P][E][D] T
     double* cs = ch_s;
     double* T = ch_s + (size_t)P * E;
@@ -1259,14 +1263,15 @@ __global__ void __launch_bounds__(256) k_cost_hess(const double* __restrict__ mu
         for (int k = tid; k < np * E; k += blockDim.x) {
             const int pl = k / E, e = k - pl * E;
             const int64_t pt = p0 + pl;
-            cs[k] = s ? s[pt * E + e] : (weights ? weights[e] : 1.0) * (mu[pt * E + e] - obs[pt * obs_ld + e]);
+            cs[k] = s ? s[pt * E + e] : (weights ? weights[(PW ? pt * w_ld : 0) + e] : 1.0) * (mu[pt * E + e] - obs[pt * obs_ld + e]);
         }
         if (C) {
             for (int64_t k = tid; k < np * ED; k += blockDim.x) {
                 const int pl = (int)(k / ED), e = (int)((k - pl * ED) / D), d = (int)(k - pl * ED - (int64_t)e * D);
                 const double* g = deriv + (p0 + pl) * ED + d;
+                const double* Cn = PW ? C + (p0 + pl) * E * E : C;
                 double v = 0.0;
-                for (int f = 0; f < E; ++f) v = fma(C[(int64_t)e * E + f], g[(int64_t)f * D], v);
+                for (int f = 0; f < E; ++f) v = fma(Cn[(int64_t)e * E + f], g[(int64_t)f * D], v);
                 T[k] = v;
             }
         }
@@ -1286,7 +1291,8 @@ __global__ void __launch_bounds__(256) k_cost_hess(const double* __restrict__ mu
                 const double* t = T + (size_t)pl * ED + j;
                 for (int e = 0; e < E; ++e) gn = fma(g[(int64_t)e * D + i], t[(int64_t)e * D], gn);
             } else {
-                for (int e = 0; e < E; ++e) gn = fma((weights ? weights[e] : 1.0) * g[(int64_t)e * D + i], g[(int64_t)e * D + j], gn);
+                const double* wn = PW && weights ? weights + pt * w_ld : weights;
+                for (int e = 0; e < E; ++e) gn = fma((wn ? wn[e] : 1.0) * g[(int64_t)e * D + i], g[(int64_t)e * D + j], gn);
             }
             const double v = a + gn;
             hess[pt * D * D + i * D + j] = v;
@@ -1299,14 +1305,16 @@ __global__ void __launch_bounds__(256) k_cost_hess(const double* __restrict__ mu
 // Launch of k_cost_hess over n points: as many points per CTA as fill its 256 threads with upper-triangle entries, within
 // 48 KB of shared memory (at least one point: a forward cost of 96 emulators at D = 256 takes 194 KB).
 int cost_hess(const double* mu, const double* obs, int64_t obs_ld, const double* weights, const double* s, const double* C,
-              const double* deriv, const double* hs, int64_t n, int E, int D, int sms, double* hess, cudaStream_t st) {
+              const double* deriv, const double* hs, int64_t n, int E, int D, int sms, double* hess, cudaStream_t st,
+              bool pw = false, int64_t w_ld = 0) {
     const int nt = D * (D + 1) / 2;
     const size_t per = (size_t)E * (C ? 1 + D : 1);
     const int P = (int)std::max<size_t>(1, std::min<size_t>(std::max(1, 256 / nt), ((size_t)48 << 10) / (per * 8)));
     const size_t smem = (size_t)P * per * 8;
     if (smem > kSmemMax) return fail(GPE_ERR_UNSUPPORTED, "cost Hessian: %zu bytes of shared memory per point", smem);
     const int grid = (int)std::min<int64_t>((n + P - 1) / P, (int64_t)sms * 8);
-    CUDA_TRY(launch_kernel(k_cost_hess, grid, 256, smem, st, mu, obs, obs_ld, weights, s, C, deriv, hs, n, E, D, P, hess));
+    CUDA_TRY(launch_kernel(pw ? k_cost_hess<true> : k_cost_hess<false>, grid, 256, smem, st, mu, obs, obs_ld, weights, s, C, deriv,
+                           hs, n, E, D, P, hess, w_ld));
     return GPE_OK;
 }
 
@@ -1356,22 +1364,27 @@ int bank_cost_walk(gpe_bank* b, const double* testing, int64_t N, bool grad, boo
     return GPE_OK;
 }
 
+// The cost calls take weights (K) shared by every point (w_ld = 0, or NULL: all 1) or one row per point, w_ld apart
+// (DESIGN 4.6f).  Cn: NULL, or (spectrum cost with per-point weights and hess) the curvature C_n (N, E, E) of the points,
+// formed beforehand by forward_cost_curv_pw (the solver keeps it across iterations).
 int bank_cost_device(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
-                     double* cost, double* grad, double* hess, cudaStream_t st, int64_t call_N = -1) {
+                     int64_t w_ld, const double*, double* cost, double* grad, double* hess, cudaStream_t st, int64_t call_N = -1) {
     const int64_t E = b->E, D = b->D;
     const int sms = b->models[0]->sms;
+    const bool pw = w_ld != 0;
     return bank_cost_walk(b, testing, N, grad != nullptr, hess != nullptr, 0, 0, st, call_N,
                           [&](double*, const double* d_mu, const double* d_der, const double* d_hes, double*, int64_t n0,
                               int64_t n) -> int {
+                              const double* w = pw ? weights + n0 * w_ld : weights;
                               if (cost || grad) {
                                   const int grid = (int)std::min<int64_t>((n + 3) / 4, (int64_t)sms * 16);
-                                  CUDA_TRY(launch_kernel(k_bank_cost, grid, 128, (size_t)4 * E * 8, st, d_mu, d_der,
-                                                         obs + n0 * obs_ld, obs_ld, weights, cost ? cost + n0 : nullptr,
-                                                         grad ? grad + n0 * D : nullptr, n, (int)E, (int)D));
+                                  CUDA_TRY(launch_kernel(pw ? k_bank_cost<true> : k_bank_cost<false>, grid, 128, (size_t)4 * E * 8,
+                                                         st, d_mu, d_der, obs + n0 * obs_ld, obs_ld, w, cost ? cost + n0 : nullptr,
+                                                         grad ? grad + n0 * D : nullptr, n, (int)E, (int)D, w_ld));
                               }
                               if (!hess) return GPE_OK;
-                              return cost_hess(d_mu, obs + n0 * obs_ld, obs_ld, weights, nullptr, nullptr, d_der, d_hes, n, (int)E,
-                                               (int)D, sms, hess + n0 * D * D, st);
+                              return cost_hess(d_mu, obs + n0 * obs_ld, obs_ld, w, nullptr, nullptr, d_der, d_hes, n, (int)E,
+                                               (int)D, sms, hess + n0 * D * D, st, pw, w_ld);
                           });
 }
 
@@ -1380,27 +1393,38 @@ int bank_cost_device(gpe_bank* b, const double* testing, int64_t N, const double
 // call, zero-padded to the basis image's width.
 //   With hess, k_forward_cost also stores s = (l o (fwd - obs)) . basis^T (n, E) in the chunk scratch, and C = basis .
 // diag(l) . basis^T (E, E) follows the partial sums in the aux area, formed once per call: the Gauss-Newton term G^T C G
-// then costs E^2 D + E D^2 per point instead of D^2 W.
+// then costs E^2 D + E D^2 per point instead of D^2 W.  With per-point weights C_n is one (E, E) matrix per point: taken
+// from Cn, or formed per chunk behind s in the chunk scratch.
 int bank_forward_cost_device(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
-                             const double* weights, double* cost, double* grad, double* hess, cudaStream_t st,
-                             int64_t call_N = -1) {
+                             const double* weights, int64_t w_ld, const double* Cn, double* cost, double* grad, double* hess,
+                             cudaStream_t st, int64_t call_N = -1) {
     const int D = b->D, W = b->W, Wp = b->Wp, E = b->E;
+    const bool pw = w_ld != 0;
     // calls of a few points spread the column groups over CTAs; their partial sums follow the aux operands in the scratch
     const int gy = forward_cost_split(call_N < 0 ? N : call_N, W);
     const int64_t part_n = gy > 1 ? (int64_t)gy * ((N + 63) / 64 * 64) * (1 + E) : 0;
-    const int64_t aux_n = 2 * (int64_t)Wp + part_n + (hess ? (int64_t)E * E : 0);
-    return bank_cost_walk(b, testing, N, grad != nullptr, hess != nullptr, aux_n, E, st, call_N,
+    const int64_t aux_n = 2 * (int64_t)Wp + part_n + (hess && !pw ? (int64_t)E * E : 0);
+    const int64_t ext_pp = E + (hess && pw && !Cn ? (int64_t)E * E : 0);
+    return bank_cost_walk(b, testing, N, grad != nullptr, hess != nullptr, aux_n, ext_pp, st, call_N,
                           [&](double* aux, const double* d_mu, const double* d_der, const double* d_hes, double* d_s,
                               int64_t n0, int64_t n) -> int {
-                              double* C = hess ? aux + 2 * Wp + part_n : nullptr;
-                              if (n0 == 0) CUDA_TRY(forward_cost_aux(weights, obs_ld == 0 ? obs : nullptr, W, Wp, aux, st));
-                              if (n0 == 0 && hess) CUDA_TRY(forward_cost_curv(b->d_basis, aux, E, Wp, C, st));
+                              const double* C = hess && !pw ? aux + 2 * Wp + part_n : nullptr;
+                              const double* w = pw ? weights + n0 * w_ld : nullptr;
+                              if (n0 == 0) CUDA_TRY(forward_cost_aux(pw ? nullptr : weights, obs_ld == 0 ? obs : nullptr, W, Wp, aux, st));
+                              if (n0 == 0 && hess && !pw) CUDA_TRY(forward_cost_curv(b->d_basis, aux, E, Wp, (double*)C, st));
                               CUDA_TRY(forward_cost_rows(d_mu, d_der, n, E, D, obs + n0 * obs_ld, obs_ld, aux, b->d_basis, W,
                                                          Wp, gy, aux + 2 * Wp, cost ? cost + n0 : nullptr,
-                                                         grad ? grad + n0 * D : nullptr, d_s, st));
+                                                         grad ? grad + n0 * D : nullptr, d_s, st, w, w_ld));
                               if (!hess) return GPE_OK;
+                              if (pw && Cn) {
+                                  C = Cn + n0 * E * E;
+                              } else if (pw) {
+                                  double* Cc = d_s + n * E;
+                                  CUDA_TRY(forward_cost_curv_pw(b->d_basis, w, w_ld, n, E, W, Wp, Cc, st));
+                                  C = Cc;
+                              }
                               return cost_hess(nullptr, nullptr, 0, nullptr, d_s, C, d_der, d_hes, n, E, D, b->models[0]->sms,
-                                               hess + n0 * D * D, st);
+                                               hess + n0 * D * D, st, pw, 0);
                           });
 }
 
@@ -1435,26 +1459,29 @@ int bank_stream(gpe_bank* b, int64_t N, const CallIo& io, const SharedCall* shar
 }
 
 // Bank cost of observations K wide (E: the bank's own outputs, W: its spectra): testing and, unless obs_ld = 0, the
-// per-point observations (idx 0) in; cost, grad, hess out (idx 1, 2, 3).
+// per-point observations (idx 0) in; cost, grad, hess out (idx 1, 2, 3); per-point weights (w_ld != 0) in (idx 4).
 CallIo cost_io(const gpe_bank* b, int64_t K, const double* testing, const double* obs, int64_t obs_ld, double* cost, double* grad,
-               double* hess) {
+               double* hess, const double* weights = nullptr, int64_t w_ld = 0) {
     CallIo io;
     io.in.add(testing, b->D);
     io.idx[0] = obs_ld != 0 ? io.in.add(obs, K) : -1;
+    io.idx[4] = w_ld != 0 ? io.in.add(weights, K) : -1;
     io.idx[1] = cost ? io.out.add(cost, 1) : -1;
     io.idx[2] = grad ? io.out.add(grad, b->D) : -1;
     io.idx[3] = hess ? io.out.add(hess, (int64_t)b->D * b->D) : -1;
     return io;
 }
 
-typedef int (*CostDevice)(gpe_bank*, const double*, int64_t, const double*, int64_t, const double*, double*, double*, double*,
-                          cudaStream_t, int64_t);
+typedef int (*CostDevice)(gpe_bank*, const double*, int64_t, const double*, int64_t, const double*, int64_t, const double*,
+                          double*, double*, double*, cudaStream_t, int64_t);
 
 // Host-resident cost call (bank_cost_device or bank_forward_cost_device, observations K wide): test points (and
 // per-point observations) stream in, cost / gradient / Hessian stream out.
 int bank_cost_stream(gpe_bank* b, int64_t K, CostDevice cost_device, int64_t N, const double* obs, int64_t obs_ld,
-                     const double* weights, const CallIo& io, const SharedCall* shared = nullptr) {
+                     const double* weights, const CallIo& io, const SharedCall* shared = nullptr, int64_t w_ld = 0) {
     if (obs_ld != 0 && obs_ld != K) return fail(GPE_ERR_INVALID, "host observations must be contiguous: obs_ld = %s or 0", K == b->E ? "E" : "W");
+    if (w_ld != 0 && w_ld != K) return fail(GPE_ERR_INVALID, "host weights must be contiguous: weights_ld = %s or 0", K == b->E ? "E" : "W");
+    if (w_ld != 0) weights = nullptr;   // streamed per chunk (idx 4), not uploaded
     // the shared observation vector and the weights are small: one upload per call, enqueued ahead of this pipeline's first
     // chunk; its later chunks (other slot streams) wait for it.  (Every chunk of the previous call has finished: the
     // buffer is free.)
@@ -1479,9 +1506,19 @@ int bank_cost_stream(gpe_bank* b, int64_t K, CostDevice cost_device, int64_t N, 
                                CUDA_TRY(cudaStreamWaitEvent(st, b->aux_ready, 0));
                            }
                            const double* d_obs = obs_ld != 0 ? io.at<const double>(di, 0) : d_obs1;
-                           return cost_device(b, (const double*)di[0], n, d_obs, obs_ld != 0 ? K : 0, d_w,
-                                              io.at<double>(dout, 1), io.at<double>(dout, 2), io.at<double>(dout, 3), st, N);
+                           const double* d_wc = w_ld != 0 ? io.at<const double>(di, 4) : d_w;
+                           return cost_device(b, (const double*)di[0], n, d_obs, obs_ld != 0 ? K : 0, d_wc, w_ld != 0 ? K : 0,
+                                              nullptr, io.at<double>(dout, 1), io.at<double>(dout, 2), io.at<double>(dout, 3), st, N);
                        });
+}
+
+// Request check of the weights of a call with observations K wide: w_ld = 0 (one shared row, or NULL), else per point,
+// >= K apart on the device and exactly K for host arrays.
+int weights_check(const double* weights, int64_t w_ld, int64_t K, bool spectra, bool host) {
+    if (w_ld != 0 && !weights) return fail(GPE_ERR_INVALID, "weights_ld = %lld but weights is NULL", (long long)w_ld);
+    if (w_ld != 0 && (w_ld < 0 || (host ? w_ld != K : w_ld < K)))
+        return fail(GPE_ERR_INVALID, "weights_ld must be 0 (one weight vector) or %s %s", host ? "=" : ">=", spectra ? "W" : "E");
+    return GPE_OK;
 }
 
 // Request check of the forward-cost calls (device: obs_ld = 0 or >= W; the host calls check obs_ld = 0 or W).
@@ -1503,28 +1540,36 @@ int forward_cost_check(gpe_bank* b, int64_t N, const double* testing, const doub
 // P pixels at a time.
 constexpr int64_t kSearchRows = 1 << 16;
 struct SearchScratch {
-    int Kp = 0, gy = 1;
+    int Kp = 0, gy = 1, Ew = 0;   // Ew: width of the ranking operand (E, or that of the per-point-weight forms)
+    bool pw = false;
     int64_t P = 0;
     double *tbl = nullptr, *ta = nullptr, *mu = nullptr, *aux = nullptr, *C = nullptr;   // table (aux, C: spectrum cost)
     double *s = nullptr, *zeros = nullptr, *pv = nullptr, *x = nullptr, *cst = nullptr;   // pixels
+    double *op = nullptr, *Cn = nullptr;                                                  // pixels, per-point weights
     int* pi = nullptr;
     int64_t* sel = nullptr;
 };
 
+// Width of the ranking operand of a search (DESIGN 4.6e, 4.6f).
+int search_width(int E, bool spectra, bool pw) { return !pw ? E : spectra ? E * (E + 1) / 2 + E : 2 * E; }
+
 // Lay out and grow the bank's search scratch for a call of call_N pixels (caller holds search_mu).
-int search_prepare(gpe_bank* b, bool spectra, int64_t K, int k, int64_t call_N, SearchScratch* sc) {
+int search_prepare(gpe_bank* b, bool spectra, int64_t K, int k, int64_t call_N, SearchScratch* sc, bool pw = false) {
     const int64_t E = b->E, D = b->D;
     sc->Kp = search_pad(K);
     sc->gy = search_split(call_N, K);
     sc->P = std::min<int64_t>(kSearchRows, call_N);
-    const int64_t P = sc->P, gy = sc->gy;
+    sc->pw = pw;
+    sc->Ew = search_width((int)E, spectra, pw);
+    const int64_t P = sc->P, gy = sc->gy, Ew = sc->Ew;
     size_t off = 0;
     auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-    const size_t o_tbl = carve(8 * (size_t)search_ks((int)E) * sc->Kp * 4), o_ta = carve(8 * (size_t)sc->Kp), o_mu = carve(8 * K * E);
-    const size_t o_aux = carve(spectra ? 16 * (size_t)b->Wp : 0), o_C = carve(spectra ? 8 * E * E : 0);
+    const size_t o_tbl = carve(8 * (size_t)search_ks((int)Ew) * sc->Kp * 4), o_ta = carve(8 * (size_t)sc->Kp), o_mu = carve(8 * K * E);
+    const size_t o_aux = carve(spectra ? 16 * (size_t)b->Wp : 0), o_C = carve(spectra && !pw ? 8 * E * E : 0);
     const size_t o_s = carve(8 * P * E), o_z = carve(spectra ? 8 * P * E : 0), o_sel = carve(8 * P * k);
     const size_t o_pv = carve(gy > 1 ? 8 * gy * P * k : 0), o_pi = carve(gy > 1 ? 4 * gy * P * k : 0);
     const size_t o_x = carve(8 * P * D), o_cst = carve(8 * P * k);
+    const size_t o_op = carve(pw ? 8 * P * Ew : 0), o_Cn = carve(pw && spectra ? 8 * P * E * E : 0);
     if (!b->search_free) CUDA_TRY(cudaEventCreateWithFlags(&b->search_free, cudaEventDisableTiming));
     if (b->search_cap < off) CUDA_TRY(cudaEventSynchronize(b->search_free));   // the old scratch may still be in use
     int rc = ensure_buf(&b->search_d, &b->search_cap, off, false);
@@ -1534,6 +1579,7 @@ int search_prepare(gpe_bank* b, bool spectra, int64_t K, int k, int64_t call_N, 
     sc->aux = spectra ? (double*)(base + o_aux) : nullptr; sc->C = spectra ? (double*)(base + o_C) : nullptr;
     sc->s = (double*)(base + o_s); sc->zeros = spectra ? (double*)(base + o_z) : nullptr; sc->sel = (int64_t*)(base + o_sel);
     sc->pv = (double*)(base + o_pv); sc->pi = (int*)(base + o_pi); sc->x = (double*)(base + o_x); sc->cst = (double*)(base + o_cst);
+    sc->op = (double*)(base + o_op); sc->Cn = (double*)(base + o_Cn);
     return GPE_OK;
 }
 
@@ -1545,33 +1591,38 @@ int search_build_table(gpe_bank* b, const SearchScratch& sc, bool spectra, const
     int rc = bank_predict_device(b, cand, K, sc.mu, nullptr, nullptr, nullptr, st, K);
     if (rc) return rc;
     if (spectra) {
-        CUDA_TRY(forward_cost_aux(weights, obs1, b->W, b->Wp, sc.aux, st));
-        CUDA_TRY(forward_cost_curv(b->d_basis, sc.aux, E, b->Wp, sc.C, st));
+        CUDA_TRY(forward_cost_aux(sc.pw ? nullptr : weights, obs1, b->W, b->Wp, sc.aux, st));
+        if (!sc.pw) CUDA_TRY(forward_cost_curv(b->d_basis, sc.aux, E, b->Wp, sc.C, st));
         CUDA_TRY(cudaMemsetAsync(sc.zeros, 0, (size_t)sc.P * E * 8, st));
     }
-    CUDA_TRY(search_table(sc.mu, K, E, sc.Kp, spectra ? nullptr : weights, sc.C, sc.tbl, sc.ta, st));
+    if (sc.pw) CUDA_TRY(search_table_pw(sc.mu, K, E, sc.Ew, sc.Kp, spectra, sc.tbl, sc.ta, st));
+    else CUDA_TRY(search_table(sc.mu, K, E, sc.Kp, spectra ? nullptr : weights, sc.C, sc.tbl, sc.ta, st));
     return GPE_OK;
 }
 
 // Pixels [0, n) of a call of call_N pixels on st, P at a time: pixel operand s (spectrum cost: s of k_forward_cost at
 // fwd = 0, i.e. -basis . (l o obs)), top-k selection, then per slot j the exact cost of candidate sel[:, j] by the cost
-// call's own path (call_N: the same kernel plans as a cost call of the call's pixels), then the final order.
+// call's own path (call_N: the same kernel plans as a cost call of the call's pixels), then the final order.  Per-point
+// weights (w_ld != 0): the operand of DESIGN 4.6f, from s and (spectrum cost) the pixels' curvature C_n.
 int search_rows(gpe_bank* b, const SearchScratch& sc, bool spectra, const double* cand, int k, const double* obs, int64_t obs_ld,
-                const double* weights, int64_t n, int64_t call_N, int64_t* idx, double* cost, cudaStream_t st) {
+                const double* weights, int64_t n, int64_t call_N, int64_t* idx, double* cost, cudaStream_t st, int64_t w_ld = 0) {
     const int E = b->E, D = b->D;
     const CostDevice cost_device = spectra ? bank_forward_cost_device : bank_cost_device;
     for (int64_t p0 = 0; p0 < n; p0 += sc.P) {
         const int64_t m = std::min(sc.P, n - p0);
         const double* o = obs + p0 * obs_ld;
+        const double* w = w_ld != 0 ? weights + p0 * w_ld : weights;
         if (spectra)
             CUDA_TRY(forward_cost_rows(sc.zeros, nullptr, m, E, D, o, obs_ld, sc.aux, b->d_basis, b->W, b->Wp, 1, nullptr, nullptr,
-                                       nullptr, sc.s, st));
-        else
+                                       nullptr, sc.s, st, w_ld != 0 ? w : nullptr, w_ld));
+        else if (w_ld == 0)
             CUDA_TRY(search_band_s(o, obs_ld, weights, m, E, sc.s, st));
-        CUDA_TRY(search_topk(sc.s, m, E, sc.tbl, sc.ta, sc.Kp, k, sc.gy, sc.pv, sc.pi, sc.sel, st));
+        if (w_ld != 0 && spectra) CUDA_TRY(forward_cost_curv_pw(b->d_basis, w, w_ld, m, E, b->W, b->Wp, sc.Cn, st));
+        if (w_ld != 0) CUDA_TRY(search_operand_pw(o, obs_ld, w, w_ld, sc.s, sc.Cn, m, E, sc.Ew, spectra, sc.op, st));
+        CUDA_TRY(search_topk(w_ld != 0 ? sc.op : sc.s, m, sc.Ew, sc.tbl, sc.ta, sc.Kp, k, sc.gy, sc.pv, sc.pi, sc.sel, st));
         for (int j = 0; j < k; ++j) {
             CUDA_TRY(search_gather(cand, D, sc.sel, k, j, m, sc.x, st));
-            int rc = cost_device(b, sc.x, m, o, obs_ld, weights, sc.cst + (int64_t)j * m, nullptr, nullptr, st, call_N);
+            int rc = cost_device(b, sc.x, m, o, obs_ld, w, w_ld, nullptr, sc.cst + (int64_t)j * m, nullptr, nullptr, st, call_N);
             if (rc) return rc;
         }
         CUDA_TRY(search_output(sc.sel, sc.cst, m, k, idx ? idx + p0 * k : nullptr, cost ? cost + p0 * k : nullptr, st));
@@ -1581,7 +1632,8 @@ int search_rows(gpe_bank* b, const SearchScratch& sc, bool spectra, const double
 
 // Request check of the search calls (device: obs_ld = 0 or >= the observation width; host: 0 or equal to it).
 int search_check(gpe_bank* b, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld, int k,
-                 const int64_t* idx, const double* cost, unsigned flags, bool host) {
+                 const int64_t* idx, const double* cost, unsigned flags, bool host, const double* weights = nullptr,
+                 int64_t w_ld = 0) {
     if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
     if (flags & ~(GPE_SOLVE_SPECTRA | GPE_HOST_PTRS)) return fail(GPE_ERR_INVALID, "unknown flag bits 0x%x", flags);
     const bool spectra = flags & GPE_SOLVE_SPECTRA;
@@ -1598,14 +1650,21 @@ int search_check(gpe_bank* b, const double* cand, int64_t K, const double* obs, 
     if (!idx && !cost) return fail(GPE_ERR_INVALID, "no output requested");
     if (search_smem(b->E) > kSmemMax || (spectra && forward_cost_smem(b->E) > kSmemMax) || b->E > 96)
         return fail(GPE_ERR_UNSUPPORTED, "the search supports banks of up to 96 emulators (got %d)", b->E);
+    int rc = weights_check(weights, w_ld, Kw, spectra, host);
+    if (rc) return rc;
+    if (w_ld != 0 && search_width(b->E, spectra, true) > 96)
+        return fail(GPE_ERR_UNSUPPORTED, "with per-point weights the %s search supports banks of up to %d emulators (got %d)",
+                    spectra ? "spectrum" : "band", spectra ? GPE_SEARCH_PW_MAX_E_SPECTRA : GPE_SEARCH_PW_MAX_E_BANDS, b->E);
     return GPE_OK;
 }
 
 // The streamed arrays of a host-resident search: per-point observations (unless shared) in; idx and cost (k 8-byte
 // columns each) out.
-CallIo search_io(int64_t Kw, const double* obs, int64_t obs_ld, int k, int64_t* idx, double* cost) {
+CallIo search_io(int64_t Kw, const double* obs, int64_t obs_ld, int k, int64_t* idx, double* cost, const double* weights = nullptr,
+                 int64_t w_ld = 0) {
     CallIo io;
     io.idx[0] = obs_ld != 0 ? io.in.add(obs, Kw) : -1;
+    io.idx[3] = w_ld != 0 ? io.in.add(weights, Kw) : -1;
     io.idx[1] = idx ? io.out.add(idx, k) : -1;
     io.idx[2] = cost ? io.out.add(cost, k) : -1;
     return io;
@@ -1615,10 +1674,10 @@ CallIo search_io(int64_t Kw, const double* obs, int64_t obs_ld, int k, int64_t* 
 // uploaded and the table is built once per call, then every chunk of pixels is searched on its slot's stream.  The
 // chunks share the per-pixel scratch: each waits for the previous one through search_free.
 int bank_search_stream(gpe_bank* b, bool spectra, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
-                       const double* weights, int k, const CallIo& io, const SharedCall* shared = nullptr) {
+                       const double* weights, int k, const CallIo& io, const SharedCall* shared = nullptr, int64_t w_ld = 0) {
     const int64_t D = b->D, Kw = spectra ? b->W : b->E;
     struct Part { const double* src; int64_t n; double* dev; };
-    Part parts[] = {{cand, K * D, nullptr}, {obs_ld == 0 ? obs : nullptr, Kw, nullptr}, {weights, Kw, nullptr}};
+    Part parts[] = {{cand, K * D, nullptr}, {obs_ld == 0 ? obs : nullptr, Kw, nullptr}, {w_ld == 0 ? weights : nullptr, Kw, nullptr}};
     size_t total = 0;
     for (const Part& p : parts) if (p.src) total += ((size_t)p.n + 31) & ~(size_t)31;
     int rc = ensure_buf((void**)&b->d_aux, &b->aux_cap, total * 8, false);
@@ -1632,7 +1691,7 @@ int bank_search_stream(gpe_bank* b, bool spectra, const double* cand, int64_t K,
     }
     std::lock_guard<std::mutex> lock(b->search_mu);
     SearchScratch sc;
-    rc = search_prepare(b, spectra, K, k, N, &sc);
+    rc = search_prepare(b, spectra, K, k, N, &sc, w_ld != 0);
     if (rc) return rc;
     CUDA_TRY(cudaStreamWaitEvent(cudaStreamLegacy, b->search_free, 0));
     rc = search_build_table(b, sc, spectra, parts[0].dev, K, parts[2].dev, parts[1].dev, cudaStreamLegacy);
@@ -1644,8 +1703,9 @@ int bank_search_stream(gpe_bank* b, bool spectra, const double* cand, int64_t K,
                        [&](int64_t, int64_t n, void* const* di, void* const* dout, cudaStream_t st) -> int {
                            CUDA_TRY(cudaStreamWaitEvent(st, b->search_free, 0));
                            const double* o = obs_ld != 0 ? io.at<const double>(di, 0) : parts[1].dev;
-                           int r = search_rows(b, sc, spectra, parts[0].dev, k, o, obs_ld != 0 ? Kw : 0, parts[2].dev, n, N,
-                                               io.at<int64_t>(dout, 1), io.at<double>(dout, 2), st);
+                           const double* w = w_ld != 0 ? io.at<const double>(di, 3) : parts[2].dev;
+                           int r = search_rows(b, sc, spectra, parts[0].dev, k, o, obs_ld != 0 ? Kw : 0, w, n, N,
+                                               io.at<int64_t>(dout, 1), io.at<double>(dout, 2), st, w_ld != 0 ? Kw : 0);
                            if (r) return r;
                            CUDA_TRY(cudaEventRecord(b->search_free, st));
                            return GPE_OK;
@@ -1656,13 +1716,17 @@ int bank_search_stream(gpe_bank* b, bool spectra, const double* cand, int64_t K,
 // Solve of N points on `st` (device arrays), in sub-chunks whose solver scratch stays within 256 MB.  Each iteration
 // evaluates the active trial points with the call's cost (cost, gradient and Hessian; call_N: the kernel plans follow the
 // call, never the active count), runs k_lm_step, compacts the active list in ascending order and reads its length back
-// through page-locked memory; the trial rows (and per-point observation rows, when the list shrank) of the survivors are
-// gathered for the next evaluation.  Synchronous: returns when the outputs are written.
+// through page-locked memory; the trial rows (and per-point observation and weight rows, when the list shrank) of the
+// survivors are gathered for the next evaluation.  Synchronous: returns when the outputs are written.
+//   Per-point weights with the spectrum cost: C_n depends on the weights only, so it is formed once per sub-chunk (Cs,
+// E^2 doubles a point) and gathered with the weight rows, never recomputed per iteration (DESIGN 4.6f).
 int bank_solve_device(gpe_bank* b, CostDevice cost_device, int64_t K, const LmProblem& pb, const double* x0, int64_t N,
                       const double* obs, int64_t obs_ld, const double* weights, double* x, double* cost, double* grad,
-                      double* hess, double* cov, int32_t* info, cudaStream_t st, int64_t call_N) {
-    const int64_t D = b->D, R = lm_state_doubles((int)D);
-    const int64_t per = R + D * D + 2 * D + 1 + (obs_ld > 0 ? K : 0) + 2;   // doubles per point, lists and flag included
+                      double* hess, double* cov, int32_t* info, cudaStream_t st, int64_t call_N, int64_t w_ld = 0) {
+    const int64_t D = b->D, R = lm_state_doubles((int)D), E = b->E;
+    const bool pw = w_ld > 0, curv = pw && cost_device == bank_forward_cost_device;
+    // doubles per point, lists and flag included
+    const int64_t per = R + D * D + 2 * D + 1 + (obs_ld > 0 ? K : 0) + (pw ? K : 0) + (curv ? 2 * E * E : 0) + 2;
     int64_t sub = std::max<int64_t>(1, std::min<int64_t>(N, (((int64_t)256 << 20) / 8) / per));
     if (const char* e = getenv("GPE_SOLVE_SUB_POINTS")) sub = std::max<int64_t>(1, std::min<int64_t>(sub, atoll(e)));   // dev aid: force sub-chunks in tests
     const size_t temp = lm_select_temp(sub);
@@ -1671,6 +1735,7 @@ int bank_solve_device(gpe_bank* b, CostDevice cost_device, int64_t K, const LmPr
     const size_t o_state = carve(8 * sub * R), o_xe = carve(8 * sub * D), o_fe = carve(8 * sub), o_ge = carve(8 * sub * D);
     const size_t o_he = carve(8 * sub * D * D), o_obs = carve(obs_ld > 0 ? 8 * sub * K : 0), o_l0 = carve(4 * sub);
     const size_t o_l1 = carve(4 * sub), o_flag = carve(4 * sub), o_cnt = carve(4), o_tmp = carve(temp);
+    const size_t o_w = carve(pw ? 8 * sub * K : 0), o_cs = carve(curv ? 8 * sub * E * E : 0), o_cc = carve(curv ? 8 * sub * E * E : 0);
     std::lock_guard<std::mutex> lock(b->solve_mu);
     int rc = ensure_buf(&b->solve_d, &b->solve_cap, off, false);
     if (rc) return rc;
@@ -1680,19 +1745,23 @@ int bank_solve_device(gpe_bank* b, CostDevice cost_device, int64_t K, const LmPr
     double* state = (double*)(base + o_state);
     double *xe = (double*)(base + o_xe), *fe = (double*)(base + o_fe), *ge = (double*)(base + o_ge), *he = (double*)(base + o_he);
     double* obs_c = (double*)(base + o_obs);
+    double *w_c = (double*)(base + o_w), *Cs = curv ? (double*)(base + o_cs) : nullptr, *C_c = (double*)(base + o_cc);
     int *lists[2] = {(int*)(base + o_l0), (int*)(base + o_l1)}, *flag = (int*)(base + o_flag), *d_cnt = (int*)(base + o_cnt);
     for (int64_t s0 = 0; s0 < N; s0 += sub) {
         const int64_t n = std::min(sub, N - s0);
         LmProblem p = pb;
         if (p.prior_mean && p.prior_ld > 0) p.prior_mean += s0 * p.prior_ld;
         const double* o = obs + s0 * obs_ld;
+        const double* w = pw ? weights + s0 * w_ld : weights;
         CUDA_TRY(lm_init(p, x0 + s0 * D, n, state, xe, lists[0], st));
+        if (curv) CUDA_TRY(forward_cost_curv_pw(b->d_basis, w, w_ld, n, (int)E, b->W, b->Wp, Cs, st));
         const double* e_obs = o;      // observation rows of the evaluation: the caller's while every point is active
-        int64_t e_ld = obs_ld, act = n;
+        const double *e_w = w, *e_C = Cs;
+        int64_t e_ld = obs_ld, e_wld = w_ld, act = n;
         for (int it = 0;; ++it) {
             int* list = lists[it & 1];
             int* next_list = lists[(it + 1) & 1];
-            rc = cost_device(b, xe, act, e_obs, e_ld, weights, fe, ge, he, st, call_N);
+            rc = cost_device(b, xe, act, e_obs, e_ld, e_w, e_wld, e_C, fe, ge, he, st, call_N);
             if (rc) return rc;
             CUDA_TRY(lm_step(p, act, list, fe, ge, he, state, flag, it == 0, st));
             CUDA_TRY(lm_select(list, flag, act, next_list, d_cnt, base + o_tmp, temp, st));
@@ -1704,6 +1773,11 @@ int bank_solve_device(gpe_bank* b, CostDevice cost_device, int64_t K, const LmPr
             const bool regather = obs_ld > 0 && next < act;
             CUDA_TRY(lm_gather(state, (int)D, next_list, next, xe, o, regather ? obs_ld : 0, K, obs_c, st));
             if (regather) { e_obs = obs_c; e_ld = K; }
+            if (pw && next < act) {
+                CUDA_TRY(lm_gather_rows(next_list, next, w, w_ld, K, w_c, st));
+                if (curv) CUDA_TRY(lm_gather_rows(next_list, next, Cs, E * E, E * E, C_c, st));
+                e_w = w_c; e_wld = K; e_C = curv ? C_c : nullptr;
+            }
             act = next;
         }
         CUDA_TRY(lm_output((int)D, n, state, x + s0 * D, cost ? cost + s0 : nullptr, grad ? grad + s0 * D : nullptr,
@@ -1766,14 +1840,16 @@ int solve_check(gpe_bank* b, int64_t N, const double* x0, const double* obs, int
 // cost / grad / hess / cov and info (8 bytes a point: one double-wide column) out.
 struct SolveIo {
     CallIo io;
-    int obs = -1, pm = -1, x = -1, cost = -1, grad = -1, hess = -1, cov = -1, info = -1;
+    int obs = -1, w = -1, pm = -1, x = -1, cost = -1, grad = -1, hess = -1, cov = -1, info = -1;
 };
 
 SolveIo solve_io(int64_t D, int64_t K, const double* x0, const double* obs, int64_t obs_ld, const gpe_solve_opts& o, double* x,
-                 double* cost, double* grad, double* hess, double* cov, int32_t* info) {
+                 double* cost, double* grad, double* hess, double* cov, int32_t* info, const double* weights = nullptr,
+                 int64_t w_ld = 0) {
     SolveIo s;
     s.io.in.add(x0, D);
     if (obs_ld != 0) s.obs = s.io.in.add(obs, K);
+    if (w_ld != 0) s.w = s.io.in.add(weights, K);
     if (o.prior_mean && o.prior_ld != 0) s.pm = s.io.in.add(o.prior_mean, D);
     s.x = s.io.out.add(x, D);
     if (cost) s.cost = s.io.out.add(cost, 1);
@@ -1791,7 +1867,7 @@ int bank_solve_stream(gpe_bank* b, bool spectra, int64_t N, const double* obs, i
                       const gpe_solve_opts& o, const SolveIo& s, const SharedCall* shared = nullptr) {
     const int64_t D = b->D, K = spectra ? b->W : b->E;
     struct Part { const double* src; int64_t n; double* dev; };
-    Part parts[] = {{obs_ld == 0 ? obs : nullptr, K, nullptr}, {weights, K, nullptr}, {o.lower, D, nullptr},
+    Part parts[] = {{obs_ld == 0 ? obs : nullptr, K, nullptr}, {s.w < 0 ? weights : nullptr, K, nullptr}, {o.lower, D, nullptr},
                     {o.upper, D, nullptr}, {o.prior_ld == 0 ? o.prior_mean : nullptr, D, nullptr}, {o.prior_prec, D * D, nullptr}};
     size_t total = 0;
     for (const Part& p : parts) if (p.src) total += (size_t)p.n;
@@ -1817,8 +1893,9 @@ int bank_solve_stream(gpe_bank* b, bool spectra, int64_t N, const double* obs, i
                            auto out = [&](int k) { return k >= 0 ? (double*)dout[k] : nullptr; };
                            return bank_solve_device(b, spectra ? bank_forward_cost_device : bank_cost_device, K, p,
                                                     (const double*)di[0], n, s.obs >= 0 ? (const double*)di[s.obs] : parts[0].dev,
-                                                    obs_ld != 0 ? K : 0, parts[1].dev, out(s.x), out(s.cost), out(s.grad),
-                                                    out(s.hess), out(s.cov), (int32_t*)dout[s.info], st, N);
+                                                    obs_ld != 0 ? K : 0, s.w >= 0 ? (const double*)di[s.w] : parts[1].dev,
+                                                    out(s.x), out(s.cost), out(s.grad), out(s.hess), out(s.cov),
+                                                    (int32_t*)dout[s.info], st, N, s.w >= 0 ? K : 0);
                        });
 }
 
@@ -2020,6 +2097,58 @@ int fan_out(gpe_multi* mm, const std::vector<Owner*>& owners, int sms, const Cal
     });
 }
 
+// The cost calls of one bank (band cost, or spectra with GPE_SOLVE_SPECTRA; host arrays with GPE_HOST_PTRS).
+int bank_cost_call(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                   int64_t w_ld, double* cost, double* grad, double* hess, unsigned flags, void* stream) {
+    const bool host = flags & GPE_HOST_PTRS, spectra = flags & GPE_SOLVE_SPECTRA;
+    if (spectra) {
+        int rc = forward_cost_check(b, N, testing, obs, obs_ld, cost, grad, hess);
+        if (rc || N == 0) return rc;
+    } else {
+        if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
+        if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
+        if (N == 0) return GPE_OK;
+        if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
+        if (!cost && !grad && !hess) return fail(GPE_ERR_INVALID, "no output requested");
+        if (!host && obs_ld != 0 && obs_ld < b->E) return fail(GPE_ERR_INVALID, "obs_ld must be 0 (one observation vector) or >= E");
+    }
+    const int64_t K = spectra ? b->W : b->E;
+    int rc = weights_check(weights, w_ld, K, spectra, host);
+    if (rc) return rc;
+    CUDA_TRY(cudaSetDevice(b->device));
+    const CostDevice cost_device = spectra ? bank_forward_cost_device : bank_cost_device;
+    if (host) {
+        std::lock_guard<std::mutex> lock(b->host_mu);
+        return bank_cost_stream(b, K, cost_device, N, obs, obs_ld, weights,
+                                cost_io(b, K, testing, obs, obs_ld, cost, grad, hess, weights, w_ld), nullptr, w_ld);
+    }
+    return cost_device(b, testing, N, obs, obs_ld, weights, w_ld, nullptr, cost, grad, hess, (cudaStream_t)stream, -1);
+}
+
+// The same on every device of a bank handle (host arrays).
+int multi_bank_cost_call(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                         int64_t w_ld, double* cost, double* grad, double* hess, bool spectra) {
+    if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
+    gpe_bank* b0 = mm->banks[0];
+    if (spectra) {
+        int rc = forward_cost_check(b0, N, testing, obs, obs_ld, cost, grad, hess);
+        if (rc || N == 0) return rc;
+    } else {
+        if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
+        if (N == 0) return GPE_OK;
+        if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
+        if (!cost && !grad && !hess) return fail(GPE_ERR_INVALID, "no output requested");
+    }
+    const int64_t K = spectra ? b0->W : b0->E;
+    int rc = weights_check(weights, w_ld, K, spectra, true);
+    if (rc) return rc;
+    const CostDevice cost_device = spectra ? bank_forward_cost_device : bank_cost_device;
+    const CallIo io = cost_io(b0, K, testing, obs, obs_ld, cost, grad, hess, weights, w_ld);
+    return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
+        return bank_cost_stream(b, K, cost_device, N, obs, obs_ld, weights, io, shared, w_ld);
+    });
+}
+
 }  // namespace
 
 extern "C" {
@@ -2150,14 +2279,14 @@ int gpe_bank_predict(gpe_bank* b, const double* testing, int64_t N, double* mu, 
 int gpe_bank_cost_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
                      double* cost, double* grad, double* hess, void* stream) {
     NvtxRange nvtx_range("gpe_bank_cost");
-    if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
-    if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
-    if (N == 0) return GPE_OK;
-    if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
-    if (!cost && !grad && !hess) return fail(GPE_ERR_INVALID, "no output requested");
-    if (obs_ld != 0 && obs_ld < b->E) return fail(GPE_ERR_INVALID, "obs_ld must be 0 (one observation vector) or >= E");
-    CUDA_TRY(cudaSetDevice(b->device));
-    return bank_cost_device(b, testing, N, obs, obs_ld, weights, cost, grad, hess, (cudaStream_t)stream);
+    return bank_cost_call(b, testing, N, obs, obs_ld, weights, 0, cost, grad, hess, 0u, stream);
+}
+
+int gpe_bank_cost_pw(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                     int64_t weights_ld, double* cost, double* grad, double* hess, unsigned flags, void* stream) {
+    NvtxRange nvtx_range("gpe_bank_cost_pw");
+    if (flags & ~(GPE_SOLVE_SPECTRA | GPE_HOST_PTRS)) return fail(GPE_ERR_INVALID, "unknown flag bits 0x%x", flags);
+    return bank_cost_call(b, testing, N, obs, obs_ld, weights, weights_ld, cost, grad, hess, flags, stream);
 }
 
 int gpe_bank_cost(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
@@ -2168,15 +2297,7 @@ int gpe_bank_cost(gpe_bank* b, const double* testing, int64_t N, const double* o
 int gpe_bank_cost_host_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                           const double* weights, double* cost, double* grad, double* hess) {
     NvtxRange nvtx_range("gpe_bank_cost_host");
-    if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
-    if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
-    if (N == 0) return GPE_OK;
-    if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
-    if (!cost && !grad && !hess) return fail(GPE_ERR_INVALID, "no output requested");
-    CUDA_TRY(cudaSetDevice(b->device));
-    std::lock_guard<std::mutex> lock(b->host_mu);
-    return bank_cost_stream(b, b->E, bank_cost_device, N, obs, obs_ld, weights,
-                            cost_io(b, b->E, testing, obs, obs_ld, cost, grad, hess));
+    return bank_cost_call(b, testing, N, obs, obs_ld, weights, 0, cost, grad, hess, GPE_HOST_PTRS, nullptr);
 }
 
 int gpe_bank_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
@@ -2187,10 +2308,7 @@ int gpe_bank_cost_host(gpe_bank* b, const double* testing, int64_t N, const doub
 int gpe_bank_forward_cost_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                              const double* weights, double* cost, double* grad, double* hess, void* stream) {
     NvtxRange nvtx_range("gpe_bank_forward_cost");
-    int rc = forward_cost_check(b, N, testing, obs, obs_ld, cost, grad, hess);
-    if (rc || N == 0) return rc;
-    CUDA_TRY(cudaSetDevice(b->device));
-    return bank_forward_cost_device(b, testing, N, obs, obs_ld, weights, cost, grad, hess, (cudaStream_t)stream);
+    return bank_cost_call(b, testing, N, obs, obs_ld, weights, 0, cost, grad, hess, GPE_SOLVE_SPECTRA, stream);
 }
 
 int gpe_bank_forward_cost(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
@@ -2201,12 +2319,7 @@ int gpe_bank_forward_cost(gpe_bank* b, const double* testing, int64_t N, const d
 int gpe_bank_forward_cost_host_ex(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                                   const double* weights, double* cost, double* grad, double* hess) {
     NvtxRange nvtx_range("gpe_bank_forward_cost_host");
-    int rc = forward_cost_check(b, N, testing, obs, obs_ld, cost, grad, hess);
-    if (rc || N == 0) return rc;
-    CUDA_TRY(cudaSetDevice(b->device));
-    std::lock_guard<std::mutex> lock(b->host_mu);
-    return bank_cost_stream(b, b->W, bank_forward_cost_device, N, obs, obs_ld, weights,
-                            cost_io(b, b->W, testing, obs, obs_ld, cost, grad, hess));
+    return bank_cost_call(b, testing, N, obs, obs_ld, weights, 0, cost, grad, hess, GPE_SOLVE_SPECTRA | GPE_HOST_PTRS, nullptr);
 }
 
 int gpe_bank_forward_cost_host(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
@@ -2214,49 +2327,62 @@ int gpe_bank_forward_cost_host(gpe_bank* b, const double* testing, int64_t N, co
     return gpe_bank_forward_cost_host_ex(b, testing, N, obs, obs_ld, weights, cost, grad, nullptr);
 }
 
-int gpe_bank_solve(gpe_bank* b, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
-                   const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess, double* cov,
-                   int32_t* info, unsigned flags, void* stream) {
+int gpe_bank_solve_pw(gpe_bank* b, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                      int64_t weights_ld, const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess,
+                      double* cov, int32_t* info, unsigned flags, void* stream) {
     NvtxRange nvtx_range("gpe_bank_solve");
     const bool host = flags & GPE_HOST_PTRS, spectra = flags & GPE_SOLVE_SPECTRA;
     gpe_solve_opts o;
     int rc = solve_check(b, N, x0, obs, obs_ld, opts, x, info, flags, host, (cudaStream_t)stream, &o);
+    if (rc == GPE_OK) rc = weights_check(weights, weights_ld, spectra ? b->W : b->E, spectra, host);
     if (rc || N == 0) return rc;
     CUDA_TRY(cudaSetDevice(b->device));
     const int64_t D = b->D, K = spectra ? b->W : b->E;
     if (host) {
         std::lock_guard<std::mutex> lock(b->host_mu);
         return bank_solve_stream(b, spectra, N, obs, obs_ld, weights, o,
-                                 solve_io(D, K, x0, obs, obs_ld, o, x, cost, grad, hess, cov, info));
+                                 solve_io(D, K, x0, obs, obs_ld, o, x, cost, grad, hess, cov, info, weights, weights_ld));
     }
     const LmProblem pb = lm_problem((int)D, o, o.lower, o.upper, o.prior_mean, o.prior_ld, o.prior_prec);
     return bank_solve_device(b, spectra ? bank_forward_cost_device : bank_cost_device, K, pb, x0, N, obs, obs_ld, weights, x,
-                             cost, grad, hess, cov, info, (cudaStream_t)stream, N);
+                             cost, grad, hess, cov, info, (cudaStream_t)stream, N, weights_ld);
 }
 
-int gpe_bank_search(gpe_bank* b, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
-                    const double* weights, int k, int64_t* idx, double* cost, unsigned flags, void* stream) {
+int gpe_bank_solve(gpe_bank* b, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                   const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess, double* cov,
+                   int32_t* info, unsigned flags, void* stream) {
+    return gpe_bank_solve_pw(b, x0, N, obs, obs_ld, weights, 0, opts, x, cost, grad, hess, cov, info, flags, stream);
+}
+
+int gpe_bank_search_pw(gpe_bank* b, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                       const double* weights, int64_t weights_ld, int k, int64_t* idx, double* cost, unsigned flags, void* stream) {
     NvtxRange nvtx_range("gpe_bank_search");
     const bool host = flags & GPE_HOST_PTRS, spectra = flags & GPE_SOLVE_SPECTRA;
-    int rc = search_check(b, cand, K, obs, N, obs_ld, k, idx, cost, flags, host);
+    int rc = search_check(b, cand, K, obs, N, obs_ld, k, idx, cost, flags, host, weights, weights_ld);
     if (rc || N == 0) return rc;
     CUDA_TRY(cudaSetDevice(b->device));
     if (host) {
         std::lock_guard<std::mutex> lock(b->host_mu);
         return bank_search_stream(b, spectra, cand, K, obs, N, obs_ld, weights, k,
-                                  search_io(spectra ? b->W : b->E, obs, obs_ld, k, idx, cost));
+                                  search_io(spectra ? b->W : b->E, obs, obs_ld, k, idx, cost, weights, weights_ld), nullptr,
+                                  weights_ld);
     }
     const cudaStream_t st = (cudaStream_t)stream;
     std::lock_guard<std::mutex> lock(b->search_mu);
     SearchScratch sc;
-    rc = search_prepare(b, spectra, K, k, N, &sc);
+    rc = search_prepare(b, spectra, K, k, N, &sc, weights_ld != 0);
     if (rc) return rc;
     CUDA_TRY(cudaStreamWaitEvent(st, b->search_free, 0));
     rc = search_build_table(b, sc, spectra, cand, K, weights, obs_ld == 0 ? obs : nullptr, st);
-    if (rc == GPE_OK) rc = search_rows(b, sc, spectra, cand, k, obs, obs_ld, weights, N, N, idx, cost, st);
+    if (rc == GPE_OK) rc = search_rows(b, sc, spectra, cand, k, obs, obs_ld, weights, N, N, idx, cost, st, weights_ld);
     if (rc) return rc;
     CUDA_TRY(cudaEventRecord(b->search_free, st));
     return GPE_OK;
+}
+
+int gpe_bank_search(gpe_bank* b, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                    const double* weights, int k, int64_t* idx, double* cost, unsigned flags, void* stream) {
+    return gpe_bank_search_pw(b, cand, K, obs, N, obs_ld, weights, 0, k, idx, cost, flags, stream);
 }
 
 int gpe_bank_project(gpe_bank* b, const double* mu, const double* deriv, int64_t N, double* fwd, double* deriv_full,
@@ -2390,16 +2516,14 @@ int gpe_multi_bank_predict(gpe_multi* mm, const double* testing, int64_t N, doub
 int gpe_multi_bank_cost_ex(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                            const double* weights, double* cost, double* grad, double* hess) {
     NvtxRange nvtx_range("gpe_multi_bank_cost");
-    if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
-    if (N < 0) return fail(GPE_ERR_INVALID, "N must be >= 0");
-    if (N == 0) return GPE_OK;
-    if (!testing || !obs) return fail(GPE_ERR_INVALID, "testing / obs is NULL");
-    if (!cost && !grad && !hess) return fail(GPE_ERR_INVALID, "no output requested");
-    gpe_bank* b0 = mm->banks[0];
-    const CallIo io = cost_io(b0, b0->E, testing, obs, obs_ld, cost, grad, hess);
-    return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
-        return bank_cost_stream(b, b->E, bank_cost_device, N, obs, obs_ld, weights, io, shared);
-    });
+    return multi_bank_cost_call(mm, testing, N, obs, obs_ld, weights, 0, cost, grad, hess, false);
+}
+
+int gpe_multi_bank_cost_pw(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                           const double* weights, int64_t weights_ld, double* cost, double* grad, double* hess, unsigned flags) {
+    NvtxRange nvtx_range("gpe_multi_bank_cost_pw");
+    if (flags & ~(GPE_SOLVE_SPECTRA | GPE_HOST_PTRS)) return fail(GPE_ERR_INVALID, "unknown flag bits 0x%x", flags);
+    return multi_bank_cost_call(mm, testing, N, obs, obs_ld, weights, weights_ld, cost, grad, hess, flags & GPE_SOLVE_SPECTRA);
 }
 
 int gpe_multi_bank_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
@@ -2410,14 +2534,7 @@ int gpe_multi_bank_cost(gpe_multi* mm, const double* testing, int64_t N, const d
 int gpe_multi_bank_forward_cost_ex(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
                                    const double* weights, double* cost, double* grad, double* hess) {
     NvtxRange nvtx_range("gpe_multi_bank_forward_cost");
-    if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
-    gpe_bank* b0 = mm->banks[0];
-    int rc = forward_cost_check(b0, N, testing, obs, obs_ld, cost, grad, hess);
-    if (rc || N == 0) return rc;
-    const CallIo io = cost_io(b0, b0->W, testing, obs, obs_ld, cost, grad, hess);
-    return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
-        return bank_cost_stream(b, b->W, bank_forward_cost_device, N, obs, obs_ld, weights, io, shared);
-    });
+    return multi_bank_cost_call(mm, testing, N, obs, obs_ld, weights, 0, cost, grad, hess, true);
 }
 
 int gpe_multi_bank_forward_cost(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
@@ -2428,14 +2545,22 @@ int gpe_multi_bank_forward_cost(gpe_multi* mm, const double* testing, int64_t N,
 int gpe_multi_bank_solve(gpe_multi* mm, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
                          const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess, double* cov,
                          int32_t* info, unsigned flags) {
+    return gpe_multi_bank_solve_pw(mm, x0, N, obs, obs_ld, weights, 0, opts, x, cost, grad, hess, cov, info, flags);
+}
+
+int gpe_multi_bank_solve_pw(gpe_multi* mm, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                            int64_t weights_ld, const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess,
+                            double* cov, int32_t* info, unsigned flags) {
     NvtxRange nvtx_range("gpe_multi_bank_solve");
     if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
     gpe_bank* b0 = mm->banks[0];
     const bool spectra = flags & GPE_SOLVE_SPECTRA;
     gpe_solve_opts o;
     int rc = solve_check(b0, N, x0, obs, obs_ld, opts, x, info, flags, true, nullptr, &o);
+    if (rc == GPE_OK) rc = weights_check(weights, weights_ld, spectra ? b0->W : b0->E, spectra, true);
     if (rc || N == 0) return rc;
-    const SolveIo s = solve_io(b0->D, spectra ? b0->W : b0->E, x0, obs, obs_ld, o, x, cost, grad, hess, cov, info);
+    const SolveIo s = solve_io(b0->D, spectra ? b0->W : b0->E, x0, obs, obs_ld, o, x, cost, grad, hess, cov, info, weights,
+                               weights_ld);
     return fan_out(mm, mm->banks, b0->models[0]->sms, s.io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
         return bank_solve_stream(b, spectra, N, obs, obs_ld, weights, o, s, shared);
     });
@@ -2443,16 +2568,21 @@ int gpe_multi_bank_solve(gpe_multi* mm, const double* x0, int64_t N, const doubl
 
 int gpe_multi_bank_search(gpe_multi* mm, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
                           const double* weights, int k, int64_t* idx, double* cost, unsigned flags) {
+    return gpe_multi_bank_search_pw(mm, cand, K, obs, N, obs_ld, weights, 0, k, idx, cost, flags);
+}
+
+int gpe_multi_bank_search_pw(gpe_multi* mm, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                             const double* weights, int64_t weights_ld, int k, int64_t* idx, double* cost, unsigned flags) {
     NvtxRange nvtx_range("gpe_multi_bank_search");
     if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
     gpe_bank* b0 = mm->banks[0];
     const bool spectra = flags & GPE_SOLVE_SPECTRA;
-    int rc = search_check(b0, cand, K, obs, N, obs_ld, k, idx, cost, flags, true);
+    int rc = search_check(b0, cand, K, obs, N, obs_ld, k, idx, cost, flags, true, weights, weights_ld);
     if (rc || N == 0) return rc;
-    const CallIo io = search_io(spectra ? b0->W : b0->E, obs, obs_ld, k, idx, cost);
+    const CallIo io = search_io(spectra ? b0->W : b0->E, obs, obs_ld, k, idx, cost, weights, weights_ld);
     // every device builds its own, identical candidate table
     return fan_out(mm, mm->banks, b0->models[0]->sms, io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
-        return bank_search_stream(b, spectra, cand, K, obs, N, obs_ld, weights, k, io, shared);
+        return bank_search_stream(b, spectra, cand, K, obs, N, obs_ld, weights, k, io, shared, weights_ld);
     });
 }
 

@@ -253,6 +253,15 @@ __global__ void k_lm_gather(const double* __restrict__ state, int D, const int* 
     }
 }
 
+// dst[i] (K) = src row list[i] (rows ld apart): the per-point weight rows and curvatures of the survivors (DESIGN 4.6f).
+__global__ void k_lm_gather_rows(const int* __restrict__ list, int64_t n, const double* __restrict__ src, int64_t ld, int64_t K,
+                                 double* __restrict__ dst) {
+    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n * K; k += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t i = k / K, c = k - i * K;
+        dst[k] = src[list[i] * ld + c];
+    }
+}
+
 // Outputs of point p (one warp).
 template <int DP>
 __device__ __forceinline__ void lm_output_point(int D, int64_t p, const double* __restrict__ state, double* __restrict__ x,
@@ -333,6 +342,11 @@ cudaError_t lm_gather(const double* state, int D, const int* list, int64_t n, do
     if (n <= 0) return cudaSuccess;
     return launch_kernel(k_lm_gather, grid_for(n * (D + (obs_ld > 0 ? K : 0)), 256), 256, 0, st, state, D, list, n, xe, obs,
                          obs_ld, K, obs_out);
+}
+
+cudaError_t lm_gather_rows(const int* list, int64_t n, const double* src, int64_t ld, int64_t K, double* dst, cudaStream_t st) {
+    if (n <= 0) return cudaSuccess;
+    return launch_kernel(k_lm_gather_rows, grid_for(n * K, 256), 256, 0, st, list, n, src, ld, K, dst);
 }
 
 cudaError_t lm_output(int D, int64_t n, const double* state, double* x, double* cost, double* grad, double* hess, double* cov,

@@ -33,6 +33,8 @@ cudaError_t lm_select(const int* list, const int* flag, int64_t n, int* list_out
 // xe[i] = xt of point list[i]; with obs_ld > 0 also obs_out[i] (K) = obs row list[i].
 cudaError_t lm_gather(const double* state, int D, const int* list, int64_t n, double* xe, const double* obs, int64_t obs_ld,
                       int64_t K, double* obs_out, cudaStream_t st);
+// dst[i] (K) = src row list[i], rows ld apart.
+cudaError_t lm_gather_rows(const int* list, int64_t n, const double* src, int64_t ld, int64_t K, double* dst, cudaStream_t st);
 // Outputs of n points from their state (any pointer but info may be NULL); cov = inv(H), NaN where H is not positive
 // definite, symmetric bit for bit.
 cudaError_t lm_output(int D, int64_t n, const double* state, double* x, double* cost, double* grad, double* hess, double* cov,

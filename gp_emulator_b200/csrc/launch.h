@@ -70,12 +70,16 @@ cudaError_t project_rows(const double* A, int64_t R, int RD, int64_t ldn, int64_
 // means mu (R, E) and gradients deriv (R, E, D); obs (R, obs_ld) or, obs_ld = 0, the shared observation in aux.
 // aux (2 Wp) is filled by forward_cost_aux: weights (NULL: 1) and the shared observation (NULL: none), zero-padded to Wp.
 cudaError_t forward_cost_aux(const double* weights, const double* obs1, int W, int Wp, double* aux, cudaStream_t st);
-// s_out (R, E) or NULL: with it, s = (l o (fwd - obs)) . basis^T is stored too, and grad may be NULL.
+// s_out (R, E) or NULL: with it, s = (l o (fwd - obs)) . basis^T is stored too, and grad may be NULL.  w_ld != 0: per-point
+// weights, row r at wts + r w_ld (the weights in aux are not read).
 cudaError_t forward_cost_rows(const double* mu, const double* deriv, int64_t R, int E, int D, const double* obs, int64_t obs_ld,
                               const double* aux, const double* b_tiled, int W, int Wp, int gy, double* part, double* cost,
-                              double* grad, double* s_out, cudaStream_t st);
+                              double* grad, double* s_out, cudaStream_t st, const double* wts = nullptr, int64_t w_ld = 0);
 // C (E, E) = basis . diag(weights in aux) . basis^T, exactly symmetric.
 cudaError_t forward_cost_curv(const double* b_tiled, const double* aux, int E, int Wp, double* C, cudaStream_t st);
+// C (n, E, E): per point n, basis . diag(wts row n, rows w_ld apart) . basis^T, summed in the order of forward_cost_curv.
+cudaError_t forward_cost_curv_pw(const double* b_tiled, const double* wts, int64_t w_ld, int64_t n, int E, int W, int Wp, double* C,
+                                cudaStream_t st);
 size_t forward_cost_smem(int E);   // dynamic shared memory of forward_cost_rows for a bank of E emulators
 // Column split gy of forward_cost_rows for a call of call_N points: > 1 (the column groups spread over gy CTAs per row tile,
 // partial sums in part (gy, R, 1 + E)) when the row tiles alone leave most SMs idle.  A function of the call, not of a chunk.
@@ -93,6 +97,11 @@ int search_split(int64_t call_N, int64_t K);
 // spectrum cost with C (E, E) otherwise
 cudaError_t search_table(const double* mu, int64_t K, int E, int Kp, const double* w, const double* C, double* tbl, double* ta,
                          cudaStream_t st);
+// Per-point weights (DESIGN 4.6f): the table of the wider operand, Ew = 2E (band) or E(E+1)/2 + E (spectrum), with a_k = 0
+cudaError_t search_table_pw(const double* mu, int64_t K, int E, int Ew, int Kp, bool spectra, double* tbl, double* ta, cudaStream_t st);
+// ... and its pixel operand op (R, Ew): band [w_r, -(w_r o obs_r)], spectrum [C_r upper triangle, diagonal halved, s_r]
+cudaError_t search_operand_pw(const double* obs, int64_t obs_ld, const double* w, int64_t w_ld, const double* s, const double* Cn,
+                              int64_t R, int E, int Ew, bool spectra, double* op, cudaStream_t st);
 // Band-cost pixel operand s (R, E) = -(w o obs)
 cudaError_t search_band_s(const double* obs, int64_t obs_ld, const double* w, int64_t R, int E, double* s, cudaStream_t st);
 // sel (R, k): per row the k candidates of the smallest a_k + s_r . m_k, in (score, index) order, -1 where none is left

@@ -312,14 +312,17 @@ __global__ void __launch_bounds__(WRG * 128, (KS <= 5 ? (WRG == 1 ? 3 : 2) : 1))
 //   aux = [weights padded to Wp with zeros | shared observation padded to Wp], so the tail group adds exact zeros.
 //   HESS (with GRAD): s itself goes to s_out (R, E) as well, the curvature coefficients of the cost's Hessian
 //   (k_cost_hess); grad may then be NULL.
+//   PW: per-point weights, row r of wts at r * w_ld, loaded beside the observations (zero past W) and used in place of
+//   the weights in aux; the product l_rw r_rw is the same one, so rows equal to the shared weights give the same bits.
 constexpr int kFcThreads = 256, kFcRows = 32, kFcPitch = 33;
-template <int KS, bool GRAD, bool HESS>
-__global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost(const double* __restrict__ mu, const double* __restrict__ deriv,
-                                                                int64_t R, int E, int D, const double* __restrict__ obs,
-                                                                int64_t obs_ld, const double* __restrict__ aux,
-                                                                const double* __restrict__ b_tiled, int W, int Wp, int nsl,
-                                                                double* __restrict__ cost, double* __restrict__ grad,
-                                                                double* __restrict__ part, double* __restrict__ s_out) {
+template <int KS, bool GRAD, bool HESS, bool PW>
+__device__ __forceinline__ void forward_cost_body(const double* __restrict__ mu, const double* __restrict__ deriv,
+                                                  int64_t R, int E, int D, const double* __restrict__ obs,
+                                                  int64_t obs_ld, const double* __restrict__ aux,
+                                                  const double* __restrict__ b_tiled, int W, int Wp, int nsl,
+                                                  double* __restrict__ cost, double* __restrict__ grad,
+                                                  double* __restrict__ part, double* __restrict__ s_out,
+                                                  const double* __restrict__ wts, int64_t w_ld) {
     extern __shared__ __align__(128) unsigned char psm[];
     constexpr int NT = KS / 2;                                   // n-tiles of 8 emulators per slice of s
     const int kstg = nsl == 1 ? KS : 8 * nsl;                    // k-steps staged per column group
@@ -371,6 +374,7 @@ __global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost(const double* __
     // of the warp's 32], zero past W
     const double* obs1 = obs_ld == 0 ? aux + Wp : nullptr;
     double ob[2][4][2];
+    double lw[2][4][2];                                          // PW: the weights of the same elements
     auto load_obs = [&](int g) {
         const int c0 = g * kProjCols + wc * 32 + 2 * (lane & 3);
 #pragma unroll
@@ -382,6 +386,7 @@ __global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost(const double* __
                 for (int h = 0; h < 2; ++h) {
                     const int w = c0 + 8 * j + h;
                     ob[i][j][h] = obs1 ? obs1[w] : ((r < R && w < W) ? obs[r * obs_ld + w] : 0.0);
+                    if (PW) lw[i][j][h] = (r < R && w < W) ? wts[r * w_ld + w] : 0.0;
                 }
         }
     };
@@ -434,7 +439,7 @@ __global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost(const double* __
 #pragma unroll
                 for (int h = 0; h < 2; ++h) {
                     const double r = f[i][j][h] - ob[i][j][h];
-                    const double u = aux[c0 + 8 * j + h] * r;
+                    const double u = (PW ? lw[i][j][h] : aux[c0 + 8 * j + h]) * r;
                     if (so == 0) c[i] = fma(u, r, c[i]);
                     f[i][j][h] = u;
                 }
@@ -517,6 +522,30 @@ __global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost(const double* __
     }
 }
 
+template <int KS, bool GRAD, bool HESS>
+__global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost(const double* __restrict__ mu, const double* __restrict__ deriv,
+                                                                int64_t R, int E, int D, const double* __restrict__ obs,
+                                                                int64_t obs_ld, const double* __restrict__ aux,
+                                                                const double* __restrict__ b_tiled, int W, int Wp, int nsl,
+                                                                double* __restrict__ cost, double* __restrict__ grad,
+                                                                double* __restrict__ part, double* __restrict__ s_out) {
+    forward_cost_body<KS, GRAD, HESS, false>(mu, deriv, R, E, D, obs, obs_ld, aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out,
+                                             nullptr, 0);
+}
+
+// Per-point weights (DESIGN 4.6f): wts (R, w_ld), l_rw = wts[r * w_ld + w].
+template <int KS, bool GRAD, bool HESS>
+__global__ void __launch_bounds__(kFcThreads, 1) k_forward_cost_pw(const double* __restrict__ mu, const double* __restrict__ deriv,
+                                                                   int64_t R, int E, int D, const double* __restrict__ obs,
+                                                                   int64_t obs_ld, const double* __restrict__ aux,
+                                                                   const double* __restrict__ b_tiled, int W, int Wp, int nsl,
+                                                                   double* __restrict__ cost, double* __restrict__ grad,
+                                                                   double* __restrict__ part, double* __restrict__ s_out,
+                                                                   const double* __restrict__ wts, int64_t w_ld) {
+    forward_cost_body<KS, GRAD, HESS, true>(mu, deriv, R, E, D, obs, obs_ld, aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out,
+                                            wts, w_ld);
+}
+
 // aux = [weights or 1, zero past W | shared observation, zero past W] (one launch per call)
 __global__ void k_forward_cost_aux(const double* __restrict__ weights, const double* __restrict__ obs1, int W, int Wp,
                                    double* __restrict__ aux) {
@@ -543,6 +572,65 @@ __global__ void k_forward_cost_curv(const double* __restrict__ b_tiled, const do
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
         if (lane == 0) C[(int64_t)e * E + f] = C[(int64_t)f * E + e] = v;
+    }
+}
+
+// Per-point curvature (DESIGN 4.6f): C_n (E, E) = basis . diag(l_n) . basis^T for the rows l_n = wts[n * w_ld + .] (zero past
+// W), summed exactly as k_forward_cost_curv sums C: lane L adds fma(b_ew l_nw, b_fw, v) over w = L, L + 32, ... < Wp in
+// order, then the same xor butterfly, so a row equal to the shared weights gives the shared C bit for bit.  One warp
+// takes a 4 x 4 tile of entries (e in block a, f in block c >= a) of one point: every lane keeps 16 sums, and per w it
+// loads l once and the two 4-wide basis columns once.  Consecutive warps take the same tile of consecutive points, so a
+// CTA reads each basis column from L1 for 8 points.  Entries e <= f < E are written to (e, f) and (f, e).
+__global__ void __launch_bounds__(256) k_forward_cost_curv_pw(const double* __restrict__ b_tiled, const double* __restrict__ wts,
+                                                              int64_t w_ld, int64_t n, int E, int W, int Wp,
+                                                              double* __restrict__ C) {
+    const int lane = threadIdx.x & 31, nb = (E + 3) / 4, ntile = nb * (nb + 1) / 2;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; k < n * ntile; k += nwarps) {
+        const int t = (int)(k / n);
+        const int64_t p = k - (int64_t)t * n;
+        int a = 0, q = t;
+        while (q >= nb - a) { q -= nb - a; ++a; }
+        const int c = a + q;
+        const double* ba = b_tiled + (size_t)a * Wp * 4;
+        const double* bc = b_tiled + (size_t)c * Wp * 4;
+        const double* l = wts + p * w_ld;
+        double v[4][4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+#pragma unroll
+            for (int j = 0; j < 4; ++j) v[i][j] = 0.0;
+        for (int w = lane; w < Wp; w += 32) {
+            const double lw = w < W ? l[w] : 0.0;
+            const double2 e01 = *reinterpret_cast<const double2*>(ba + 4 * (size_t)w);
+            const double2 e23 = *reinterpret_cast<const double2*>(ba + 4 * (size_t)w + 2);
+            const double2 f01 = *reinterpret_cast<const double2*>(bc + 4 * (size_t)w);
+            const double2 f23 = *reinterpret_cast<const double2*>(bc + 4 * (size_t)w + 2);
+            const double be[4] = {e01.x * lw, e01.y * lw, e23.x * lw, e23.y * lw}, bf[4] = {f01.x, f01.y, f23.x, f23.y};
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) v[i][j] = fma(be[i], bf[j], v[i][j]);
+        }
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) v[i][j] += __shfl_xor_sync(0xffffffffu, v[i][j], o);
+            }
+        if (lane < 16) {
+            double out = 0.0;
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) if (lane == 4 * i + j) out = v[i][j];
+            const int e = 4 * a + (lane >> 2), f = 4 * c + (lane & 3);
+            if (e <= f && f < E) {
+                double* Cp = C + p * E * E;
+                Cp[(int64_t)e * E + f] = Cp[(int64_t)f * E + e] = out;
+            }
+        }
     }
 }
 
@@ -595,9 +683,18 @@ cudaError_t forward_cost_curv(const double* b_tiled, const double* aux, int E, i
     return launch_kernel(k_forward_cost_curv, (unsigned)std::min<int64_t>((warps + 7) / 8, 4096), 256, 0, st, b_tiled, aux, E, Wp, C);
 }
 
+cudaError_t forward_cost_curv_pw(const double* b_tiled, const double* wts, int64_t w_ld, int64_t n, int E, int W, int Wp, double* C,
+                                cudaStream_t st) {
+    if (n <= 0) return cudaSuccess;
+    const int nb = (E + 3) / 4;
+    const int64_t warps = n * (nb * (nb + 1) / 2);
+    return launch_kernel(k_forward_cost_curv_pw, (unsigned)std::min<int64_t>((warps + 7) / 8, (int64_t)148 * 64), 256, 0, st,
+                         b_tiled, wts, w_ld, n, E, W, Wp, C);
+}
+
 cudaError_t forward_cost_rows(const double* mu, const double* deriv, int64_t R, int E, int D, const double* obs, int64_t obs_ld,
                               const double* aux, const double* b_tiled, int W, int Wp, int gy, double* part, double* cost,
-                              double* grad, double* s_out, cudaStream_t st) {
+                              double* grad, double* s_out, cudaStream_t st, const double* wts, int64_t w_ld) {
     const int nsl = (E + 31) / 32, ks = (E + 3) / 4;
     const size_t smem = forward_cost_smem(E);
     const dim3 grid((unsigned)((R + kFcRows - 1) / kFcRows), (unsigned)gy);
@@ -609,10 +706,24 @@ cudaError_t forward_cost_rows(const double* mu, const double* deriv, int64_t R, 
                                aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out)                                            \
                : launch_kernel(k_forward_cost<KSV, false, false>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs,       \
                                obs_ld, aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out)
-    if (nsl == 1 && ks <= 4) GPE_FC(4);
-    else if (nsl == 1 && ks <= 6) GPE_FC(6);
-    else GPE_FC(8);
+#define GPE_FC_PW(KSV)                                                                                                       \
+    e = s_out ? launch_kernel(k_forward_cost_pw<KSV, true, true>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs,        \
+                              obs_ld, aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out, wts, w_ld)                          \
+        : grad ? launch_kernel(k_forward_cost_pw<KSV, true, false>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs,      \
+                               obs_ld, aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out, wts, w_ld)                         \
+               : launch_kernel(k_forward_cost_pw<KSV, false, false>, grid, kFcThreads, smem, st, mu, deriv, R, E, D, obs,    \
+                               obs_ld, aux, b_tiled, W, Wp, nsl, cost, grad, part, s_out, wts, w_ld)
+    if (w_ld != 0) {
+        if (nsl == 1 && ks <= 4) GPE_FC_PW(4);
+        else if (nsl == 1 && ks <= 6) GPE_FC_PW(6);
+        else GPE_FC_PW(8);
+    } else {
+        if (nsl == 1 && ks <= 4) GPE_FC(4);
+        else if (nsl == 1 && ks <= 6) GPE_FC(6);
+        else GPE_FC(8);
+    }
 #undef GPE_FC
+#undef GPE_FC_PW
     if (e != cudaSuccess || gy == 1) return e;
     const unsigned fgrid = (unsigned)((R * (D + 1) + 127) / 128);
     return s_out ? launch_kernel(k_forward_cost_finish<true>, fgrid, 128, 0, st, part, deriv, R, E, D, gy, cost, grad, s_out)

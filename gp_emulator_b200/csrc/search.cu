@@ -248,6 +248,56 @@ __global__ void k_search_band_s(const double* __restrict__ obs, int64_t obs_ld, 
     }
 }
 
+// Per-point weights (DESIGN 4.6f): both costs stay a_k + s_n . m'_k + c_n with a wider pixel operand and table row, and
+// a_k = 0 (NaN past K):
+//   band cost:      m'_k = [1/2 m_k o m_k, m_k] (2E)                pixel [w_n, -w_n o o_n]
+//   spectrum cost:  m'_k = [m_ke m_kf for e <= f, m_k] (E(E+1)/2 + E)   pixel [C_n upper triangle, diagonal halved, s_n]
+// (the upper triangle row by row).  tbl [search_ks(Ew)][Kp][4], zero past Ew and K.
+__global__ void k_search_table_pw(const double* __restrict__ mu, int64_t K, int E, int Ew, int ksa, int Kp, bool spectra,
+                                  double* __restrict__ tbl, double* __restrict__ ta) {
+    const int nq = spectra ? E * (E + 1) / 2 : E;
+    for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < Kp; c += (int64_t)gridDim.x * blockDim.x) {
+        const double* m = mu + c * E;
+        int e = 0, f = 0;
+        for (int q = 0; q < 4 * ksa; ++q) {
+            double v = 0.0;
+            if (c < K && q < nq) {
+                v = spectra ? m[e] * m[f] : 0.5 * (m[q] * m[q]);
+                if (spectra && ++f == E) { ++e; f = e; }
+            } else if (c < K && q < Ew) {
+                v = m[q - nq];
+            }
+            tbl[((size_t)(q >> 2) * Kp + c) * 4 + (q & 3)] = v;
+        }
+        ta[c] = c < K ? 0.0 : __longlong_as_double(0x7ff8000000000000LL);
+    }
+}
+
+// Per-point-weight pixel operand op (R, Ew): band [w_r, -(w_r o obs_r)]; spectrum [C_r (e <= f, diagonal halved), s_r] from
+// the curvature Cn (R, E, E) and s (R, E).
+__global__ void k_search_operand_pw(const double* __restrict__ obs, int64_t obs_ld, const double* __restrict__ w, int64_t w_ld,
+                                    const double* __restrict__ s, const double* __restrict__ Cn, int64_t R, int E, int Ew,
+                                    bool spectra, double* __restrict__ op) {
+    const int nq = spectra ? E * (E + 1) / 2 : E;
+    for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < R * Ew; q += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t r = q / Ew;
+        const int j = (int)(q - r * Ew);
+        double v;
+        if (!spectra) {
+            v = j < E ? w[r * w_ld + j] : -(w[r * w_ld + j - E] * obs[r * obs_ld + j - E]);
+        } else if (j < nq) {
+            int e = 0, t = j;
+            while (t >= E - e) { t -= E - e; ++e; }
+            const int f = e + t;
+            v = Cn[(r * E + e) * E + f];
+            if (e == f) v *= 0.5;
+        } else {
+            v = s[r * E + j - nq];
+        }
+        op[q] = v;
+    }
+}
+
 // x (R, D) = cand[sel[r, j]] (candidate 0 for an empty slot: its cost is discarded).
 __global__ void k_search_gather(const double* __restrict__ cand, int D, const int64_t* __restrict__ sel, int k, int j, int64_t R,
                                 double* __restrict__ x) {
@@ -313,6 +363,15 @@ int search_split(int64_t call_N, int64_t K) {
 cudaError_t search_table(const double* mu, int64_t K, int E, int Kp, const double* w, const double* C, double* tbl, double* ta,
                          cudaStream_t st) {
     return launch_kernel(k_search_table, grid_for(Kp, 128), 128, 0, st, mu, K, E, search_ks(E), Kp, w, C, tbl, ta);
+}
+
+cudaError_t search_table_pw(const double* mu, int64_t K, int E, int Ew, int Kp, bool spectra, double* tbl, double* ta, cudaStream_t st) {
+    return launch_kernel(k_search_table_pw, grid_for(Kp, 128), 128, 0, st, mu, K, E, Ew, search_ks(Ew), Kp, spectra, tbl, ta);
+}
+
+cudaError_t search_operand_pw(const double* obs, int64_t obs_ld, const double* w, int64_t w_ld, const double* s, const double* Cn,
+                              int64_t R, int E, int Ew, bool spectra, double* op, cudaStream_t st) {
+    return launch_kernel(k_search_operand_pw, grid_for(R * Ew, 256), 256, 0, st, obs, obs_ld, w, w_ld, s, Cn, R, E, Ew, spectra, op);
 }
 
 cudaError_t search_band_s(const double* obs, int64_t obs_ld, const double* w, int64_t R, int E, double* s, cudaStream_t st) {

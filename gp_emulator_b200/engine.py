@@ -82,6 +82,16 @@ def _auto_pinned_empty(shape):
     return a
 
 
+def _weights_ld(shape, K, N):
+    """Row pitch of the weights of a call with observations K wide: 0 for one (K,) vector shared by every point (or
+    None), K for one row per point (N, K)."""
+    if shape is None or tuple(shape) == (K,):
+        return 0
+    if tuple(shape) == (N, K):
+        return K
+    raise ValueError(f"weights must be ({K},) or ({N}, {K})")
+
+
 def _check_out(out, k, shape):
     a = out[k]
     if not isinstance(a, np.ndarray) or a.shape != shape or a.dtype != np.float64 or not a.flags.c_contiguous:
@@ -505,7 +515,13 @@ class DeviceBank(_Handle):
         (``gpe_bank_cost``).  ``obs`` is (E,) -- one observation for every point -- or (N, E); ``weights`` (E,) or None.
         ``want_hess``: also ``hess (N, D, D)``, the exact input Hessian of the cost (``gpe_bank_cost_ex``).
         numpy in -> numpy out (streamed below the C ABI, all devices of the bank); torch CUDA in -> torch CUDA out
-        (asynchronous on the current stream, single-device banks)."""
+        (asynchronous on the current stream, single-device banks).
+
+        Per-point weights: ``weights`` may also be (N, K) -- one row per point, e.g. 1 / sigma^2 of the point's own
+        uncertainties -- through the ``_pw`` entry points (include/gpemu.h, DESIGN 4.6f); rows all equal to a vector w give
+        the (K,) call's results bit for bit.  A weight of 0 with a finite observation masks that entry exactly (the result
+        does not depend on the observation's value); a NaN observation still gives NaN.  Data that marks gaps with NaN:
+        ``weights = np.where(np.isnan(obs), 0.0, weights); obs = np.where(np.isnan(obs), 0.0, obs)``."""
         lib = _lib.load()
         return self._reduce(testing, obs, weights, want_grad, want_hess, self.E,
                             lib.gpe_multi_bank_cost_ex if self.multi else lib.gpe_bank_cost_host_ex, lib.gpe_bank_cost_ex)
@@ -517,7 +533,8 @@ class DeviceBank(_Handle):
         spectra never leave the kernel.  ``obs`` is (W,) -- one observed spectrum for every point -- or (N, W);
         ``weights`` (W,) or None.  ``want_hess``: also ``hess (N, D, D)``, the exact input Hessian of the cost
         (``gpe_bank_forward_cost_ex``).  numpy in -> numpy out (streamed below the C ABI, all devices of the bank); torch
-        CUDA in -> torch CUDA out (asynchronous on the current stream, single-device banks)."""
+        CUDA in -> torch CUDA out (asynchronous on the current stream, single-device banks).  Per-point weights (N, W)
+        as in ``cost``."""
         if self.W == 0:
             raise GpemuError("bank has no basis functions to project onto")
         lib = _lib.load()
@@ -527,8 +544,10 @@ class DeviceBank(_Handle):
 
     def _reduce(self, testing, obs, weights, want_grad, want_hess, K, host_fn, device_fn):
         """Shape checks and routing of the cost calls (observations K wide): host arrays to host_fn, CUDA tensors to
-        device_fn on the current stream."""
+        device_fn on the current stream; per-point (N, K) weights to the ``_pw`` entry points."""
         D = self.D
+        lib = _lib.load()
+        flags = _lib.SOLVE_SPECTRA if device_fn is lib.gpe_bank_forward_cost_ex else 0
         if not _is_torch(testing):
             th = f64c(testing)
             if th.ndim != 2 or th.shape[1] != D:
@@ -544,16 +563,21 @@ class DeviceBank(_Handle):
             wt = None
             if weights is not None:
                 wt = f64c(weights.cpu().numpy() if _is_torch(weights) else weights)
-                if wt.shape != (K,):
-                    raise ValueError(f"weights must be ({K},)")
+            w_ld = _weights_ld(None if wt is None else wt.shape, K, N)
             out = {"cost": np.empty(N)}
             if want_grad:
                 out["grad"] = np.empty((N, D))
             if want_hess:
                 out["hess"] = np.empty((N, D, D))
-            if N > 0:
-                check(host_fn(self._h, addr(th), N, addr(o), obs_ld, addr(wt), addr(out["cost"]), addr(out.get("grad")),
-                              addr(out.get("hess"))))
+            outs = (addr(out["cost"]), addr(out.get("grad")), addr(out.get("hess")))
+            if N > 0 and w_ld:
+                if self.multi:
+                    check(lib.gpe_multi_bank_cost_pw(self._h, addr(th), N, addr(o), obs_ld, addr(wt), w_ld, *outs, flags))
+                else:
+                    check(lib.gpe_bank_cost_pw(self._h, addr(th), N, addr(o), obs_ld, addr(wt), w_ld, *outs, flags | HOST_PTRS,
+                                               None))
+            elif N > 0:
+                check(host_fn(self._h, addr(th), N, addr(o), obs_ld, addr(wt), *outs))
             return out
         if self.multi:
             raise ValueError("a multi-device bank takes host arrays; use one DeviceBank per device for CUDA tensors")
@@ -575,15 +599,18 @@ class DeviceBank(_Handle):
         if weights is not None:
             wt = torch.as_tensor(np.asarray(weights, dtype=np.float64) if not _is_torch(weights) else weights,
                                  dtype=torch.float64, device=dev).contiguous()
-            if tuple(wt.shape) != (K,):
-                raise ValueError(f"weights must be ({K},)")
+        w_ld = _weights_ld(None if wt is None else tuple(wt.shape), K, N)
         out = {"cost": torch.empty(N, dtype=torch.float64, device=dev)}
         if want_grad:
             out["grad"] = torch.empty(N, D, dtype=torch.float64, device=dev)
         if want_hess:
             out["hess"] = torch.empty(N, D, D, dtype=torch.float64, device=dev)
-        check(device_fn(self._h, addr(t), N, addr(o), obs_ld, addr(wt), addr(out["cost"]),
-                        addr(out.get("grad")), addr(out.get("hess")), _current_stream_ptr(self.device)))
+        outs = (addr(out["cost"]), addr(out.get("grad")), addr(out.get("hess")))
+        if w_ld:
+            check(lib.gpe_bank_cost_pw(self._h, addr(t), N, addr(o), obs_ld, addr(wt), w_ld, *outs, flags,
+                                       _current_stream_ptr(self.device)))
+        else:
+            check(device_fn(self._h, addr(t), N, addr(o), obs_ld, addr(wt), *outs, _current_stream_ptr(self.device)))
         return out
 
     def search(self, candidates, obs, weights=None, k=1):
@@ -595,12 +622,15 @@ class DeviceBank(_Handle):
         call of the same N points.  Candidates are ranked by the expanded form ``a_k + s_n . m_k`` of the cost, whose
         rounding may swap candidates whose costs differ by about ``E u (|a_k| + sum_e |s_ne m_ke|)`` (include/gpemu.h).
         A point with fewer than k candidates of non-NaN score gets ``idx = -1`` and ``cost = NaN`` in its last slots.
+        ``weights`` may be (N, E), one row per point (``gpe_bank_search_pw``; banks of up to ``SEARCH_PW_MAX_E_BANDS`` (48)
+        emulators), with the masking rules of ``cost``.
         numpy in -> numpy out (all devices of the bank); a torch CUDA tensor among ``candidates`` / ``obs`` -> torch CUDA
         out (asynchronous on the current stream, single-device banks)."""
         return self._search(False, candidates, obs, weights, k)
 
     def forward_search(self, candidates, obs, weights=None, k=1):
-        """``search`` with the spectrum cost of ``forward_cost``: ``obs`` (W,) or (N, W), ``weights`` (W,) or None."""
+        """``search`` with the spectrum cost of ``forward_cost``: ``obs`` (W,) or (N, W), ``weights`` (W,), (N, W) or None.
+        With per-point weights the search takes banks of up to ``SEARCH_PW_MAX_E_SPECTRA`` (12) emulators."""
         if self.W == 0:
             raise GpemuError("bank has no basis functions to project onto")
         return self._search(True, candidates, obs, weights, k)
@@ -633,9 +663,17 @@ class DeviceBank(_Handle):
             N, obs_ld = shape(o)[0], K_obs
         else:
             raise ValueError(f"obs must be ({K_obs},) or (N, {K_obs})")
-        if wt is not None and shape(wt) != (K_obs,):
-            raise ValueError(f"weights must be ({K_obs},)")
+        w_ld = _weights_ld(None if wt is None else shape(wt), K_obs, N)
         out = {"idx": empty((N, k), np.int64), "cost": empty((N, k), np.float64)}
+        if w_ld:
+            args = (addr(c), shape(c)[0], addr(o), N, obs_ld, addr(wt), w_ld, k, addr(out["idx"]), addr(out["cost"]))
+            if _is_torch(c):
+                check(lib.gpe_bank_search_pw(self._h, *args, flags, _current_stream_ptr(self.device)))
+            elif self.multi:
+                check(lib.gpe_multi_bank_search_pw(self._h, *args, flags))
+            else:
+                check(lib.gpe_bank_search_pw(self._h, *args, flags | HOST_PTRS, None))
+            return out
         args = (addr(c), shape(c)[0], addr(o), N, obs_ld, addr(wt), k, addr(out["idx"]), addr(out["cost"]))
         if _is_torch(c):
             check(lib.gpe_bank_search(self._h, *args, flags, _current_stream_ptr(self.device)))
@@ -653,7 +691,8 @@ class DeviceBank(_Handle):
         bounded Levenberg-Marquardt on the exact Hessian, every iteration on the device (``gpe_bank_solve``; the
         algorithm and the stopping tests are stated in include/gpemu.h).
 
-        ``x0`` (N, D) starting points; ``obs`` (E,) or (N, E); ``weights`` (E,) or None; ``lower`` / ``upper`` (D,) or
+        ``x0`` (N, D) starting points; ``obs`` (E,) or (N, E); ``weights`` (E,), (N, E) or None (per-point rows as in
+        ``cost``: ``gpe_bank_solve_pw``, and with 1 / sigma^2 of each point ``cov`` is its Laplace posterior); ``lower`` / ``upper`` (D,) or
         None (entries may be infinite); ``prior_mean`` (D,) or (N, D), ``prior_precision`` (D, D).  Returns a dict:
         ``x`` (N, D), ``cost`` (N,), ``grad`` (N, D) and ``hess`` (N, D, D) at x (prior included), ``cov`` (N, D, D) =
         inv(hess) with ``want_cov`` (NaN where hess is not positive definite), ``status`` (N,) int32 (``SOLVE_*`` of
@@ -757,8 +796,8 @@ class DeviceBank(_Handle):
         else:
             raise ValueError(f"obs must be ({K},) or ({N}, {K})")
         wt, lo, hi, pm, pp = (arr(a) for a in (weights, lower, upper, prior_mean, prior_precision))
-        for name, a, want in (("weights", wt, (K,)), ("lower", lo, (D,)), ("upper", hi, (D,)),
-                              ("prior_precision", pp, (D, D))):
+        w_ld = _weights_ld(None if wt is None else shape(wt), K, N)
+        for name, a, want in (("lower", lo, (D,)), ("upper", hi, (D,)), ("prior_precision", pp, (D, D))):
             if a is not None and shape(a) != want:
                 raise ValueError(f"{name} must be {want}")
         prior_ld = 0
@@ -776,7 +815,15 @@ class DeviceBank(_Handle):
         flags = _lib.SOLVE_SPECTRA if spectra else 0
         args = (addr(x0), N, addr(o), obs_ld, addr(wt), C.byref(opts), addr(out["x"]), addr(out["cost"]),
                 addr(out["grad"]), addr(out["hess"]), addr(out.get("cov")), addr(info))
-        if dev:
+        if w_ld:
+            args = args[:5] + (w_ld,) + args[5:]
+            if dev:
+                check(lib.gpe_bank_solve_pw(self._h, *args, flags, _current_stream_ptr(self.device)))
+            elif self.multi:
+                check(lib.gpe_multi_bank_solve_pw(self._h, *args, flags))
+            else:
+                check(lib.gpe_bank_solve_pw(self._h, *args, flags | HOST_PTRS, None))
+        elif dev:
             check(lib.gpe_bank_solve(self._h, *args, flags, _current_stream_ptr(self.device)))
         elif self.multi:
             check(lib.gpe_multi_bank_solve(self._h, *args, flags))

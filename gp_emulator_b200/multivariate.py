@@ -13,6 +13,7 @@ import shutil
 
 import numpy as np
 
+from . import _lib
 from .engine import DeviceBank, resolve_devices
 from .gaussian_process import GaussianProcess
 
@@ -171,7 +172,10 @@ class MultivariateEmulator(object):
         the exact Hessian in ``y`` (for Newton steps; with weights 1 / sigma^2, ``inv(hess)`` at the optimum is the
         Laplace approximation of the posterior covariance).
 
-        ``obs`` (N_full,) is shared by every point, (N, N_full) is one per point; ``weights`` (N_full,) or None (all 1).
+        ``obs`` (N_full,) is shared by every point, (N, N_full) is one per point; ``weights`` (N_full,), (N, N_full) -- one
+        row per point, e.g. 1 / sigma^2 of each pixel's own noise -- or None (all 1).  A weight of 0 with a finite
+        observation masks that entry exactly; a NaN observation still gives NaN, so mask NaN gaps with
+        ``weights = np.where(np.isnan(obs), 0.0, weights); obs = np.where(np.isnan(obs), 0.0, obs)``.
         Returns the requested items in the order cost, grad, hess -- one point: ``float``, ``(N_params,)``,
         ``(N_params, N_params)``; N points: ``(N,)``, ``(N, N_params)``, ``(N, N_params, N_params)`` -- and the cost
         alone, not in a tuple, when it is the only one.  Host arrays or CUDA tensors, as ``predict``.
@@ -191,7 +195,8 @@ class MultivariateEmulator(object):
     def search(self, obs, candidates=None, k=1, weights=None):
         """The ``k`` parameter vectors of the table ``candidates`` (K, N_params) whose reconstructed output fits ``obs``
         best, by ``cost`` (``DeviceBank.forward_search``); ``candidates=None`` searches the training design ``y_train``.
-        ``obs`` (N_full,) is one observation, (N, N_full) one per point.  Returns ``{"idx", "cost"}``, each ``(k,)`` for
+        ``obs`` (N_full,) is one observation, (N, N_full) one per point; ``weights`` as in ``cost`` (per-point rows: at most
+        ``SEARCH_PW_MAX_E_SPECTRA`` (12) principal components).  Returns ``{"idx", "cost"}``, each ``(k,)`` for
         one observation and ``(N, k)`` for N, in ascending order of (cost, index); ``idx`` -1 / ``cost`` NaN where fewer
         than k candidates have a finite ranking score.  Host arrays or CUDA tensors, as ``predict``."""
         cand = np.atleast_2d(self.y_train) if candidates is None else candidates
@@ -207,6 +212,8 @@ class MultivariateEmulator(object):
         Laplace approximation of the posterior covariance.
 
         ``y0`` (N_params,) or (N, N_params) starting points; ``obs`` (N_full,) shared or (N, N_full) one per point;
+        ``weights`` (N_full,), (N, N_full) one row per point (with 1 / sigma^2 of each point, ``cov`` is its own Laplace
+        posterior), or None;
         ``lower`` / ``upper`` (N_params,) or None; ``m`` (N_params,) or (N, N_params), ``P`` (N_params, N_params).
         Returns a dict ``x``, ``cost``, ``grad``, ``hess``, ``cov`` (with ``do_cov``), ``status``, ``n_iter`` -- one point:
         ``(N_params,)``, ``float``, ``(N_params,)``, ``(N_params, N_params)``, ..., ``int``, ``int``; N points: the same with
@@ -222,6 +229,9 @@ class MultivariateEmulator(object):
         if y0 is None:
             cand = np.atleast_2d(self.y_train) if candidates is None else candidates
             one = len(obs.shape) == 1
+            if weights is not None and len(weights.shape) == 2 and self.n_pcs > _lib.SEARCH_PW_MAX_E_SPECTRA:
+                raise ValueError(f"with per-point weights the candidate search takes at most {_lib.SEARCH_PW_MAX_E_SPECTRA} "
+                                 f"principal components (this emulator has {self.n_pcs}): give the starting points y0")
             out = bank.forward_invert(None, obs, weights, lower=lower, upper=upper, prior_mean=m, prior_precision=P,
                                       max_iter=max_iter, ftol=ftol, xtol=xtol, gtol=gtol, want_cov=do_cov,
                                       candidates=cand, n_starts=n_starts)

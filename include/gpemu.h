@@ -322,6 +322,51 @@ int gpe_bank_search(gpe_bank* b, const double* cand, int64_t K, const double* ob
 int gpe_multi_bank_search(gpe_multi* mm, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
                           const double* weights, int k, int64_t* idx, double* cost, unsigned flags);
 
+/* Per-point observation weights (DESIGN 4.6f): the cost, solve and search calls above with weights (N, K) -- one row per
+ * point, as obs (K = E, or W with GPE_SOLVE_SPECTRA):
+ *   weights_ld = 0       one (K) vector shared by every point: the calls above, bit for bit;
+ *   weights_ld >= K      rows weights_ld apart (device pointers; host arrays: weights_ld = K exactly);
+ *   weights == NULL      all weights 1 (weights_ld must then be 0).
+ * The formulas are those of gpe_bank_cost_ex and gpe_bank_forward_cost_ex with w_e -> w_ne and l_w -> l_nw; for the spectrum
+ * cost s_n = (l_n o r_n) . basis^T, C_n = basis . diag(l_n) . basis^T (one (E, E) matrix per point) and
+ * hess_n = sum_e s_ne H_ne + G_n^T C_n G_n.  With weights 1 / sigma_n^2, sigma_n the point's own uncertainties, the cost is a
+ * negative log-likelihood and cov = inv(hess) of the solve is the Laplace posterior covariance.
+ *   Equivalence: a call whose weight rows all equal a vector w returns, bit for bit, what the shared-w call returns (cost,
+ * grad and hess of both costs; x, cost, grad, hess, cov and info of the solve; idx and cost of the search).
+ *   Masking: a weight of 0 with a FINITE observation masks that entry: every term it enters is an exact zero, so the result
+ * does not depend on the observation's value, bit for bit.  NaN semantics are unchanged (numpy's): a NaN observation gives
+ * NaN even where its weight is 0.  Data that marks gaps with NaN is masked by
+ *     weights = np.where(np.isnan(obs), 0.0, weights);  obs = np.where(np.isnan(obs), 0.0, obs)
+ *   flags: GPE_SOLVE_SPECTRA selects the spectrum cost; GPE_HOST_PTRS host arrays (streamed in chunks, synchronous).  The
+ * multi-device calls take host arrays on every device of a handle (GPE_HOST_PTRS implied).  Results do not depend on
+ * chunking, pointer placement, the device count or the order of the points (weight rows permuted with them).
+ *   gpe_bank_cost_pw: outputs as gpe_bank_cost_ex / gpe_bank_forward_cost_ex (any non-empty subset of cost, grad, hess).
+ *   gpe_bank_solve_pw: as gpe_bank_solve; C_n is formed once per point, not per iteration.
+ *   gpe_bank_search_pw: as gpe_bank_search; the ranking stays one skinny GEMM with a wider operand, a_k = 0:
+ *     band cost:      m'_k = [1/2 m_k o m_k, m_k], pixel [w_n, -w_n o obs_n]  (2E wide: banks of up to 48 emulators)
+ *                     score error about 2E u (sum_e |w_ne| (m_ke^2 / 2 + |obs_ne m_ke|))
+ *     spectrum cost:  m'_k = [m_ke m_kf for e <= f, m_k], pixel [C_n (e <= f, diagonal halved), s_n]
+ *                     (E(E+1)/2 + E wide: banks of up to 12 emulators)
+ *                     score error about (E(E+1)/2 + E) u (sum_{e<=f} |C_nef m_ke m_kf| + sum_e |s_ne m_ke|)
+ *     Larger banks: GPE_ERR_UNSUPPORTED.  The returned costs are those of gpe_bank_cost_pw, bit for bit, as in
+ *     gpe_bank_search. */
+int gpe_bank_cost_pw(gpe_bank* b, const double* testing, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                     int64_t weights_ld, double* cost, double* grad, double* hess, unsigned flags, void* stream);
+int gpe_bank_solve_pw(gpe_bank* b, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                      int64_t weights_ld, const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess,
+                      double* cov, int32_t* info, unsigned flags, void* stream);
+int gpe_bank_search_pw(gpe_bank* b, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                       const double* weights, int64_t weights_ld, int k, int64_t* idx, double* cost, unsigned flags, void* stream);
+int gpe_multi_bank_cost_pw(gpe_multi* mm, const double* testing, int64_t N, const double* obs, int64_t obs_ld,
+                           const double* weights, int64_t weights_ld, double* cost, double* grad, double* hess, unsigned flags);
+int gpe_multi_bank_solve_pw(gpe_multi* mm, const double* x0, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
+                            int64_t weights_ld, const gpe_solve_opts* opts, double* x, double* cost, double* grad, double* hess,
+                            double* cov, int32_t* info, unsigned flags);
+int gpe_multi_bank_search_pw(gpe_multi* mm, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
+                             const double* weights, int64_t weights_ld, int k, int64_t* idx, double* cost, unsigned flags);
+#define GPE_SEARCH_PW_MAX_E_BANDS 48
+#define GPE_SEARCH_PW_MAX_E_SPECTRA 12
+
 /* PCA back-projection of bank means: fwd (N, W) = mu (N, E) @ basis (E, W)
  * (the accumulation `fwd += pred_mu * basis_functions[i]`, gp_emulator/multivariate_gp.py:216, batched
  * over N points), and optionally deriv_full (N, D, W) = sum_e deriv[n, e, d] * basis[e, w] (:218).
