@@ -81,6 +81,27 @@ def main():
           "the truth" % (np.round(res["x"][3], 4), np.round(sd[3], 4), np.round(y_test[3], 4),
                          100 * np.mean(np.abs(res["x"] - y_test) <= 3 * sd)))
 
+    rs = np.random.RandomState(5)                                             # 3d. time series with cloudy dates
+    S, T = 200, 46                                                            # 200 pixels x 46 dates a season
+    ph = rs.uniform(0, 2 * np.pi, (S, 1, len(dists)))
+    y_ts = (lower + upper) / 2 + 0.3 * (upper - lower) * np.sin(2 * np.pi * np.arange(T)[None, :, None] / T + ph)
+    obs_ts = toy_model(y_ts.reshape(-1, len(dists)), wl) + sigma * rs.standard_normal((S * T, len(wl)))
+    cloudy = rs.random_sample(S * T) < 0.4                                    # 40 % of the dates masked
+    w_ts = np.where(cloudy[:, None], 0.0, 1.0 / sigma ** 2) * np.ones(len(wl))
+    obs_ts[cloudy] = 0.0                                                      # no data there: any finite value, weight 0
+    y0 = table[emu.search(obs_ts, candidates=table, k=1)["idx"][:, 0]]       # starts per date from the table ...
+    y0[cloudy] = 0.5 * (lower + upper)                                        # ... and the box centre where it is cloudy
+    per_date = emu.invert(obs_ts, y0, weights=w_ts, bounds=(lower, upper), do_cov=False)
+    step = 0.3 * (upper - lower) * 2 * np.pi / T                              # largest change of y between dates
+    ts = emu.invert_series(obs_ts.reshape(S, T, -1), y0.reshape(S, T, -1), smooth=(np.diag(1.0 / step ** 2), None),
+                           weights=w_ts.reshape(S, T, -1), bounds=(lower, upper), do_cov=False)
+    err = lambda x: np.abs(x.reshape(-1, len(dists)) - y_ts.reshape(-1, len(dists)))
+    rms = lambda e, m: np.sqrt(np.mean(e[m] ** 2))
+    print("time series, %d pixels x %d dates, %d %% cloudy: rmse on cloudy dates %.4f per date, %.4f jointly; on clear "
+          "dates %.4f per date, %.4f jointly; series status counts %s" % (
+        S, T, round(100 * cloudy.mean()), rms(err(per_date["x"]), cloudy), rms(err(ts["x"]), cloudy),
+        rms(err(per_date["x"]), ~cloudy), rms(err(ts["x"]), ~cloudy), np.bincount(ts["status"], minlength=4).tolist()))
+
     bands = [40, 120, 200, 280, 360]                                          # 4. per-band GPs
     from gp_emulator_b200.training import fit_bank
     gps, _ = fit_bank(y_train, X_train[:, bands].T, n_tries=10)              # all bands x starts in one batch

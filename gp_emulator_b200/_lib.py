@@ -40,7 +40,7 @@ SYMBOLS = (
     "gpe_trainer_create", "gpe_trainer_eval", "gpe_trainer_destroy", "gpe_bank_solve", "gpe_multi_bank_solve",
     "gpe_bank_search", "gpe_multi_bank_search",
     "gpe_bank_cost_pw", "gpe_bank_solve_pw", "gpe_bank_search_pw", "gpe_multi_bank_cost_pw", "gpe_multi_bank_solve_pw",
-    "gpe_multi_bank_search_pw",
+    "gpe_multi_bank_search_pw", "gpe_bank_solve_series", "gpe_multi_bank_solve_series",
 )
 
 
@@ -159,6 +159,13 @@ def load():
     lib.gpe_multi_bank_search_pw.restype = C.c_int
     lib.gpe_multi_bank_search_pw.argtypes = [C.c_void_p, dp, C.c_int64, dp, C.c_int64, C.c_int64, dp, C.c_int64, C.c_int, dp,
                                              dp, C.c_uint]
+    # time series: (S, T) after the handle, smooth_prec and coupling after opts
+    lib.gpe_bank_solve_series.restype = C.c_int
+    lib.gpe_bank_solve_series.argtypes = [C.c_void_p, C.c_int64, C.c_int64, dp, dp, C.c_int64, dp, C.c_int64, so, dp, dp, dp, dp,
+                                          dp, dp, dp, dp, C.c_uint, C.c_void_p]
+    lib.gpe_multi_bank_solve_series.restype = C.c_int
+    lib.gpe_multi_bank_solve_series.argtypes = [C.c_void_p, C.c_int64, C.c_int64, dp, dp, C.c_int64, dp, C.c_int64, so, dp, dp,
+                                                dp, dp, dp, dp, dp, dp, C.c_uint]
     lib.gpe_bank_project.restype = C.c_int
     lib.gpe_bank_project.argtypes = [C.c_void_p, dp, dp, C.c_int64, dp, dp, C.c_void_p]
     lib.gpe_bank_forward.restype = C.c_int

@@ -1788,6 +1788,93 @@ int bank_solve_device(gpe_bank* b, CostDevice cost_device, int64_t K, const LmPr
     return GPE_OK;
 }
 
+// Solve of S series of T dates on `st` (device arrays; DESIGN 4.6g): bank_solve_device with series as the list entries.
+// Each evaluation is act T rows of the call's cost (call_N: the call's row count), k_lm_series_step steps every active
+// series, and the series that stay active are expanded into their rows for the row gathers of the point solver.  Scratch
+// within 256 MB, in whole series.
+int bank_series_solve_device(gpe_bank* b, CostDevice cost_device, int64_t K, const LmProblem& pb, const LmSeries& sp0,
+                             const double* x0, int64_t S, const double* obs, int64_t obs_ld, const double* weights,
+                             double* x, double* cost, double* grad, double* hess, double* cov, int32_t* info, cudaStream_t st,
+                             int64_t call_N, int64_t w_ld = 0) {
+    const int64_t D = b->D, R = lm_state_doubles((int)D), E = b->E, T = sp0.T;
+    const bool pw = w_ld > 0, curv = pw && cost_device == bank_forward_cost_device;
+    // doubles per series: per row those of the point solver (the row lists counted as a double), the block factors, and
+    // the series list and flag
+    const int64_t per_row = R + D * D + 2 * D + 1 + (obs_ld > 0 ? K : 0) + (pw ? K : 0) + (curv ? 2 * E * E : 0) + 2;
+    const int64_t per = T * per_row + lm_series_scratch_doubles((int)D, (int)T) + 2;
+    const int64_t cap = (((int64_t)256 << 20) / 8);
+    if (per > cap)
+        return fail(GPE_ERR_UNSUPPORTED, "one series of %lld dates needs %lld MB of solver scratch, beyond the 256 MB limit",
+                    (long long)T, (long long)((per * 8) >> 20));
+    int64_t sub = std::max<int64_t>(1, std::min<int64_t>(S, cap / per));
+    if (const char* e = getenv("GPE_SOLVE_SUB_POINTS")) sub = std::max<int64_t>(1, std::min<int64_t>(sub, atoll(e)));   // dev aid: series here
+    const int64_t rows_max = sub * T;
+    const size_t temp = lm_select_temp(sub);
+    size_t off = 0;
+    auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
+    const size_t o_state = carve(8 * rows_max * R), o_xe = carve(8 * rows_max * D), o_fe = carve(8 * rows_max);
+    const size_t o_ge = carve(8 * rows_max * D), o_he = carve(8 * rows_max * D * D), o_obs = carve(obs_ld > 0 ? 8 * rows_max * K : 0);
+    const size_t o_l0 = carve(4 * rows_max), o_l1 = carve(4 * sub), o_rows = carve(4 * rows_max), o_flag = carve(4 * sub);
+    const size_t o_cnt = carve(4), o_tmp = carve(temp), o_w = carve(pw ? 8 * rows_max * K : 0);
+    const size_t o_cs = carve(curv ? 8 * rows_max * E * E : 0), o_cc = carve(curv ? 8 * rows_max * E * E : 0);
+    const size_t o_scr = carve(8 * sub * lm_series_scratch_doubles((int)D, (int)T));
+    std::lock_guard<std::mutex> lock(b->solve_mu);
+    int rc = ensure_buf(&b->solve_d, &b->solve_cap, off, false);
+    if (rc) return rc;
+    if (!b->solve_count) CUDA_TRY(cudaMallocHost((void**)&b->solve_count, sizeof(int)));
+    if (!b->solve_ev) CUDA_TRY(cudaEventCreateWithFlags(&b->solve_ev, cudaEventDisableTiming));
+    char* base = (char*)b->solve_d;
+    double* state = (double*)(base + o_state);
+    double *xe = (double*)(base + o_xe), *fe = (double*)(base + o_fe), *ge = (double*)(base + o_ge), *he = (double*)(base + o_he);
+    double* obs_c = (double*)(base + o_obs);
+    double *w_c = (double*)(base + o_w), *Cs = curv ? (double*)(base + o_cs) : nullptr, *C_c = (double*)(base + o_cc);
+    int *lists[2] = {(int*)(base + o_l0), (int*)(base + o_l1)}, *flag = (int*)(base + o_flag), *d_cnt = (int*)(base + o_cnt);
+    int* rows = (int*)(base + o_rows);
+    LmSeries sp = sp0;
+    sp.scratch = (double*)(base + o_scr);
+    for (int64_t s0 = 0; s0 < S; s0 += sub) {
+        const int64_t n = std::min(sub, S - s0), r0 = s0 * T;
+        LmProblem p = pb;
+        if (p.prior_mean && p.prior_ld > 0) p.prior_mean += r0 * p.prior_ld;
+        const double* o = obs + r0 * obs_ld;
+        const double* w = pw ? weights + r0 * w_ld : weights;
+        // lm_init numbers the rows: the first n entries of the list are then the series 0 .. n-1
+        CUDA_TRY(lm_init(p, x0 + r0 * D, n * T, state, xe, lists[0], st));
+        if (curv) CUDA_TRY(forward_cost_curv_pw(b->d_basis, w, w_ld, n * T, (int)E, b->W, b->Wp, Cs, st));
+        const double* e_obs = o;
+        const double *e_w = w, *e_C = Cs;
+        int64_t e_ld = obs_ld, e_wld = w_ld, act = n;
+        for (int it = 0;; ++it) {
+            int* list = lists[it & 1];
+            int* next_list = lists[(it + 1) & 1];
+            rc = cost_device(b, xe, act * T, e_obs, e_ld, e_w, e_wld, e_C, fe, ge, he, st, call_N);
+            if (rc) return rc;
+            CUDA_TRY(lm_series_step(p, sp, act, list, fe, ge, he, state, flag, it == 0, st));
+            CUDA_TRY(lm_select(list, flag, act, next_list, d_cnt, base + o_tmp, temp, st));
+            CUDA_TRY(cudaMemcpyAsync(b->solve_count, d_cnt, sizeof(int), cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaEventRecord(b->solve_ev, st));
+            CUDA_TRY(cudaEventSynchronize(b->solve_ev));
+            const int64_t next = *b->solve_count;
+            if (next == 0) break;
+            const bool regather = obs_ld > 0 && next < act;
+            CUDA_TRY(lm_series_rows(next_list, next, (int)T, rows, st));
+            CUDA_TRY(lm_gather(state, (int)D, rows, next * T, xe, o, regather ? obs_ld : 0, K, obs_c, st));
+            if (regather) { e_obs = obs_c; e_ld = K; }
+            if (pw && next < act) {
+                CUDA_TRY(lm_gather_rows(rows, next * T, w, w_ld, K, w_c, st));
+                if (curv) CUDA_TRY(lm_gather_rows(rows, next * T, Cs, E * E, E * E, C_c, st));
+                e_w = w_c; e_wld = K; e_C = curv ? C_c : nullptr;
+            }
+            act = next;
+        }
+        CUDA_TRY(lm_series_output(p, sp, n, state, x + r0 * D, cost ? cost + s0 : nullptr, grad ? grad + r0 * D : nullptr,
+                                  hess ? hess + r0 * D * D : nullptr, cov ? cov + r0 * D * D : nullptr, info + 2 * s0, st));
+    }
+    CUDA_TRY(cudaEventRecord(b->solve_ev, st));
+    CUDA_TRY(cudaEventSynchronize(b->solve_ev));
+    return GPE_OK;
+}
+
 constexpr gpe_solve_opts kSolveDefaults = {GPE_SOLVE_DEFAULT_MAX_ITER, 1e-10, 1e-10, 0.0, 1e-3, nullptr, nullptr, nullptr, 0, nullptr};
 
 LmProblem lm_problem(int D, const gpe_solve_opts& o, const double* lower, const double* upper, const double* prior_mean,
@@ -1836,6 +1923,34 @@ int solve_check(gpe_bank* b, int64_t N, const double* x0, const double* obs, int
     return GPE_OK;
 }
 
+// Request check of the series arguments (DESIGN 4.6g): S >= 0, T >= 1, R (D, D) finite and exactly symmetric, coupling
+// (T - 1) finite and >= 0 or NULL.  Device pointers are read with a D2H copy on the call's stream `st`.
+int series_check(gpe_bank* b, int64_t S, int64_t T, const double* R, const double* coupling, bool host, cudaStream_t st) {
+    if (S < 0) return fail(GPE_ERR_INVALID, "S must be >= 0");
+    if (T < 1 || T > (1 << 24)) return fail(GPE_ERR_INVALID, "T must be in [1, 2^24] (got %lld)", (long long)T);
+    if (!R) return fail(GPE_ERR_INVALID, "smooth_prec is NULL");
+    const int D = b->D;
+    if (D > GPE_SOLVE_MAX_D) return fail(GPE_ERR_UNSUPPORTED, "the solver supports D <= %d (got %d)", GPE_SOLVE_MAX_D, D);
+    std::vector<double> r((size_t)D * D), c(coupling ? (size_t)(T - 1) : 0);
+    if (host) {
+        memcpy(r.data(), R, r.size() * 8);
+        if (!c.empty()) memcpy(c.data(), coupling, c.size() * 8);
+    } else {
+        CUDA_TRY(cudaSetDevice(b->device));
+        CUDA_TRY(cudaMemcpyAsync(r.data(), R, r.size() * 8, cudaMemcpyDeviceToHost, st));
+        if (!c.empty()) CUDA_TRY(cudaMemcpyAsync(c.data(), coupling, c.size() * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    for (int i = 0; i < D; ++i)
+        for (int j = 0; j < D; ++j) {
+            if (!std::isfinite(r[i * D + j])) return fail(GPE_ERR_INVALID, "smooth_prec[%d, %d] is not finite", i, j);
+            if (r[i * D + j] != r[j * D + i]) return fail(GPE_ERR_INVALID, "smooth_prec is not symmetric at (%d, %d)", i, j);
+        }
+    for (size_t t = 0; t < c.size(); ++t)
+        if (!(std::isfinite(c[t]) && c[t] >= 0.0)) return fail(GPE_ERR_INVALID, "coupling[%zu] must be finite and >= 0", t);
+    return GPE_OK;
+}
+
 // The streamed arrays of a host-resident solve: x0 and, when per point, obs and the prior means in; x, the optional
 // cost / grad / hess / cov and info (8 bytes a point: one double-wide column) out.
 struct SolveIo {
@@ -1843,19 +1958,20 @@ struct SolveIo {
     int obs = -1, w = -1, pm = -1, x = -1, cost = -1, grad = -1, hess = -1, cov = -1, info = -1;
 };
 
+// T > 1: the unit is a series of T rows (cost and info stay one per series).
 SolveIo solve_io(int64_t D, int64_t K, const double* x0, const double* obs, int64_t obs_ld, const gpe_solve_opts& o, double* x,
                  double* cost, double* grad, double* hess, double* cov, int32_t* info, const double* weights = nullptr,
-                 int64_t w_ld = 0) {
+                 int64_t w_ld = 0, int64_t T = 1) {
     SolveIo s;
-    s.io.in.add(x0, D);
-    if (obs_ld != 0) s.obs = s.io.in.add(obs, K);
-    if (w_ld != 0) s.w = s.io.in.add(weights, K);
-    if (o.prior_mean && o.prior_ld != 0) s.pm = s.io.in.add(o.prior_mean, D);
-    s.x = s.io.out.add(x, D);
+    s.io.in.add(x0, T * D);
+    if (obs_ld != 0) s.obs = s.io.in.add(obs, T * K);
+    if (w_ld != 0) s.w = s.io.in.add(weights, T * K);
+    if (o.prior_mean && o.prior_ld != 0) s.pm = s.io.in.add(o.prior_mean, T * D);
+    s.x = s.io.out.add(x, T * D);
     if (cost) s.cost = s.io.out.add(cost, 1);
-    if (grad) s.grad = s.io.out.add(grad, D);
-    if (hess) s.hess = s.io.out.add(hess, D * D);
-    if (cov) s.cov = s.io.out.add(cov, D * D);
+    if (grad) s.grad = s.io.out.add(grad, T * D);
+    if (hess) s.hess = s.io.out.add(hess, T * D * D);
+    if (cov) s.cov = s.io.out.add(cov, T * D * D);
     s.info = s.io.out.add(info, 1);
     return s;
 }
@@ -1863,20 +1979,23 @@ SolveIo solve_io(int64_t D, int64_t K, const double* x0, const double* obs, int6
 // Host-resident solve through the bank's pipeline (caller holds b->host_mu): the small per-call operands (shared
 // observation, weights, bounds, shared prior mean, precision) are uploaded once, then every chunk is solved by
 // bank_solve_device as its chunk launch.  A chunk's solve blocks this pipeline's thread until it has finished.
+//   series (host R and coupling): N series, each chunk solved by bank_series_solve_device; R and coupling are uploaded too.
 int bank_solve_stream(gpe_bank* b, bool spectra, int64_t N, const double* obs, int64_t obs_ld, const double* weights,
-                      const gpe_solve_opts& o, const SolveIo& s, const SharedCall* shared = nullptr) {
-    const int64_t D = b->D, K = spectra ? b->W : b->E;
+                      const gpe_solve_opts& o, const SolveIo& s, const SharedCall* shared = nullptr,
+                      const LmSeries* series = nullptr) {
+    const int64_t D = b->D, K = spectra ? b->W : b->E, T = series ? series->T : 1;
     struct Part { const double* src; int64_t n; double* dev; };
     Part parts[] = {{obs_ld == 0 ? obs : nullptr, K, nullptr}, {s.w < 0 ? weights : nullptr, K, nullptr}, {o.lower, D, nullptr},
-                    {o.upper, D, nullptr}, {o.prior_ld == 0 ? o.prior_mean : nullptr, D, nullptr}, {o.prior_prec, D * D, nullptr}};
+                    {o.upper, D, nullptr}, {o.prior_ld == 0 ? o.prior_mean : nullptr, D, nullptr}, {o.prior_prec, D * D, nullptr},
+                    {series ? series->R : nullptr, D * D, nullptr}, {series ? series->coupling : nullptr, T - 1, nullptr}};
     size_t total = 0;
-    for (const Part& p : parts) if (p.src) total += (size_t)p.n;
+    for (const Part& p : parts) if (p.src && p.n > 0) total += (size_t)p.n;
     if (total > 0) {
         int rc = ensure_buf((void**)&b->d_aux, &b->aux_cap, total * 8, false);
         if (rc) return rc;
         double* at = b->d_aux;
         for (Part& p : parts) {
-            if (!p.src) continue;
+            if (!p.src || p.n == 0) continue;
             CUDA_TRY(cudaMemcpyAsync(at, p.src, (size_t)p.n * 8, cudaMemcpyHostToDevice, cudaStreamLegacy));
             p.dev = at;
             at += p.n;
@@ -1891,6 +2010,13 @@ int bank_solve_stream(gpe_bank* b, bool spectra, int64_t N, const double* obs, i
                            LmProblem p = pb;
                            if (s.pm >= 0) { p.prior_mean = (const double*)di[s.pm]; p.prior_ld = D; }
                            auto out = [&](int k) { return k >= 0 ? (double*)dout[k] : nullptr; };
+                           if (series)
+                               return bank_series_solve_device(
+                                   b, spectra ? bank_forward_cost_device : bank_cost_device, K, p,
+                                   LmSeries{(int)T, parts[7].dev, parts[6].dev, nullptr}, (const double*)di[0], n,
+                                   s.obs >= 0 ? (const double*)di[s.obs] : parts[0].dev, obs_ld != 0 ? K : 0,
+                                   s.w >= 0 ? (const double*)di[s.w] : parts[1].dev, out(s.x), out(s.cost), out(s.grad),
+                                   out(s.hess), out(s.cov), (int32_t*)dout[s.info], st, N * T, s.w >= 0 ? K : 0);
                            return bank_solve_device(b, spectra ? bank_forward_cost_device : bank_cost_device, K, p,
                                                     (const double*)di[0], n, s.obs >= 0 ? (const double*)di[s.obs] : parts[0].dev,
                                                     obs_ld != 0 ? K : 0, s.w >= 0 ? (const double*)di[s.w] : parts[1].dev,
@@ -2354,6 +2480,32 @@ int gpe_bank_solve(gpe_bank* b, const double* x0, int64_t N, const double* obs, 
     return gpe_bank_solve_pw(b, x0, N, obs, obs_ld, weights, 0, opts, x, cost, grad, hess, cov, info, flags, stream);
 }
 
+int gpe_bank_solve_series(gpe_bank* b, int64_t S, int64_t T, const double* x0, const double* obs, int64_t obs_ld,
+                          const double* weights, int64_t weights_ld, const gpe_solve_opts* opts, const double* smooth_prec,
+                          const double* coupling, double* x, double* cost, double* grad, double* hess, double* cov,
+                          int32_t* info, unsigned flags, void* stream) {
+    NvtxRange nvtx_range("gpe_bank_solve_series");
+    const bool host = flags & GPE_HOST_PTRS, spectra = flags & GPE_SOLVE_SPECTRA;
+    if (!b) return fail(GPE_ERR_INVALID, "bank is NULL");
+    int rc = series_check(b, S, T, smooth_prec, coupling, host, (cudaStream_t)stream);
+    gpe_solve_opts o;
+    if (rc == GPE_OK) rc = solve_check(b, S * T, x0, obs, obs_ld, opts, x, info, flags, host, (cudaStream_t)stream, &o);
+    if (rc == GPE_OK) rc = weights_check(weights, weights_ld, spectra ? b->W : b->E, spectra, host);
+    if (rc || S == 0) return rc;
+    CUDA_TRY(cudaSetDevice(b->device));
+    const int64_t D = b->D, K = spectra ? b->W : b->E;
+    const LmSeries sp{(int)T, coupling, smooth_prec, nullptr};
+    if (host) {
+        std::lock_guard<std::mutex> lock(b->host_mu);
+        return bank_solve_stream(b, spectra, S, obs, obs_ld, weights, o,
+                                 solve_io(D, K, x0, obs, obs_ld, o, x, cost, grad, hess, cov, info, weights, weights_ld, T),
+                                 nullptr, &sp);
+    }
+    const LmProblem pb = lm_problem((int)D, o, o.lower, o.upper, o.prior_mean, o.prior_ld, o.prior_prec);
+    return bank_series_solve_device(b, spectra ? bank_forward_cost_device : bank_cost_device, K, pb, sp, x0, S, obs, obs_ld,
+                                    weights, x, cost, grad, hess, cov, info, (cudaStream_t)stream, S * T, weights_ld);
+}
+
 int gpe_bank_search_pw(gpe_bank* b, const double* cand, int64_t K, const double* obs, int64_t N, int64_t obs_ld,
                        const double* weights, int64_t weights_ld, int k, int64_t* idx, double* cost, unsigned flags, void* stream) {
     NvtxRange nvtx_range("gpe_bank_search");
@@ -2563,6 +2715,27 @@ int gpe_multi_bank_solve_pw(gpe_multi* mm, const double* x0, int64_t N, const do
                                weights_ld);
     return fan_out(mm, mm->banks, b0->models[0]->sms, s.io, N, -1, [&](gpe_bank* b, const SharedCall* shared) {
         return bank_solve_stream(b, spectra, N, obs, obs_ld, weights, o, s, shared);
+    });
+}
+
+int gpe_multi_bank_solve_series(gpe_multi* mm, int64_t S, int64_t T, const double* x0, const double* obs, int64_t obs_ld,
+                                const double* weights, int64_t weights_ld, const gpe_solve_opts* opts, const double* smooth_prec,
+                                const double* coupling, double* x, double* cost, double* grad, double* hess, double* cov,
+                                int32_t* info, unsigned flags) {
+    NvtxRange nvtx_range("gpe_multi_bank_solve_series");
+    if (!mm || mm->banks.empty()) return fail(GPE_ERR_INVALID, "handle is NULL or not a bank handle");
+    gpe_bank* b0 = mm->banks[0];
+    const bool spectra = flags & GPE_SOLVE_SPECTRA;
+    int rc = series_check(b0, S, T, smooth_prec, coupling, true, nullptr);
+    gpe_solve_opts o;
+    if (rc == GPE_OK) rc = solve_check(b0, S * T, x0, obs, obs_ld, opts, x, info, flags, true, nullptr, &o);
+    if (rc == GPE_OK) rc = weights_check(weights, weights_ld, spectra ? b0->W : b0->E, spectra, true);
+    if (rc || S == 0) return rc;
+    const SolveIo s = solve_io(b0->D, spectra ? b0->W : b0->E, x0, obs, obs_ld, o, x, cost, grad, hess, cov, info, weights,
+                               weights_ld, T);
+    const LmSeries sp{(int)T, coupling, smooth_prec, nullptr};
+    return fan_out(mm, mm->banks, b0->models[0]->sms, s.io, S, -1, [&](gpe_bank* b, const SharedCall* shared) {
+        return bank_solve_stream(b, spectra, S, obs, obs_ld, weights, o, s, shared, &sp);
     });
 }
 

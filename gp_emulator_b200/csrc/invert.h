@@ -40,4 +40,25 @@ cudaError_t lm_gather_rows(const int* list, int64_t n, const double* src, int64_
 cudaError_t lm_output(int D, int64_t n, const double* state, double* x, double* cost, double* grad, double* hess, double* cov,
                       int32_t* info, cudaStream_t st);
 
+
+// ---- time series (gpe_bank_solve_series, DESIGN 4.6g) ----
+// The rows n = s T + t of a series keep the per-point state; the series' scalars live in those of its row s T.
+struct LmSeries {
+    int T;
+    const double* coupling;    // (T - 1) or NULL (all 1)
+    const double* R;           // (D, D) smoothness precision
+    double* scratch;           // lm_series_scratch_doubles per series of the launch: the block factors L_t, M_t
+};
+__host__ __device__ inline int64_t lm_series_scratch_doubles(int D, int T) { return 2 * (int64_t)T * D * D; }
+// One LM step for the n active series list[0 .. n): evaluation rows i T + t (f, g, H without prior and coupling) -> state
+// of series list[i]; ge is overwritten.  flag[i] = 1 where the series stays active (trial rows in the state's xt).
+cudaError_t lm_series_step(const LmProblem& pb, const LmSeries& sp, int64_t n, const int* list, const double* fe, double* ge,
+                           const double* he, double* state, int* flag, bool first, cudaStream_t st);
+// rows (n T) = the rows of the series list[0 .. n), in order.
+cudaError_t lm_series_rows(const int* list, int64_t n, int T, int* rows, cudaStream_t st);
+// Outputs of n series: x, grad (n T, D), hess and cov (n T, D, D) diagonal blocks, cost (n), info (n, 2); any but x and info
+// may be NULL.  cov: NaN blocks where H is not positive definite, each block symmetric bit for bit.
+cudaError_t lm_series_output(const LmProblem& pb, const LmSeries& sp, int64_t n, double* state, double* x, double* cost,
+                             double* grad, double* hess, double* cov, int32_t* info, cudaStream_t st);
+
 }  // namespace gpe

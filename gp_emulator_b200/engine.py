@@ -718,6 +718,40 @@ class DeviceBank(_Handle):
         return self._solve(True, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
                            lambda0, want_cov, candidates, n_starts)
 
+    def invert_series(self, x0, obs, weights=None, smooth_precision=None, coupling=None, lower=None, upper=None,
+                      prior_mean=None, prior_precision=None, max_iter=_lib.SOLVE_DEFAULT_MAX_ITER, ftol=1e-10, xtol=1e-10,
+                      gtol=0.0, lambda0=1e-3, want_cov=False):
+        """Per series of T dates, the inputs that minimise the summed band cost of ``cost`` plus the optional Gaussian
+        prior of ``invert`` on every date plus a temporal smoothness prior,
+        ``1/2 sum_t coupling[t-1] (x_t - x_t-1)^T smooth_precision (x_t - x_t-1)``, inside the box: the Levenberg-Marquardt
+        of ``invert`` on the block-tridiagonal Hessian of the whole series, every iteration on the device
+        (``gpe_bank_solve_series``; the objective and the algorithm are stated in include/gpemu.h).
+
+        ``x0`` (S, T, D) or (T, D) for one series; ``obs`` (E,) or (S, T, E); ``weights`` (E,), (S, T, E) or None -- a date
+        whose weights are all 0 is masked and filled in by the smoothness prior; ``smooth_precision`` (D, D) symmetric PSD,
+        required; ``coupling`` (T - 1,) >= 0 or None (all 1): with 1 / (days between dates) the prior is a random walk over
+        irregular dates, a 0 cuts the chain; ``prior_mean`` (D,) or (S, T, D); the other arguments as ``invert``.  Returns
+        ``x`` and ``grad`` (S, T, D), ``hess`` (S, T, D, D) the diagonal blocks of the Hessian (the off-diagonal ones are
+        ``-coupling[t-1] smooth_precision``), ``cov`` (S, T, D, D) the diagonal blocks of its inverse with ``want_cov``,
+        ``cost``, ``status`` and ``n_iter`` (S,) -- without the leading S (scalars for the last three) for one series.
+        numpy in -> numpy out (all devices of the bank); torch CUDA in -> torch CUDA out (single-device banks)."""
+        if smooth_precision is None:
+            raise ValueError("smooth_precision (D, D) is required")
+        return self._solve(False, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
+                           lambda0, want_cov, series=(smooth_precision, coupling))
+
+    def forward_invert_series(self, x0, obs, weights=None, smooth_precision=None, coupling=None, lower=None, upper=None,
+                              prior_mean=None, prior_precision=None, max_iter=_lib.SOLVE_DEFAULT_MAX_ITER, ftol=1e-10,
+                              xtol=1e-10, gtol=0.0, lambda0=1e-3, want_cov=False):
+        """``invert_series`` with the spectrum cost of ``forward_cost``: ``obs`` (W,) or (S, T, W), ``weights`` (W,),
+        (S, T, W) or None."""
+        if self.W == 0:
+            raise GpemuError("bank has no basis functions to project onto")
+        if smooth_precision is None:
+            raise ValueError("smooth_precision (D, D) is required")
+        return self._solve(True, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
+                           lambda0, want_cov, series=(smooth_precision, coupling))
+
     def _solve_from_candidates(self, spectra, candidates, n_starts, obs, weights, solve):
         """Multi-start solve: ``solve(x0)`` from each of the ``n_starts`` best candidates, the best result per point."""
         found = self._search(spectra, candidates, obs, weights, n_starts)
@@ -756,7 +790,7 @@ class DeviceBank(_Handle):
         return best
 
     def _solve(self, spectra, x0, obs, weights, lower, upper, prior_mean, prior_precision, max_iter, ftol, xtol, gtol,
-               lambda0, want_cov, candidates=None, n_starts=1):
+               lambda0, want_cov, candidates=None, n_starts=1, series=None):
         if x0 is None:
             if candidates is None:
                 raise ValueError("give the starting points x0 or a candidate table")
@@ -785,6 +819,22 @@ class DeviceBank(_Handle):
             empty = np.empty
             info_empty = lambda n: np.empty((n, 2), dtype=np.int32)
         x0 = arr(x0)
+        if series is not None:
+            # series: the (S, T, ...) arrays become rows n = s T + t of the point solver's arguments
+            if len(shape(x0)) == 3 and shape(x0)[2] == D:
+                lead = tuple(shape(x0)[:2])
+            elif len(shape(x0)) == 2 and shape(x0)[1] == D:
+                lead = (shape(x0)[0],)
+            else:
+                raise ValueError(f"x0 must be (S, T, {D}) or (T, {D})")
+            S, T = (lead[0], lead[1]) if len(lead) == 2 else (1, lead[0])
+            rows = lambda a, w: a.reshape(S * T, w) if a is not None and tuple(shape(a)) == lead + (w,) else a
+            x0, obs, weights, prior_mean = rows(x0, D), rows(arr(obs), K), rows(arr(weights), K), rows(arr(prior_mean), D)
+            smooth, cpl = arr(series[0]), arr(series[1])
+            if shape(smooth) != (D, D):
+                raise ValueError(f"smooth_precision must be ({D}, {D})")
+            if cpl is not None and shape(cpl) != (T - 1,):
+                raise ValueError(f"coupling must be ({T - 1},)")
         if len(shape(x0)) != 2 or shape(x0)[1] != D:
             raise ValueError(f"x0 must be (N, {D})")
         N = shape(x0)[0]
@@ -808,13 +858,31 @@ class DeviceBank(_Handle):
                 raise ValueError(f"prior_mean must be ({D},) or ({N}, {D})")
         opts = _lib.SolveOpts(int(max_iter), float(ftol), float(xtol), float(gtol), float(lambda0), addr(lo), addr(hi),
                               addr(pm), prior_ld, addr(pp))
-        out = {"x": empty((N, D)), "cost": empty(N), "grad": empty((N, D)), "hess": empty((N, D, D))}
+        n_out = N if series is None else S
+        out = {"x": empty((N, D)), "cost": empty(n_out), "grad": empty((N, D)), "hess": empty((N, D, D))}
         if want_cov:
             out["cov"] = empty((N, D, D))
-        info = info_empty(N)
+        info = info_empty(n_out)
         flags = _lib.SOLVE_SPECTRA if spectra else 0
         args = (addr(x0), N, addr(o), obs_ld, addr(wt), C.byref(opts), addr(out["x"]), addr(out["cost"]),
                 addr(out["grad"]), addr(out["hess"]), addr(out.get("cov")), addr(info))
+        if series is not None:
+            args = (S, T, addr(x0), addr(o), obs_ld, addr(wt), w_ld, C.byref(opts), addr(smooth), addr(cpl)) + args[6:]
+            if dev:
+                check(lib.gpe_bank_solve_series(self._h, *args, flags, _current_stream_ptr(self.device)))
+            elif self.multi:
+                check(lib.gpe_multi_bank_solve_series(self._h, *args, flags))
+            else:
+                check(lib.gpe_bank_solve_series(self._h, *args, flags | HOST_PTRS, None))
+            out["status"], out["n_iter"] = info[:, 0], info[:, 1]
+            one = len(lead) == 1
+            for key in ("x", "grad", "hess", "cov"):
+                if key in out:
+                    out[key] = out[key].reshape(lead + tuple(shape(out[key])[1:]))
+            if one:
+                for key in ("cost", "status", "n_iter"):
+                    out[key] = out[key][0]
+            return out
         if w_ld:
             args = args[:5] + (w_ld,) + args[5:]
             if dev:

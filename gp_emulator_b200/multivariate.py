@@ -252,6 +252,27 @@ class MultivariateEmulator(object):
             return one
         return out
 
+    def invert_series(self, obs, y0, smooth, weights=None, bounds=None, prior=None, max_iter=50, ftol=1e-10, xtol=1e-10,
+                      gtol=0.0, do_cov=True):
+        """Retrieve the parameters of every date of a time series jointly: per series, the minimiser of the summed ``cost``
+        of its dates (plus the per-date prior ``prior = (m, P)``) plus a smoothness prior
+        ``1/2 sum_t c_t (y_t - y_t-1)^T R (y_t - y_t-1)`` with ``smooth = (R, coupling)`` -- ``coupling`` (T - 1,) the c_t,
+        e.g. 1 / (days between dates), or None for all 1 -- inside ``bounds`` (``DeviceBank.forward_invert_series``).
+        Dates whose weights are all 0 (cloudy) are filled in by the prior.
+
+        ``obs`` (N_full,) shared or (S, T, N_full); ``y0`` (S, T, N_params) or (T, N_params) starting points, required (seed
+        it per date from ``search``); ``weights`` (N_full,), (S, T, N_full) or None.  Returns ``x``, ``grad``, ``hess``
+        (diagonal blocks), ``cov`` (with ``do_cov``: diagonal blocks of the posterior covariance), ``cost``, ``status``,
+        ``n_iter``, with leading (S, T) or (T,) as ``y0``.  Host arrays or CUDA tensors, as ``predict``."""
+        if y0 is None:
+            raise ValueError("invert_series needs the starting points y0 (seed them per date from search)")
+        R, coupling = smooth
+        lower, upper = bounds if bounds is not None else (None, None)
+        m, P = prior if prior is not None else (None, None)
+        return self._device_bank().forward_invert_series(y0, obs, weights, smooth_precision=R, coupling=coupling, lower=lower,
+                                                         upper=upper, prior_mean=m, prior_precision=P, max_iter=max_iter,
+                                                         ftol=ftol, xtol=xtol, gtol=gtol, want_cov=do_cov)
+
     def predict_pcs(self, y, do_unc=True, do_deriv=True):
         """PC-space outputs for N points: dict with mu (N, P), var (N, P), deriv (N, P, D)."""
         return self._device_bank().predict(np.atleast_2d(y), want_var=do_unc, want_deriv=do_deriv)

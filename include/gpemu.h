@@ -367,6 +367,44 @@ int gpe_multi_bank_search_pw(gpe_multi* mm, const double* cand, int64_t K, const
 #define GPE_SEARCH_PW_MAX_E_BANDS 48
 #define GPE_SEARCH_PW_MAX_E_SPECTRA 12
 
+/* Time series (DESIGN 4.6g): S series of T dates each, inverted jointly under a prior that the state changes smoothly
+ * in time.  Row n = s T + t holds the state x_st (D) of date t of series s.  Per series, the X in the box lower <= x <= upper
+ * that minimises
+ *   f_s(X) = sum_t [ cost(x_st; obs_st, w_st) + 1/2 (x_st - m_st)^T P (x_st - m_st) ]
+ *          + 1/2 sum_{t=1}^{T-1} c_t (x_st - x_s,t-1)^T R (x_st - x_s,t-1)
+ * with cost the band cost of gpe_bank_cost_pw (default) or, with GPE_SOLVE_SPECTRA, its spectrum cost; the prior (m, P)
+ * optional as in gpe_bank_solve.  R (D, D) is the smoothness precision (symmetric, PSD); coupling holds c_1 .. c_{T-1}
+ * >= 0, shared by every series, or is NULL (all 1).  With c_t = 1 / (days between dates t - 1 and t) the prior is a random
+ * walk over irregular dates; c_t = 0 cuts the chain there.
+ *   The gradient is per date, g_t = grad_t + P (x_t - m_t) + c_t R (x_t - x_t-1) - c_{t+1} R (x_t+1 - x_t), and the
+ * Hessian is block-tridiagonal: H_tt = hess_t + P + (c_t + c_{t+1}) R (c_0 = c_T = 0) and H_t,t-1 = -c_t R.
+ *   The algorithm is the Levenberg-Marquardt of gpe_bank_solve applied per series: the free set is taken per (t, d); the
+ * scale is s = max(|H_dd|, 1e-12 max |H_dd| over the series' free set); the step solves the damped, free-set-masked
+ * block-tridiagonal system by a block Cholesky over the dates; damping, accept / reject on f_s and the stopping tests are
+ * those of gpe_bank_solve with maxima over the whole series.  A series is GPE_SOLVE_NONFINITE when f_s is not finite at
+ * the clipped start.  With T = 1 every output equals gpe_bank_solve_pw's, bit for bit, whatever R.
+ * Outputs at the returned X: x (S T, D); cost (S) = f_s; grad (S T, D); hess (S T, D, D) the diagonal blocks H_tt or NULL;
+ * cov (S T, D, D) the diagonal blocks of inv(H) (undamped, all variables), symmetric bit for bit, NaN blocks for a series
+ * whose H is not positive definite, or NULL; info (S, 2) = (status, evaluations after the first).
+ *   - The off-diagonal blocks of H are -c_t R; they are not returned.
+ *   - With no prior, the per-date misfit at the result is one gpe_bank_cost_pw call on the returned x.
+ *   - Ragged series are padded to a common T with dates of zero weight (and any finite observation).
+ * Arguments: x0 (S T, D); obs (S T, K) with obs_ld >= K or (K) with obs_ld = 0; weights (K), (S T, K) rows weights_ld
+ * apart, or NULL, as gpe_bank_solve_pw; opts as gpe_bank_solve (prior_mean rows are per row n); S >= 0, 1 <= T <= 2^24,
+ * D <= 32.  R must be finite and exactly symmetric, coupling finite and >= 0 (GPE_ERR_INVALID otherwise).  Placement, the
+ * synchronous return and the independence of chunking, pointer placement, the device count and the order of the series
+ * are those of gpe_bank_solve; a chunk never splits a series.  A series whose solver scratch alone exceeds 256 MB:
+ * GPE_ERR_UNSUPPORTED. */
+int gpe_bank_solve_series(gpe_bank* b, int64_t S, int64_t T, const double* x0, const double* obs, int64_t obs_ld,
+                          const double* weights, int64_t weights_ld, const gpe_solve_opts* opts, const double* smooth_prec,
+                          const double* coupling, double* x, double* cost, double* grad, double* hess, double* cov,
+                          int32_t* info, unsigned flags, void* stream);
+/* The same on every device of a bank handle; host arrays (GPE_HOST_PTRS is implied). */
+int gpe_multi_bank_solve_series(gpe_multi* mm, int64_t S, int64_t T, const double* x0, const double* obs, int64_t obs_ld,
+                                const double* weights, int64_t weights_ld, const gpe_solve_opts* opts, const double* smooth_prec,
+                                const double* coupling, double* x, double* cost, double* grad, double* hess, double* cov,
+                                int32_t* info, unsigned flags);
+
 /* PCA back-projection of bank means: fwd (N, W) = mu (N, E) @ basis (E, W)
  * (the accumulation `fwd += pred_mu * basis_functions[i]`, gp_emulator/multivariate_gp.py:216, batched
  * over N points), and optionally deriv_full (N, D, W) = sum_e deriv[n, e, d] * basis[e, w] (:218).
